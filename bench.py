@@ -1,14 +1,13 @@
 #!/usr/bin/env python
 """Benchmark of the WindGNN GCN-GRU forward hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
-One "step" = `passes_per_step` forwards of the workload (BASELINE.json configs[1]: the shipped
-34-station checkpoint, batch 4096 windows of 168 hours) per GPU; `passes_per_step` is chosen after the
-warm-up so that the K timed steps last >= `--min-seconds` (default 2 s: sustained clocks, >= 20
-nvidia-smi samples inside the timed region).  With N > 1 (launched through ``torch.distributed.run``)
-every rank runs the same per-GPU batch on its own device (weak scaling: the sequence batch is sharded,
-no collective on the data path).
+One "step" = one forward of the workload (BASELINE.json configs[1]: the shipped 34-station checkpoint,
+batch 4096 windows of 168 hours) per GPU; exactly K steps are timed, after max(W, 3) untimed ones.  At
+about 5 ms per step, K >= 400 gives a timed region of 2 s (sustained clocks, >= 20 nvidia-smi samples inside
+it).  With N > 1 (launched through ``torch.distributed.run``) every rank runs the same per-GPU batch on
+its own device (weak scaling: the sequence batch is sharded, no collective on the data path).
 
 Prints ONE JSON line (rank 0):
   value         sequences/s with the inputs resident in HBM (CUDA events, max over ranks)
@@ -28,6 +27,10 @@ Prints ONE JSON line (rank 0):
 
 ``--impl reference`` times the reference's CPU forward alone on the full configs[1] step (4096 windows
 per step), all host threads.
+
+``--dump-outputs DIR`` writes what the timed path returned in its last timed step (rank 0) as
+DIR/<name>.npy, float32.  The inputs are seeded, so two builds run with the same arguments can be
+compared output for output.  An output above 64 MB is cut to a fixed sample of windows (see dump_output).
 """
 
 from __future__ import annotations
@@ -81,6 +84,22 @@ def load_workload(S_=34):
     idx = list(range(7)) if S_ == 7 else [i for i, n in enumerate(c["names"]) if n != "Enchant 2 AGCM"]
     latlon = np.array([[c["lat"][i], c["lon"][i]] for i in idx], dtype=np.float64)
     return sd, latlon
+
+
+DUMP_MAX_BYTES = 64_000_000
+
+
+def dump_output(out_dir: str, name: str, y: torch.Tensor) -> None:
+    """Save `y` [B, ...] as out_dir/<name>.npy in float32.  If it is larger than DUMP_MAX_BYTES, only the
+    windows rows = sorted(default_rng(0).choice(B, n, replace=False)) are saved, n as many as fit: the
+    same rows for the same B, whichever build wrote the file."""
+    y = y.detach()
+    n = min(y.shape[0], DUMP_MAX_BYTES // (4 * max(1, math.prod(y.shape[1:]))))
+    if n < y.shape[0]:
+        rows = np.sort(np.random.default_rng(0).choice(y.shape[0], n, replace=False))
+        y = y[torch.from_numpy(rows).to(y.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"{name}.npy"), y.to(torch.float32).cpu().numpy())
 
 
 class ClockSampler:
@@ -251,8 +270,10 @@ def run_reference(args, rank: int):
         fn(adj32, x[: min(256, n_seq)])
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        fn(adj32, x)
+        y = fn(adj32, x)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, "y", y)
     value = n_seq * args.steps / dt
     what = ("the reference's own GraphConvLayer / nn.GRU modules (oracle/_ref, unmodified), batched through its "
             "sub-modules" if kind == "reference" else "the oracle's torch-CPU port (oracle/_ref absent)")
@@ -310,18 +331,21 @@ def timed_events(ctx: Ctx, fn, steps: int, warmup: int, clocks: ClockSampler | N
     return ctx.max_over_ranks(e0.elapsed_time(e1))
 
 
-def scaled_leg(ctx: Ctx, which: str, steps: int, warmup: int, lib_peak: float, batch4096: int = 256):
+def scaled_leg(ctx: Ctx, which: str, steps: int, warmup: int, lib_peak: float, batch4096: int = 256,
+               dump_dir: str | None = None):
     """One of the other BASELINE configs as a sub-object (device-resident throughput; parity for these shapes
     is in tests/test_parity_gpu.py).
       fwd7     configs[0]: shipped 7-station checkpoint, 4096 windows per GPU (weak)
       fwd34_1m configs[2]: 2^20 windows in total, rank r owns a contiguous 1/world of them, streamed through the
                library in resident pieces of <= 131072 windows (one synthetic piece reused) (strong)
-      fwd4096  configs[3]: 4096-station kNN(8) graph, GCN_GRU(13,128,13,53248,128), T=24, 256 windows per GPU (weak)"""
+      fwd4096  configs[3]: 4096-station kNN(8) graph, GCN_GRU(13,128,13,53248,128), T=24, 256 windows per GPU (weak)
+    With `dump_dir`, rank 0 saves the output of the last timed step (fwd34_1m: of its last piece) there."""
     import windgnn_b200
     from windgnn_b200.shard import shard_range
 
     dev, rank, world = ctx.dev, ctx.rank, ctx.world
     gen = torch.Generator(device=dev).manual_seed(99 + rank)
+    last = {}
     if which == "fwd34_1m":
         sd, latlon = load_workload()
         model = windgnn_b200.GCN_GRU(F, F, F, I, H)
@@ -338,7 +362,7 @@ def scaled_leg(ctx: Ctx, which: str, steps: int, warmup: int, lib_peak: float, b
 
         def step():
             for _ in range(n_pieces):
-                model(adj, x)
+                last["y"] = model(adj, x)
     elif which == "fwd7":
         sd, latlon = load_workload(7)
         model = windgnn_b200.GCN_GRU(F, F, F, 13 * 7, 21)
@@ -351,7 +375,7 @@ def scaled_leg(ctx: Ctx, which: str, steps: int, warmup: int, lib_peak: float, b
         name = "7-station forward (wind_gnn_7.pth), T=168, 4096 windows per GPU (BASELINE.json configs[0], batched)"
 
         def step():
-            model(adj, x)
+            last["y"] = model(adj, x)
     else:
         S4, Fh4, H4, T4, B4 = 4096, 128, 128, 24, batch4096
         torch.manual_seed(4)
@@ -370,10 +394,12 @@ def scaled_leg(ctx: Ctx, which: str, steps: int, warmup: int, lib_peak: float, b
                 "variant C)")
 
         def step():
-            model(adj, x)
+            last["y"] = model(adj, x)
     model = model.to(dev).eval()
     with torch.no_grad():
         ms = timed_events(ctx, step, steps, warmup)
+    if dump_dir and rank == 0:
+        dump_output(dump_dir, "y", last["y"])
     value = units * steps / (ms * 1e-3)
     tfl = fl * value / world / 1e12
     tensor = None
@@ -390,7 +416,7 @@ def scaled_leg(ctx: Ctx, which: str, steps: int, warmup: int, lib_peak: float, b
            "hbm_gbs_algorithmic_per_gpu": by * value / world / 1e9, "flop_per_seq": fl}
     if tensor is not None:
         out["tensor_path"] = tensor
-    del x, model, adj
+    del x, model, adj, last
     torch.cuda.empty_cache()
     return out
 
@@ -432,12 +458,12 @@ def h2d_ceiling(ctx: Ctx, xh: torch.Tensor, oh: torch.Tensor, reps: int = 4):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps (one forward of the batch each)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
-    ap.add_argument("--batch", type=int, default=B_PER_GPU, help="sequences per GPU per pass")
+    ap.add_argument("--batch", type=int, default=B_PER_GPU, help="sequences per GPU per step")
     ap.add_argument("--min-seconds", type=float, default=2.0,
-                    help="minimum length of the timed region; a step becomes several passes over the batch if needed")
+                    help="minimum length of the timed region of the host-buffer (e2e) leg")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-tensor-path", action="store_true")
@@ -453,7 +479,12 @@ def main():
                          "the other names print that config alone")
     ap.add_argument("--train-batch", type=int, default=512,
                     help="windows per GPU of the training-step measurement (BASELINE.json configs[4]: 4096 over 8 GPUs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="save the output of the last timed step as DIR/y.npy (float32; above 64 MB a fixed sample "
+                         "of windows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -482,12 +513,12 @@ def main():
         ctx.dist = dist
 
     warmup = max(args.warmup, 3)
-    steps = max(args.steps, 1)
+    steps = args.steps
     Bg = args.batch
     ffma_peak = lib.wg_measure_ffma_tflops(local_rank, 10)
 
     if args.workload != "fwd34":
-        leg = scaled_leg(ctx, args.workload, steps, warmup, ffma_peak, Bg if Bg != B_PER_GPU else 256)
+        leg = scaled_leg(ctx, args.workload, steps, warmup, ffma_peak, Bg if Bg != B_PER_GPU else 256, args.dump_outputs)
         if rank == 0:
             print(json.dumps({
                 "metric": METRIC, "value": leg["value"], "unit": UNIT, "n_gpus": world, "steps": steps,
@@ -516,21 +547,16 @@ def main():
     # ---------------- device-resident throughput (`value`) ----------------
     holder = {}
 
-    def one_pass():
+    def one_step():
         holder["y"] = model(adj, x)
 
     with torch.no_grad():
-        ms_probe = timed_events(ctx, one_pass, 3, warmup) / 3      # also the warm-up
-        passes = max(1, min(256, math.ceil(args.min_seconds * 1e3 / (steps * ms_probe))))
-
-        def one_step():
-            for _ in range(passes):
-                one_pass()
-
         with ClockSampler(local_rank) as clocks:
-            ms = timed_events(ctx, one_step, steps, 1, clocks)
+            ms = timed_events(ctx, one_step, steps, warmup, clocks)
     y = holder["y"]
-    value = world * Bg * passes * steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_output(args.dump_outputs, "y", y)
+    value = world * Bg * steps / (ms * 1e-3)
     n_chunks = (Bg + 148 * 32 - 1) // (148 * 32)
     launches_per_pass = 1 + 3 * n_chunks  # pack + (gcn, inproj, recur) per internal chunk
 
@@ -541,15 +567,14 @@ def main():
         try:
             with torch.no_grad():
                 def tc_step():
-                    for _ in range(passes):
-                        holder["yt"] = model(adj, x)
+                    holder["yt"] = model(adj, x)
 
                 ms_t = timed_events(ctx, tc_step, steps, 2)
             yt = holder["yt"]
             err = float((yt - y).abs().max() / y.abs().max())
             tensor_path = {"precision": "tensor-core path (tcgen05, error-compensated split operands, fp32 accumulate)",
-                           "value": world * Bg * passes * steps / (ms_t * 1e-3), "unit": UNIT,
-                           "ms_per_pass": ms_t / steps / passes,
+                           "value": world * Bg * steps / (ms_t * 1e-3), "unit": UNIT,
+                           "ms_per_pass": ms_t / steps,
                            "max_abs_diff_vs_fp32_path_normalised": err, "parity_bar": 1e-5}
             del yt
             holder.pop("yt", None)
@@ -779,8 +804,8 @@ def main():
         inproj_bytes = rows * (I + 3 * H) * 4        # U read once + GI written once
         inproj_tflops = inproj_flops / (stage_ms["inproj"] * 1e-3) / 1e12
         nominal_peak = 148 * 128 * 2 * float(peaks.get("sm_max_mhz", 1965.0)) * 1e6 / 1e12
-        path_tflops = FLOP_PER_SEQ * Bg * passes * steps / (ms * 1e-3) / 1e12  # per GPU
-        hbm_gbs = BYTES_PER_SEQ * Bg * passes * steps / (ms * 1e-3) / 1e9      # per GPU, algorithmic
+        path_tflops = FLOP_PER_SEQ * Bg * steps / (ms * 1e-3) / 1e12  # per GPU
+        hbm_gbs = BYTES_PER_SEQ * Bg * steps / (ms * 1e-3) / 1e9      # per GPU, algorithmic
         kname = "inproj_kernel" if flags == 0 else "inproj_tc2_kernel"
         traffic, traffic_note = ncu_traffic_bytes(kname, inproj_bytes)
         stage_flops = {"gcn": 2 * (2 * S * S * F + 2 * S * F * F) * rows, "inproj": inproj_flops,
@@ -827,10 +852,9 @@ def main():
                        "workload": "34-station GCN-GRU forward (wind_gnn_34.pth), T=168, batch 4096 per GPU "
                                    "(BASELINE.json configs[1])", "S": S, "T": T, "batch_per_gpu": Bg,
                        "global_batch": Bg * world, "parallelism": f"sequence-sharded x{world}, no collective",
-                       "passes_per_step": passes, "ms_per_pass": ms / steps / passes,
                        "l2_policy": "inputs (1.22 GB per pass) larger than L2",
                        "station_sequence_predictions_per_s": value * S},
-            "clocks": clocks.summary(), "e2e": e2e, "gpu_launches": launches_per_pass * passes * steps,
+            "clocks": clocks.summary(), "e2e": e2e, "gpu_launches": launches_per_pass * steps,
             "roofline": roofline, "cpu_baseline": cpu, "gpu_eager": gpu_eager, "tensor_path": tensor_path,
             "train_step": train_step, "batch1": batch1, "scaled": scaled,
         }
