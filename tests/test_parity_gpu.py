@@ -181,8 +181,8 @@ def test_full_size_chunking_and_sharding_invariance(full34):
 
 
 def test_small_batch_recurrence_is_bit_identical_to_the_throughput_kernel(full34):
-    """Up to 1,184 sequences the 4-sequence-per-CTA recurrence runs, above that the 32-sequence one
-    (csrc/recur.cuh): same summation order, same gate expressions -> the same bits, for a single
+    """Up to 1,184 sequences the 4-sequence-per-CTA recurrence (gru_recur_regw_kernel) runs, above that
+    gru_recur_unit_kernel: same summation order, same gate expressions -> the same bits, for a single
     window (the reference's batch-1 call, main.py:102), ragged CTAs and the 7-station model."""
     model, adj, x, y = full34
     with torch.no_grad():
@@ -327,9 +327,12 @@ def _scaled_model(S, Fh, H, seed):
     return m
 
 
-@pytest.mark.parametrize("S,Fh,H,B,T,k", [(300, 128, 128, 3, 6, 8), (96, 40, 30, 5, 4, 3), (150, 13, 36, 2, 5, 8)])
+@pytest.mark.parametrize("S,Fh,H,B,T,k", [(300, 128, 128, 3, 6, 8), (96, 40, 30, 5, 4, 3), (150, 13, 36, 2, 5, 8),
+                                           (300, 320, 48, 2, 3, 8), (4600, 16, 32, 1, 2, 4)])
 def test_sparse_graph_path_vs_oracle(S, Fh, H, B, T, k):
-    """CSR adjacency path (large kNN graph, wide GCN hidden layer) against the oracle."""
+    """CSR adjacency path (large kNN graph, wide GCN hidden layer) against the oracle.  The last two cases run
+    gcn_sparse_l1_kernel / gcn_sparse_l2_kernel: F_hid = 320 is wider than the constant bank of
+    gcn_sparse_plan_kernel, and a 4600-station slab does not fit shared memory."""
     from oracle import knn_graph_f64, synthetic_coordinates
 
     adj = knn_graph_f64(synthetic_coordinates(S, seed=S), k).astype(np.float32)

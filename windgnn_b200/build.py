@@ -67,7 +67,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     objs = []
     for src, extra in UNITS:
         obj = os.path.join(BUILD, src.replace(".cu", ".o"))
-        env_extra = os.environ.get("WG_NVCC_FLAGS", "").split()  # experiment knobs, e.g. -DWG_RC_ALTERNATE=0
+        env_extra = os.environ.get("WG_NVCC_FLAGS", "").split()  # experiment builds, e.g. -DWG_RC_TRACE
         cmd = [nvcc, *ARCH, *COMMON, *extra, *env_extra, "-c", os.path.join(CSRC, src), "-o", obj]
         if verbose:
             cmd.insert(1, "-Xptxas=-v")

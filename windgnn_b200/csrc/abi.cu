@@ -19,7 +19,6 @@
 #include "gemm_kb.cuh"
 #include "gru_bwd.cuh"
 #include "inproj.cuh"
-#include "inproj_tc.cuh"
 #include "inproj_tc2.cuh"
 #include "recur.cuh"
 #include "recur_tc.cuh"
@@ -78,7 +77,7 @@ struct Plan {
     bool sparse;   // CSR graph path: adds the Z scratch of the sparse GCN kernels
     bool sq;       // CSR graph path on gcn_sparse_plan_kernel (constant-bank weights + gather plan)
     size_t off_sqw, off_sqplan;
-    bool tc;       // tensor-core (3xTF32 tcgen05) input projection: U and w_ih kept as hi + lo
+    bool tc;       // tensor-core input projection (inproj_tc2.cuh): w_ih packed as fp16 hi + lo
     wg::Tc2Shape tc2;
     size_t off_wp, off_bias, off_wht, off_whu, off_bhn, off_u, off_gi, off_z, total;
     bool tc_recur;             // tensor-core recurrence (recur_tc.cuh): W_hh packed as fp16 hi + lo
@@ -95,8 +94,6 @@ long long default_chunk(long long B, size_t bytes_per_seq) {
     }
     return B < c ? (B < 1 ? 1 : B) : c;
 }
-
-bool force_legacy();
 
 int make_plan(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int H, long long chunk,
               bool sparse = false, int flags = 0) {
@@ -148,7 +145,7 @@ int make_plan(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int H,
     // sparse path scratch: row-major U (rows x S*Fo) + one [Fo][S] row per resident CTA
     p.off_z = o;    if (sparse) o = align_up(o + (rows + wg::kNumSMs) * (size_t)S * Fo * 4);
     // second-generation CSR kernel: weights staged for the constant bank + the gather plan
-    p.sq = sparse && Fi <= wg::kSpF && Fo <= wg::kSpF && Fh <= wg::kSqMaxFh && !force_legacy() &&
+    p.sq = sparse && Fi <= wg::kSpF && Fo <= wg::kSpF && Fh <= wg::kSqMaxFh &&
            wg::gcn_sparse_plan_smem_bytes(S, Fi, Fo) <= (size_t)wg::kMaxSmemOptin;
     p.off_sqw = o;    if (p.sq) o = align_up(o + sizeof(wg::SqWeights));
     p.off_sqplan = o; if (p.sq) o = align_up(o + wg::sq_plan_bytes(S));
@@ -216,8 +213,7 @@ __global__ void pack_params_kernel(const float* __restrict__ w_ih, const float* 
 // ---------------------------------------------------------------------------------------------
 template <int FP, int SG, bool EXACT, int LAYERS, bool TILED>
 int launch_gcn_t(const float* X, const float* adj, const float* W1, const float* b1, const float* W2,
-                 const float* b2, float* out, float* out_lo, long long R, int S, int Fi, int Fh, int Fo, int ldo,
-                 cudaStream_t st) {
+                 const float* b2, float* out, long long R, int S, int Fi, int Fh, int Fo, int ldo, cudaStream_t st) {
     const int NSG = wg::ceil_div(S, SG);
     if (NSG > wg::kGcnThreads)
         return fail(WG_ERR_UNSUPPORTED, "S=%d too large for the dense GCN kernel", S);
@@ -250,8 +246,7 @@ int launch_gcn_t(const float* X, const float* adj, const float* W1, const float*
     long long grid = (long long)wg::kNumSMs * per_sm;
     if (grid > nblocks) grid = nblocks;
     if (grid < 1) return WG_OK;
-    kern<<<(unsigned)grid, wg::kGcnThreads, smem, st>>>(X, adj, W1, b1, W2, b2, out, out_lo, R, S, Fi, Fh, Fo, ldo,
-                                                        RB);
+    kern<<<(unsigned)grid, wg::kGcnThreads, smem, st>>>(X, adj, W1, b1, W2, b2, out, R, S, Fi, Fh, Fo, ldo, RB);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
@@ -260,8 +255,6 @@ int launch_gcn_t(const float* X, const float* adj, const float* W1, const float*
 int pick_sg(int S) {
     return wg::ceil_div(S, 7) * 7 <= wg::ceil_div(S, 4) * 4 ? 7 : 4;
 }
-
-bool force_legacy();
 
 // second-generation fused two-layer kernel (gcn_rows.cuh): lane = row, output straight into the tiles
 int launch_gcn_rows(const float* X, const float* adj, const float* W1, const float* b1, const float* W2,
@@ -281,16 +274,22 @@ int launch_gcn_rows(const float* X, const float* adj, const float* W1, const flo
     return WG_OK;
 }
 
+// Testing knob: WG_FORCE_LEGACY=1 runs the fused two-layer GCN on gcn_kernel where gcn_rows_kernel would run, so
+// that the tests can compare the two (they are bit-identical).  It selects nothing else.
+bool force_legacy() {
+    const char* e = getenv("WG_FORCE_LEGACY");
+    return e && e[0] == '1';
+}
+
 template <int LAYERS, bool TILED>
 int launch_gcn(const float* X, const float* adj, const float* W1, const float* b1, const float* W2,
-               const float* b2, float* out, float* out_lo, long long R, int S, int Fi, int Fh, int Fo, int ldo,
-               cudaStream_t st) {
-    if (LAYERS == 2 && TILED && out_lo == nullptr && wg::gcn_rows_applies(S, Fi, Fh, Fo) && !force_legacy() &&
+               const float* b2, float* out, long long R, int S, int Fi, int Fh, int Fo, int ldo, cudaStream_t st) {
+    if (LAYERS == 2 && TILED && wg::gcn_rows_applies(S, Fi, Fh, Fo) && !force_legacy() &&
         wg::gcn_rows_smem_floats(S) * 4 <= (size_t)wg::kMaxSmemOptin)
         return launch_gcn_rows(X, adj, W1, b1, W2, b2, out, R, S, ldo, st);
     const int fmax = Fi > Fh ? (Fi > Fo ? Fi : Fo) : (Fh > Fo ? Fh : Fo);
 #define WG_GCN(FP, SG, EX) \
-    launch_gcn_t<FP, SG, EX, LAYERS, TILED>(X, adj, W1, b1, W2, b2, out, out_lo, R, S, Fi, Fh, Fo, ldo, st)
+    launch_gcn_t<FP, SG, EX, LAYERS, TILED>(X, adj, W1, b1, W2, b2, out, R, S, Fi, Fh, Fo, ldo, st)
     if (Fi == 13 && Fh == 13 && Fo == 13) return pick_sg(S) == 7 ? WG_GCN(13, 7, true) : WG_GCN(13, 4, true);
     if (fmax <= 16) return WG_GCN(16, 4, false);
 #undef WG_GCN
@@ -330,25 +329,8 @@ int launch_gcn_sparse(const Plan& p, void* ws, const Csr& g, const float* x, con
         WG_CUDA(cudaGetLastError());
         return WG_OK;
     }
-    // a whole row's [S, F] slab fits shared memory: the row-resident fused kernel
-    const size_t smem_row = wg::gcn_sparse_row_smem_bytes(p.S, p.Fi, p.Fh, p.Fo);
-    if (smem_row <= (size_t)wg::kMaxSmemOptin && rows >= 1) {
-        auto kern = (p.Fi <= 13 && p.Fo <= 13) ? wg::gcn_sparse_row_kernel<13> : wg::gcn_sparse_row_kernel<16>;
-        WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_row));
-        const unsigned grid = (unsigned)(rows < wg::kNumSMs ? rows : wg::kNumSMs);
-        // off_z: [rows][S*Fo] row-major U, then gridDim per-CTA Z rows
-        float* urow = ws_ptr<float>(ws, p.off_z);
-        float* zscr = urow + (size_t)rows * p.S * p.Fo;
-        kern<<<grid, wg::kSrThreads, smem_row, st>>>(x, g.rowptr, g.colidx, g.vals, w1, b1, w2, b2, zscr, urow, rows,
-                                                     p.S, p.Fi, p.Fh, p.Fo);
-        WG_CUDA(cudaGetLastError());
-        const long long rt = (rows + wg::kSpThreads - 1) / wg::kSpThreads * wg::kSpThreads;  // whole tiles (zero rows)
-        const dim3 tg((unsigned)((p.IP + 31) / 32), (unsigned)(rt / 32));
-        if (tg.y > 65535u) return fail(WG_ERR_UNSUPPORTED, "sparse GCN: chunk of %lld rows too large", rows);
-        wg::rows_to_tiles_kernel<<<tg, 256, 0, st>>>(urow, ws_ptr<float>(ws, p.off_u), rows, p.S * p.Fo, p.S * p.Fo, p.IP);
-        WG_CUDA(cudaGetLastError());
-        return WG_OK;
-    }
+    // gcn_sparse_plan_kernel does not apply (hidden width above its constant bank, or a slab too large for
+    // shared memory): the two lane = row kernels
     const size_t smem = ((size_t)2 * p.Fh * wg::kSpF + p.Fh) * 4;
     if (smem > (size_t)wg::kMaxSmemOptin)
         return fail(WG_ERR_UNSUPPORTED, "sparse GCN: hidden width %d too large", p.Fh);
@@ -403,42 +385,33 @@ int launch_inproj(const Plan& p, void* ws, long long rows, cudaStream_t st) {
     return WG_OK;
 }
 
-template <int NW, bool WS, bool SAVE = false>
-int launch_recur_t(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave = nullptr,
-                   int ldsave = 0) {
+// FP32 recurrence of the hidden sizes gru_recur_unit_kernel cannot fit (H = 125 .. 360): W_hh^T read through L1 / L2
+int launch_recur_wide(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st) {
     // stage h in shared memory for bulk stores when it fits, else store every step directly
     int TS = wg::recur_stage_steps(p.H);
-    size_t smem = wg::recur_smem_floats(p.KP, p.NPR, p.GP, WS, p.H, TS) * 4;
+    size_t smem = wg::recur_smem_floats(p.KP, p.GP, p.H, TS) * 4;
     if (smem > (size_t)wg::kMaxSmemOptin) {
         TS = 0;
-        smem = wg::recur_smem_floats(p.KP, p.NPR, p.GP, WS) * 4;
+        smem = wg::recur_smem_floats(p.KP, p.GP) * 4;
     }
-    auto kern = wg::gru_recur_kernel<NW, WS, SAVE>;
-    WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (smem > (size_t)wg::kMaxSmemOptin)
+        return fail(WG_ERR_UNSUPPORTED, "GRU hidden size %d: state does not fit shared memory", p.H);
+    WG_CUDA(cudaFuncSetAttribute(wg::gru_recur_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const long long grid = (Bc + wg::kRcBT - 1) / wg::kRcBT;
     if (grid < 1) return WG_OK;
-    kern<<<(unsigned)grid, NW * 32, smem, st>>>(ws_ptr<float>(ws, p.off_gi), ws_ptr<float>(ws, p.off_wht),
-                                               ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H, p.GP,
-                                               p.KP, p.NPR, TS, gsave, ldsave);
+    wg::gru_recur_kernel<<<(unsigned)grid, wg::kRcWarps * 32, smem, st>>>(
+        ws_ptr<float>(ws, p.off_gi), ws_ptr<float>(ws, p.off_wht), ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H,
+        p.GP, p.KP, p.NPR, TS);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
 
-template <bool WS>
-int launch_recur_ws(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st) {
-    // warps per 16-sequence group: one per 80-column block (1, 2, 4 or 8; more blocks are looped)
-    const int blocks = p.NPR / wg::kRcCB;
-    if (blocks <= 1) return launch_recur_t<2, WS>(p, ws, out, Bc, st);
-    if (blocks <= 2) return launch_recur_t<4, WS>(p, ws, out, Bc, st);
-    if (blocks <= 4) return launch_recur_t<8, WS>(p, ws, out, Bc, st);
-    return launch_recur_t<16, WS>(p, ws, out, Bc, st);
-}
-
-// few sequences (the reference's batch-1 calls, small shards): 4 per CTA, bit-identical results
+// few sequences (the reference's batch-1 calls, small shards) of the shipped models: W_hh in registers for their
+// contraction lengths (H = 102 -> 104, H = 21 -> 24), 4 sequences per CTA, bit-identical results
 bool recur_small_applies(const Plan& p, long long Bc) {
-    // up to two waves of 4-sequence CTAs (~0.55 ms each at T = 168) beat one pass of the 32-sequence kernel (1.4 ms)
-    return Bc <= 2LL * wg::kRsBT * wg::kNumSMs && p.NPR / 2 <= wg::kRsCols &&
-           wg::recur_small_smem_floats(p.KP, p.NPR, p.GP) * 4 <= (size_t)wg::kMaxSmemOptin;
+    // up to two waves of 4-sequence CTAs
+    return Bc <= 2LL * wg::kRsBT * wg::kNumSMs && (p.KP == 104 || p.KP == 24) && p.NPR <= wg::kRwThreads &&
+           wg::recur_regw_smem_floats(p.KP, p.NPR, p.GP) * 4 <= (size_t)wg::kMaxSmemOptin;
 }
 template <bool SAVE, int NB, int KPT>
 int launch_recur_regw_t(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
@@ -460,34 +433,14 @@ int launch_recur_regw(const Plan& p, void* ws, float* out, long long Bc, cudaStr
     if (Bc == 2) return launch_recur_regw_t<SAVE, 2, KPT>(p, ws, out, Bc, st, gsave, ldsave);
     return launch_recur_regw_t<SAVE, 1, KPT>(p, ws, out, Bc, st, gsave, ldsave);
 }
-
 template <bool SAVE>
 int launch_recur_small(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
     if (Bc < 1) return WG_OK;
-    // W_hh in registers for the contraction lengths of the shipped models (H = 102 -> 104, H = 21 -> 24)
-    if (p.NPR <= wg::kRwThreads && p.KP == 104) return launch_recur_regw<SAVE, 104>(p, ws, out, Bc, st, gsave, ldsave);
-    if (p.NPR <= wg::kRwThreads && p.KP == 24) return launch_recur_regw<SAVE, 24>(p, ws, out, Bc, st, gsave, ldsave);
-    const size_t smem = wg::recur_small_smem_floats(p.KP, p.NPR, p.GP) * 4;
-    // FMA chains per thread = sequences per CTA that can exist
-    auto kern = Bc >= 4 ? wg::gru_recur_small_kernel<SAVE, 4>
-              : Bc == 3 ? wg::gru_recur_small_kernel<SAVE, 3>
-              : Bc == 2 ? wg::gru_recur_small_kernel<SAVE, 2> : wg::gru_recur_small_kernel<SAVE, 1>;
-    WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const long long grid = (Bc + wg::kRsBT - 1) / wg::kRsBT;
-    kern<<<(unsigned)grid, wg::kRsThreads, smem, st>>>(ws_ptr<float>(ws, p.off_gi), ws_ptr<float>(ws, p.off_wht),
-                                                      ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H, p.GP, p.KP,
-                                                      p.NPR, gsave, ldsave);
-    WG_CUDA(cudaGetLastError());
-    return WG_OK;
+    if (p.KP == 104) return launch_recur_regw<SAVE, 104>(p, ws, out, Bc, st, gsave, ldsave);
+    return launch_recur_regw<SAVE, 24>(p, ws, out, Bc, st, gsave, ldsave);
 }
 
 // ---- second-generation throughput recurrence (recur_unit.cuh) ----
-}  // namespace
-namespace {
-bool force_legacy() {   // testing knob: WG_FORCE_LEGACY=1 selects the first-generation kernels (bit-identical results)
-    const char* e = getenv("WG_FORCE_LEGACY");
-    return e && e[0] == '1';
-}
 // sequences per group: the R in [4, 8] that needs the fewest (waves x R) for this batch
 int recur_u_pick_r(long long Bc, int ngrp) {
     int best = wg::kRuMaxR;
@@ -500,16 +453,8 @@ int recur_u_pick_r(long long Bc, int ngrp) {
     }
     return best;
 }
-// FMA-pipe hand-over between the two one-warp groups of a scheduler (recur_unit.cuh).  Measured
-// (scripts/handover_ab.py, profiles/r02_handover_ab.json): H = 21, 4096 sequences: 0.395 -> 0.358 ms.  Two-warp
-// groups (H = 102) own their scheduler and need none.  WG_RU_HANDOVER=0 switches it off (results are identical).
-bool recur_handover(int wpg) {
-    const char* e = getenv("WG_RU_HANDOVER");
-    return wpg == 1 && !(e && e[0] == '0');
-}
 bool recur_unit_applies(const Plan& p) {
-    return !force_legacy() && wg::recur_u_applies(p.H) &&
-           wg::recur_u_smem_floats(p.H, wg::kRuMinR) * 4 <= (size_t)wg::kMaxSmemOptin;
+    return wg::recur_u_applies(p.H) && wg::recur_u_smem_floats(p.H, wg::kRuMinR) * 4 <= (size_t)wg::kMaxSmemOptin;
 }
 template <int R, int WPG, bool SAVE, int HT>
 int launch_recur_unit_t(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
@@ -519,9 +464,12 @@ int launch_recur_unit_t(const Plan& p, void* ws, float* out, long long Bc, cudaS
     const int per_cta = (wg::kRuWarps / WPG) * R;
     const long long grid = (Bc + per_cta - 1) / per_cta;
     if (grid < 1) return WG_OK;
+    // FMA-pipe hand-over between the two one-warp groups of a scheduler (profiles/r02_handover_ab.json: H = 21, 4096
+    // sequences: 0.395 -> 0.358 ms, identical results).  Two-warp groups (H = 102) own their scheduler and need none.
+    const int handover = WPG == 1 ? 1 : 0;
     kern<<<(unsigned)grid, wg::kRuThreads, smem, st>>>(ws_ptr<float>(ws, p.off_gi), ws_ptr<float>(ws, p.off_whu),
                                                       ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H, gsave, ldsave,
-                                                      recur_handover(WPG) ? 1 : 0);
+                                                      handover);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
@@ -550,14 +498,7 @@ int launch_recur_unit(const Plan& p, void* ws, float* out, long long Bc, cudaStr
 int launch_recur_save(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
     if (recur_small_applies(p, Bc)) return launch_recur_small<true>(p, ws, out, Bc, st, gsave, ldsave);
     if (recur_unit_applies(p)) return launch_recur_unit<true>(p, ws, out, Bc, st, gsave, ldsave);
-    const size_t smem_ws = wg::recur_smem_floats(p.KP, p.NPR, p.GP, true) * 4;
-    if (smem_ws > (size_t)wg::kMaxSmemOptin)
-        return fail(WG_ERR_UNSUPPORTED, "training: GRU hidden size %d does not fit the shared-memory recurrence", p.H);
-    const int blocks = p.NPR / wg::kRcCB;
-    if (blocks <= 1) return launch_recur_t<2, true, true>(p, ws, out, Bc, st, gsave, ldsave);
-    if (blocks <= 2) return launch_recur_t<4, true, true>(p, ws, out, Bc, st, gsave, ldsave);
-    if (blocks <= 4) return launch_recur_t<8, true, true>(p, ws, out, Bc, st, gsave, ldsave);
-    return launch_recur_t<16, true, true>(p, ws, out, Bc, st, gsave, ldsave);
+    return fail(WG_ERR_UNSUPPORTED, "training: GRU hidden size %d does not fit the shared-memory recurrence", p.H);
 }
 
 int launch_recur_tc(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st) {
@@ -576,11 +517,7 @@ int launch_recur(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t
     if (p.tc_recur) return launch_recur_tc(p, ws, out, Bc, st);   // the tensor path: one kernel for every batch size
     if (recur_small_applies(p, Bc)) return launch_recur_small<false>(p, ws, out, Bc, st, nullptr, 0);
     if (recur_unit_applies(p)) return launch_recur_unit<false>(p, ws, out, Bc, st, nullptr, 0);
-    const size_t smem_ws = wg::recur_smem_floats(p.KP, p.NPR, p.GP, true) * 4;
-    if (smem_ws <= (size_t)wg::kMaxSmemOptin) return launch_recur_ws<true>(p, ws, out, Bc, st);
-    const size_t smem_nows = wg::recur_smem_floats(p.KP, p.NPR, p.GP, false) * 4;
-    if (smem_nows <= (size_t)wg::kMaxSmemOptin) return launch_recur_ws<false>(p, ws, out, Bc, st);
-    return fail(WG_ERR_UNSUPPORTED, "GRU hidden size %d: state does not fit shared memory", p.H);
+    return launch_recur_wide(p, ws, out, Bc, st);
 }
 
 int launch_pack(const Plan& p, void* ws, const float* w_ih, const float* w_hh, const float* b_ih,
@@ -608,8 +545,8 @@ int launch_pack(const Plan& p, void* ws, const float* w_ih, const float* w_hh, c
 int run_chunk(const Plan& p, void* ws, const float* adj, const float* x, const float* w1, const float* b1,
               const float* w2, const float* b2, float* out, long long Bc, cudaStream_t st) {
     const long long rows = Bc * p.T;
-    int rc = launch_gcn<2, true>(x, adj, w1, b1, w2, b2, ws_ptr<float>(ws, p.off_u), nullptr, rows, p.S, p.Fi, p.Fh,
-                                 p.Fo, p.IP, st);
+    int rc = launch_gcn<2, true>(x, adj, w1, b1, w2, b2, ws_ptr<float>(ws, p.off_u), rows, p.S, p.Fi, p.Fh, p.Fo,
+                                 p.IP, st);
     if (rc) return rc;
     rc = launch_inproj(p, ws, rows, st);
     if (rc) return rc;
@@ -718,6 +655,11 @@ size_t param_count(int S, int Fi, int Fh, int Fo, int H) {
     return (size_t)Fi * Fh + Fh + (size_t)Fh * Fo + Fo + G * I + G * H + G + G;
 }
 
+// Largest GRU hidden size training accepts: the bound of the recurrence it was built and tested with (W_hh^T resident
+// in shared memory beside the state of 32 sequences).  The gate-saving recurrence that runs now
+// (gru_recur_unit_kernel or gru_recur_regw_kernel) serves every H up to it.
+constexpr int kTrainMaxH = 106;
+
 int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, int Fo, int H) {
     int rc = make_plan(tp.f, B, T, S, Fi, Fh, Fo, H, B > 0 ? B : 1, false, 0);
     if (rc) return rc;
@@ -743,7 +685,7 @@ int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, in
             wg::gru_bwd_smem_floats(tp.HP, tp.GR, tp.bt_gb) * 4 > (size_t)wg::kMaxSmemOptin)
             return fail(WG_ERR_UNSUPPORTED, "training: GRU hidden size %d too large for the shared-memory BPTT kernel", H);
     }
-    if (wg::recur_smem_floats(p.KP, p.NPR, p.GP, true) * 4 > (size_t)wg::kMaxSmemOptin)
+    if (H > kTrainMaxH)
         return fail(WG_ERR_UNSUPPORTED, "training: GRU hidden size %d does not fit the shared-memory recurrence", H);
     tp.rows = (B > 0 ? B : 1) * (long long)T;
     tp.grid_gb = (int)(((B > 0 ? B : 1) + tp.bt_gb - 1) / tp.bt_gb);
@@ -901,8 +843,8 @@ int wg_stage_gcn_f32(const float* adj, const float* x, const float* w1, const fl
     if ((rc = check_ws(p, workspace, workspace_bytes))) return rc;
     DeviceGuard g(device);
     WG_CUDA(g.err);
-    return launch_gcn<2, true>(x, adj, w1, b1, w2, b2, ws_ptr<float>(workspace, p.off_u), nullptr, (long long)Bc * T, S,
-                               F_in, F_hid, F_out, p.IP, static_cast<cudaStream_t>(stream));
+    return launch_gcn<2, true>(x, adj, w1, b1, w2, b2, ws_ptr<float>(workspace, p.off_u), (long long)Bc * T, S, F_in,
+                               F_hid, F_out, p.IP, static_cast<cudaStream_t>(stream));
 }
 
 int wg_stage_inproj_f32(int64_t Bc, int T, int S, int F_in, int F_hid, int F_out, int H, int64_t chunk,
@@ -1177,8 +1119,8 @@ int wg_gcn_layer_f32(const float* adj, const float* attr, const float* weight, c
     DeviceGuard g(device);
     WG_CUDA(g.err);
     // single layer: "hidden" plays the role of the output width
-    return launch_gcn<1, false>(attr, adj, weight, bias, nullptr, nullptr, out, nullptr, R, S, F_in, F_out, F_out,
-                                S * F_out, static_cast<cudaStream_t>(stream));
+    return launch_gcn<1, false>(attr, adj, weight, bias, nullptr, nullptr, out, R, S, F_in, F_out, F_out, S * F_out,
+                                static_cast<cudaStream_t>(stream));
 }
 
 
@@ -1214,8 +1156,8 @@ int wg_gcn_gru_forward_train_f32(const float* adj, const float* x, const float* 
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const Plan& p = tp.f;
     if ((rc = launch_pack(p, workspace, w_ih, w_hh, b_ih, b_hh, st))) return rc;
-    if ((rc = launch_gcn<2, true>(x, adj, w1, b1, w2, b2, ws_ptr<float>(workspace, p.off_u), nullptr, tp.rows, S, F_in,
-                                  F_hid, F_out, p.IP, st)))
+    if ((rc = launch_gcn<2, true>(x, adj, w1, b1, w2, b2, ws_ptr<float>(workspace, p.off_u), tp.rows, S, F_in, F_hid,
+                                  F_out, p.IP, st)))
         return rc;
     if ((rc = launch_inproj(p, workspace, tp.rows, st))) return rc;
     return launch_recur_save(p, workspace, out, B, st, ws_ptr<float>(workspace, tp.off_gates), tp.LD4);
@@ -1403,10 +1345,6 @@ int wg_adam_step_f32(float* param, const float* grad, float* exp_avg, float* exp
 int wg_debug_read_unit_trace(long long* host, int n) {
     if (n > 8 * 256 * 5) n = 8 * 256 * 5;
     return (int)cudaMemcpyFromSymbol(host, wg::g_ru_trace, sizeof(long long) * n);
-}
-int wg_debug_read_trace(long long* host, int n) {
-    if (n > 2 * 8 * 256) n = 2 * 8 * 256;
-    return (int)cudaMemcpyFromSymbol(host, wg::g_rc_trace, sizeof(long long) * n);
 }
 #endif
 

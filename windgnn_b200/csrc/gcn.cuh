@@ -24,12 +24,8 @@
 namespace wg {
 
 constexpr int kGcnThreads = 128;
-#ifndef WG_GCN_UNROLL
-#define WG_GCN_UNROLL 2  // aggregation loop unroll (measured: 1.88 -> 1.82 ms at S = 34)
-#endif
-#ifndef WG_GCN_MINB
-#define WG_GCN_MINB 3  // resident CTAs per SM the register budget is planned for (<= 168 regs)
-#endif
+constexpr int kGcnUnroll = 2;      // aggregation loop unroll (measured: 1.88 -> 1.82 ms at S = 34)
+constexpr int kGcnMinBlocks = 3;   // resident CTAs per SM the register budget is planned for (<= 168 regs)
 constexpr int kGcnFS = 16;   // feature slots of the packed weight table
 constexpr int kUTileRows = 128;  // rows per K-major tile of the tiled output (= inproj BM)
 
@@ -69,8 +65,7 @@ __device__ __noinline__ void gcn_layer_inplace(float* __restrict__ buf, const fl
         const float* xrow = buf + (size_t)row_local * RS;
         const float* arow = adjT + q * 8;
         const int astride = NSG * 8;
-        constexpr int kUnroll = WG_GCN_UNROLL;
-#pragma unroll kUnroll
+#pragma unroll kGcnUnroll
         for (int sp = 0; sp < S; ++sp) {
             float a[8];
             {
@@ -135,11 +130,10 @@ __device__ __noinline__ void gcn_layer_inplace(float* __restrict__ buf, const fl
 // TILED: out is [ceil(R/128)][ldo][128] (K-major row tiles, zero padded columns) else [R][ldo]
 // row-major with ldo == S * F_last.
 template <int FP, int SG, bool EXACT, int LAYERS, bool TILED>
-__global__ void __launch_bounds__(kGcnThreads, WG_GCN_MINB)
+__global__ void __launch_bounds__(kGcnThreads, kGcnMinBlocks)
     gcn_kernel(const float* __restrict__ X, const float* __restrict__ adj, const float* __restrict__ W1,
                const float* __restrict__ b1, const float* __restrict__ W2, const float* __restrict__ b2,
-               float* __restrict__ out, float* __restrict__ out_lo, long long R, int S, int Fi, int Fh, int Fo,
-               int ldo, int RB) {
+               float* __restrict__ out, long long R, int S, int Fi, int Fh, int Fo, int ldo, int RB) {
     extern __shared__ __align__(16) float smem[];
     const int NSG = ceil_div(S, SG);
     const int tid = threadIdx.x;
@@ -218,31 +212,7 @@ __global__ void __launch_bounds__(kGcnThreads, WG_GCN_MINB)
             gcn_layer_inplace<FP, SG, EXACT>(buf, adjT, w2d, b2s, S, Fh, Fo, RS, NSG, row_local, q, active);
 
         // ---- store the final slab ----
-        if (TILED && out_lo != nullptr) {
-            // tensor-core layout (inproj_tc.cuh): out / out_lo [(r / 128)][c / 4][r % 128][4] hold the
-            // TF32-rounded value and the remainder; a lane owns one row and writes 16 bytes per
-            // column quad, so a warp store covers nrows * 16 contiguous bytes
-            for (int rl = tid & 31; rl < nrows; rl += 32) {
-                const long long r = r0 + rl;
-                const size_t base = ((size_t)(r / kUTileRows) * (ldo >> 2) * kUTileRows + (r % kUTileRows)) * 4;
-                const float* srcr = buf + rl * RS;
-                for (int cq = tid >> 5; cq < (ldo >> 2); cq += kGcnThreads / 32) {
-                    float hi[4], lo[4];
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        const int c = 4 * cq + j;
-                        const float v = c < out_cols ? srcr[c] : 0.0f;
-                        uint32_t t;
-                        asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(t) : "f"(v));
-                        hi[j] = __uint_as_float(t);
-                        lo[j] = v - hi[j];
-                    }
-                    const size_t o = base + (size_t)cq * kUTileRows * 4;
-                    *reinterpret_cast<float4*>(out + o) = make_float4(hi[0], hi[1], hi[2], hi[3]);
-                    *reinterpret_cast<float4*>(out_lo + o) = make_float4(lo[0], lo[1], lo[2], lo[3]);
-                }
-            }
-        } else if (TILED) {
+        if (TILED) {
             // out[(r / 128)][c][r % 128]: a lane owns one row of the block (its tile offset is fixed),
             // each warp walks the columns; a store instruction writes nrows consecutive floats
             for (int rl = tid & 31; rl < nrows; rl += 32) {

@@ -35,10 +35,7 @@ constexpr int kGrRows = 32;     // rows per block (= lanes)
 constexpr int kGrF = 13;        // feature width served
 constexpr int kGrFS = 16;       // feature stride of the layer-1 result in shared memory
 constexpr int kGrAP = 12;       // adjacency floats per (s', warp): up to 6 station pairs
-#ifndef WG_GR_MAXP
-#define WG_GR_MAXP 5
-#endif
-constexpr int kGrMaxPairs = WG_GR_MAXP;  // station pairs per warp (accumulators: 5 x 13 float2 = 130 registers)
+constexpr int kGrMaxPairs = 5;  // station pairs per warp (accumulators: 5 x 13 float2 = 130 registers)
 constexpr int kGrMaxWarps = 8;
 
 __host__ __device__ inline int gcn_rows_warps(int S) { return ceil_div(ceil_div(S, 2), kGrMaxPairs); }
@@ -53,12 +50,7 @@ __host__ __device__ inline int gcn_rows_rs2(int S) { return S * kGrFS + 4; }
 // is bit-identical to the 5/4/4/4 split, whose light warps spent 20 % of their time at the CTA barriers
 // (ncu: 16 % of all warp samples) waiting for the warp with five pairs.
 constexpr int kGrXS = 28;   // exchange row stride (floats): 13 float2, padded; 8 lanes x 16 B cover all 32 banks
-#ifndef WG_GR_BALANCED
-#define WG_GR_BALANCED 1   // 0: the 5/4/4/4 split (A/B runs)
-#endif
-__host__ __device__ inline bool gcn_rows_balanced(int S) {
-    return WG_GR_BALANCED && WG_GR_MAXP >= 5 && ceil_div(S, 2) == 17;
-}
+__host__ __device__ inline bool gcn_rows_balanced(int S) { return ceil_div(S, 2) == 17; }
 // warp w's slice: features / output columns 3w .. 3w + 3 (0-3, 3-6, 6-9, 9-12; the boundary columns are computed
 // by two warps — the same value, stored twice — so that all four warps run ONE instruction stream: with a slice per
 // template instantiation the four warps of a CTA executed four copies of the block code and the kernel ran at
@@ -230,27 +222,14 @@ __device__ __forceinline__ void gr_transform_chunk(float2 (&o)[NPW][4], const fl
 }
 
 // ReLU; NaN propagates like torch.relu.  One FMNMX.NAN instead of FSETP + FSEL (the epilogues run 884 of these per
-// row); WG_GR_EPI=0 restores the r02 epilogue for A/B runs.
-#ifndef WG_GR_EPI
-#define WG_GR_EPI 1
-#endif
+// row).
 __device__ __forceinline__ float gr_relu(float u) {
-#if WG_GR_EPI
     float r;
     asm("max.NaN.f32 %0, %1, 0f00000000;" : "=f"(r) : "f"(u));
     return r;
-#else
-    return u < 0.0f ? 0.0f : u;
-#endif
 }
 // (o.x + b, o.y + b): one FADD2 for the two stations of a pair
-__device__ __forceinline__ float2 gr_bias(float2 o, float b) {
-#if WG_GR_EPI
-    return __fadd2_rn(o, make_float2(b, b));
-#else
-    return make_float2(o.x + b, o.y + b);
-#endif
-}
+__device__ __forceinline__ float2 gr_bias(float2 o, float b) { return __fadd2_rn(o, make_float2(b, b)); }
 
 // One row block through both layers for a warp that owns NPW station pairs starting at station s0.
 // SHARED (balanced mode): additionally this warp's feature / column slice f0 .. f0 + 3 of the shared pair
@@ -372,11 +351,7 @@ __device__ __forceinline__ void gr_block(float* __restrict__ buf, const float* _
 }
 
 // X [R][S][13] -> out [ceil(R/128)][ldo][128] (K-major row tiles, columns >= S*13 zero)
-#ifndef WG_GR_LB_T
-#define WG_GR_LB_T (kGrMaxWarps * 32)
-#define WG_GR_LB_B 1
-#endif
-__global__ void __launch_bounds__(WG_GR_LB_T, WG_GR_LB_B)
+__global__ void __launch_bounds__(kGrMaxWarps * 32, 1)
     gcn_rows_kernel(const float* __restrict__ X, const float* __restrict__ adj, const float* __restrict__ W1,
                     const float* __restrict__ b1, const float* __restrict__ W2, const float* __restrict__ b2,
                     float* __restrict__ out, long long R, int S, int ldo) {
@@ -476,18 +451,12 @@ __global__ void __launch_bounds__(WG_GR_LB_T, WG_GR_LB_B)
         gr_block<N, false>(buf, arow, astride, w1d, b1s, w2d, b2s, S, s0, lane, row_ok, out_col0, ldo,        \
                            pad_warp, nsrc, nbytes, bar, xch, 0);                                              \
         break;
-        if (WG_GR_MAXP >= 5 && balanced) {   // one instruction stream for the four warps; the slice offset is a runtime value
+        if (balanced) {   // one instruction stream for the four warps; the slice offset is a runtime value
             gr_block<4, true>(buf, arow, astride, w1d, b1s, w2d, b2s, S, s0, lane, row_ok, out_col0, ldo, pad_warp,
                               nsrc, nbytes, bar, xch, kGrSliceStep * w);
         } else {
             switch (npw) {   // warp-uniform
-                WG_GR(1) WG_GR(2) WG_GR(3)
-#if WG_GR_MAXP >= 4
-                WG_GR(4)
-#endif
-#if WG_GR_MAXP >= 5
-                WG_GR(5)
-#endif
+                WG_GR(1) WG_GR(2) WG_GR(3) WG_GR(4) WG_GR(5)
                 default: break;
             }
         }

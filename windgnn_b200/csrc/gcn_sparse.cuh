@@ -14,6 +14,10 @@
 // Mapping: a CTA = 128 consecutive rows (one K-major output tile of the projection GEMM) x a
 // chunk of stations; lane = row, so the CSR entries and the weights are warp-uniform (broadcast)
 // and the tiled output store is coalesced; each lane gathers its own row's F-wide station slabs.
+//
+// These two kernels serve the CSR graphs that gcn_sparse_plan_kernel (gcn_sparse_plan.cuh) cannot:
+// a hidden width above the kSqMaxFh its constant bank holds, or a row slab S * max(F_in, F_out)
+// too large for shared memory.  They gather from HBM with one sector per lane.
 #pragma once
 
 #include "wg_common.cuh"
@@ -129,236 +133,6 @@ __global__ void __launch_bounds__(kSpThreads)
     // zero the K padding once (the CTA of the last station chunk does it)
     if (s1 == S)
         for (int c = S * Fo; c < ldo; ++c) ut[(size_t)c * kSpThreads] = 0.0f;
-}
-
-// ---------------------------------------------------------------------------------------------
-// Row-resident variant: ONE kernel for both layers, a CTA owns one (sequence, timestep) row at a
-// time and keeps that row's whole [S, F] slab in shared memory (S * 13 * 4 B = 213 KB at S = 4096:
-// it fits beside the 17 KB of weights), so every neighbour gather is a shared-memory read and
-// HBM sees X once and U once.  Thread = station (stations tid, tid + 512, ... two at a time):
-//   pass 1: agg = (A.X)[s] from the slab -> h = relu(agg.W1 + b1) (128 wide, registers only) ->
-//           z = h.W2; both contractions are FFMA2 on STATION pairs with the weight as the scalar
-//           operand: h2[(s, s')] += w1[f][fh] * (agg_s[f], agg_s'[f]);  z2[f][(s, s')] += w2[fh][f] * h2.
-//           Z goes to a per-CTA scratch row in HBM/L2 as [F_out][S] (coalesced), is bulk-copied
-//           back over the slab once every thread is done with X;
-//   pass 2: U[s] = relu((A.Z)[s] + b2), written row-major (coalesced); rows_to_tiles_kernel then re-lays
-//           it into the projection GEMM's K-major 128-row tiles (a 4-byte scatter from here would
-//           double the DRAM write traffic through partial sectors).
-// (Tried: stations handed out in degree order so that a warp's neighbour lists have equal length — slower,
-// 15.4 vs 13.7 ms: the CSR reads of a warp stop being contiguous.)
-// The lane = row kernels above gather from HBM with one sector per lane; at S = 4096 this
-// variant is what runs (8x fewer bytes through L2, FMA-bound instead of latency-bound).
-constexpr int kSrThreads = 512;   // 16 warps: the gather passes are latency-bound and the row pins the CTA count at 1
-constexpr int kSrGroup = 2;       // stations per thread per group (FFMA2 pairs along stations)
-constexpr int kSrPairs = kSrGroup / 2;
-
-__host__ __device__ inline size_t gcn_sparse_row_smem_bytes(int S, int Fi, int Fh, int Fo) {
-    const int FS = Fi > Fo ? Fi : Fo;
-    return ((size_t)round_up(S * FS, 4) + 2 * (size_t)Fh * kSpF + round_up(Fh, 4) + kSpF) * 4 + 16;
-}
-
-// FW: compile-time bound on F_in and F_out (13 for the reference's feature set, else 16)
-template <int FW>
-__global__ void __launch_bounds__(kSrThreads, 1)
-    gcn_sparse_row_kernel(const float* __restrict__ X, const int* __restrict__ rowptr,
-                          const int* __restrict__ colidx, const float* __restrict__ vals,
-                          const float* __restrict__ W1, const float* __restrict__ b1,
-                          const float* __restrict__ W2, const float* __restrict__ b2, float* __restrict__ Zscr,
-                          float* __restrict__ U, long long R, int S, int Fi, int Fh, int Fo) {
-    extern __shared__ __align__(16) float smem[];
-    const int FS = Fi > Fo ? Fi : Fo;
-    float* slab = smem;                                    // X row [S][Fi], then Z row [Fo][S]
-    float* w1t = slab + round_up(S * FS, 4);               // [Fh][16]: w1t[fh][f] = W1[f][fh]
-    float* w2p = w1t + (size_t)Fh * kSpF;                  // [Fh][16]: w2p[fh][fo] = W2[fh][fo]
-    float* b1s = w2p + (size_t)Fh * kSpF;                  // [Fh]
-    float* b2s = b1s + round_up(Fh, 4);                    // [16]
-    uint64_t* bar = reinterpret_cast<uint64_t*>(b2s + kSpF);
-    const int tid = threadIdx.x;
-    for (int e = tid; e < Fh * kSpF; e += kSrThreads) {
-        const int fh = e / kSpF, f = e % kSpF;
-        w1t[e] = f < Fi ? W1[(size_t)f * Fh + fh] : 0.0f;
-        w2p[e] = f < Fo ? W2[(size_t)fh * Fo + f] : 0.0f;
-    }
-    for (int e = tid; e < Fh; e += kSrThreads) b1s[e] = b1[e];
-    if (tid < kSpF) b2s[tid] = tid < Fo ? b2[tid] : 0.0f;
-    if (tid == 0) {
-        mbar_init(bar, 1);
-        fence_mbar_init();
-    }
-    __syncthreads();
-    float* zrow = Zscr + (size_t)blockIdx.x * Fo * S;      // this CTA's scratch row, [Fo][S]
-    const unsigned xbytes = (unsigned)((size_t)S * Fi * 4), zbytes = (unsigned)((size_t)S * Fo * 4);
-    const bool z_bulk = (zbytes & 15) == 0 && (reinterpret_cast<uintptr_t>(zrow) & 15) == 0;
-    unsigned phase = 0;
-
-    for (long long r = blockIdx.x; r < R; r += gridDim.x) {
-        // ---- the row's X slab: one bulk copy ----
-        const float* xr = X + (size_t)r * S * Fi;
-        if ((xbytes & 15) == 0 && (reinterpret_cast<uintptr_t>(xr) & 15) == 0) {
-            if (tid == 0) {
-                mbar_expect_tx(bar, xbytes);
-                bulk_g2s(slab, xr, xbytes, bar);
-            }
-            mbar_wait(bar, phase);
-            phase ^= 1;
-        } else {
-            for (int e = tid; e < S * Fi; e += kSrThreads) slab[e] = __ldg(xr + e);
-            __syncthreads();
-        }
-        // ---- pass 1 ----
-        for (int base = 0; base < S; base += kSrThreads * kSrGroup) {
-            float2 ag[FW][kSrPairs];
-#pragma unroll
-            for (int f = 0; f < FW; ++f)
-#pragma unroll
-                for (int q = 0; q < kSrPairs; ++q) ag[f][q] = make_float2(0.0f, 0.0f);
-            // the four stations' neighbour lists are walked together (four independent load chains
-            // per step; a finished list contributes a = 0 against slab row 0)
-            int eb[kSrGroup], en[kSrGroup], nmax = 0;
-#pragma unroll
-            for (int i = 0; i < kSrGroup; ++i) {
-                const int s = base + tid + i * kSrThreads;
-                eb[i] = s < S ? __ldg(rowptr + s) : 0;
-                en[i] = s < S ? __ldg(rowptr + s + 1) - eb[i] : 0;
-                nmax = en[i] > nmax ? en[i] : nmax;
-            }
-#pragma unroll 2
-            for (int j = 0; j < nmax; ++j) {
-                float a[kSrGroup];
-                const float* xs[kSrGroup];
-#pragma unroll
-                for (int i = 0; i < kSrGroup; ++i) {
-                    const bool ok = j < en[i];
-                    a[i] = ok ? __ldg(vals + eb[i] + j) : 0.0f;
-                    xs[i] = slab + (size_t)(ok ? __ldg(colidx + eb[i] + j) : 0) * Fi;
-                }
-#pragma unroll
-                for (int i = 0; i < kSrGroup; ++i) {
-#pragma unroll
-                    for (int f = 0; f < FW; ++f) {
-                        if (f < Fi) {
-                            if (i & 1) ag[f][i >> 1].y = fmaf(a[i], xs[i][f], ag[f][i >> 1].y);
-                            else ag[f][i >> 1].x = fmaf(a[i], xs[i][f], ag[f][i >> 1].x);
-                        }
-                    }
-                }
-            }
-            float2 z[FW][kSrPairs];
-#pragma unroll
-            for (int f = 0; f < FW; ++f)
-#pragma unroll
-                for (int q = 0; q < kSrPairs; ++q) z[f][q] = make_float2(0.0f, 0.0f);
-#pragma unroll 2
-            for (int fh = 0; fh < Fh; ++fh) {
-                float2 h[kSrPairs];
-#pragma unroll
-                for (int q = 0; q < kSrPairs; ++q) h[q] = make_float2(0.0f, 0.0f);
-#pragma unroll
-                for (int v = 0; v < kSpF / 4; ++v) {
-                    const float4 w = *reinterpret_cast<const float4*>(w1t + fh * kSpF + 4 * v);
-                    const float wv[4] = {w.x, w.y, w.z, w.w};
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        if (4 * v + j < FW) {
-#pragma unroll
-                            for (int q = 0; q < kSrPairs; ++q)
-                                h[q] = __ffma2_rn(make_float2(wv[j], wv[j]), ag[4 * v + j][q], h[q]);
-                        }
-                    }
-                }
-                const float bb = b1s[fh];
-#pragma unroll
-                for (int q = 0; q < kSrPairs; ++q) {
-                    h[q].x += bb; h[q].y += bb;
-                    h[q].x = h[q].x < 0.0f ? 0.0f : h[q].x;   // ReLU of layer 1
-                    h[q].y = h[q].y < 0.0f ? 0.0f : h[q].y;
-                }
-#pragma unroll
-                for (int v = 0; v < kSpF / 4; ++v) {
-                    const float4 w = *reinterpret_cast<const float4*>(w2p + fh * kSpF + 4 * v);
-                    const float wv[4] = {w.x, w.y, w.z, w.w};
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        if (4 * v + j < FW) {
-#pragma unroll
-                            for (int q = 0; q < kSrPairs; ++q)
-                                z[4 * v + j][q] = __ffma2_rn(make_float2(wv[j], wv[j]), h[q], z[4 * v + j][q]);
-                        }
-                    }
-                }
-            }
-#pragma unroll
-            for (int i = 0; i < kSrGroup; ++i) {
-                const int s = base + tid + i * kSrThreads;
-                if (s < S) {
-#pragma unroll
-                    for (int f = 0; f < FW; ++f)
-                        if (f < Fo) zrow[(size_t)f * S + s] = (i & 1) ? z[f][i >> 1].y : z[f][i >> 1].x;
-                }
-            }
-        }
-        // ---- Z row back over the slab (every thread is done with X; the scratch row is L2-hot) ----
-        __threadfence();
-        asm volatile("fence.proxy.async;\n" ::: "memory");   // generic-proxy stores -> visible to the bulk copy
-        __syncthreads();
-        if (z_bulk) {
-            if (tid == 0) {
-                mbar_expect_tx(bar, zbytes);
-                bulk_g2s(slab, zrow, zbytes, bar);
-            }
-            mbar_wait(bar, phase);
-            phase ^= 1;
-        } else {
-            for (int e = tid; e < S * Fo; e += kSrThreads) slab[e] = zrow[e];
-            __syncthreads();
-        }
-        // ---- pass 2: U[s] = relu((A.Z)[s] + b2), tiled store ----
-        float* urow = U + (size_t)r * S * Fo;   // row-major [R][S * Fo]; rows_to_tiles_kernel re-lays it
-        for (int base = 0; base < S; base += kSrThreads * kSrGroup) {
-            float acc[kSrGroup][FW];
-            int eb[kSrGroup], en[kSrGroup], nmax = 0;
-#pragma unroll
-            for (int i = 0; i < kSrGroup; ++i) {
-                const int s = base + tid + i * kSrThreads;
-                eb[i] = s < S ? __ldg(rowptr + s) : 0;
-                en[i] = s < S ? __ldg(rowptr + s + 1) - eb[i] : 0;
-                nmax = en[i] > nmax ? en[i] : nmax;
-#pragma unroll
-                for (int f = 0; f < FW; ++f) acc[i][f] = 0.0f;
-            }
-#pragma unroll 2
-            for (int j = 0; j < nmax; ++j) {
-                float a[kSrGroup];
-                const float* zs[kSrGroup];
-#pragma unroll
-                for (int i = 0; i < kSrGroup; ++i) {
-                    const bool ok = j < en[i];
-                    a[i] = ok ? __ldg(vals + eb[i] + j) : 0.0f;
-                    zs[i] = slab + (ok ? __ldg(colidx + eb[i] + j) : 0);
-                }
-#pragma unroll
-                for (int i = 0; i < kSrGroup; ++i)
-#pragma unroll
-                    for (int f = 0; f < FW; ++f)
-                        if (f < Fo) acc[i][f] = fmaf(a[i], zs[i][(size_t)f * S], acc[i][f]);
-            }
-#pragma unroll
-            for (int i = 0; i < kSrGroup; ++i) {
-                const int s = base + tid + i * kSrThreads;
-                if (s < S) {
-#pragma unroll
-                    for (int f = 0; f < FW; ++f) {
-                        if (f < Fo) {
-                            float v = acc[i][f] + b2s[f];
-                            v = v < 0.0f ? 0.0f : v;
-                            urow[(size_t)s * Fo + f] = v;
-                        }
-                    }
-                }
-            }
-        }
-        __syncthreads();   // the slab is free for the next row's bulk copy
-    }
 }
 
 // Urow [R][lds] row-major (first K columns used) -> U tiles [ceil(R/128)][ldo][128] (K-major), columns

@@ -3,10 +3,10 @@
 // Reference arithmetic as in gcn_sparse.cuh (src/step5_gcn_layer_model.py:13-23 twice, via
 // src/step6_gcn_gru_combined_model.py:17,20), layer 2 evaluated as relu(A.(G1.W2) + b2).
 //
-// ncu on gcn_sparse_row_kernel (profiles/r01_sparse_ncu_summary.md) showed the shared-memory pipe as the bound,
-// not the FMA pipe: 1.59 G wavefronts per launch, half of them the warp-uniform LDS.128 weight reads of the
-// dense phase (2 wavefronts each) and half the neighbour gathers (2.7 wavefronts per LDS: the 32 lanes of a
-// warp read 32 random slab rows).  This kernel removes both:
+// ncu on the first-generation row-resident kernel (profiles/r01_sparse_ncu_summary.md) showed the shared-memory
+// pipe as the bound, not the FMA pipe: 1.59 G wavefronts per launch, half of them the warp-uniform LDS.128 weight
+// reads of the dense phase (2 wavefronts each) and half the neighbour gathers (2.7 wavefronts per LDS: the 32 lanes
+// of a warp read 32 random slab rows).  This kernel removes both:
 //   * W1, W2, b1, b2 live in CONSTANT memory and reach FFMA2 as uniform-register operands (LDCU): the dense
 //     phase issues no shared-memory instruction at all and a thread covers FOUR stations (two FFMA2 pairs),
 //     68 TFLOP/s in isolation (scripts/probes/dense_probe.cu) against 52 with LDS.128 weights;
@@ -17,8 +17,8 @@
 //     entry (col, val) of a step is one coalesced 8-byte load per lane.  Blocks the plan cannot hold
 //     (a station with more than 64 neighbours, or more than kSqPlanCap steps) keep the CSR order.
 // The order in which a station's neighbours are added is the plan's (a pure function of the graph), so results
-// are deterministic and independent of batch size / chunking; they differ from gcn_sparse_row_kernel's by
-// rounding only.
+// are deterministic and independent of batch size / chunking; they differ from the CSR-order sums of
+// gcn_sparse_l1_kernel / gcn_sparse_l2_kernel by rounding only.
 // Both passes write f-major rows ([F][S], coalesced from the thread = station mapping); fmajor_to_tiles_kernel
 // re-lays U into the projection GEMM's K-major 128-row tiles.
 #pragma once

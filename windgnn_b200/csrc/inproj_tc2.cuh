@@ -5,7 +5,7 @@
 //
 // Reference: the `gi = W_ih u + b_ih` half of nn.GRU, src/step6_gcn_gru_combined_model.py:11,23.
 //
-// inproj_tc_kernel (first generation, TF32 hi / lo copies of both operands in HBM) moved 11.1 GB from L2
+// The first-generation kernel (kind::tf32, hi / lo copies of both operands in HBM) moved 11.1 GB from L2
 // for 2.06 GB of algorithmic operand bytes and was L2-bound with the tensor pipe 49 % busy (ncu r01).
 // Here the GCN kernel's ordinary fp32 tiles are the A operand: a stage's [32 k][128 rows] fp32 block
 // arrives by one bulk copy, four converter warps split it into fp16 hi / lo in the UMMA K-major layout
@@ -27,8 +27,8 @@
 
 #include <cuda_fp16.h>
 
-#include "inproj_tc.cuh"
 #include "recur_tc.cuh"
+#include "tcgen05.cuh"
 #include "wg_common.cuh"
 
 namespace wg {

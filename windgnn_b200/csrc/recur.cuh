@@ -7,11 +7,13 @@
 //     h' = (h - n) * z + n
 // gi (with b_ih, and b_hh for r and z, already added) comes from the input-projection kernel.
 //
-// A CTA owns 32 sequences for all T steps.  W_hh^T ([k][n], zero padded to KP x NP) lives in
-// shared memory for the whole kernel, the hidden state of the 32 sequences too; nothing but gi
-// (read) and h (written) touches HBM inside the time loop.  The warps form TWO independent
-// groups of 16 sequences that only ever synchronise among themselves (named barriers), so one
-// group's gate phase (MUFU-bound) overlaps the other group's GEMM (FMA-bound).  Per step:
+// gru_recur_kernel serves the hidden sizes that gru_recur_unit_kernel (recur_unit.cuh) cannot fit in
+// shared memory, H = 125 .. 360.  A CTA owns 32 sequences for all T steps.  W_hh^T ([k][n], zero
+// padded to KP x NP; too large for shared memory at these sizes) is read through L1 / L2 every step,
+// the hidden state of the 32 sequences lives in shared memory; nothing but gi (read) and h
+// (written) touches HBM inside the time loop.  The 16 warps form TWO independent groups of 16
+// sequences that only ever synchronise among themselves (named barriers), so one group's gate phase
+// (MUFU-bound) overlaps the other group's GEMM (FMA-bound).  Per step:
 //   GEMM  : acc[b][n] = sum_k h[b][k] * W[k][n] on the FMA pipe with packed FFMA2 (sm_100a):
 //           acc2[b][(n, n+1)] += h[b][k] (scalar operand, broadcast) * (W[k][n], W[k][n+1]).
 //           A warp covers 16 sequences x 80 gate columns, a thread 4 x 10 (five column pairs);
@@ -30,6 +32,7 @@ namespace wg {
 
 constexpr int kRcBT = 32;    // sequences per CTA (two groups of 16)
 constexpr int kRcCB = 80;    // gate columns per warp
+constexpr int kRcWarps = 16;   // eight per group; a warp loops over every eighth 80-column block
 
 __host__ __device__ inline int recur_np(int G) { return round_up(G, kRcCB); }
 // hidden-state rows: KP floats padded so that four consecutive rows start in distinct bank groups
@@ -37,9 +40,8 @@ __host__ __device__ inline int recur_hs_stride(int KP) { return ((KP / 4) & 1) ?
 // timesteps staged in shared memory per bulk store of h: the smallest count that makes one
 // sequence's staged block (TS * H floats) a multiple of 16 bytes
 __host__ __device__ inline int recur_stage_steps(int H) { return (H % 4 == 0) ? 1 : (H % 2 == 0) ? 2 : 4; }
-__host__ __device__ inline size_t recur_smem_floats(int KP, int NP, int GP, bool w_smem, int H = 0, int TS = 0) {
+__host__ __device__ inline size_t recur_smem_floats(int KP, int GP, int H = 0, int TS = 0) {
     size_t n = (size_t)round_up(kRcBT * TS * H, 4);  // staging of h for the bulk stores (TS = 0: none)
-    if (w_smem) n += (size_t)KP * NP;
     n += (size_t)kRcBT * recur_hs_stride(KP);  // hs
     n += (size_t)kRcBT * GP;                   // gi tile (r,z columns become gi + gh)
     n += (size_t)kRcBT * KP;                   // gh of the n gate
@@ -57,23 +59,6 @@ __device__ __forceinline__ void cp_async8(void* smem_dst, const void* gmem_src) 
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(smem_u32(smem_dst)), "l"(gmem_src) : "memory");
 }
 
-#ifndef WG_GATE_EXP
-#define WG_GATE_EXP 0
-#endif
-#ifndef WG_GEMM_EXP
-#define WG_GEMM_EXP 0
-#endif
-#ifdef WG_RC_TRACE
-// debug build only: per-phase clock stamps of CTA 0 (8 stamps per step per group)
-__device__ long long g_rc_trace[2 * 8 * 256];
-#define WG_TRACE(slot)                                                                          \
-    do {                                                                                        \
-        if (blockIdx.x == 0 && gtid == 0 && t < 256) g_rc_trace[(grp * 256 + t) * 8 + (slot)] = clock64(); \
-    } while (0)
-#else
-#define WG_TRACE(slot) do { } while (0)
-#endif
-
 // one operand fragment: four k's of this thread's 4 rows and 10 columns
 struct RcFrag {
     float4 h[4];      // h[i] = hs[row i][k .. k+3]
@@ -82,21 +67,17 @@ struct RcFrag {
     float2 wc[4];     // W[k + kk][cC .. cC+1]
 };
 
-// SAVE (training forward): the gate values the backward pass needs are written beside h:
-// gsave[b, t, :] = [r | z | n | hn] with hn = W_hn h + b_hn, row stride ldsave (gru_bwd.cuh).
-template <int NWARPS, bool W_SMEM, bool SAVE = false>
-__global__ void __launch_bounds__(NWARPS * 32, 1)
+__global__ void __launch_bounds__(kRcWarps * 32, 1)
     gru_recur_kernel(const float* __restrict__ GI, const float* __restrict__ WhT,
                      const float* __restrict__ bhn, float* __restrict__ out, long long B, int T, int H,
-                     int ldg, int KP, int NP, int TS, float* __restrict__ gsave = nullptr, int ldsave = 0) {
-    constexpr int NT = NWARPS * 32;
-    constexpr int WG = NWARPS / 2;   // warps per group
+                     int ldg, int KP, int NP, int TS) {
+    constexpr int NT = kRcWarps * 32;
+    constexpr int WG = kRcWarps / 2;   // warps per group
     constexpr int NG = WG * 32;      // threads per group
     constexpr int GB = kRcBT / 2;    // sequences per group
     extern __shared__ __align__(16) float smem[];
     const int RS = recur_hs_stride(KP);
-    float* Ws = smem;
-    float* hs = smem + (W_SMEM ? (size_t)KP * NP : 0);
+    float* hs = smem;
     float* gis = hs + kRcBT * RS;          // [32][ldg]
     float* ghn = gis + kRcBT * ldg;        // [32][KP]
     float* bns = ghn + kRcBT * KP;         // [KP]
@@ -104,7 +85,6 @@ __global__ void __launch_bounds__(NWARPS * 32, 1)
     // bulk (TMA) stores of h need 16-byte aligned, 16-byte-multiple spans per sequence
     const bool bulk_ok = TS > 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0 && (((long long)T * H) & 3) == 0 &&
                          ((TS * H) & 3) == 0;
-    const float* Wsrc = W_SMEM ? Ws : WhT;
 
     const int tid = threadIdx.x;
     const int lane = tid & 31;
@@ -115,12 +95,6 @@ __global__ void __launch_bounds__(NWARPS * 32, 1)
     const long long b0 = (long long)blockIdx.x * kRcBT;
     const int H2 = 2 * H;
 
-    if (W_SMEM) {
-        const int n4 = KP * NP / 4;
-        const float4* src = reinterpret_cast<const float4*>(WhT);
-        float4* dst = reinterpret_cast<float4*>(Ws);
-        for (int e = tid; e < n4; e += NT) dst[e] = __ldg(src + e);
-    }
     for (int e = tid; e < kRcBT * RS; e += NT) hs[e] = 0.0f;
     for (int e = tid; e < kRcBT * ldg; e += NT) gis[e] = 0.0f;
     for (int e = tid; e < kRcBT * KP; e += NT) ghn[e] = 0.0f;
@@ -158,14 +132,7 @@ __global__ void __launch_bounds__(NWARPS * 32, 1)
 
     const float* hrow = hs + rbase * RS;
     const int h_step = 4 * RS;
-#ifndef WG_RC_ALTERNATE
-#define WG_RC_ALTERNATE 1
-#endif
     for (int t = 0; t < T; ++t) {
-        WG_TRACE(0);
-#if WG_RC_ALTERNATE == 2
-        group_barrier(5, NT);  // experiment: both groups start every step together
-#elif WG_RC_ALTERNATE
         // The two groups take turns on the FMA pipe: group 0 runs GEMM(t) while group 1 does the
         // merge / gates of step t-1, then they swap.  Barrier 3: "group 0 finished its GEMM",
         // barrier 4: "group 1 finished its GEMM" (arrive = signal, sync = wait; NT participants).
@@ -174,9 +141,7 @@ __global__ void __launch_bounds__(NWARPS * 32, 1)
         } else {
             group_barrier(3, NT);
         }
-#endif
         // ================= GEMM + merge =================
-        WG_TRACE(1);
         bool handed_over = false;
         for (int cb = gwarp; cb < n_cb; cb += WG) {
             const int cA = cb * kRcCB + ln * 4, cB = cA + 32, cC = cb * kRcCB + 64 + ln * 2;
@@ -187,22 +152,16 @@ __global__ void __launch_bounds__(NWARPS * 32, 1)
                 for (int p = 0; p < 5; ++p) acc[i][p] = make_float2(0.0f, 0.0f);
 
             const float* hp = hrow;            // + 4 floats per fragment
-            const float* wp = Wsrc + cA;       // + 4 * NP floats per fragment
+            const float* wp = WhT + cA;        // + 4 * NP floats per fragment
             auto load_frag = [&](RcFrag& f) {
 #pragma unroll
                 for (int i = 0; i < 4; ++i) f.h[i] = *reinterpret_cast<const float4*>(hp + i * h_step);
 #pragma unroll
                 for (int kk = 0; kk < 4; ++kk) {
                     const float* w = wp + kk * NP;
-                    if (W_SMEM) {
-                        f.wa[kk] = *reinterpret_cast<const float4*>(w);
-                        f.wb[kk] = *reinterpret_cast<const float4*>(w + 32);
-                        f.wc[kk] = *reinterpret_cast<const float2*>(w + 64 - 2 * ln);
-                    } else {
-                        f.wa[kk] = __ldg(reinterpret_cast<const float4*>(w));
-                        f.wb[kk] = __ldg(reinterpret_cast<const float4*>(w + 32));
-                        f.wc[kk] = __ldg(reinterpret_cast<const float2*>(w + 64 - 2 * ln));
-                    }
+                    f.wa[kk] = __ldg(reinterpret_cast<const float4*>(w));
+                    f.wb[kk] = __ldg(reinterpret_cast<const float4*>(w + 32));
+                    f.wc[kk] = __ldg(reinterpret_cast<const float2*>(w + 64 - 2 * ln));
                 }
                 hp += 4;
                 wp += 4 * NP;
@@ -228,14 +187,6 @@ __global__ void __launch_bounds__(NWARPS * 32, 1)
                 RcFrag fa, fb;
                 load_frag(fa);
                 int k4 = 4;
-#if WG_GEMM_EXP == 1
-                load_frag(fb);   // experiment: no loads inside the loop (wrong results, timing only)
-#pragma unroll 1
-                for (; k4 + 4 < KP; k4 += 8) {
-                    mma_frag(fa);
-                    mma_frag(fb);
-                }
-#else
 #pragma unroll 1
                 for (; k4 + 4 < KP; k4 += 8) {
                     load_frag(fb);
@@ -243,7 +194,6 @@ __global__ void __launch_bounds__(NWARPS * 32, 1)
                     load_frag(fa);
                     mma_frag(fb);
                 }
-#endif
                 if (k4 < KP) {   // even number of fragments: one more pair
                     load_frag(fb);
                     mma_frag(fa);
@@ -252,14 +202,11 @@ __global__ void __launch_bounds__(NWARPS * 32, 1)
                     mma_frag(fa);
                 }
             }
-#if WG_RC_ALTERNATE == 1
             if (cb + WG >= n_cb) {  // last column block of this warp: hand the FMA pipe over
                 if (grp == 0) group_arrive(3, NT);
                 else if (t + 1 < T) group_arrive(4, NT);
                 handed_over = true;
             }
-#endif
-            WG_TRACE(2);
             cp_async_wait<0>();  // this thread's chunks of gi(t) have landed
             // merge: r/z columns accumulate onto gi (vector read-modify-write), n-gate columns go to
             // ghn; a chunk that straddles a gate boundary (or the padding) takes the element path.
@@ -299,18 +246,12 @@ __global__ void __launch_bounds__(NWARPS * 32, 1)
             merge_chunk(cB, IntC<4>{}, 2);
             merge_chunk(cC, IntC<2>{}, 4);
         }
-#if WG_RC_ALTERNATE == 1
         if (!handed_over) {  // a warp without a column block still takes part in the hand-over
             if (grp == 0) group_arrive(3, NT);
             else if (t + 1 < T) group_arrive(4, NT);
         }
-#else
-        (void)handed_over;
-#endif
-        WG_TRACE(3);
         if (bulk_ok && gtid < GB) bulk_wait_read();  // the previous bulk store has read its staging rows
         group_barrier(1 + grp, NG);
-        WG_TRACE(4);
 
         // ================= gate phase =================
         // A thread owns hidden unit(s) j and walks the group's 16 sequences: every address is a
@@ -336,13 +277,6 @@ __global__ void __launch_bounds__(NWARPS * 32, 1)
                 const float hn = gn[bl * KP] + bn;
                 const float n = tanh_f(g[bl * ldg + H2] + r * hn);
                 hnew[bl] = (hp[bl * RS] - n) * z + n;
-                if (SAVE && b0 + grp * GB + bl < B) {
-                    float* gs = gsave + ((size_t)(b0 + grp * GB + bl) * T + t) * ldsave + j;
-                    gs[0] = r;
-                    gs[H] = z;
-                    gs[H2] = n;
-                    gs[H2 + H] = hn;
-                }
             }
 #pragma unroll
             for (int bl = 0; bl < GB; ++bl) {
@@ -352,9 +286,7 @@ __global__ void __launch_bounds__(NWARPS * 32, 1)
             }
         }
         if (TS > 0) asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");  // staged h -> async proxy
-        WG_TRACE(5);
         group_barrier(1 + grp, NG);
-        WG_TRACE(6);
         if (TS > 0 && ((t % TS) == TS - 1 || t == T - 1)) {
             // flush the staged steps t0 .. t of this group's 16 sequences to out[b][t0 .. t][:]
             const int t0 = t - (t % TS), nst = t - t0 + 1;
@@ -377,224 +309,25 @@ __global__ void __launch_bounds__(NWARPS * 32, 1)
             }
         }
         if (t + 1 < T) prefetch_gi(t + 1);  // lands during the next GEMM
-        WG_TRACE(7);
     }
     if (bulk_ok && gtid < GB) bulk_wait_read();  // shared memory must outlive the last bulk store's reads
 }
 
-}  // namespace wg
-
-namespace wg {
-
 // ---------------------------------------------------------------------------------------------
-// Small-batch recurrence: 4 sequences per CTA.
+// Small-batch recurrence: 4 sequences per CTA, W_hh IN REGISTERS (compile-time contraction length KPT).
 //
-// gru_recur_kernel above is a throughput kernel: 32 sequences per CTA, ~8 us per timestep whatever
-// the batch — 1.4 ms for T = 168 even for ONE window, which is the reference's own call pattern
-// (`model(adj_matrix, batch_x)` with batch 1, src/main.py:66,102) and the per-GPU shard of the
-// training configuration.  When the batch does not fill the SMs at 32 per CTA this kernel runs
-// instead: same data flow (W_hh^T resident in shared memory, gi of the next step prefetched with
-// cp.async, h kept in shared memory), but a CTA owns only 4 sequences, so a step is a
-// [4 x H].[H x 3H] product (thread tile 4 sequences x 2 gate columns, FFMA2) + 408 gate items and
-// takes a few microseconds.
-//
-// Every output's sum runs over k = 0 .. KP-1 ascending in ONE FFMA chain, and the merge / gate
-// expressions are the ones of gru_recur_kernel, so both kernels produce bit-identical results
-// (chunking / sharding invariance is tested bit-exactly).
+// The throughput kernels spend a fixed time per timestep whatever the batch; a few sequences — the
+// reference's own call pattern (`model(adj_matrix, batch_x)` with batch 1, src/main.py:66,102) or a
+// small per-GPU shard — leave most of the machine idle.  For the contraction lengths of the shipped
+// models (KP = 24: the 7-station model, KP = 104: the 34-station model) this kernel runs instead
+// when the batch is small.  A thread owns one gate COLUMN and keeps its KPT weights in registers for
+// the whole kernel (streaming W_hh^T — 127 KB at H = 102 — out of shared memory cost ~1000 cycles of
+// LSU time per step even for ONE sequence); a step's product is KPT FFMAs per sequence in one
+// dependent chain (k ascending: bit-identical to every other recurrence kernel), fed by broadcast
+// 16-byte loads of h.  Shared memory holds only h, gi (double buffered, prefetched with cp.async one
+// step ahead) and gh (17 KB).  Serves 3H (padded) <= 320.
 // ---------------------------------------------------------------------------------------------
-constexpr int kRsBT = 4;        // sequences per CTA
-constexpr int kRsCols = 192;     // gate-column pairs a CTA can hold (3H <= 384)
-constexpr int kRsThreads = 2 * kRsCols;   // 12 warps: the product runs on the first NP / 2 threads, the gate math on all
-
-__host__ __device__ inline size_t recur_small_smem_floats(int KP, int NP, int GP) {
-    size_t n = (size_t)KP * NP;            // W_hh^T
-    n += (size_t)kRsBT * (KP + 4);         // hs
-    n += 2 * (size_t)kRsBT * GP;           // gi tiles (double buffered)
-    n += (size_t)kRsBT * NP;               // gh = h . W_hh^T of the current step
-    n += (size_t)KP;                       // b_hn
-    return n;
-}
-
-// One step's product for one gate-column pair and the NS sequences of the CTA that exist:
-// gh[i][2cp .. 2cp+1] = sum_k h[i][k] * W_hh^T[k][2cp .. 2cp+1], k ascending in ONE FFMA2 chain per sequence.
-// Stages of KS k's (8 for one or two chains, 4 for three or four), double buffered in registers: a stage's FMAs
-// (>= 36 cycles) cover the shared-memory latency of the next stage's operands even with a single chain.
-// N4: number of 4-k groups actually used of the stage (the last stage of a KS = 8 loop may be half full).
-template <int NS, int KS, int N4>
-__device__ __forceinline__ void rs_load(const float* __restrict__ wp, const float* __restrict__ hs, int k, int NP, int RS,
-                                        float4 (&hh)[NS][KS / 4], float2 (&ww)[KS]) {
-#pragma unroll
-    for (int i = 0; i < NS; ++i)
-#pragma unroll
-        for (int q = 0; q < N4; ++q) hh[i][q] = *reinterpret_cast<const float4*>(hs + i * RS + k + 4 * q);
-#pragma unroll
-    for (int kk = 0; kk < 4 * N4; ++kk) ww[kk] = *reinterpret_cast<const float2*>(wp + (size_t)(k + kk) * NP);
-}
-template <int NS, int KS, int N4>
-__device__ __forceinline__ void rs_fma(float2 (&acc)[NS], const float4 (&hh)[NS][KS / 4], const float2 (&ww)[KS]) {
-#pragma unroll
-    for (int kk = 0; kk < 4 * N4; ++kk) {
-#pragma unroll
-        for (int i = 0; i < NS; ++i) {
-            const float4 q = hh[i][kk >> 2];
-            const float a = (kk & 3) == 0 ? q.x : (kk & 3) == 1 ? q.y : (kk & 3) == 2 ? q.z : q.w;
-            acc[i] = __ffma2_rn(make_float2(a, a), ww[kk], acc[i]);
-        }
-    }
-}
-template <int NS>
-__device__ __forceinline__ void rs_gemm(const float* __restrict__ wp, const float* __restrict__ hs, float* __restrict__ gh,
-                                        int KP, int NP, int RS) {
-    constexpr int KS = NS <= 2 ? 8 : 4, G4 = KS / 4;
-    float2 acc[NS];
-#pragma unroll
-    for (int i = 0; i < NS; ++i) acc[i] = make_float2(0.0f, 0.0f);
-    float4 hA[NS][G4], hB[NS][G4];
-    float2 wA[KS], wB[KS];
-    // KP is a multiple of 4: `full` stages of KS, then (KS = 8 only) possibly one half stage (`tail`)
-    const int full = KP / KS;
-    const bool tail = (KP % KS) != 0;
-    if (full > 0) rs_load<NS, KS, G4>(wp, hs, 0, NP, RS, hA, wA);
-    else if (tail) rs_load<NS, KS, 1>(wp, hs, 0, NP, RS, hA, wA);
-    int s8 = 0;
-#pragma unroll 1
-    for (; s8 + 2 <= full; s8 += 2) {
-        rs_load<NS, KS, G4>(wp, hs, (s8 + 1) * KS, NP, RS, hB, wB);
-        rs_fma<NS, KS, G4>(acc, hA, wA);
-        if (s8 + 2 < full) rs_load<NS, KS, G4>(wp, hs, (s8 + 2) * KS, NP, RS, hA, wA);
-        else if (tail) rs_load<NS, KS, 1>(wp, hs, (s8 + 2) * KS, NP, RS, hA, wA);
-        rs_fma<NS, KS, G4>(acc, hB, wB);
-    }
-    if (s8 < full) {   // one full stage left in A
-        if (tail) rs_load<NS, KS, 1>(wp, hs, (s8 + 1) * KS, NP, RS, hB, wB);
-        rs_fma<NS, KS, G4>(acc, hA, wA);
-        if (tail) rs_fma<NS, KS, 1>(acc, hB, wB);
-    } else if (tail) {
-        rs_fma<NS, KS, 1>(acc, hA, wA);
-    }
-#pragma unroll
-    for (int i = 0; i < NS; ++i) *reinterpret_cast<float2*>(gh + i * NP) = acc[i];
-}
-
-// NB: FMA chains per thread = min(4, batch) (a kernel parameter rather than a per-CTA switch: with the four
-// variants inlined behind one switch ptxas hoists across the cases and spills).
-template <bool SAVE, int NB>
-__global__ void __launch_bounds__(kRsThreads, 1)
-    gru_recur_small_kernel(const float* __restrict__ GI, const float* __restrict__ WhT, const float* __restrict__ bhn,
-                           float* __restrict__ out, long long B, int T, int H, int ldg, int KP, int NP,
-                           float* __restrict__ gsave, int ldsave) {
-    extern __shared__ __align__(16) float smem[];
-    const int RS = KP + 4;
-    float* Ws = smem;                          // [KP][NP]
-    float* hs = Ws + (size_t)KP * NP;          // [4][RS]
-    float* gis = hs + kRsBT * RS;              // [2][4][ldg]
-    float* ghs = gis + 2 * kRsBT * ldg;        // [4][NP]
-    float* bns = ghs + kRsBT * NP;             // [KP]
-    const int tid = threadIdx.x;
-    const long long b0 = (long long)blockIdx.x * kRsBT;
-    const int H2 = 2 * H;
-
-    {
-        const int n4 = KP * NP / 4;
-        const float4* src = reinterpret_cast<const float4*>(WhT);
-        float4* dst = reinterpret_cast<float4*>(Ws);
-        for (int e = tid; e < n4; e += kRsThreads) dst[e] = __ldg(src + e);
-    }
-    for (int e = tid; e < kRsBT * RS; e += kRsThreads) hs[e] = 0.0f;
-    for (int e = tid; e < 2 * kRsBT * ldg; e += kRsThreads) gis[e] = 0.0f;
-    for (int e = tid; e < kRsBT * NP; e += kRsThreads) ghs[e] = 0.0f;
-    for (int e = tid; e < KP; e += kRsThreads) bns[e] = e < H ? __ldg(bhn + e) : 0.0f;
-
-    // gi rows of step t -> buffer (t & 1): 16-byte chunks (ldg is a multiple of 4, rows 16-byte aligned).  The
-    // copies are issued by the UPPER half of the CTA (the lower half runs the product and should start on it at
-    // once); each of those threads owns fixed chunks whose source advances by one row per step — no index
-    // arithmetic inside the time loop.
-    const int chunks = ldg >> 2;
-    constexpr int kPfThreads = kRsThreads - kRsCols, kPfMax = (kRsBT * (4 * 128) / 4 + kPfThreads - 1) / kPfThreads;
-    const float* pf_src[kPfMax];
-    int pf_off[kPfMax];       // float offset inside a gi buffer, -1: no chunk
-    bool pf_ok[kPfMax];
-#pragma unroll
-    for (int q = 0; q < kPfMax; ++q) {
-        const int e = (tid - kRsCols) + q * kPfThreads;
-        const bool mine = tid >= kRsCols && e < kRsBT * chunks;
-        const int b = mine ? e / chunks : 0, c = mine ? e - b * chunks : 0;
-        pf_ok[q] = mine && (b0 + b < B);
-        pf_off[q] = mine ? b * ldg + 4 * c : -1;
-        pf_src[q] = GI + ((size_t)(pf_ok[q] ? b0 + b : 0) * T) * ldg + 4 * c;
-    }
-    // every thread commits a group (empty for the lower half): the waits below count groups
-#define WG_RS_PREFETCH(t_)                                                                              \
-    do {                                                                                                \
-        float* dstb_ = gis + ((t_) & 1) * kRsBT * ldg;                                                  \
-        _Pragma("unroll") for (int q = 0; q < kPfMax; ++q)                                              \
-            if (pf_off[q] >= 0) cp_async16(dstb_ + pf_off[q], pf_src[q] + (size_t)(t_) * ldg, pf_ok[q]); \
-        cp_async_commit();                                                                              \
-    } while (0)
-    __syncthreads();
-    WG_RS_PREFETCH(0);
-
-    // GEMM coordinates: the first NP / 2 threads own one gate-column pair each, for the NB = min(4, batch)
-    // sequences a CTA can have: NB FMA chains per thread (round 1 always ran 4 — for the reference's batch-1 calls three
-    // quarters of the FMAs went to sequences that do not exist).  The k loop (rs_gemm) is software-pipelined by
-    // hand (ncu: the loop waited on LDS).
-    // Every output's sum is still ONE chain over k ascending: bit-identical to every other recurrence kernel.
-    const int cp = tid;
-    const int nb = (int)((B - b0) < kRsBT ? (B - b0) : kRsBT);   // sequences of this CTA that exist
-    const bool gemm_thread = cp < (NP >> 1);
-
-    for (int t = 0; t < T; ++t) {
-        if (t + 1 < T) WG_RS_PREFETCH(t + 1);
-        const float* g = gis + (t & 1) * kRsBT * ldg;
-        if (t > 0 && gemm_thread)   // h_{-1} = 0: the product is zero at t == 0 (ghs was zeroed above)
-            rs_gemm<NB>(Ws + 2 * cp, hs, ghs + 2 * cp, KP, NP, RS);
-        // gi(t) was committed one step ago (or before the loop); only step t+1's group may still be in flight
-        if (t + 1 < T) cp_async_wait<1>(); else cp_async_wait<0>();
-        __syncthreads();   // gi(t) and gh(t) complete
-        // gates: one (sequence, hidden unit) item per thread-slot, lanes along the hidden index; gi + gh is the
-        // same single addition the throughput kernel's merge performs.  H <= 128 here (the launcher requires
-        // NP / 2 <= kRsThreads), so the unrolled slots cover every item
-#pragma unroll
-        for (int u = 0; u < (kRsBT * 128 + kRsThreads - 1) / kRsThreads; ++u) {
-            const int e = tid + u * kRsThreads;
-            if (e < nb * H) {
-                const int b = e / H, j = e - b * H;
-                const float* gr = g + b * ldg + j;
-                const float* gh = ghs + b * NP + j;
-                const float r = sigmoid_f(gr[0] + gh[0]);
-                const float z = sigmoid_f(gr[H] + gh[H]);
-                const float hn = gh[H2] + bns[j];
-                const float n = tanh_f(gr[H2] + r * hn);
-                const float hnew = (hs[b * RS + j] - n) * z + n;
-                hs[b * RS + j] = hnew;
-                if (b0 + b < B) {
-                    out[((size_t)(b0 + b) * T + t) * H + j] = hnew;
-                    if (SAVE) {
-                        float* gs = gsave + ((size_t)(b0 + b) * T + t) * ldsave + j;
-                        gs[0] = r;
-                        gs[H] = z;
-                        gs[H2] = n;
-                        gs[H2 + H] = hn;
-                    }
-                }
-            }
-        }
-        __syncthreads();   // h(t) visible before the next GEMM; gi buffer (t & 1) and gh free again
-    }
-#undef WG_RS_PREFETCH
-}
-
-// ---------------------------------------------------------------------------------------------
-// Small-batch recurrence with W_hh IN REGISTERS (compile-time contraction length KPT).
-//
-// gru_recur_small_kernel streams W_hh^T (127 KB at H = 102) out of shared memory every timestep: ~1000
-// cycles of LSU time per step even when the CTA holds ONE sequence, which is the reference's own
-// call pattern (`model(adj_matrix, batch_x)` with batch 1, src/main.py:66,102).  Here a thread owns one
-// gate COLUMN and keeps its KPT weights in registers for the whole kernel; a step's product is KPT
-// FFMAs per sequence in one dependent chain (k ascending: bit-identical to every other recurrence
-// kernel), fed by broadcast 16-byte loads of h.  Shared memory holds only h, gi and gh (17 KB).
-// Gate math, gi prefetch and outputs as in gru_recur_small_kernel.  Serves 3H (padded) <= 320.
-// ---------------------------------------------------------------------------------------------
+constexpr int kRsBT = 4;          // sequences per CTA
 constexpr int kRwThreads = 320;   // 10 warps >= the 306 gate columns of H = 102
 
 __host__ __device__ inline size_t recur_regw_smem_floats(int KP, int NP, int GP) {

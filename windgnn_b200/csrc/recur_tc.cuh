@@ -11,7 +11,7 @@
 // significant bits, and fp16 x fp16 products are exact in the fp32 accumulator):
 //     D ~= A_hi.B_hi + A_hi.B_lo + A_lo.B_hi          (kind::f16, M = 128, N = 16, K = 16)
 // The A_hi.B_hi products go to one TMEM accumulator, the two corrections to a second one (TMEM
-// accumulation truncates — inproj_tc.cuh — so the small terms are kept apart from the big ones and the
+// accumulation truncates — tcgen05.cuh — so the small terms are kept apart from the big ones and the
 // two are added with round-to-nearest in the epilogue).  The dropped lo.lo term is 2^-22 relative.
 //
 // Why this layout: with the hidden unit on the M axis, TMEM lane j of all three gate tiles holds
@@ -36,8 +36,8 @@
 
 #include <cuda_fp16.h>
 
-#include "inproj_tc.cuh"
 #include "recur.cuh"
+#include "tcgen05.cuh"
 #include "wg_common.cuh"
 
 namespace wg {

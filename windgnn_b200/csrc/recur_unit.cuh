@@ -23,8 +23,9 @@
 // (4 .. 8) so that the grid is one full wave: 4096 sequences -> 147 CTAs of 4 x 7.
 //
 // Every output's sum runs over k ascending in one FMA chain and the gate expressions are those of
-// gru_recur_kernel / gru_recur_small_kernel: the three kernels are bit-identical (tested), so the
-// kernel choice — which depends on the batch size — never changes a result.
+// gru_recur_regw_kernel (recur.cuh), which takes the small batches of the shipped models: the two
+// kernels are bit-identical (tested), so the kernel choice — which depends on the batch size — never
+// changes a result.
 #pragma once
 
 #include "recur.cuh"
