@@ -64,7 +64,11 @@ struct DeviceGuard {
 constexpr size_t kAlign = 256;
 size_t align_up(size_t v) { return (v + kAlign - 1) / kAlign * kAlign; }
 
-// Everything the three stages need to agree on.
+// kGcnNone: no dense gcn_kernel instantiation serves the feature widths
+enum GcnKind { kGcnRows, kGcn13x7, kGcn13x4, kGcn16x4, kGcnNone, kGcnSparsePlan, kGcnSparseLanes };
+enum RecurKind { kRecurTc, kRecurUnit, kRecurWide };
+
+// Everything the stages need to agree on: shapes, workspace layout and the kernel of every stage.
 struct Plan {
     int T, S, Fi, Fh, Fo, H;
     long long chunk;
@@ -74,14 +78,19 @@ struct Plan {
     int GP;        // leading dim of GI: G rounded up to 8
     int KP;        // K of the recurrent GEMM: H rounded up to 4
     int NPR;       // columns of packed w_hh^T: G rounded up to 80 (one warp's column block)
+    int n_bias;    // packed bias entries: one per packed w_ih row of either projection, at least 512
     bool sparse;   // CSR graph path: adds the Z scratch of the sparse GCN kernels
-    bool sq;       // CSR graph path on gcn_sparse_plan_kernel (constant-bank weights + gather plan)
-    size_t off_sqw, off_sqplan;
+    GcnKind gcn;
+    size_t sq_smem;                             // gcn_sparse_plan_kernel: dynamic shared memory,
+    size_t off_sqw, off_sqsteps, off_sqpairs;   // its constant-bank weights and gather plan (steps, pairs)
     bool tc;       // tensor-core input projection (inproj_tc2.cuh): w_ih packed as fp16 hi + lo
     wg::Tc2Shape tc2;
+    RecurKind recur;   // small chunks may run gru_recur_regw_kernel instead (launch_recur)
+    bool regw;         // the contraction length fits gru_recur_regw_kernel, which then takes small chunks
+    bool whu;          // W_hh^T packed for gru_recur_unit_kernel: whenever that kernel serves H, on every path
+    int ru_wpg, ru_ht; // gru_recur_unit_kernel: warps per group, compile-time H (102 or 21) or 0
     size_t off_wp, off_bias, off_wht, off_whu, off_bhn, off_u, off_gi, off_z, total;
-    bool tc_recur;             // tensor-core recurrence (recur_tc.cuh): W_hh packed as fp16 hi + lo
-    size_t off_whh_hi, off_whh_lo;
+    size_t off_whh_hi, off_whh_lo;   // kRecurTc: W_hh packed as fp16 hi + lo
 };
 
 long long default_chunk(long long B, size_t bytes_per_seq) {
@@ -93,6 +102,20 @@ long long default_chunk(long long B, size_t bytes_per_seq) {
         if (c < wg::kRcBT) c = wg::kRcBT;
     }
     return B < c ? (B < 1 ? 1 : B) : c;
+}
+
+// gcn_kernel instantiation for the feature widths (the single layer passes F_out as F_hid): the exact 13-wide one
+// with 7 or 4 stations per thread, whichever pads S less (ties: 7), else the generic 16-wide one
+GcnKind dense_gcn_kind(int S, int Fi, int Fh, int Fo) {
+    if (Fi == 13 && Fh == 13 && Fo == 13) return wg::ceil_div(S, 7) * 7 <= wg::ceil_div(S, 4) * 4 ? kGcn13x7 : kGcn13x4;
+    return Fi <= 16 && Fh <= 16 && Fo <= 16 ? kGcn16x4 : kGcnNone;
+}
+
+// Testing knob: WG_FORCE_LEGACY=1 runs the fused two-layer GCN on gcn_kernel where gcn_rows_kernel would run, so
+// that the tests can compare the two (they are bit-identical).  It selects nothing else.
+bool force_legacy() {
+    const char* e = getenv("WG_FORCE_LEGACY");
+    return e && e[0] == '1';
 }
 
 int make_plan(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int H, long long chunk,
@@ -123,19 +146,46 @@ int make_plan(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int H,
         p.chunk = chunk > 0 ? chunk : default_chunk(B, per_seq);
         if (p.chunk > B && B > 0) p.chunk = B;
     }
+    // GCN: the CSR graph on the second-generation kernel when its weights fit the constant bank and its slab fits
+    // shared memory; the dense graph on gcn_rows_kernel when that kernel serves the shape
+    p.sq_smem = wg::gcn_sparse_plan_smem_bytes(S, Fi, Fo);
+    if (sparse)
+        p.gcn = Fi <= wg::kSpF && Fo <= wg::kSpF && Fh <= wg::kSqMaxFh && p.sq_smem <= (size_t)wg::kMaxSmemOptin
+                    ? kGcnSparsePlan : kGcnSparseLanes;
+    else if (wg::gcn_rows_applies(S, Fi, Fh, Fo) && wg::gcn_rows_smem_floats(S) * 4 <= (size_t)wg::kMaxSmemOptin &&
+             !force_legacy())
+        p.gcn = kGcnRows;
+    else
+        p.gcn = dense_gcn_kind(S, Fi, Fh, Fo);
+    p.whu = wg::recur_u_applies(H);
+    if (p.tc && wg::recur_tc_applies(H) && wg::recur_tc_smem_bytes(H) <= (size_t)wg::kMaxSmemOptin)
+        p.recur = kRecurTc;
+    else if (p.whu && wg::recur_u_smem_floats(H, wg::kRuMinR) * 4 <= (size_t)wg::kMaxSmemOptin)
+        p.recur = kRecurUnit;
+    else
+        p.recur = kRecurWide;
+    // small chunks (the reference's batch-1 calls, small shards) of the shipped models: W_hh in registers for their
+    // contraction lengths (H = 102 -> 104, H = 21 -> 24), 4 sequences per CTA, bit-identical results
+    p.regw = (p.KP == 104 || p.KP == 24) && p.NPR <= wg::kRwThreads &&
+             wg::recur_regw_smem_floats(p.KP, p.NPR, p.GP) * 4 <= (size_t)wg::kMaxSmemOptin;
+    // H = 102 and H = 21 (the shipped 34- and 7-station models, 3 x S) have their own instantiations with
+    // compile-time strides; for the odd H = 21 this also folds the alignment branches of the gate phase
+    // (ncu: 55 % of the generic kernel's samples sat in that branchy code at H = 21)
+    p.ru_wpg = wg::recur_u_wpg(H);
+    p.ru_ht = H == 102 || H == 21 ? H : 0;
     size_t o = 0;
-    const int wrows = p.tc ? (p.tc2.NP > p.NPB ? p.tc2.NP : p.NPB) : p.NPB;
+    const int wrows = p.tc && p.tc2.NP > p.NPB ? p.tc2.NP : p.NPB;
+    p.n_bias = wrows > 512 ? wrows : 512;
     // packed w_ih: fp32 [N/64][K][64] for the FFMA GEMM, or fp16 hi + lo stage blocks for the tensor cores
-    p.off_wp = o;   o = align_up(o + (p.tc ? wg::tc2_w_halves(p.tc2) * 2 : (size_t)wrows * p.IP * 4));
-    p.off_bias = o; o = align_up(o + (size_t)(wrows > 512 ? wrows : 512) * 4);
+    p.off_wp = o;   o = align_up(o + (p.tc ? wg::tc2_w_halves(p.tc2) * 2 : (size_t)p.NPB * p.IP * 4));
+    p.off_bias = o; o = align_up(o + (size_t)p.n_bias * 4);
     p.off_wht = o;  o = align_up(o + (size_t)p.KP * p.NPR * 4);
-    p.off_whu = o;  // [k][gate][unit] (recur_unit.cuh), only for hidden sizes that kernel serves
-    if (wg::recur_u_applies(H)) o = align_up(o + (size_t)p.KP * 3 * wg::recur_u_hp2(H) * 4);
+    p.off_whu = o;  // [k][gate][unit] (recur_unit.cuh)
+    if (p.whu) o = align_up(o + (size_t)p.KP * 3 * wg::recur_u_hp2(H) * 4);
     p.off_bhn = o;  o = align_up(o + (size_t)p.KP * 4);
-    p.tc_recur = (flags & WG_FLAG_TENSOR_CORES) != 0 && wg::recur_tc_applies(H) &&
-                 wg::recur_tc_smem_bytes(H) <= (size_t)wg::kMaxSmemOptin;
-    p.off_whh_hi = o; if (p.tc_recur) o = align_up(o + wg::recur_tc_w_halves(H) * 2);
-    p.off_whh_lo = o; if (p.tc_recur) o = align_up(o + wg::recur_tc_w_halves(H) * 2);
+    const bool tc_recur = p.recur == kRecurTc;
+    p.off_whh_hi = o; if (tc_recur) o = align_up(o + wg::recur_tc_w_halves(H) * 2);
+    p.off_whh_lo = o; if (tc_recur) o = align_up(o + wg::recur_tc_w_halves(H) * 2);
     const size_t rows = (size_t)p.chunk * T;
     const size_t rows_tiled = (rows + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows;
     p.off_u = o;    o = align_up(o + rows_tiled * p.IP * 4);  // K-major 128-row tiles
@@ -144,21 +194,23 @@ int make_plan(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int H,
     p.off_gi = o;   o = align_up(o + rows_gi * p.GP * 4);
     // sparse path scratch: row-major U (rows x S*Fo) + one [Fo][S] row per resident CTA
     p.off_z = o;    if (sparse) o = align_up(o + (rows + wg::kNumSMs) * (size_t)S * Fo * 4);
-    // second-generation CSR kernel: weights staged for the constant bank + the gather plan
-    p.sq = sparse && Fi <= wg::kSpF && Fo <= wg::kSpF && Fh <= wg::kSqMaxFh &&
-           wg::gcn_sparse_plan_smem_bytes(S, Fi, Fo) <= (size_t)wg::kMaxSmemOptin;
-    p.off_sqw = o;    if (p.sq) o = align_up(o + sizeof(wg::SqWeights));
-    p.off_sqplan = o; if (p.sq) o = align_up(o + wg::sq_plan_bytes(S));
+    // second-generation CSR kernel: weights staged for the constant bank + the gather plan (one step count per
+    // 32-station block, padded to 4, then the gather pairs)
+    const bool sq = p.gcn == kGcnSparsePlan;
+    p.off_sqw = o;     if (sq) o = align_up(o + sizeof(wg::SqWeights));
+    p.off_sqsteps = o;
+    p.off_sqpairs = o + (size_t)wg::round_up(wg::ceil_div(S, 32), 4) * sizeof(int);
+    if (sq) o = align_up(o + wg::sq_plan_bytes(S));
     p.total = o;
     return WG_OK;
 }
 
-int check_ws(const Plan& p, const void* ws, size_t bytes) {
-    if (!ws) return fail(WG_ERR_WORKSPACE, "workspace is NULL (need %zu bytes)", p.total);
+int check_ws(const void* ws, size_t bytes, size_t need) {
+    if (!ws) return fail(WG_ERR_WORKSPACE, "workspace is NULL (need %zu bytes)", need);
     if (reinterpret_cast<uintptr_t>(ws) % kAlign)
         return fail(WG_ERR_WORKSPACE, "workspace must be %zu-byte aligned", kAlign);
-    if (bytes < p.total)
-        return fail(WG_ERR_WORKSPACE, "workspace too small: %zu bytes given, %zu needed", bytes, p.total);
+    if (bytes < need)
+        return fail(WG_ERR_WORKSPACE, "workspace too small: %zu bytes given, %zu needed", bytes, need);
     return WG_OK;
 }
 
@@ -251,9 +303,18 @@ int launch_gcn_t(const float* X, const float* adj, const float* W1, const float*
     return WG_OK;
 }
 
-// stations per thread: 7 or 4, whichever pads S less (ties: 7)
-int pick_sg(int S) {
-    return wg::ceil_div(S, 7) * 7 <= wg::ceil_div(S, 4) * 4 ? 7 : 4;
+template <int LAYERS, bool TILED>
+int launch_gcn_dense(GcnKind k, const float* X, const float* adj, const float* W1, const float* b1, const float* W2,
+                     const float* b2, float* out, long long R, int S, int Fi, int Fh, int Fo, int ldo,
+                     cudaStream_t st) {
+#define WG_GCN(FP, SG, EX) \
+    launch_gcn_t<FP, SG, EX, LAYERS, TILED>(X, adj, W1, b1, W2, b2, out, R, S, Fi, Fh, Fo, ldo, st)
+    if (k == kGcn13x7) return WG_GCN(13, 7, true);
+    if (k == kGcn13x4) return WG_GCN(13, 4, true);
+    if (k == kGcn16x4) return WG_GCN(16, 4, false);
+#undef WG_GCN
+    const int fmax = Fi > Fh ? (Fi > Fo ? Fi : Fo) : (Fh > Fo ? Fh : Fo);
+    return fail(WG_ERR_UNSUPPORTED, "GCN feature width %d > 16 is not built into the dense kernel", fmax);
 }
 
 // second-generation fused two-layer kernel (gcn_rows.cuh): lane = row, output straight into the tiles
@@ -274,51 +335,29 @@ int launch_gcn_rows(const float* X, const float* adj, const float* W1, const flo
     return WG_OK;
 }
 
-// Testing knob: WG_FORCE_LEGACY=1 runs the fused two-layer GCN on gcn_kernel where gcn_rows_kernel would run, so
-// that the tests can compare the two (they are bit-identical).  It selects nothing else.
-bool force_legacy() {
-    const char* e = getenv("WG_FORCE_LEGACY");
-    return e && e[0] == '1';
-}
-
-template <int LAYERS, bool TILED>
-int launch_gcn(const float* X, const float* adj, const float* W1, const float* b1, const float* W2,
-               const float* b2, float* out, long long R, int S, int Fi, int Fh, int Fo, int ldo, cudaStream_t st) {
-    if (LAYERS == 2 && TILED && wg::gcn_rows_applies(S, Fi, Fh, Fo) && !force_legacy() &&
-        wg::gcn_rows_smem_floats(S) * 4 <= (size_t)wg::kMaxSmemOptin)
-        return launch_gcn_rows(X, adj, W1, b1, W2, b2, out, R, S, ldo, st);
-    const int fmax = Fi > Fh ? (Fi > Fo ? Fi : Fo) : (Fh > Fo ? Fh : Fo);
-#define WG_GCN(FP, SG, EX) \
-    launch_gcn_t<FP, SG, EX, LAYERS, TILED>(X, adj, W1, b1, W2, b2, out, R, S, Fi, Fh, Fo, ldo, st)
-    if (Fi == 13 && Fh == 13 && Fo == 13) return pick_sg(S) == 7 ? WG_GCN(13, 7, true) : WG_GCN(13, 4, true);
-    if (fmax <= 16) return WG_GCN(16, 4, false);
-#undef WG_GCN
-    return fail(WG_ERR_UNSUPPORTED, "GCN feature width %d > 16 is not built into the dense kernel", fmax);
-}
-
-struct Csr {
+// The graph of a forward: the dense adjacency, or the CSR arrays when Plan::sparse.
+struct Graph {
+    const float* adj;
     const int* rowptr;
     const int* colidx;
     const float* vals;
 };
 
-int launch_gcn_sparse(const Plan& p, void* ws, const Csr& g, const float* x, const float* w1, const float* b1,
+int launch_gcn_sparse(const Plan& p, void* ws, const Graph& g, const float* x, const float* w1, const float* b1,
                       const float* w2, const float* b2, long long rows, cudaStream_t st) {
     if (p.Fi > wg::kSpF || p.Fo > wg::kSpF)
         return fail(WG_ERR_UNSUPPORTED, "sparse GCN: F_in / F_out must be <= %d (got %d / %d)", wg::kSpF, p.Fi, p.Fo);
-    if (p.sq && rows >= 1) {   // second generation: constant-bank weights + gather plan (prepare_sparse ran)
-        const size_t smem = wg::gcn_sparse_plan_smem_bytes(p.S, p.Fi, p.Fo);
+    if (p.gcn == kGcnSparsePlan && rows >= 1) {   // constant-bank weights + gather plan (prepare_sparse ran)
         const bool narrow = p.Fi <= 13 && p.Fo <= 13, exact = p.Fi == 13 && p.Fo == 13;
         auto kern = exact ? wg::gcn_sparse_plan_kernel<13, true>
                           : narrow ? wg::gcn_sparse_plan_kernel<13, false> : wg::gcn_sparse_plan_kernel<16, false>;
-        WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.sq_smem));
         const unsigned grid = (unsigned)(rows < wg::kNumSMs ? rows : wg::kNumSMs);
         float* urow = ws_ptr<float>(ws, p.off_z);   // [rows][Fo][S] f-major U, then gridDim per-CTA Z rows
         float* zscr = urow + (size_t)rows * p.S * p.Fo;
-        const int* steps = ws_ptr<int>(ws, p.off_sqplan);
-        const int2* plan = reinterpret_cast<const int2*>(steps + wg::round_up(wg::ceil_div(p.S, 32), 4));
-        kern<<<grid, wg::kSqThreads, smem, st>>>(x, g.rowptr, g.colidx, g.vals, steps, plan, zscr, urow, rows, p.S,
-                                                 p.Fi, p.Fh, p.Fo);
+        kern<<<grid, wg::kSqThreads, p.sq_smem, st>>>(x, g.rowptr, g.colidx, g.vals, ws_ptr<int>(ws, p.off_sqsteps),
+                                                      ws_ptr<int2>(ws, p.off_sqpairs), zscr, urow, rows, p.S, p.Fi,
+                                                      p.Fh, p.Fo);
         WG_CUDA(cudaGetLastError());
         const long long rt = (rows + wg::kSpThreads - 1) / wg::kSpThreads * wg::kSpThreads;  // whole tiles (zero rows)
         const dim3 tg((unsigned)((p.S + 31) / 32), (unsigned)(rt / 32));
@@ -352,6 +391,15 @@ int launch_gcn_sparse(const Plan& p, void* ws, const Csr& g, const float* x, con
                                                              s_chunk);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
+}
+
+// The plan's two-layer GCN over `rows` = sequences x steps, into the projection's U tiles.
+int launch_gcn(const Plan& p, void* ws, const Graph& g, const float* x, const float* w1, const float* b1,
+               const float* w2, const float* b2, long long rows, cudaStream_t st) {
+    float* u = ws_ptr<float>(ws, p.off_u);
+    if (p.gcn == kGcnRows) return launch_gcn_rows(x, g.adj, w1, b1, w2, b2, u, rows, p.S, p.IP, st);
+    if (p.sparse) return launch_gcn_sparse(p, ws, g, x, w1, b1, w2, b2, rows, st);
+    return launch_gcn_dense<2, true>(p.gcn, x, g.adj, w1, b1, w2, b2, u, rows, p.S, p.Fi, p.Fh, p.Fo, p.IP, st);
 }
 
 int launch_inproj_tc(const Plan& p, void* ws, long long rows, cudaStream_t st) {
@@ -406,40 +454,6 @@ int launch_recur_wide(const Plan& p, void* ws, float* out, long long Bc, cudaStr
     return WG_OK;
 }
 
-// few sequences (the reference's batch-1 calls, small shards) of the shipped models: W_hh in registers for their
-// contraction lengths (H = 102 -> 104, H = 21 -> 24), 4 sequences per CTA, bit-identical results
-bool recur_small_applies(const Plan& p, long long Bc) {
-    // up to two waves of 4-sequence CTAs
-    return Bc <= 2LL * wg::kRsBT * wg::kNumSMs && (p.KP == 104 || p.KP == 24) && p.NPR <= wg::kRwThreads &&
-           wg::recur_regw_smem_floats(p.KP, p.NPR, p.GP) * 4 <= (size_t)wg::kMaxSmemOptin;
-}
-template <bool SAVE, int NB, int KPT>
-int launch_recur_regw_t(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
-    const size_t smem = wg::recur_regw_smem_floats(KPT, p.NPR, p.GP) * 4;
-    auto kern = wg::gru_recur_regw_kernel<SAVE, NB, KPT>;
-    WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const long long grid = (Bc + wg::kRsBT - 1) / wg::kRsBT;
-    kern<<<(unsigned)grid, wg::kRwThreads, smem, st>>>(ws_ptr<float>(ws, p.off_gi), ws_ptr<float>(ws, p.off_wht),
-                                                      ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H, p.GP, p.NPR,
-                                                      gsave, ldsave);
-    WG_CUDA(cudaGetLastError());
-    return WG_OK;
-}
-template <bool SAVE, int KPT>
-int launch_recur_regw(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
-    // FMA chains per thread = sequences per CTA that can exist (the reference's batch-1 calls run one)
-    if (Bc >= 4) return launch_recur_regw_t<SAVE, 4, KPT>(p, ws, out, Bc, st, gsave, ldsave);
-    if (Bc == 3) return launch_recur_regw_t<SAVE, 3, KPT>(p, ws, out, Bc, st, gsave, ldsave);
-    if (Bc == 2) return launch_recur_regw_t<SAVE, 2, KPT>(p, ws, out, Bc, st, gsave, ldsave);
-    return launch_recur_regw_t<SAVE, 1, KPT>(p, ws, out, Bc, st, gsave, ldsave);
-}
-template <bool SAVE>
-int launch_recur_small(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
-    if (Bc < 1) return WG_OK;
-    if (p.KP == 104) return launch_recur_regw<SAVE, 104>(p, ws, out, Bc, st, gsave, ldsave);
-    return launch_recur_regw<SAVE, 24>(p, ws, out, Bc, st, gsave, ldsave);
-}
-
 // ---- second-generation throughput recurrence (recur_unit.cuh) ----
 // sequences per group: the R in [4, 8] that needs the fewest (waves x R) for this batch
 int recur_u_pick_r(long long Bc, int ngrp) {
@@ -453,52 +467,59 @@ int recur_u_pick_r(long long Bc, int ngrp) {
     }
     return best;
 }
-bool recur_unit_applies(const Plan& p) {
-    return wg::recur_u_applies(p.H) && wg::recur_u_smem_floats(p.H, wg::kRuMinR) * 4 <= (size_t)wg::kMaxSmemOptin;
+
+using RegwKernel = decltype(&wg::gru_recur_regw_kernel<false, 1, 24>);
+template <bool SAVE, int KPT>
+RegwKernel regw_kernel(int nb) {
+    const RegwKernel k[4] = {wg::gru_recur_regw_kernel<SAVE, 1, KPT>, wg::gru_recur_regw_kernel<SAVE, 2, KPT>,
+                             wg::gru_recur_regw_kernel<SAVE, 3, KPT>, wg::gru_recur_regw_kernel<SAVE, 4, KPT>};
+    return k[nb - 1];
 }
-template <int R, int WPG, bool SAVE, int HT>
-int launch_recur_unit_t(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
-    const size_t smem = wg::recur_u_smem_floats(p.H, R) * 4;
-    auto kern = wg::gru_recur_unit_kernel<R, WPG, SAVE, HT>;
+int launch_recur_regw(const Plan& p, void* ws, float* out, long long Bc, int nb, cudaStream_t st, float* gsave,
+                      int ldsave) {
+    if (Bc < 1) return WG_OK;
+    const RegwKernel kern = gsave ? (p.KP == 104 ? regw_kernel<true, 104>(nb) : regw_kernel<true, 24>(nb))
+                                  : (p.KP == 104 ? regw_kernel<false, 104>(nb) : regw_kernel<false, 24>(nb));
+    const size_t smem = wg::recur_regw_smem_floats(p.KP, p.NPR, p.GP) * 4;
     WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int per_cta = (wg::kRuWarps / WPG) * R;
+    const long long grid = (Bc + wg::kRsBT - 1) / wg::kRsBT;
+    kern<<<(unsigned)grid, wg::kRwThreads, smem, st>>>(ws_ptr<float>(ws, p.off_gi), ws_ptr<float>(ws, p.off_wht),
+                                                      ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H, p.GP, p.NPR,
+                                                      gsave, ldsave);
+    WG_CUDA(cudaGetLastError());
+    return WG_OK;
+}
+
+using UnitKernel = decltype(&wg::gru_recur_unit_kernel<4, 1, false, 0>);
+template <int WPG, bool SAVE, int HT>
+UnitKernel unit_kernel(int r) {
+    const UnitKernel k[5] = {wg::gru_recur_unit_kernel<4, WPG, SAVE, HT>, wg::gru_recur_unit_kernel<5, WPG, SAVE, HT>,
+                             wg::gru_recur_unit_kernel<6, WPG, SAVE, HT>, wg::gru_recur_unit_kernel<7, WPG, SAVE, HT>,
+                             wg::gru_recur_unit_kernel<8, WPG, SAVE, HT>};
+    return k[r - wg::kRuMinR];
+}
+template <bool SAVE>
+UnitKernel unit_kernel(const Plan& p, int r) {
+    if (p.ru_ht == 102) return unit_kernel<2, SAVE, 102>(r);
+    if (p.ru_ht == 21) return unit_kernel<1, SAVE, 21>(r);
+    return p.ru_wpg == 1 ? unit_kernel<1, SAVE, 0>(r) : unit_kernel<2, SAVE, 0>(r);
+}
+int launch_recur_unit(const Plan& p, void* ws, float* out, long long Bc, int r, cudaStream_t st, float* gsave,
+                      int ldsave) {
+    const UnitKernel kern = gsave ? unit_kernel<true>(p, r) : unit_kernel<false>(p, r);
+    const size_t smem = wg::recur_u_smem_floats(p.H, r) * 4;
+    WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int per_cta = (wg::kRuWarps / p.ru_wpg) * r;
     const long long grid = (Bc + per_cta - 1) / per_cta;
     if (grid < 1) return WG_OK;
     // FMA-pipe hand-over between the two one-warp groups of a scheduler (profiles/r02_handover_ab.json: H = 21, 4096
     // sequences: 0.395 -> 0.358 ms, identical results).  Two-warp groups (H = 102) own their scheduler and need none.
-    const int handover = WPG == 1 ? 1 : 0;
+    const int handover = p.ru_wpg == 1 ? 1 : 0;
     kern<<<(unsigned)grid, wg::kRuThreads, smem, st>>>(ws_ptr<float>(ws, p.off_gi), ws_ptr<float>(ws, p.off_whu),
                                                       ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H, gsave, ldsave,
                                                       handover);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
-}
-template <bool SAVE>
-int launch_recur_unit(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
-    const int wpg = wg::recur_u_wpg(p.H);
-    int r = recur_u_pick_r(Bc, wg::kRuWarps / wpg);
-    while (r > wg::kRuMinR && wg::recur_u_smem_floats(p.H, r) * 4 > (size_t)wg::kMaxSmemOptin) --r;
-    // H = 102 and H = 21 (the shipped 34- and 7-station models, 3 x S) have their own instantiations with
-    // compile-time strides; for the odd H = 21 this also folds the alignment branches of the gate phase
-    // (ncu: 55 % of the generic kernel's samples sat in that branchy code at H = 21)
-#define WG_RU(RR)                                                                                          \
-    case RR:                                                                                               \
-        if (p.H == 102) return launch_recur_unit_t<RR, 2, SAVE, 102>(p, ws, out, Bc, st, gsave, ldsave);   \
-        if (p.H == 21) return launch_recur_unit_t<RR, 1, SAVE, 21>(p, ws, out, Bc, st, gsave, ldsave);     \
-        return wpg == 1 ? launch_recur_unit_t<RR, 1, SAVE, 0>(p, ws, out, Bc, st, gsave, ldsave)           \
-                        : launch_recur_unit_t<RR, 2, SAVE, 0>(p, ws, out, Bc, st, gsave, ldsave);
-    switch (r) {
-        WG_RU(4) WG_RU(5) WG_RU(6) WG_RU(7) WG_RU(8)
-    }
-#undef WG_RU
-    return fail(WG_ERR_UNSUPPORTED, "recurrence: no kernel for R = %d", r);
-}
-
-// training forward: the same recurrence, additionally saving [r | z | n | hn] per (sequence, step)
-int launch_recur_save(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
-    if (recur_small_applies(p, Bc)) return launch_recur_small<true>(p, ws, out, Bc, st, gsave, ldsave);
-    if (recur_unit_applies(p)) return launch_recur_unit<true>(p, ws, out, Bc, st, gsave, ldsave);
-    return fail(WG_ERR_UNSUPPORTED, "training: GRU hidden size %d does not fit the shared-memory recurrence", p.H);
 }
 
 int launch_recur_tc(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st) {
@@ -513,27 +534,37 @@ int launch_recur_tc(const Plan& p, void* ws, float* out, long long Bc, cudaStrea
     return WG_OK;
 }
 
-int launch_recur(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st) {
-    if (p.tc_recur) return launch_recur_tc(p, ws, out, Bc, st);   // the tensor path: one kernel for every batch size
-    if (recur_small_applies(p, Bc)) return launch_recur_small<false>(p, ws, out, Bc, st, nullptr, 0);
-    if (recur_unit_applies(p)) return launch_recur_unit<false>(p, ws, out, Bc, st, nullptr, 0);
+// The recurrence of one chunk: the plan's kernel, except that up to two waves of 4-sequence CTAs run
+// gru_recur_regw_kernel where it serves the contraction length (FMA chains per thread = sequences per CTA that can
+// exist: the reference's batch-1 calls run one).  gsave: the training forward, which also saves [r | z | n | hn] per
+// (sequence, step), row stride ldsave.
+int launch_recur(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
+    if (p.recur != kRecurTc && p.regw && Bc <= 2LL * wg::kRsBT * wg::kNumSMs)
+        return launch_recur_regw(p, ws, out, Bc, Bc >= 4 ? 4 : (int)Bc, st, gsave, ldsave);
+    if (p.recur == kRecurUnit) {
+        int r = recur_u_pick_r(Bc, wg::kRuWarps / p.ru_wpg);
+        while (r > wg::kRuMinR && wg::recur_u_smem_floats(p.H, r) * 4 > (size_t)wg::kMaxSmemOptin) --r;
+        return launch_recur_unit(p, ws, out, Bc, r, st, gsave, ldsave);
+    }
+    if (gsave)   // the two kernels above are the ones that save gates
+        return fail(WG_ERR_UNSUPPORTED, "training: GRU hidden size %d does not fit the shared-memory recurrence", p.H);
+    if (p.recur == kRecurTc) return launch_recur_tc(p, ws, out, Bc, st);   // the tensor path: every batch size
     return launch_recur_wide(p, ws, out, Bc, st);
 }
 
 int launch_pack(const Plan& p, void* ws, const float* w_ih, const float* w_hh, const float* b_ih,
                 const float* b_hh, cudaStream_t st) {
-    const int wrows = p.tc ? (p.tc2.NP > p.NPB ? p.tc2.NP : p.NPB) : p.NPB;
     pack_params_kernel<<<wg::kNumSMs * 2, 256, 0, st>>>(
         w_ih, w_hh, b_ih, b_hh, ws_ptr<float>(ws, p.off_wp), ws_ptr<float>(ws, p.off_bias),
-        ws_ptr<float>(ws, p.off_wht), wg::recur_u_applies(p.H) ? ws_ptr<float>(ws, p.off_whu) : nullptr,
-        ws_ptr<float>(ws, p.off_bhn), p.I, p.H, p.IP, p.NPB, p.KP, p.NPR, p.tc ? 0 : 1, wrows > 512 ? wrows : 512);
+        ws_ptr<float>(ws, p.off_wht), p.whu ? ws_ptr<float>(ws, p.off_whu) : nullptr, ws_ptr<float>(ws, p.off_bhn),
+        p.I, p.H, p.IP, p.NPB, p.KP, p.NPR, p.tc ? 0 : 1, p.n_bias);
     WG_CUDA(cudaGetLastError());
     if (p.tc) {
         wg::pack_wih_tc2_kernel<<<wg::kNumSMs * 2, 256, 0, st>>>(w_ih, ws_ptr<__half>(ws, p.off_wp), p.G, p.I, p.tc2.KP,
                                                                 p.tc2.n_nt, p.tc2.N_each);
         WG_CUDA(cudaGetLastError());
     }
-    if (p.tc_recur) {
+    if (p.recur == kRecurTc) {
         wg::pack_whh_tc_kernel<<<wg::kNumSMs, 256, 0, st>>>(w_hh, ws_ptr<__half>(ws, p.off_whh_hi),
                                                            ws_ptr<__half>(ws, p.off_whh_lo), p.H);
         WG_CUDA(cudaGetLastError());
@@ -541,17 +572,20 @@ int launch_pack(const Plan& p, void* ws, const float* w_ih, const float* w_hh, c
     return WG_OK;
 }
 
-// One chunk (Bc <= plan.chunk sequences) through the three stages.
-int run_chunk(const Plan& p, void* ws, const float* adj, const float* x, const float* w1, const float* b1,
-              const float* w2, const float* b2, float* out, long long Bc, cudaStream_t st) {
+// One chunk (Bc <= plan.chunk sequences) through the three stages; gsave / ldsave: see launch_recur.
+int run_chunk(const Plan& p, void* ws, const Graph& g, const float* x, const float* w1, const float* b1,
+              const float* w2, const float* b2, float* out, long long Bc, cudaStream_t st, float* gsave = nullptr,
+              int ldsave = 0) {
     const long long rows = Bc * p.T;
-    int rc = launch_gcn<2, true>(x, adj, w1, b1, w2, b2, ws_ptr<float>(ws, p.off_u), rows, p.S, p.Fi, p.Fh, p.Fo,
-                                 p.IP, st);
+    int rc = launch_gcn(p, ws, g, x, w1, b1, w2, b2, rows, st);
     if (rc) return rc;
     rc = launch_inproj(p, ws, rows, st);
     if (rc) return rc;
-    return launch_recur(p, ws, out, Bc, st);
+    return launch_recur(p, ws, out, Bc, st, gsave, ldsave);
 }
+
+// Per-device tables (constant-bank ordering below, host-path streams): DeviceGuard has rejected a negative index.
+constexpr int kMaxDevices = 64;
 
 // Per-call setup of the second-generation CSR kernel: weights into the constant bank, gather plan.
 // The constant bank is one per device: forwards on different streams are ordered through an event (a later
@@ -559,19 +593,20 @@ int run_chunk(const Plan& p, void* ws, const float* adj, const float* x, const f
 // the caller holds from prepare_sparse to finish_sparse.
 std::mutex g_sq_mu;
 struct SqDeviceState { cudaEvent_t ev = nullptr; cudaStream_t last = nullptr; bool recorded = false; };
-SqDeviceState g_sq_dev[64];
+SqDeviceState g_sq_dev[kMaxDevices];
 
-int prepare_sparse(const Plan& p, void* ws, const Csr& g, const float* w1, const float* b1, const float* w2,
+int prepare_sparse(const Plan& p, void* ws, const Graph& g, const float* w1, const float* b1, const float* w2,
                    const float* b2, int device, cudaStream_t st) {
+    if (device >= kMaxDevices) return fail(WG_ERR_BAD_ARG, "device index %d out of range", device);
     wg::SqWeights* stage = ws_ptr<wg::SqWeights>(ws, p.off_sqw);
     wg::sq_pack_weights_kernel<<<32, 256, 0, st>>>(w1, b1, w2, b2, stage, p.Fi, p.Fh, p.Fo);
     WG_CUDA(cudaGetLastError());
-    int* steps = ws_ptr<int>(ws, p.off_sqplan);
-    int2* plan = reinterpret_cast<int2*>(steps + wg::round_up(wg::ceil_div(p.S, 32), 4));
     const int wbs = wg::ceil_div(p.S, 32);
-    wg::csr_plan_kernel<<<wg::ceil_div(wbs, 4), 128, 0, st>>>(g.rowptr, g.colidx, g.vals, p.S, steps, plan);
+    wg::csr_plan_kernel<<<wg::ceil_div(wbs, 4), 128, 0, st>>>(g.rowptr, g.colidx, g.vals, p.S,
+                                                             ws_ptr<int>(ws, p.off_sqsteps),
+                                                             ws_ptr<int2>(ws, p.off_sqpairs));
     WG_CUDA(cudaGetLastError());
-    SqDeviceState& d = g_sq_dev[device & 63];
+    SqDeviceState& d = g_sq_dev[device];
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     cudaStreamIsCapturing(st, &cap);
     if (cap == cudaStreamCaptureStatusNone && d.recorded && d.last != st) WG_CUDA(cudaStreamWaitEvent(st, d.ev, 0));
@@ -579,7 +614,7 @@ int prepare_sparse(const Plan& p, void* ws, const Csr& g, const float* w1, const
     return WG_OK;
 }
 int finish_sparse(int device, cudaStream_t st) {
-    SqDeviceState& d = g_sq_dev[device & 63];
+    SqDeviceState& d = g_sq_dev[device];
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     cudaStreamIsCapturing(st, &cap);
     if (cap != cudaStreamCaptureStatusNone) return WG_OK;
@@ -590,20 +625,57 @@ int finish_sparse(int device, cudaStream_t st) {
     return WG_OK;
 }
 
-int run_chunk_csr(const Plan& p, void* ws, const Csr& g, const float* x, const float* w1, const float* b1,
-                  const float* w2, const float* b2, float* out, long long Bc, cudaStream_t st) {
-    const long long rows = Bc * p.T;
-    int rc = launch_gcn_sparse(p, ws, g, x, w1, b1, w2, b2, rows, st);
-    if (rc) return rc;
-    rc = launch_inproj(p, ws, rows, st);
-    if (rc) return rc;
-    return launch_recur(p, ws, out, Bc, st);
-}
-
 bool any_null(std::initializer_list<const void*> ps) {
     for (const void* q : ps)
         if (!q) return true;
     return false;
+}
+
+// The device-buffer forward of either graph form: pack the parameters, then every chunk through the three stages.
+// On gcn_sparse_plan_kernel the CSR graph also holds the constant bank from prepare_sparse to finish_sparse.
+int forward(bool sparse, const Graph& g, const float* x, const float* w1, const float* b1, const float* w2,
+            const float* b2, const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, float* out,
+            long long B, int T, int S, int Fi, int Fh, int Fo, int H, long long chunk, int flags, void* ws,
+            size_t ws_bytes, int device, void* stream) {
+    Plan p;
+    int rc = make_plan(p, B, T, S, Fi, Fh, Fo, H, chunk, sparse, flags);
+    if (rc) return rc;
+    if (B == 0) return WG_OK;
+    const bool no_graph = p.sparse ? any_null({g.rowptr, g.colidx, g.vals}) : !g.adj;
+    if (no_graph || any_null({x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out}))
+        return fail(WG_ERR_BAD_ARG, "null pointer argument");
+    if ((rc = check_ws(ws, ws_bytes, p.total))) return rc;
+    DeviceGuard dg(device);
+    WG_CUDA(dg.err);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if ((rc = launch_pack(p, ws, w_ih, w_hh, b_ih, b_hh, st))) return rc;
+    const bool sq = p.gcn == kGcnSparsePlan;
+    std::unique_lock<std::mutex> sq_lock(g_sq_mu, std::defer_lock);
+    if (sq) {
+        sq_lock.lock();
+        if ((rc = prepare_sparse(p, ws, g, w1, b1, w2, b2, device, st))) return rc;
+    }
+    const size_t x_seq = (size_t)p.T * p.S * p.Fi, o_seq = (size_t)p.T * p.H;
+    for (long long b0 = 0; b0 < B; b0 += p.chunk) {
+        const long long Bc = (B - b0) < p.chunk ? (B - b0) : p.chunk;
+        rc = run_chunk(p, ws, g, x + (size_t)b0 * x_seq, w1, b1, w2, b2, out + (size_t)b0 * o_seq, Bc, st);
+        if (rc) return rc;
+    }
+    return sq ? finish_sparse(device, st) : WG_OK;
+}
+
+// The wg_stage_* entry points: plan one chunk, check Bc, the workspace and the device, then run `launch`.
+template <typename Launch>
+int run_stage(long long Bc, int T, int S, int Fi, int Fh, int Fo, int H, long long chunk, int flags, void* ws,
+              size_t ws_bytes, int device, void* stream, Launch launch) {
+    Plan p;
+    int rc = make_plan(p, chunk, T, S, Fi, Fh, Fo, H, chunk, false, flags);
+    if (rc) return rc;
+    if (Bc < 0 || Bc > p.chunk) return fail(WG_ERR_BAD_ARG, "Bc=%lld outside [0, chunk=%lld]", Bc, p.chunk);
+    if ((rc = check_ws(ws, ws_bytes, p.total))) return rc;
+    DeviceGuard g(device);
+    WG_CUDA(g.err);
+    return launch(p, static_cast<cudaStream_t>(stream));
 }
 
 
@@ -823,53 +895,31 @@ int wg_stage_pack_f32(const float* w_ih, const float* w_hh, const float* b_ih, c
                       int S, int F_in, int F_hid, int F_out, int H, int64_t chunk, int flags, void* workspace,
                       size_t workspace_bytes, int device, void* stream) {
     if (any_null({w_ih, w_hh, b_ih, b_hh})) return fail(WG_ERR_BAD_ARG, "null parameter pointer");
-    Plan p;
-    int rc = make_plan(p, chunk, T, S, F_in, F_hid, F_out, H, chunk, false, flags);
-    if (rc) return rc;
-    if ((rc = check_ws(p, workspace, workspace_bytes))) return rc;
-    DeviceGuard g(device);
-    WG_CUDA(g.err);
-    return launch_pack(p, workspace, w_ih, w_hh, b_ih, b_hh, static_cast<cudaStream_t>(stream));
+    auto launch = [&](const Plan& p, cudaStream_t st) { return launch_pack(p, workspace, w_ih, w_hh, b_ih, b_hh, st); };
+    return run_stage(0, T, S, F_in, F_hid, F_out, H, chunk, flags, workspace, workspace_bytes, device, stream, launch);
 }
 
 int wg_stage_gcn_f32(const float* adj, const float* x, const float* w1, const float* b1, const float* w2,
                      const float* b2, int64_t Bc, int T, int S, int F_in, int F_hid, int F_out, int H,
                      int64_t chunk, int flags, void* workspace, size_t workspace_bytes, int device, void* stream) {
     if (any_null({adj, x, w1, b1, w2, b2})) return fail(WG_ERR_BAD_ARG, "null pointer");
-    Plan p;
-    int rc = make_plan(p, chunk, T, S, F_in, F_hid, F_out, H, chunk, false, flags);
-    if (rc) return rc;
-    if (Bc < 0 || Bc > p.chunk) return fail(WG_ERR_BAD_ARG, "Bc=%lld outside [0, chunk=%lld]", (long long)Bc, p.chunk);
-    if ((rc = check_ws(p, workspace, workspace_bytes))) return rc;
-    DeviceGuard g(device);
-    WG_CUDA(g.err);
-    return launch_gcn<2, true>(x, adj, w1, b1, w2, b2, ws_ptr<float>(workspace, p.off_u), (long long)Bc * T, S, F_in,
-                               F_hid, F_out, p.IP, static_cast<cudaStream_t>(stream));
+    auto launch = [&](const Plan& p, cudaStream_t st) {
+        return launch_gcn(p, workspace, Graph{adj}, x, w1, b1, w2, b2, Bc * T, st);
+    };
+    return run_stage(Bc, T, S, F_in, F_hid, F_out, H, chunk, flags, workspace, workspace_bytes, device, stream, launch);
 }
 
 int wg_stage_inproj_f32(int64_t Bc, int T, int S, int F_in, int F_hid, int F_out, int H, int64_t chunk,
                         int flags, void* workspace, size_t workspace_bytes, int device, void* stream) {
-    Plan p;
-    int rc = make_plan(p, chunk, T, S, F_in, F_hid, F_out, H, chunk, false, flags);
-    if (rc) return rc;
-    if (Bc < 0 || Bc > p.chunk) return fail(WG_ERR_BAD_ARG, "Bc=%lld outside [0, chunk=%lld]", (long long)Bc, p.chunk);
-    if ((rc = check_ws(p, workspace, workspace_bytes))) return rc;
-    DeviceGuard g(device);
-    WG_CUDA(g.err);
-    return launch_inproj(p, workspace, (long long)Bc * T, static_cast<cudaStream_t>(stream));
+    auto launch = [&](const Plan& p, cudaStream_t st) { return launch_inproj(p, workspace, Bc * T, st); };
+    return run_stage(Bc, T, S, F_in, F_hid, F_out, H, chunk, flags, workspace, workspace_bytes, device, stream, launch);
 }
 
 int wg_stage_recur_f32(float* out, int64_t Bc, int T, int S, int F_in, int F_hid, int F_out, int H,
                        int64_t chunk, int flags, void* workspace, size_t workspace_bytes, int device, void* stream) {
     if (!out) return fail(WG_ERR_BAD_ARG, "null output pointer");
-    Plan p;
-    int rc = make_plan(p, chunk, T, S, F_in, F_hid, F_out, H, chunk, false, flags);
-    if (rc) return rc;
-    if (Bc < 0 || Bc > p.chunk) return fail(WG_ERR_BAD_ARG, "Bc=%lld outside [0, chunk=%lld]", (long long)Bc, p.chunk);
-    if ((rc = check_ws(p, workspace, workspace_bytes))) return rc;
-    DeviceGuard g(device);
-    WG_CUDA(g.err);
-    return launch_recur(p, workspace, out, Bc, static_cast<cudaStream_t>(stream));
+    auto launch = [&](const Plan& p, cudaStream_t st) { return launch_recur(p, workspace, out, Bc, st, nullptr, 0); };
+    return run_stage(Bc, T, S, F_in, F_hid, F_out, H, chunk, flags, workspace, workspace_bytes, device, stream, launch);
 }
 
 int wg_gcn_gru_forward_f32(const float* adj, const float* x, const float* w1, const float* b1,
@@ -877,25 +927,8 @@ int wg_gcn_gru_forward_f32(const float* adj, const float* x, const float* w1, co
                            const float* b_ih, const float* b_hh, float* out, int64_t B, int T, int S,
                            int F_in, int F_hid, int F_out, int H, int64_t chunk, int flags, void* workspace,
                            size_t workspace_bytes, int device, void* stream) {
-    Plan p;
-    int rc = make_plan(p, B, T, S, F_in, F_hid, F_out, H, chunk, false, flags);
-    if (rc) return rc;
-    if (B == 0) return WG_OK;
-    if (any_null({adj, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out}))
-        return fail(WG_ERR_BAD_ARG, "null pointer argument");
-    if ((rc = check_ws(p, workspace, workspace_bytes))) return rc;
-    DeviceGuard g(device);
-    WG_CUDA(g.err);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if ((rc = launch_pack(p, workspace, w_ih, w_hh, b_ih, b_hh, st))) return rc;
-    const size_t x_seq = (size_t)T * S * F_in, o_seq = (size_t)T * H;
-    for (long long b0 = 0; b0 < B; b0 += p.chunk) {
-        const long long Bc = (B - b0) < p.chunk ? (B - b0) : p.chunk;
-        rc = run_chunk(p, workspace, adj, x + (size_t)b0 * x_seq, w1, b1, w2, b2, out + (size_t)b0 * o_seq,
-                       Bc, st);
-        if (rc) return rc;
-    }
-    return WG_OK;
+    return forward(false, Graph{adj}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, B, T,
+                   S, F_in, F_hid, F_out, H, chunk, flags, workspace, workspace_bytes, device, stream);
 }
 
 size_t wg_gcn_gru_csr_workspace_bytes(int64_t B, int T, int S, int F_in, int F_hid, int F_out, int H,
@@ -911,56 +944,38 @@ int wg_gcn_gru_forward_csr_f32(const int32_t* rowptr, const int32_t* colidx, con
                                float* out, int64_t B, int T, int S, int F_in, int F_hid, int F_out, int H,
                                int64_t chunk, int flags, void* workspace, size_t workspace_bytes, int device,
                                void* stream) {
-    Plan p;
-    int rc = make_plan(p, B, T, S, F_in, F_hid, F_out, H, chunk, true, flags);
-    if (rc) return rc;
-    if (B == 0) return WG_OK;
-    if (any_null({rowptr, colidx, vals, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out}))
-        return fail(WG_ERR_BAD_ARG, "null pointer argument");
-    if ((rc = check_ws(p, workspace, workspace_bytes))) return rc;
-    DeviceGuard g(device);
-    WG_CUDA(g.err);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if ((rc = launch_pack(p, workspace, w_ih, w_hh, b_ih, b_hh, st))) return rc;
-    const Csr csr{rowptr, colidx, vals};
-    const size_t x_seq = (size_t)T * S * F_in, o_seq = (size_t)T * H;
-    std::unique_lock<std::mutex> sq_lock(g_sq_mu, std::defer_lock);
-    if (p.sq) {
-        sq_lock.lock();
-        if ((rc = prepare_sparse(p, workspace, csr, w1, b1, w2, b2, device, st))) return rc;
-    }
-    for (long long b0 = 0; b0 < B; b0 += p.chunk) {
-        const long long Bc = (B - b0) < p.chunk ? (B - b0) : p.chunk;
-        rc = run_chunk_csr(p, workspace, csr, x + (size_t)b0 * x_seq, w1, b1, w2, b2, out + (size_t)b0 * o_seq,
-                           Bc, st);
-        if (rc) return rc;
-    }
-    if (p.sq) return finish_sparse(device, st);
-    return WG_OK;
-}
-
-// ---- host-buffer variant: H2D / compute / D2H of consecutive chunks overlapped ----------------
-// Two compute lanes (streams, each with its own scratch) so that the latency-bound recurrence of chunk c
-// overlaps the GCN / projection of chunk c+1; three staging slots each for x and out.
-// workspace = [ compute workspace 0 | compute workspace 1 | x staging 0..2 | out staging 0..2 ]
-constexpr int kHostLanes = 2;
-constexpr int kHostSlots = 3;
-constexpr long long kHostDefaultChunk = 256;   // measured best piece size for the 34-station model (DESIGN.md, section 5)
-
-size_t wg_gcn_gru_host_workspace_bytes(int64_t B, int T, int S, int F_in, int F_hid, int F_out, int H,
-                                       int64_t chunk, int flags) {
-    Plan p;
-    if (chunk == 0) chunk = kHostDefaultChunk;   // the host path pipelines: a piece small enough to overlap copies
-    if (make_plan(p, B, T, S, F_in, F_hid, F_out, H, chunk, false, flags)) return 0;
-    const size_t xs = align_up((size_t)p.chunk * T * S * F_in * 4);
-    const size_t os = align_up((size_t)p.chunk * T * H * 4);
-    const size_t ps = align_up((size_t)p.chunk * H * 4);   // de-normalised last step (wg_gcn_gru_predict_host_f32)
-    return kHostLanes * align_up(p.total) + kHostSlots * (xs + os + ps);
+    return forward(true, Graph{nullptr, rowptr, colidx, vals}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, B, T, S,
+                   F_in, F_hid, F_out, H, chunk, flags, workspace, workspace_bytes, device, stream);
 }
 
 }  // extern "C"
 
 namespace {
+
+// ---- host-buffer variant: H2D / compute / D2H of consecutive chunks overlapped ----------------
+// Two compute lanes (streams, each with its own scratch) so that the latency-bound recurrence of chunk c
+// overlaps the GCN / projection of chunk c+1; three staging slots each for x, out and pred.
+constexpr int kHostLanes = 2;
+constexpr int kHostSlots = 3;
+constexpr long long kHostDefaultChunk = 256;   // measured best piece size for the 34-station model (DESIGN.md, section 5)
+
+// workspace = [ compute workspace 0 | compute workspace 1 | x staging 0..2 | out staging 0..2 | pred staging 0..2 ]
+struct HostLayout {
+    size_t lane, xs, os, ps;   // bytes of one compute workspace and of one x / out / pred staging slot
+    size_t total;
+};
+int host_plan(Plan& p, HostLayout& L, long long B, int T, int S, int Fi, int Fh, int Fo, int H, long long chunk,
+              int flags) {
+    if (chunk == 0) chunk = kHostDefaultChunk;   // the host path pipelines: a piece small enough to overlap copies
+    int rc = make_plan(p, B, T, S, Fi, Fh, Fo, H, chunk, false, flags);
+    if (rc) return rc;
+    L.lane = align_up(p.total);
+    L.xs = align_up((size_t)p.chunk * T * S * Fi * 4);
+    L.os = align_up((size_t)p.chunk * T * H * 4);
+    L.ps = align_up((size_t)p.chunk * H * 4);   // de-normalised last step (wg_gcn_gru_predict_host_f32)
+    L.total = kHostLanes * L.lane + kHostSlots * (L.xs + L.os + L.ps);
+    return WG_OK;
+}
 
 // Internal streams and events of the host-buffer entry points: created once per (host thread, device) and
 // reused by every later call of that thread (creating 4 streams + 9 events per call cost ~0.1 ms).
@@ -969,11 +984,10 @@ struct HostCtx {
     cudaStream_t s_in = nullptr, s_out = nullptr, s_cmp[kHostLanes] = {};
     cudaEvent_t ev_in[kHostSlots] = {}, ev_cmp[kHostSlots] = {}, ev_out[kHostSlots] = {};
 };
-constexpr int kMaxDevices = 64;
 thread_local HostCtx g_host_ctx[kMaxDevices];
 
 int host_ctx(int device, HostCtx** out) {
-    if (device < 0 || device >= kMaxDevices) return fail(WG_ERR_BAD_ARG, "device index %d out of range", device);
+    if (device >= kMaxDevices) return fail(WG_ERR_BAD_ARG, "device index %d out of range", device);
     HostCtx& c = g_host_ctx[device];
     if (!c.ready) {
         WG_CUDA(cudaStreamCreateWithFlags(&c.s_in, cudaStreamNonBlocking));
@@ -997,21 +1011,13 @@ int host_pipeline(const float* adj, const float* x_host, const float* w1, const 
                   int flags, void* workspace, size_t workspace_bytes, int device, bool last_only, double vmin,
                   double vmax) {
     Plan p;
-    if (chunk == 0) chunk = kHostDefaultChunk;
-    int rc = make_plan(p, B, T, S, F_in, F_hid, F_out, H, chunk, false, flags);
+    HostLayout L;
+    int rc = host_plan(p, L, B, T, S, F_in, F_hid, F_out, H, chunk, flags);
     if (rc) return rc;
     if (B == 0) return WG_OK;
     if (any_null({adj, x_host, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, dst_host}))
         return fail(WG_ERR_BAD_ARG, "null pointer argument");
-    const size_t xs = align_up((size_t)p.chunk * T * S * F_in * 4);
-    const size_t os = align_up((size_t)p.chunk * T * H * 4);
-    const size_t ps = align_up((size_t)p.chunk * H * 4);
-    const size_t wsz = align_up(p.total);
-    const size_t need = kHostLanes * wsz + kHostSlots * (xs + os + ps);
-    if (!workspace || reinterpret_cast<uintptr_t>(workspace) % kAlign)
-        return fail(WG_ERR_WORKSPACE, "workspace NULL or not %zu-byte aligned", kAlign);
-    if (workspace_bytes < need)
-        return fail(WG_ERR_WORKSPACE, "workspace too small: %zu bytes given, %zu needed", workspace_bytes, need);
+    if ((rc = check_ws(workspace, workspace_bytes, L.total))) return rc;
     DeviceGuard g(device);
     WG_CUDA(g.err);
     HostCtx* cx = nullptr;
@@ -1019,14 +1025,15 @@ int host_pipeline(const float* adj, const float* x_host, const float* w1, const 
 
     char* base = static_cast<char*>(workspace);
     void* lane_ws[kHostLanes];
-    for (int l = 0; l < kHostLanes; ++l) lane_ws[l] = base + l * wsz;
+    for (int l = 0; l < kHostLanes; ++l) lane_ws[l] = base + l * L.lane;
+    char* slots = base + kHostLanes * L.lane;
     float* xdev[kHostSlots];
     float* odev[kHostSlots];
     float* pdev[kHostSlots];
     for (int i = 0; i < kHostSlots; ++i) {
-        xdev[i] = reinterpret_cast<float*>(base + kHostLanes * wsz + i * xs);
-        odev[i] = reinterpret_cast<float*>(base + kHostLanes * wsz + kHostSlots * xs + i * os);
-        pdev[i] = reinterpret_cast<float*>(base + kHostLanes * wsz + kHostSlots * (xs + os) + i * ps);
+        xdev[i] = reinterpret_cast<float*>(slots + i * L.xs);
+        odev[i] = reinterpret_cast<float*>(slots + kHostSlots * L.xs + i * L.os);
+        pdev[i] = reinterpret_cast<float*>(slots + kHostSlots * (L.xs + L.os) + i * L.ps);
     }
     int result = WG_OK;
 #define WG_CUDA_H(expr)                                                                         \
@@ -1040,13 +1047,11 @@ int host_pipeline(const float* adj, const float* x_host, const float* w1, const 
         }                                                                                       \
     } while (0)
 
+    auto synced = [](int code) { cudaDeviceSynchronize(); return code; };   // an error leaves no copy in flight
     const long long n_chunks = (B + p.chunk - 1) / p.chunk;
-    for (int l = 0; l < kHostLanes && l < n_chunks; ++l) {   // each lane packs the parameters into its own scratch
-        if ((rc = launch_pack(p, lane_ws[l], w_ih, w_hh, b_ih, b_hh, cx->s_cmp[l]))) {
-            cudaDeviceSynchronize();
-            return rc;
-        }
-    }
+    for (int l = 0; l < kHostLanes && l < n_chunks; ++l)   // each lane packs the parameters into its own scratch
+        if ((rc = launch_pack(p, lane_ws[l], w_ih, w_hh, b_ih, b_hh, cx->s_cmp[l]))) return synced(rc);
+    const Graph graph{adj};
     const size_t x_seq = (size_t)T * S * F_in, o_seq = (size_t)T * H;
     for (long long c = 0; c < n_chunks; ++c) {
         const int sl = (int)(c % kHostSlots), lane = (int)(c % kHostLanes);
@@ -1061,16 +1066,11 @@ int host_pipeline(const float* adj, const float* x_host, const float* w1, const 
         // the lane's scratch is free because chunk c - lanes ran on the same stream
         WG_CUDA_H(cudaStreamWaitEvent(cx->s_cmp[lane], cx->ev_in[sl], 0));
         if (c >= kHostSlots) WG_CUDA_H(cudaStreamWaitEvent(cx->s_cmp[lane], cx->ev_out[sl], 0));
-        if ((rc = run_chunk(p, lane_ws[lane], adj, xdev[sl], w1, b1, w2, b2, odev[sl], Bc, cx->s_cmp[lane]))) {
-            cudaDeviceSynchronize();
-            return rc;
-        }
-        if (last_only) {   // only 3S floats per window leave the GPU (src/main.py:103,116)
-            if ((rc = wg_denorm_last_step_f32(odev[sl], pdev[sl], Bc, T, H, vmin, vmax, device, cx->s_cmp[lane]))) {
-                cudaDeviceSynchronize();
-                return rc;
-            }
-        }
+        if ((rc = run_chunk(p, lane_ws[lane], graph, xdev[sl], w1, b1, w2, b2, odev[sl], Bc, cx->s_cmp[lane])))
+            return synced(rc);
+        if (last_only &&   // only 3S floats per window leave the GPU (src/main.py:103,116)
+            (rc = wg_denorm_last_step_f32(odev[sl], pdev[sl], Bc, T, H, vmin, vmax, device, cx->s_cmp[lane])))
+            return synced(rc);
         WG_CUDA_H(cudaEventRecord(cx->ev_cmp[sl], cx->s_cmp[lane]));
         WG_CUDA_H(cudaStreamWaitEvent(cx->s_out, cx->ev_cmp[sl], 0));
         if (last_only)
@@ -1091,6 +1091,14 @@ int host_pipeline(const float* adj, const float* x_host, const float* w1, const 
 }  // namespace
 
 extern "C" {
+
+size_t wg_gcn_gru_host_workspace_bytes(int64_t B, int T, int S, int F_in, int F_hid, int F_out, int H,
+                                       int64_t chunk, int flags) {
+    Plan p;
+    HostLayout L;
+    if (host_plan(p, L, B, T, S, F_in, F_hid, F_out, H, chunk, flags)) return 0;
+    return L.total;
+}
 
 int wg_gcn_gru_forward_host_f32(const float* adj, const float* x_host, const float* w1, const float* b1,
                                 const float* w2, const float* b2, const float* w_ih, const float* w_hh,
@@ -1119,8 +1127,8 @@ int wg_gcn_layer_f32(const float* adj, const float* attr, const float* weight, c
     DeviceGuard g(device);
     WG_CUDA(g.err);
     // single layer: "hidden" plays the role of the output width
-    return launch_gcn<1, false>(attr, adj, weight, bias, nullptr, nullptr, out, R, S, F_in, F_out, F_out, S * F_out,
-                                static_cast<cudaStream_t>(stream));
+    return launch_gcn_dense<1, false>(dense_gcn_kind(S, F_in, F_out, F_out), attr, adj, weight, bias, nullptr, nullptr,
+                                      out, R, S, F_in, F_out, F_out, S * F_out, static_cast<cudaStream_t>(stream));
 }
 
 
@@ -1147,20 +1155,13 @@ int wg_gcn_gru_forward_train_f32(const float* adj, const float* x, const float* 
     if (B == 0) return WG_OK;
     if (any_null({adj, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out}))
         return fail(WG_ERR_BAD_ARG, "null pointer argument");
-    if (!workspace || reinterpret_cast<uintptr_t>(workspace) % kAlign)
-        return fail(WG_ERR_WORKSPACE, "workspace NULL or not %zu-byte aligned", kAlign);
-    if (workspace_bytes < tp.total)
-        return fail(WG_ERR_WORKSPACE, "workspace too small: %zu bytes given, %zu needed", workspace_bytes, tp.total);
+    if ((rc = check_ws(workspace, workspace_bytes, tp.total))) return rc;
     DeviceGuard g(device);
     WG_CUDA(g.err);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const Plan& p = tp.f;
-    if ((rc = launch_pack(p, workspace, w_ih, w_hh, b_ih, b_hh, st))) return rc;
-    if ((rc = launch_gcn<2, true>(x, adj, w1, b1, w2, b2, ws_ptr<float>(workspace, p.off_u), tp.rows, S, F_in, F_hid,
-                                  F_out, p.IP, st)))
-        return rc;
-    if ((rc = launch_inproj(p, workspace, tp.rows, st))) return rc;
-    return launch_recur_save(p, workspace, out, B, st, ws_ptr<float>(workspace, tp.off_gates), tp.LD4);
+    if ((rc = launch_pack(tp.f, workspace, w_ih, w_hh, b_ih, b_hh, st))) return rc;
+    return run_chunk(tp.f, workspace, Graph{adj}, x, w1, b1, w2, b2, out, B, st,
+                     ws_ptr<float>(workspace, tp.off_gates), tp.LD4);
 }
 
 int wg_gcn_gru_backward_f32(const float* adj, const float* x, const float* w1, const float* b1, const float* w2,
@@ -1181,10 +1182,7 @@ int wg_gcn_gru_backward_f32(const float* adj, const float* x, const float* w1, c
         WG_CUDA(cudaMemsetAsync(grads, 0, n_params * 4, st));
         return WG_OK;
     }
-    if (!workspace || reinterpret_cast<uintptr_t>(workspace) % kAlign)
-        return fail(WG_ERR_WORKSPACE, "workspace NULL or not %zu-byte aligned", kAlign);
-    if (workspace_bytes < tp.total)
-        return fail(WG_ERR_WORKSPACE, "workspace too small: %zu bytes given, %zu needed", workspace_bytes, tp.total);
+    if ((rc = check_ws(workspace, workspace_bytes, tp.total))) return rc;
     // flat gradient layout = state_dict order
     float* d_w1 = grads;
     float* d_b1 = d_w1 + (size_t)F_in * F_hid;
