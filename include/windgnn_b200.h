@@ -231,7 +231,8 @@ int wg_denorm_last_step_f32(const float* out, float* pred, int64_t B, int T, int
  *   optimizer.step()  (torch.optim.Adam, :52,:77)    -> wg_adam_step_f32
  * FP32 throughout, dense adjacency, F_in / F_hid / F_out <= 16, H <= 106 (the limit the
  * planner enforces: W_hh and the recurrent state resident in shared
- * memory; the shipped models).
+ * memory; the shipped models).  B * T may be at most 2,097,024 rows (16,383 tiles of 128): the
+ * backward re-lays the input-gate gradients in one pass, and the planner rejects larger batches.
  *
  * The forward is the inference path's three kernels; the recurrence additionally saves the gate
  * values [r | z | n | W_hn h + b_hn] per (sequence, step).  `workspace` (sized by

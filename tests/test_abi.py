@@ -108,6 +108,14 @@ def test_training_planning_and_validation():
     assert rc == _lib.WG_ERR_WORKSPACE
     rc = lib.wg_gcn_gru_backward_f32(*([None] * 11), 2, *dims34, None, 0, 0, None)
     assert rc == _lib.WG_ERR_BAD_ARG and "null" in _lib.last_error()
+    # B*T is bounded by the one-pass dU stage: 12482 x 168 rows plan, 12483 x 168 are rejected before any launch
+    assert lib.wg_gcn_gru_train_workspace_bytes(12482, *dims34) > 0
+    assert lib.wg_gcn_gru_train_workspace_bytes(12483, *dims34) == 0
+    assert "rows" in _lib.last_error()
+    rc = lib.wg_gcn_gru_forward_train_f32(*([fake] * 11), 12483, *dims34, None, 0, 0, None)
+    assert rc == _lib.WG_ERR_UNSUPPORTED and "rows" in _lib.last_error()
+    rc = lib.wg_gcn_gru_backward_f32(*([fake] * 11), 12483, *dims34, None, 0, 0, None)
+    assert rc == _lib.WG_ERR_UNSUPPORTED and "rows" in _lib.last_error()
     assert lib.wg_mse_loss_grad_f32(None, None, 0, None, None, None, 0, 0, None) == _lib.WG_ERR_BAD_ARG
     assert lib.wg_adam_step_f32(None, None, None, None, 10, 1e-3, 0.9, 0.999, 1e-8, 0, 1.0, 0, None) == _lib.WG_ERR_BAD_ARG
     assert lib.wg_adam_step_f32(None, None, None, None, 0, 1e-3, 0.9, 0.999, 1e-8, 1, 1.0, 0, None) == _lib.WG_OK

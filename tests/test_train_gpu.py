@@ -208,12 +208,15 @@ def test_training_rejects_what_it_does_not_support():
                                      # gru_bwd_regw_kernel (padded hidden size 24 / 104): batches that select its
                                      # 8-, 16- and 28-sequence CTAs (the goldens above run the 4-sequence one)
                                      (7, 21, 700, 3), (7, 22, 1500, 3), (8, 24, 2500, 2),
-                                     (34, 102, 700, 2), (34, 101, 1300, 2), (34, 103, 2400, 2)])
+                                     (34, 102, 700, 2), (34, 101, 1300, 2), (34, 103, 2400, 2),
+                                     # gcn_bwd_kernel<13> (13-wide features, 48 < S): 60 stations, and 90 stations,
+                                     # whose shared memory cuts the row block down to 2 rows
+                                     (60, 30, 40, 3), (90, 45, 20, 2)])
 def test_gradients_ragged_model_shapes(S, H, B, T):
     """Random models with odd station counts / hidden sizes (H odd, even-not-multiple-of-4, near the
     shared-memory limit of the recurrence), batches that end inside a CTA and inside a GEMM tile, a batch past the
-    16-sequence BPTT switch, and every CTA size of the register-resident BPTT kernel: every GEMM edge predicate,
-    unaligned leading dimension and padded column is exercised."""
+    16-sequence BPTT switch, every CTA size of the register-resident BPTT kernel, and station counts past the
+    row-per-lane GCN backward: every GEMM edge predicate, unaligned leading dimension and padded column is exercised."""
     torch.manual_seed(S * 100 + B)
     m = windgnn_b200.GCN_GRU(13, 13, 13, 13 * S, H)
     with torch.no_grad():

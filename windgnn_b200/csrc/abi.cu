@@ -534,20 +534,23 @@ int launch_recur_tc(const Plan& p, void* ws, float* out, long long Bc, cudaStrea
     return WG_OK;
 }
 
+// whether a chunk of Bc sequences runs gru_recur_regw_kernel (launch_recur)
+bool regw_serves(const Plan& p, long long Bc) {
+    return p.recur != kRecurTc && p.regw && Bc <= 2LL * wg::kRsBT * wg::kNumSMs;
+}
+
 // The recurrence of one chunk: the plan's kernel, except that up to two waves of 4-sequence CTAs run
 // gru_recur_regw_kernel where it serves the contraction length (FMA chains per thread = sequences per CTA that can
 // exist: the reference's batch-1 calls run one).  gsave: the training forward, which also saves [r | z | n | hn] per
-// (sequence, step), row stride ldsave.
+// (sequence, step), row stride ldsave; only the regw and unit kernels save gates, and make_train_plan accepts only the
+// shapes that reach one of them.
 int launch_recur(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
-    if (p.recur != kRecurTc && p.regw && Bc <= 2LL * wg::kRsBT * wg::kNumSMs)
-        return launch_recur_regw(p, ws, out, Bc, Bc >= 4 ? 4 : (int)Bc, st, gsave, ldsave);
+    if (regw_serves(p, Bc)) return launch_recur_regw(p, ws, out, Bc, Bc >= 4 ? 4 : (int)Bc, st, gsave, ldsave);
     if (p.recur == kRecurUnit) {
         int r = recur_u_pick_r(Bc, wg::kRuWarps / p.ru_wpg);
         while (r > wg::kRuMinR && wg::recur_u_smem_floats(p.H, r) * 4 > (size_t)wg::kMaxSmemOptin) --r;
         return launch_recur_unit(p, ws, out, Bc, r, st, gsave, ldsave);
     }
-    if (gsave)   // the two kernels above are the ones that save gates
-        return fail(WG_ERR_UNSUPPORTED, "training: GRU hidden size %d does not fit the shared-memory recurrence", p.H);
     if (p.recur == kRecurTc) return launch_recur_tc(p, ws, out, Bc, st);   // the tensor path: every batch size
     return launch_recur_wide(p, ws, out, Bc, st);
 }
@@ -631,20 +634,20 @@ bool any_null(std::initializer_list<const void*> ps) {
     return false;
 }
 
-// The device-buffer forward of either graph form: pack the parameters, then every chunk through the three stages.
-// On gcn_sparse_plan_kernel the CSR graph also holds the constant bank from prepare_sparse to finish_sparse.
-int forward(bool sparse, const Graph& g, const float* x, const float* w1, const float* b1, const float* w2,
-            const float* b2, const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, float* out,
-            long long B, int T, int S, int Fi, int Fh, int Fo, int H, long long chunk, int flags, void* ws,
-            size_t ws_bytes, int device, void* stream) {
-    Plan p;
-    int rc = make_plan(p, B, T, S, Fi, Fh, Fo, H, chunk, sparse, flags);
-    if (rc) return rc;
+// The device-buffer forward of a finished plan, on either graph form: pack the parameters, then every chunk through
+// the three stages.  need: the workspace bytes to check (the training plan adds its regions to the forward's);
+// gsave / ldsave: see launch_recur.  On gcn_sparse_plan_kernel the CSR graph also holds the constant bank from
+// prepare_sparse to finish_sparse.
+int forward(const Plan& p, size_t need, const Graph& g, const float* x, const float* w1, const float* b1,
+            const float* w2, const float* b2, const float* w_ih, const float* w_hh, const float* b_ih,
+            const float* b_hh, float* out, long long B, void* ws, size_t ws_bytes, int device, void* stream,
+            float* gsave = nullptr, int ldsave = 0) {
     if (B == 0) return WG_OK;
     const bool no_graph = p.sparse ? any_null({g.rowptr, g.colidx, g.vals}) : !g.adj;
     if (no_graph || any_null({x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out}))
         return fail(WG_ERR_BAD_ARG, "null pointer argument");
-    if ((rc = check_ws(ws, ws_bytes, p.total))) return rc;
+    int rc = check_ws(ws, ws_bytes, need);
+    if (rc) return rc;
     DeviceGuard dg(device);
     WG_CUDA(dg.err);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -658,7 +661,8 @@ int forward(bool sparse, const Graph& g, const float* x, const float* w1, const 
     const size_t x_seq = (size_t)p.T * p.S * p.Fi, o_seq = (size_t)p.T * p.H;
     for (long long b0 = 0; b0 < B; b0 += p.chunk) {
         const long long Bc = (B - b0) < p.chunk ? (B - b0) : p.chunk;
-        rc = run_chunk(p, ws, g, x + (size_t)b0 * x_seq, w1, b1, w2, b2, out + (size_t)b0 * o_seq, Bc, st);
+        rc = run_chunk(p, ws, g, x + (size_t)b0 * x_seq, w1, b1, w2, b2, out + (size_t)b0 * o_seq, Bc, st,
+                       gsave ? gsave + (size_t)b0 * p.T * ldsave : nullptr, ldsave);
         if (rc) return rc;
     }
     return sq ? finish_sparse(device, st) : WG_OK;
@@ -697,20 +701,46 @@ __global__ void pack_wih_bwd_kernel(const float* __restrict__ w_ih, float* __res
 // ---------------------------------------------------------------------------------------------
 // training step: forward that saves the gate values, backward (BPTT + GEMMs + GCN backward)
 // ---------------------------------------------------------------------------------------------
+// BPTT kernels: gru_bwd_regw_kernel<BT, HPT> (W_hh in registers, HPT = 104 or 24) in the CTA sizes kGbRegwBT, else
+// gru_bwd_kernel<BT> with 4 or kGbBT sequences per CTA
+using GbRegwKernel = decltype(&wg::gru_bwd_regw_kernel<4, 24>);
+using GbKernel = decltype(&wg::gru_bwd_kernel<4>);
+constexpr int kGbRegwBT[4] = {4, 8, 16, 28};
+template <int HPT>
+GbRegwKernel gb_regw_kernel(int i) {
+    const GbRegwKernel k[4] = {wg::gru_bwd_regw_kernel<4, HPT>, wg::gru_bwd_regw_kernel<8, HPT>,
+                               wg::gru_bwd_regw_kernel<16, HPT>, wg::gru_bwd_regw_kernel<28, HPT>};
+    return k[i];
+}
+
+// GCN backward kernel: gcn_bwd_rows_kernel (13 / 13 / 13 features, S <= 48), else gcn_bwd_kernel<13> (exactly 13
+// features everywhere) or gcn_bwd_kernel<16>
+enum GcnBwdKind { kGcnBwdRows, kGcnBwd13, kGcnBwd16 };
+
 struct TrainPlan {
     Plan f;            // the forward's plan (chunk == B, FP32 path, dense graph)
     int LD4;           // row stride of the gate / DG buffers: 4H rounded up to 4
-    int HP, GR, bt_gb; // gru_bwd: H rounded up to 4, padded contraction length, sequences per CTA
-    bool gb_regw;      // gru_bwd_regw_kernel (W_hh in registers; HP = 104 or 24), else gru_bwd_kernel
     long long rows;    // B * T
-    int grid_gb;       // CTAs of the backward recurrence
-    int grid_gcn, rb_gcn, sg_gcn, fp_gcn, parts_gcn;   // parts_gcn: partial gradient sets the GCN backward writes
-    bool gcn_rows;       // gcn_bwd_rows_kernel (13 / 13 / 13 features, S <= 48), else gcn_bwd_kernel
-    size_t smem_gcn;
-    int splits_hh_a, splits_hh_b, splits_ih;
-    int ldu, KPd, NPd;  // dU row stride (I rounded up to 4); K / N of the dU GEMM padded for inproj_kernel
-    int mt_ih, nt_ih;       // dW_ih on gemm_kb_kernel: tiles over the input features / the gate columns
+    // 1. BPTT: exactly one of gb_regw and gb is set
+    GbRegwKernel gb_regw;
+    GbKernel gb;
+    int HP, GR;        // H rounded up to 4; gru_bwd_kernel: padded contraction length
+    int gb_threads, gb_grid, gb_parts;   // gb_parts: bias partial sets the kernel writes (3 per CTA on gb_regw, else 2)
+    size_t gb_smem;
+    // 2. dW_hh on sgemm_kernel: K splits of the r / z and of the n product
+    int splits_hh_a, splits_hh_b;
+    // 3. dW_ih on gemm_kb_kernel: tiles over the input features / the gate columns, splits of the B*T rows
+    int mt_ih, nt_ih, splits_ih;
     long long kt_per_ih;    // k-tiles (16 rows) per split
+    // 4. dU on inproj_kernel
+    int ldu, KPd, NPd;  // dU row stride (I rounded up to 4); K / N of the dU GEMM padded for inproj_kernel
+    dim3 tg_du;         // rows_to_tiles_kernel: dGI into K-major 128-row tiles
+    long long mt_du;    // inproj_kernel: row tiles
+    int nt_du;          //                column tiles
+    // 5. GCN backward
+    GcnBwdKind gcn;
+    int grid_gcn, rb_gcn, parts_gcn;   // parts_gcn: partial gradient sets the GCN backward writes
+    size_t smem_gcn;
     size_t off_gates, off_dg, off_dgt, off_wpb, off_zb, off_du, off_biasp, off_gcnp, off_splitk, total;
 };
 
@@ -733,45 +763,50 @@ size_t param_count(int S, int Fi, int Fh, int Fo, int H) {
 constexpr int kTrainMaxH = 106;
 
 int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, int Fo, int H) {
-    int rc = make_plan(tp.f, B, T, S, Fi, Fh, Fo, H, B > 0 ? B : 1, false, 0);
+    const long long Bn = B > 0 ? B : 1;   // B = 0 plans one sequence: the backward then only zeroes the gradients
+    int rc = make_plan(tp.f, B, T, S, Fi, Fh, Fo, H, Bn, false, 0);
     if (rc) return rc;
     const Plan& p = tp.f;
     if (Fi > 16 || Fh > 16 || Fo > 16)
         return fail(WG_ERR_UNSUPPORTED, "training: GCN feature widths must be <= 16 (got %d / %d / %d)", Fi, Fh, Fo);
     tp.LD4 = wg::round_up(4 * H, 4);
     tp.HP = wg::round_up(H, 4);
-    tp.gb_regw = tp.HP == 104 || tp.HP == 24;
-    if (tp.gb_regw) {
+    int bt;   // sequences per BPTT CTA
+    if (tp.HP == 104 || tp.HP == 24) {
         // W_hh in registers: the smallest CTA size that still makes the grid one wave (28 sequences fit)
-        const long long Bn = B > 0 ? B : 1;
-        tp.bt_gb = 28;
-        for (int bt : {4, 8, 16, 28})
-            if ((Bn + bt - 1) / bt <= wg::kNumSMs) { tp.bt_gb = bt; break; }
-        tp.GR = wg::gru_bwd_gr(H, 4);
+        int i = 0;
+        while (i < 3 && (Bn + kGbRegwBT[i] - 1) / kGbRegwBT[i] > wg::kNumSMs) ++i;
+        bt = kGbRegwBT[i];
+        tp.gb_regw = tp.HP == 104 ? gb_regw_kernel<104>(i) : gb_regw_kernel<24>(i);
+        tp.gb = nullptr;
+        tp.gb_threads = wg::kGrwThreads;
+        tp.gb_smem = wg::gru_bwd_regw_smem_floats(tp.HP, bt) * 4;
     } else {
         // 16 sequences per CTA when that fills the machine, else 4 (the recurrence is latency-bound: with few
         // sequences per GPU — configs[4]: 512 — more, lighter CTAs shorten every one of the T serial steps)
-        tp.bt_gb = (B > 0 ? B : 1) > 4LL * wg::kNumSMs ? wg::kGbBT : 4;
-        tp.GR = wg::gru_bwd_gr(H, tp.bt_gb);
-        if (tp.HP > 128 || (tp.HP / 4) * (tp.bt_gb / 4) * wg::gru_bwd_ksplit(tp.bt_gb) > wg::kGbThreads ||
-            wg::gru_bwd_smem_floats(tp.HP, tp.GR, tp.bt_gb) * 4 > (size_t)wg::kMaxSmemOptin)
+        bt = Bn > 4LL * wg::kNumSMs ? wg::kGbBT : 4;
+        tp.GR = wg::gru_bwd_gr(H, bt);
+        tp.gb_smem = wg::gru_bwd_smem_floats(tp.HP, tp.GR, bt) * 4;
+        if (tp.HP > 128 || (tp.HP / 4) * (bt / 4) * wg::gru_bwd_ksplit(bt) > wg::kGbThreads ||
+            tp.gb_smem > (size_t)wg::kMaxSmemOptin)
             return fail(WG_ERR_UNSUPPORTED, "training: GRU hidden size %d too large for the shared-memory BPTT kernel", H);
+        tp.gb_regw = nullptr;
+        tp.gb = bt == 4 ? wg::gru_bwd_kernel<4> : wg::gru_bwd_kernel<wg::kGbBT>;
+        tp.gb_threads = wg::kGbThreads;
     }
-    if (H > kTrainMaxH)
+    tp.gb_grid = (int)((Bn + bt - 1) / bt);
+    tp.gb_parts = tp.gb_grid * (tp.gb_regw ? 3 : 2);
+    // the forward's recurrence saves the gates: only gru_recur_regw_kernel and gru_recur_unit_kernel do (launch_recur)
+    if (H > kTrainMaxH || !(regw_serves(p, B) || p.recur == kRecurUnit))
         return fail(WG_ERR_UNSUPPORTED, "training: GRU hidden size %d does not fit the shared-memory recurrence", H);
-    tp.rows = (B > 0 ? B : 1) * (long long)T;
-    tp.grid_gb = (int)(((B > 0 ? B : 1) + tp.bt_gb - 1) / tp.bt_gb);
-    // GCN backward geometry (same station grouping as the forward)
-    // 4 stations per thread: the slabs bound the CTA to ~24 rows, so the narrower station group is what
-    // puts 7 warps instead of 4 on the SM
-    tp.sg_gcn = 4;
-    tp.fp_gcn = (Fi == 13 && Fh == 13 && Fo == 13) ? 13 : 16;
+    tp.rows = Bn * T;
     tp.ldu = wg::round_up(p.I, 4);
     tp.KPd = wg::round_up(p.G, wg::kIpBK);
     tp.NPd = wg::round_up(p.I, wg::kIpBN);
-    tp.gcn_rows = wg::gcn_bwd_rows_applies(S, Fi, Fh, Fo) &&
-                  wg::gcn_bwd_rows_smem_floats(S, tp.ldu) * 4 <= (size_t)wg::kMaxSmemOptin;
-    if (tp.gcn_rows) {
+    // GCN backward geometry (same station grouping as the forward)
+    if (wg::gcn_bwd_rows_applies(S, Fi, Fh, Fo) &&
+        wg::gcn_bwd_rows_smem_floats(S, tp.ldu) * 4 <= (size_t)wg::kMaxSmemOptin) {
+        tp.gcn = kGcnBwdRows;
         tp.rb_gcn = wg::kGb2Rows;
         tp.smem_gcn = wg::gcn_bwd_rows_smem_floats(S, tp.ldu) * 4;
         const long long nblk = (tp.rows + wg::kGb2Rows - 1) / wg::kGb2Rows;
@@ -779,13 +814,14 @@ int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, in
         tp.grid_gcn = (int)(nblk < (long long)per_sm * wg::kNumSMs ? nblk : (long long)per_sm * wg::kNumSMs);
         tp.parts_gcn = tp.grid_gcn * wg::kGb2Slices;
     } else {
-        const int NSG = wg::ceil_div(S, tp.sg_gcn);
+        tp.gcn = Fi == 13 && Fh == 13 && Fo == 13 ? kGcnBwd13 : kGcnBwd16;
+        const int NSG = wg::ceil_div(S, wg::kGbwSG);
         if (NSG > wg::kGcnThreads) return fail(WG_ERR_UNSUPPORTED, "training: S=%d too large for the dense GCN kernels", S);
         int RB = wg::kGbwThreads / NSG;
         const int cols = S * Fi;
         const int need = (cols % 4 == 0) ? 1 : (cols % 2 == 0) ? 2 : 4;
         if (RB > need) RB -= RB % need;
-        auto smem_of = [&](int rb) { return wg::gcn_bwd_smem_floats<4>(S, tp.ldu, rb) * 4; };
+        auto smem_of = [&](int rb) { return wg::gcn_bwd_smem_floats(S, tp.ldu, rb) * 4; };
         while (smem_of(RB) > (size_t)wg::kMaxSmemOptin && RB > 1) RB = (RB > need) ? RB - need : RB - 1;
         if (smem_of(RB) > (size_t)wg::kMaxSmemOptin)
             return fail(WG_ERR_UNSUPPORTED, "training: S=%d does not fit the shared-memory GCN backward", S);
@@ -795,19 +831,18 @@ int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, in
         tp.grid_gcn = (int)(nblk < wg::kNumSMs ? nblk : wg::kNumSMs);
         tp.parts_gcn = tp.grid_gcn * (wg::kGbwThreads / 16);
     }
+    // dU stage: dGI re-laid into K-major 128-row tiles by one pass of 32-row blocks (at most 65535 of them)
+    const long long rt = (tp.rows + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows;
+    if (rt / 32 > 65535) return fail(WG_ERR_UNSUPPORTED, "training: B*T = %lld rows exceed one pass", tp.rows);
+    tp.tg_du = dim3((unsigned)((tp.KPd + 31) / 32), (unsigned)(rt / 32));
+    tp.mt_du = rt / wg::kIpBM;
+    tp.nt_du = tp.NPd / wg::kIpBN;
     tp.splits_hh_a = pick_splits(2 * H, H, tp.rows);
     tp.splits_hh_b = pick_splits(H, H, tp.rows);
-    size_t o = p.total;
-    tp.off_gates = o; o = align_up(o + (size_t)tp.rows * tp.LD4 * 4);
-    tp.off_dg = o;    o = align_up(o + (size_t)tp.rows * tp.LD4 * 4);
+    // dW_ih on gemm_kb_kernel<64, 160, 0>: tiles over (i, g), the B*T rows split so that the grid is one wave
+    tp.mt_ih = (p.IP + wg::KbWih::kBM - 1) / wg::KbWih::kBM;
+    tp.nt_ih = (p.G + wg::KbWih::kBN - 1) / wg::KbWih::kBN;
     {
-        const size_t rt = ((size_t)tp.rows + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows;
-        tp.off_dgt = o; o = align_up(o + rt * tp.KPd * 4);            // dGI in K-major 128-row tiles
-        tp.off_wpb = o; o = align_up(o + (size_t)tp.NPd * tp.KPd * 4);  // w_ih packed for dU = dGI . w_ih
-        tp.off_zb = o;  o = align_up(o + (size_t)tp.NPd * 4);           // zero bias (written by the pack kernel)
-        // dW_ih on gemm_kb_kernel<64, 160, 0>: tiles over (i, g), the B*T rows split so that the grid is one wave
-        tp.mt_ih = (p.IP + wg::KbWih::kBM - 1) / wg::KbWih::kBM;
-        tp.nt_ih = (p.G + wg::KbWih::kBN - 1) / wg::KbWih::kBN;
         const long long ktall = (tp.rows + wg::kKbBK - 1) / wg::kKbBK;
         long long sp = (3LL * wg::kNumSMs) / ((long long)tp.mt_ih * tp.nt_ih);   // one wave at 3 CTAs per SM
         if (sp < 1) sp = 1;
@@ -815,8 +850,14 @@ int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, in
         tp.kt_per_ih = (ktall + sp - 1) / sp;
         tp.splits_ih = (int)((ktall + tp.kt_per_ih - 1) / tp.kt_per_ih);
     }
+    size_t o = p.total;
+    tp.off_gates = o; o = align_up(o + (size_t)tp.rows * tp.LD4 * 4);
+    tp.off_dg = o;    o = align_up(o + (size_t)tp.rows * tp.LD4 * 4);
+    tp.off_dgt = o;   o = align_up(o + (size_t)rt * tp.KPd * 4);              // dGI in K-major 128-row tiles
+    tp.off_wpb = o;   o = align_up(o + (size_t)tp.NPd * tp.KPd * 4);          // w_ih packed for dU = dGI . w_ih
+    tp.off_zb = o;    o = align_up(o + (size_t)tp.NPd * 4);                   // zero bias (written by the pack kernel)
     tp.off_du = o;    o = align_up(o + (size_t)tp.rows * tp.ldu * 4);
-    tp.off_biasp = o; o = align_up(o + (size_t)tp.grid_gb * 3 * tp.LD4 * 4);   // 3 partial sets per CTA (regw), else 2
+    tp.off_biasp = o; o = align_up(o + (size_t)tp.gb_grid * 3 * tp.LD4 * 4);  // 3 partial sets per CTA (regw), else 2
     tp.off_gcnp = o;  o = align_up(o + (size_t)tp.parts_gcn * (2 * 256 + 32) * 4);
     size_t sk = (size_t)tp.splits_hh_a * 2 * H * H;
     if ((size_t)tp.splits_hh_b * H * H > sk) sk = (size_t)tp.splits_hh_b * H * H;
@@ -842,19 +883,6 @@ int splitk_gemm(const wg::SgOperand& A, const wg::SgOperand& Bo, long long M, in
     WG_CUDA(cudaGetLastError());
     const long long total = M * N;
     wg::sg_reduce_kernel<<<(unsigned)((total * 8 + 255) / 256), 256, 0, st>>>(part, splits, M, N, out, s_m, s_n, N);
-    WG_CUDA(cudaGetLastError());
-    return WG_OK;
-}
-
-template <int FP, int SG>
-int launch_gcn_bwd_t(const TrainPlan& tp, void* ws, const float* x, const float* adj, const float* w1, const float* b1,
-                     const float* w2, const float* b2, cudaStream_t st) {
-    const Plan& p = tp.f;
-    auto kern = wg::gcn_bwd_kernel<FP, SG>;
-    WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_gcn));
-    kern<<<tp.grid_gcn, wg::kGbwThreads, tp.smem_gcn, st>>>(x, ws_ptr<float>(ws, tp.off_du), adj, w1, b1, w2, b2,
-                                                           ws_ptr<float>(ws, tp.off_gcnp), tp.rows, p.S, p.Fi, p.Fh,
-                                                           p.Fo, tp.rb_gcn, tp.ldu);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
@@ -927,8 +955,10 @@ int wg_gcn_gru_forward_f32(const float* adj, const float* x, const float* w1, co
                            const float* b_ih, const float* b_hh, float* out, int64_t B, int T, int S,
                            int F_in, int F_hid, int F_out, int H, int64_t chunk, int flags, void* workspace,
                            size_t workspace_bytes, int device, void* stream) {
-    return forward(false, Graph{adj}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, B, T,
-                   S, F_in, F_hid, F_out, H, chunk, flags, workspace, workspace_bytes, device, stream);
+    Plan p;
+    const int rc = make_plan(p, B, T, S, F_in, F_hid, F_out, H, chunk, false, flags);
+    return rc ? rc : forward(p, p.total, Graph{adj}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, B, workspace,
+                             workspace_bytes, device, stream);
 }
 
 size_t wg_gcn_gru_csr_workspace_bytes(int64_t B, int T, int S, int F_in, int F_hid, int F_out, int H,
@@ -944,8 +974,10 @@ int wg_gcn_gru_forward_csr_f32(const int32_t* rowptr, const int32_t* colidx, con
                                float* out, int64_t B, int T, int S, int F_in, int F_hid, int F_out, int H,
                                int64_t chunk, int flags, void* workspace, size_t workspace_bytes, int device,
                                void* stream) {
-    return forward(true, Graph{nullptr, rowptr, colidx, vals}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, B, T, S,
-                   F_in, F_hid, F_out, H, chunk, flags, workspace, workspace_bytes, device, stream);
+    Plan p;
+    const int rc = make_plan(p, B, T, S, F_in, F_hid, F_out, H, chunk, true, flags);
+    return rc ? rc : forward(p, p.total, Graph{nullptr, rowptr, colidx, vals}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih,
+                             b_hh, out, B, workspace, workspace_bytes, device, stream);
 }
 
 }  // extern "C"
@@ -1150,18 +1182,11 @@ int wg_gcn_gru_forward_train_f32(const float* adj, const float* x, const float* 
                                  int F_in, int F_hid, int F_out, int H, void* workspace, size_t workspace_bytes,
                                  int device, void* stream) {
     TrainPlan tp;
-    int rc = make_train_plan(tp, B, T, S, F_in, F_hid, F_out, H);
+    const int rc = make_train_plan(tp, B, T, S, F_in, F_hid, F_out, H);
     if (rc) return rc;
-    if (B == 0) return WG_OK;
-    if (any_null({adj, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out}))
-        return fail(WG_ERR_BAD_ARG, "null pointer argument");
-    if ((rc = check_ws(workspace, workspace_bytes, tp.total))) return rc;
-    DeviceGuard g(device);
-    WG_CUDA(g.err);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if ((rc = launch_pack(tp.f, workspace, w_ih, w_hh, b_ih, b_hh, st))) return rc;
-    return run_chunk(tp.f, workspace, Graph{adj}, x, w1, b1, w2, b2, out, B, st,
-                     ws_ptr<float>(workspace, tp.off_gates), tp.LD4);
+    float* gates = workspace ? ws_ptr<float>(workspace, tp.off_gates) : nullptr;   // forward() rejects a NULL workspace
+    return forward(tp.f, tp.total, Graph{adj}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, B, workspace,
+                   workspace_bytes, device, stream, gates, tp.LD4);
 }
 
 int wg_gcn_gru_backward_f32(const float* adj, const float* x, const float* w1, const float* b1, const float* w2,
@@ -1201,29 +1226,17 @@ int wg_gcn_gru_backward_f32(const float* adj, const float* x, const float* w1, c
     const long long rows = tp.rows;
 
     // 1. BPTT through the recurrence: DG = [da_r | da_z | da_n | da_n r], bias partials
-    {
-        if (tp.gb_regw) {
-            using KernT = void (*)(const float*, const float*, const float*, const float*, float*, float*, long long, int, int, int);
-            KernT kern = nullptr;
-            if (tp.HP == 104)
-                kern = tp.bt_gb == 4 ? wg::gru_bwd_regw_kernel<4, 104> : tp.bt_gb == 8 ? wg::gru_bwd_regw_kernel<8, 104>
-                     : tp.bt_gb == 16 ? wg::gru_bwd_regw_kernel<16, 104> : wg::gru_bwd_regw_kernel<28, 104>;
-            else
-                kern = tp.bt_gb == 4 ? wg::gru_bwd_regw_kernel<4, 24> : tp.bt_gb == 8 ? wg::gru_bwd_regw_kernel<8, 24>
-                     : tp.bt_gb == 16 ? wg::gru_bwd_regw_kernel<16, 24> : wg::gru_bwd_regw_kernel<28, 24>;
-            const size_t smem = wg::gru_bwd_regw_smem_floats(tp.HP, tp.bt_gb) * 4;
-            WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            kern<<<tp.grid_gb, wg::kGrwThreads, smem, st>>>(gates, out, d_out, w_hh, DG, biasp, B, T, H, tp.LD4);
-        } else {
-            const size_t smem = wg::gru_bwd_smem_floats(tp.HP, tp.GR, tp.bt_gb) * 4;
-            auto kern = tp.bt_gb == 4 ? wg::gru_bwd_kernel<4> : wg::gru_bwd_kernel<wg::kGbBT>;
-            WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            kern<<<tp.grid_gb, wg::kGbThreads, smem, st>>>(gates, out, d_out, w_hh, DG, biasp, B, T, H, tp.LD4, tp.HP, tp.GR);
-        }
-        WG_CUDA(cudaGetLastError());
-        wg::gru_bias_grad_kernel<<<(4 * H + 127) / 128, 128, 0, st>>>(biasp, tp.grid_gb * (tp.gb_regw ? 3 : 2), H, tp.LD4, d_bih, d_bhh);
-        WG_CUDA(cudaGetLastError());
+    if (tp.gb_regw) {
+        WG_CUDA(cudaFuncSetAttribute(tp.gb_regw, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.gb_smem));
+        tp.gb_regw<<<tp.gb_grid, tp.gb_threads, tp.gb_smem, st>>>(gates, out, d_out, w_hh, DG, biasp, B, T, H, tp.LD4);
+    } else {
+        WG_CUDA(cudaFuncSetAttribute(tp.gb, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.gb_smem));
+        tp.gb<<<tp.gb_grid, tp.gb_threads, tp.gb_smem, st>>>(gates, out, d_out, w_hh, DG, biasp, B, T, H, tp.LD4, tp.HP,
+                                                              tp.GR);
     }
+    WG_CUDA(cudaGetLastError());
+    wg::gru_bias_grad_kernel<<<(4 * H + 127) / 128, 128, 0, st>>>(biasp, tp.gb_parts, H, tp.LD4, d_bih, d_bhh);
+    WG_CUDA(cudaGetLastError());
     const int dg_vec = (tp.LD4 % 4 == 0) && aligned16(DG);
     // 2. dW_hh = dGH^T . H_prev   (H_prev[b, t] = out[b, t-1], 0 at t = 0)
     {
@@ -1268,33 +1281,30 @@ int wg_gcn_gru_backward_f32(const float* adj, const float* x, const float* w1, c
         float* DGt = ws_ptr<float>(workspace, tp.off_dgt);
         float* wpb = ws_ptr<float>(workspace, tp.off_wpb);
         float* zb = ws_ptr<float>(workspace, tp.off_zb);
-        const long long rt = (rows + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows;
-        const dim3 tg((unsigned)((tp.KPd + 31) / 32), (unsigned)(rt / 32));
-        if (tg.y > 65535u) return fail(WG_ERR_UNSUPPORTED, "training: B*T = %lld rows exceed one pass", rows);
-        wg::rows_to_tiles_kernel<<<tg, 256, 0, st>>>(DG, DGt, rows, p.G, tp.LD4, tp.KPd);
+        wg::rows_to_tiles_kernel<<<tp.tg_du, 256, 0, st>>>(DG, DGt, rows, p.G, tp.LD4, tp.KPd);
         WG_CUDA(cudaGetLastError());
         pack_wih_bwd_kernel<<<wg::kNumSMs, 256, 0, st>>>(w_ih, wpb, zb, p.G, p.I, tp.KPd, tp.NPd);
         WG_CUDA(cudaGetLastError());
-        const long long m_tiles = rt / wg::kIpBM;
-        const int n_tiles = tp.NPd / wg::kIpBN;
         WG_CUDA(cudaFuncSetAttribute(wg::inproj_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, wg::kIpSmemBytes));
-        wg::inproj_kernel<<<(unsigned)(m_tiles * n_tiles), wg::kIpThreads, wg::kIpSmemBytes, st>>>(
-            DGt, wpb, zb, dU, rows, tp.KPd, tp.ldu, n_tiles);
+        wg::inproj_kernel<<<(unsigned)(tp.mt_du * tp.nt_du), wg::kIpThreads, wg::kIpSmemBytes, st>>>(
+            DGt, wpb, zb, dU, rows, tp.KPd, tp.ldu, tp.nt_du);
         WG_CUDA(cudaGetLastError());
     }
     // 5. GCN backward: dW1, db1, dW2, db2
-    if (tp.gcn_rows) {
+    float* gcnp = ws_ptr<float>(workspace, tp.off_gcnp);
+    if (tp.gcn == kGcnBwdRows) {
         WG_CUDA(cudaFuncSetAttribute(wg::gcn_bwd_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_gcn));
-        wg::gcn_bwd_rows_kernel<<<tp.grid_gcn, wg::kGb2Threads, tp.smem_gcn, st>>>(
-            x, dU, adj, w1, b1, w2, b2, ws_ptr<float>(workspace, tp.off_gcnp), tp.rows, p.S, tp.ldu);
-        WG_CUDA(cudaGetLastError());
+        wg::gcn_bwd_rows_kernel<<<tp.grid_gcn, wg::kGb2Threads, tp.smem_gcn, st>>>(x, dU, adj, w1, b1, w2, b2, gcnp, rows,
+                                                                                 p.S, tp.ldu);
     } else {
-        if (tp.fp_gcn == 13) rc = launch_gcn_bwd_t<13, 4>(tp, workspace, x, adj, w1, b1, w2, b2, st);
-        else rc = launch_gcn_bwd_t<16, 4>(tp, workspace, x, adj, w1, b1, w2, b2, st);
-        if (rc) return rc;
+        auto kern = tp.gcn == kGcnBwd13 ? wg::gcn_bwd_kernel<13> : wg::gcn_bwd_kernel<16>;
+        WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_gcn));
+        kern<<<tp.grid_gcn, wg::kGbwThreads, tp.smem_gcn, st>>>(x, dU, adj, w1, b1, w2, b2, gcnp, rows, p.S, p.Fi, p.Fh,
+                                                               p.Fo, tp.rb_gcn, tp.ldu);
     }
+    WG_CUDA(cudaGetLastError());
     wg::gcn_bwd_finish_kernel<<<(2 * 256 + 32 + 7) / 8, 256, 0, st>>>(
-        ws_ptr<float>(workspace, tp.off_gcnp), tp.parts_gcn, F_in, F_hid, F_out, d_w1, d_b1, d_w2, d_b2);
+        gcnp, tp.parts_gcn, F_in, F_hid, F_out, d_w1, d_b1, d_w2, d_b2);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }

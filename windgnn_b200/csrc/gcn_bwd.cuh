@@ -11,7 +11,7 @@
 // intermediate state that would otherwise go through HBM).
 //
 // Same decomposition as the forward kernel (gcn.cuh): a CTA owns RB rows, the X and dU row
-// blocks arrive by ONE bulk async copy each, a thread owns SG stations of one row and does the
+// blocks arrive by ONE bulk async copy each, a thread owns kGbwSG = 4 stations of one row and does the
 // S-long aggregations with FFMA2 on feature pairs.  The slabs live in shared memory with 16
 // floats per station so that the two 13 x 13 outer-product reductions (sum over all stations of
 // all rows of the block) run as a small register-tiled GEMM: thread = 4 x 4 output tile x one of
@@ -29,12 +29,16 @@ constexpr int kGbwW = 16;   // width of the zero-padded weight tables
 constexpr int kGbwFS = 20;  // floats per station in the padded slabs: 16 used + 4 so that the stations a warp's
                             // lanes own (consecutive stations, 80 B apart) fall into distinct bank groups
 constexpr int kGbwThreads = 256;
+// stations per thread: the slabs bound the CTA to ~24 rows, so the narrower station group is what puts 7 warps
+// instead of 4 on the SM
+constexpr int kGbwSG = 4;
 // padded slab row stride: + 4 floats so that the rows a warp touches at once start in different banks
 __host__ __device__ inline int gcn_bwd_row_stride(int S) { return S * kGbwFS + 4; }
 
-template <int SG>
+// The adjacency tables keep 8 floats per (station, group) although the kernel reads 4: this size decides the row
+// block RB, and RB the grouping of the partial sums, so the gradient bits depend on it.
 __host__ __device__ inline size_t gcn_bwd_smem_floats(int S, int ldu, int RB) {
-    const int NSG = ceil_div(S, SG);
+    const int NSG = ceil_div(S, kGbwSG);
     size_t n = 0;
     n += 2 * (size_t)S * NSG * 8;          // adjT (A[own][sp]) and adjN (A[sp][own])
     n += 3 * (size_t)kGbwW * kGbwW;        // W1, W2, W2^T (zero padded 16 x 16)
@@ -48,24 +52,17 @@ __host__ __device__ inline size_t gcn_bwd_smem_floats(int S, int ldu, int RB) {
 // acc[i][fp] = sum_sp tab[sp][q][i] * (x[sp][2fp], x[sp][2fp+1]); x rows `stride` floats apart,
 // features >= flim read as zero (dense input slab) or are zero padding (stride 16 slabs).
 // VEC: the slab is a padded one (16 floats per station, 16-byte aligned): features come by LDS.128.
-template <int FPP, int SG, bool VEC>
-__device__ __forceinline__ void gcn_bwd_agg(float2 (&acc)[SG][FPP], const float* __restrict__ xrow, int stride,
+template <int FPP, bool VEC>
+__device__ __forceinline__ void gcn_bwd_agg(float2 (&acc)[kGbwSG][FPP], const float* __restrict__ xrow, int stride,
                                             int flim, const float* __restrict__ arow, int astride, int S) {
 #pragma unroll
-    for (int i = 0; i < SG; ++i)
+    for (int i = 0; i < kGbwSG; ++i)
 #pragma unroll
         for (int fp = 0; fp < FPP; ++fp) acc[i][fp] = make_float2(0.0f, 0.0f);
 #pragma unroll 2
     for (int sp = 0; sp < S; ++sp) {
-        float a[8];
-        {
-            const float4 t0 = *reinterpret_cast<const float4*>(arow + (size_t)sp * astride);
-            a[0] = t0.x; a[1] = t0.y; a[2] = t0.z; a[3] = t0.w;
-            if (SG > 4) {
-                const float4 t1 = *reinterpret_cast<const float4*>(arow + (size_t)sp * astride + 4);
-                a[4] = t1.x; a[5] = t1.y; a[6] = t1.z; a[7] = t1.w;
-            }
-        }
+        const float4 t = *reinterpret_cast<const float4*>(arow + (size_t)sp * astride);
+        const float a[kGbwSG] = {t.x, t.y, t.z, t.w};
         float x[2 * FPP + 2];
         if (VEC) {
 #pragma unroll
@@ -80,7 +77,7 @@ __device__ __forceinline__ void gcn_bwd_agg(float2 (&acc)[SG][FPP], const float*
             for (int f = 0; f < 2 * FPP; ++f) x[f] = f < flim ? xrow[sp * stride + f] : 0.0f;
         }
 #pragma unroll
-        for (int i = 0; i < SG; ++i) {
+        for (int i = 0; i < kGbwSG; ++i) {
             const float2 aa = make_float2(a[i], a[i]);
 #pragma unroll
             for (int fp = 0; fp < FPP; ++fp)
@@ -89,17 +86,17 @@ __device__ __forceinline__ void gcn_bwd_agg(float2 (&acc)[SG][FPP], const float*
     }
 }
 
-// o[i][0..1] = sum_f in[i][f] * (W[f][fo0 .. fo0+3]) for this thread's SG stations
-template <int FPP, int SG>
-__device__ __forceinline__ void gcn_bwd_xform4(float2 (&o)[SG][2], const float2 (&in)[SG][FPP],
+// o[i][0..1] = sum_f in[i][f] * (W[f][fo0 .. fo0+3]) for this thread's kGbwSG stations
+template <int FPP>
+__device__ __forceinline__ void gcn_bwd_xform4(float2 (&o)[kGbwSG][2], const float2 (&in)[kGbwSG][FPP],
                                                const float* __restrict__ Wn, int fo0) {
 #pragma unroll
-    for (int i = 0; i < SG; ++i) o[i][0] = o[i][1] = make_float2(0.0f, 0.0f);
+    for (int i = 0; i < kGbwSG; ++i) o[i][0] = o[i][1] = make_float2(0.0f, 0.0f);
 #pragma unroll
     for (int f = 0; f < 2 * FPP; ++f) {
         const float4 w = *reinterpret_cast<const float4*>(Wn + f * kGbwW + fo0);
 #pragma unroll
-        for (int i = 0; i < SG; ++i) {
+        for (int i = 0; i < kGbwSG; ++i) {
             const float av = (f & 1) ? in[i][f >> 1].y : in[i][f >> 1].x;
             o[i][0] = __ffma2_rn(make_float2(av, av), make_float2(w.x, w.y), o[i][0]);
             o[i][1] = __ffma2_rn(make_float2(av, av), make_float2(w.z, w.w), o[i][1]);
@@ -109,7 +106,7 @@ __device__ __forceinline__ void gcn_bwd_xform4(float2 (&o)[SG][2], const float2 
 
 // FP: compile-time bound on the feature widths (13 for the reference's models, else 16).
 // part: [gridDim.x * 8][2 * 256 + 32] per-thread-slice partials (dW1 16x16, dW2 16x16, db1 16, db2 16).
-template <int FP, int SG>
+template <int FP>
 __global__ void __launch_bounds__(kGbwThreads, 1)
     gcn_bwd_kernel(const float* __restrict__ X, const float* __restrict__ dU, const float* __restrict__ adj,
                    const float* __restrict__ W1, const float* __restrict__ b1, const float* __restrict__ W2,
@@ -117,10 +114,9 @@ __global__ void __launch_bounds__(kGbwThreads, 1)
                    int Fo, int RB, int ldu) {
     constexpr int FPP = (FP + 1) / 2;
     extern __shared__ __align__(16) float smem[];
-    const int NSG = ceil_div(S, SG);
+    const int NSG = ceil_div(S, kGbwSG);
     const int tid = threadIdx.x;
-    constexpr int TS = SG > 4 ? 8 : 4;   // table floats per station group (LDS.128 granules)
-    const int astride = NSG * TS;
+    const int astride = NSG * kGbwSG;   // table floats per row of the adjacency tables (one LDS.128 per group)
     const int SR = gcn_bwd_row_stride(S);   // padded slab row stride
 
     float* adjT = smem;
@@ -136,12 +132,12 @@ __global__ void __launch_bounds__(kGbwThreads, 1)
     float* sd = s2 + (size_t)RB * SR;          // dU (dense)
     uint64_t* bar = reinterpret_cast<uint64_t*>(sd + round_up(RB * ldu, 4));
 
-    for (int e = tid; e < S * NSG * TS; e += kGbwThreads) {
-        const int sp = e / (NSG * TS);
-        const int c = e % (NSG * TS);
-        const int qq = c / TS, i = c % TS;
+    for (int e = tid; e < S * NSG * kGbwSG; e += kGbwThreads) {
+        const int sp = e / (NSG * kGbwSG);
+        const int c = e % (NSG * kGbwSG);
+        const int qq = c / kGbwSG, i = c % kGbwSG;
         const int s = qq + NSG * i;       // thread qq owns stations qq, qq + NSG, ... (lanes = consecutive stations)
-        const bool ok = i < SG && s < S;
+        const bool ok = s < S;
         adjT[e] = ok ? adj[(size_t)s * S + sp] : 0.0f;
         adjN[e] = ok ? adj[(size_t)sp * S + s] : 0.0f;
     }
@@ -220,16 +216,16 @@ __global__ void __launch_bounds__(kGbwThreads, 1)
             __syncthreads();
         }
         const bool active = row_local < nrows && tid < RB * NSG;
-        unsigned mask1[SG];
-        float2 acc[SG][FPP];
+        unsigned mask1[kGbwSG];
+        float2 acc[kGbwSG][FPP];
 
         // ---- P1: AX = A.X (own stations) ; G1 = relu(AX.W1 + b1) ----
         if (active)
-            gcn_bwd_agg<FPP, SG, false>(acc, s0 + (size_t)row_local * in_cols, Fi, Fi, adjT + q * TS, astride, S);
+            gcn_bwd_agg<FPP, false>(acc, s0 + (size_t)row_local * in_cols, Fi, Fi, adjT + q * kGbwSG, astride, S);
         __syncthreads();   // every read of the dense X block is done: s0 becomes the padded AX slab
         if (active) {
 #pragma unroll
-            for (int i = 0; i < SG; ++i) {
+            for (int i = 0; i < kGbwSG; ++i) {
                 mask1[i] = 0u;
                 const int s = q + NSG * i;
                 if (s < S) {
@@ -241,11 +237,11 @@ __global__ void __launch_bounds__(kGbwThreads, 1)
             }
 #pragma unroll 1
             for (int fo0 = 0; fo0 < kGbwW; fo0 += 4) {
-                float2 o[SG][2];
-                gcn_bwd_xform4<FPP, SG>(o, acc, w1d, fo0);
+                float2 o[kGbwSG][2];
+                gcn_bwd_xform4<FPP>(o, acc, w1d, fo0);
                 const float4 bb = *reinterpret_cast<const float4*>(b1s + fo0);
 #pragma unroll
-                for (int i = 0; i < SG; ++i) {
+                for (int i = 0; i < kGbwSG; ++i) {
                     const int s = q + NSG * i;
                     if (s < S) {
                         float4 g;
@@ -263,11 +259,11 @@ __global__ void __launch_bounds__(kGbwThreads, 1)
 
         // ---- P2: AG = A.G1 ; dZ2 = dU * [AG.W2 + b2 > 0] ----
         if (active)
-            gcn_bwd_agg<FPP, SG, true>(acc, s1 + (size_t)row_local * SR, kGbwFS, 2 * FPP, adjT + q * TS, astride, S);
+            gcn_bwd_agg<FPP, true>(acc, s1 + (size_t)row_local * SR, kGbwFS, 2 * FPP, adjT + q * kGbwSG, astride, S);
         __syncthreads();   // every read of G1 is done: s1 becomes AG
         if (active) {
 #pragma unroll
-            for (int i = 0; i < SG; ++i) {
+            for (int i = 0; i < kGbwSG; ++i) {
                 const int s = q + NSG * i;
                 if (s < S) {
                     float* ag = s1 + (size_t)row_local * SR + s * kGbwFS;
@@ -278,11 +274,11 @@ __global__ void __launch_bounds__(kGbwThreads, 1)
             }
 #pragma unroll 1
             for (int fo0 = 0; fo0 < kGbwW; fo0 += 4) {
-                float2 o[SG][2];
-                gcn_bwd_xform4<FPP, SG>(o, acc, w2d, fo0);
+                float2 o[kGbwSG][2];
+                gcn_bwd_xform4<FPP>(o, acc, w2d, fo0);
                 const float4 bb = *reinterpret_cast<const float4*>(b2s + fo0);
 #pragma unroll
-                for (int i = 0; i < SG; ++i) {
+                for (int i = 0; i < kGbwSG; ++i) {
                     const int s = q + NSG * i;
                     if (s < S) {
                         const float* du = sd + (size_t)row_local * du_cols + s * Fo + fo0;
@@ -302,7 +298,7 @@ __global__ void __launch_bounds__(kGbwThreads, 1)
         reduce(s1, s2, nrows, aw2, ab2);
         if (active) {   // own dZ2 rows into registers (reads only) before anyone overwrites s2
 #pragma unroll
-            for (int i = 0; i < SG; ++i) {
+            for (int i = 0; i < kGbwSG; ++i) {
                 const int s = q + NSG * i;
                 const float* dz = s2 + (size_t)row_local * SR + (s < S ? s : 0) * kGbwFS;
 #pragma unroll
@@ -313,10 +309,10 @@ __global__ void __launch_bounds__(kGbwThreads, 1)
         if (active) {
 #pragma unroll 1
             for (int fo0 = 0; fo0 < kGbwW; fo0 += 4) {
-                float2 o[SG][2];
-                gcn_bwd_xform4<FPP, SG>(o, acc, w2t, fo0);
+                float2 o[kGbwSG][2];
+                gcn_bwd_xform4<FPP>(o, acc, w2t, fo0);
 #pragma unroll
-                for (int i = 0; i < SG; ++i) {
+                for (int i = 0; i < kGbwSG; ++i) {
                     const int s = q + NSG * i;
                     if (s < S)
                         *reinterpret_cast<float4*>(s2 + (size_t)row_local * SR + s * kGbwFS + fo0) =
@@ -328,9 +324,9 @@ __global__ void __launch_bounds__(kGbwThreads, 1)
 
         // ---- P4: dG1 = A^T dAG ; dZ1 = dG1 * [G1 > 0] -> s1 ----
         if (active) {
-            gcn_bwd_agg<FPP, SG, true>(acc, s2 + (size_t)row_local * SR, kGbwFS, 2 * FPP, adjN + q * TS, astride, S);
+            gcn_bwd_agg<FPP, true>(acc, s2 + (size_t)row_local * SR, kGbwFS, 2 * FPP, adjN + q * kGbwSG, astride, S);
 #pragma unroll
-            for (int i = 0; i < SG; ++i) {
+            for (int i = 0; i < kGbwSG; ++i) {
                 const int s = q + NSG * i;
                 if (s < S) {
                     float* dz = s1 + (size_t)row_local * SR + s * kGbwFS;
