@@ -72,6 +72,11 @@ const char* wg_last_error(void);
  *   to the same 1e-5 parity bar.  Operand magnitudes must stay inside the fp16 range (|x| < 65504;
  *   the GCN outputs and the weights of the shipped models are O(1)).  Results do not depend on how
  *   a batch is split.  The workspace must be sized with the same flags.
+ *
+ * The workspace queries of the forward (this one, the CSR and the host-buffer ones below) return 0
+ * for every shape (dims, chunk and flags) their entry point rejects, and wg_last_error() says why.
+ * The entry point checks the shape first and returns the same code and text before it looks at
+ * pointers or the workspace and before it launches anything.
  * ---------------------------------------------------------------------------------- */
 size_t wg_gcn_gru_workspace_bytes(int64_t B, int T, int S, int F_in, int F_hid, int F_out, int H,
                                   int64_t chunk, int flags);

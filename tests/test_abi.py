@@ -90,6 +90,30 @@ def test_argument_validation_happens_before_cuda():
     assert rc == _lib.WG_ERR_WORKSPACE and "aligned" in _lib.last_error()
 
 
+@pytest.mark.parametrize("csr,dims,reason", [
+    (False, (4, 168, 7, 20, 20, 13, 21, 0, 0), "GCN feature width 20 > 16"),
+    (False, (4, 8, 520, 16, 16, 16, 21, 0, 0), "S=520 too large for the dense GCN kernel"),
+    (False, (4, 8, 600, 13, 13, 13, 21, 0, 0), "S=600 too large for the dense GCN kernel"),   # the 13 x 4 kernel
+    (False, (4, 8, 200, 16, 16, 16, 21, 0, 0), "dense GCN needs"),
+    (False, (4, 8, 34, 13, 13, 13, 400, 0, 0), "GRU hidden size 400: state does not fit"),
+    (True, (2, 3, 4, 20, 20, 13, 12, 0, 0), "sparse GCN: F_in / F_out must be <= 16 (got 20 / 13)"),
+    (True, (2, 3, 300, 13, 2000, 13, 24, 0, 0), "sparse GCN: hidden width 2000 too large"),
+    (True, (20000, 168, 300, 13, 32, 13, 24, 20000, 0), "sparse GCN: chunk of 3360000 rows too large"),
+    (True, (2, 3, 300, 13, 32, 13, 400, 0, 0), "GRU hidden size 400: state does not fit"),
+])
+def test_kernel_limits_are_checked_at_planning(csr, dims, reason):
+    """A shape that no kernel of the plan serves gets no workspace, and the forward rejects it before it looks at the
+    workspace, so that nothing launches."""
+    lib = _lib.load()
+    query, entry, n_ptrs = ((lib.wg_gcn_gru_csr_workspace_bytes, lib.wg_gcn_gru_forward_csr_f32, 13) if csr else
+                            (lib.wg_gcn_gru_workspace_bytes, lib.wg_gcn_gru_forward_f32, 11))
+    assert query(*dims) == 0
+    assert reason in _lib.last_error()
+    fake = ctypes.c_void_p(8)   # non-null, never dereferenced; the workspace stays NULL so that nothing can launch
+    assert entry(*([fake] * n_ptrs), *dims, None, 0, 0, None) == _lib.WG_ERR_UNSUPPORTED
+    assert reason in _lib.last_error()
+
+
 def test_training_planning_and_validation():
     lib = _lib.load()
     dims34 = (168, 34, 13, 13, 13, 102)
@@ -102,6 +126,11 @@ def test_training_planning_and_validation():
     assert trn - fwd >= 512 * 168 * (2 * 408 + 442) * 4
     assert lib.wg_gcn_gru_train_workspace_bytes(512, 168, 34, 13, 32, 13, 102) == 0
     assert "feature widths" in _lib.last_error()
+    # the training limits are reported before the forward's, which these shapes exceed too
+    assert lib.wg_gcn_gru_train_workspace_bytes(4, 8, 520, 16, 16, 16, 21) == 0
+    assert _lib.last_error() == "training: S=520 too large for the dense GCN kernels"
+    assert lib.wg_gcn_gru_train_workspace_bytes(4, 8, 200, 16, 16, 16, 21) == 0
+    assert _lib.last_error() == "training: S=200 does not fit the shared-memory GCN backward"
     assert lib.wg_mse_workspace_bytes() >= 8
     fake = ctypes.c_void_p(8)
     rc = lib.wg_gcn_gru_forward_train_f32(*([fake] * 11), 2, *dims34, None, 0, 0, None)

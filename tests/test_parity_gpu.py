@@ -392,6 +392,20 @@ def test_errors_are_reported_not_thrown_across_the_abi():
     with pytest.raises(_lib.WindGNNError) as ei:
         m(torch.eye(4, device=DEV), torch.zeros((2, 3, 4, 20), device=DEV))
     assert ei.value.code == _lib.WG_ERR_UNSUPPORTED
+    # the code is the library's own, whichever limit the shape exceeds; planning rejects both, so nothing launches
+    S = 80700   # S * F_out = 1,049,100 > 2^20
+    eye = torch.arange(S + 1, dtype=torch.int32, device=DEV)
+    params = [torch.zeros(shp, device=DEV) for shp in ((13, 13), (13,), (13, 13), (13,), (3, S * 13), (3, 1), (3,), (3,))]
+    with pytest.raises(_lib.WindGNNError) as ei:
+        ops.gcn_gru_forward_csr(eye, eye[:S], torch.ones(S, device=DEV), torch.zeros((1, 1, S, 13), device=DEV),
+                                *params)
+    assert ei.value.code == _lib.WG_ERR_UNSUPPORTED and "dimension too large" in str(ei.value)
+    H = 400     # the wide recurrence's state does not fit shared memory
+    params = [torch.zeros(shp, device=DEV) for shp in ((13, 13), (13,), (13, 13), (13,), (3 * H, 4 * 13), (3 * H, H),
+                                                        (3 * H,), (3 * H,))]
+    with pytest.raises(_lib.WindGNNError) as ei:
+        ops.gcn_gru_forward_host(torch.eye(4, device=DEV), torch.zeros((2, 3, 4, 13)), params)
+    assert ei.value.code == _lib.WG_ERR_UNSUPPORTED and f"GRU hidden size {H}" in str(ei.value)
     bad = _model(7)
     with pytest.raises(RuntimeError):
         bad(torch.eye(7, device=DEV), torch.zeros((2, 3, 9, 13), device=DEV))   # S mismatch

@@ -195,6 +195,9 @@ def test_training_rejects_what_it_does_not_support():
     model = _model(7)
     with pytest.raises(RuntimeError):
         train.forward_train(_adj(7).cpu(), torch.zeros(1, 2, 7, 13), [p.data.cpu() for p in _params(model)])
+    with pytest.raises(_lib.WindGNNError) as ei:   # T = 0 is an invalid argument, not an unsupported shape
+        train.forward_train(_adj(7), torch.zeros(1, 0, 7, 13, device=DEV), [p.data for p in _params(model)])
+    assert ei.value.code == _lib.WG_ERR_BAD_ARG and "non-positive" in str(ei.value)
     lib = _lib.load()
     assert lib.wg_gcn_gru_train_workspace_bytes(4, 8, 7, 13, 32, 13, 21) == 0      # hidden GCN width > 16
     assert "feature widths" in _lib.last_error()

@@ -64,11 +64,11 @@ struct DeviceGuard {
 constexpr size_t kAlign = 256;
 size_t align_up(size_t v) { return (v + kAlign - 1) / kAlign * kAlign; }
 
-// kGcnNone: no dense gcn_kernel instantiation serves the feature widths
-enum GcnKind { kGcnRows, kGcn13x7, kGcn13x4, kGcn16x4, kGcnNone, kGcnSparsePlan, kGcnSparseLanes };
+enum GcnKind { kGcnRows, kGcn13x7, kGcn13x4, kGcn16x4, kGcnSparsePlan, kGcnSparseLanes };
 enum RecurKind { kRecurTc, kRecurUnit, kRecurWide };
 
-// Everything the stages need to agree on: shapes, workspace layout and the kernel of every stage.
+// Everything the stages need to agree on: shapes, workspace layout, the kernel of every stage and the launch geometry
+// that depends only on the shape.
 struct Plan {
     int T, S, Fi, Fh, Fo, H;
     long long chunk;
@@ -81,14 +81,19 @@ struct Plan {
     int n_bias;    // packed bias entries: one per packed w_ih row of either projection, at least 512
     bool sparse;   // CSR graph path: adds the Z scratch of the sparse GCN kernels
     GcnKind gcn;
-    size_t sq_smem;                             // gcn_sparse_plan_kernel: dynamic shared memory,
-    size_t off_sqw, off_sqsteps, off_sqpairs;   // its constant-bank weights and gather plan (steps, pairs)
+    size_t gcn_smem;   // dynamic shared memory of the GCN kernel (the lane kernels: of gcn_sparse_l1_kernel)
+    int gcn_rb;        // gcn_kernel: rows per block
+    int gcn_threads;   // gcn_rows_kernel: block size
+    size_t off_sqw, off_sqsteps, off_sqpairs;   // gcn_sparse_plan_kernel: constant-bank weights, gather plan (steps, pairs)
     bool tc;       // tensor-core input projection (inproj_tc2.cuh): w_ih packed as fp16 hi + lo
     wg::Tc2Shape tc2;
     RecurKind recur;   // small chunks may run gru_recur_regw_kernel instead (launch_recur)
     bool regw;         // the contraction length fits gru_recur_regw_kernel, which then takes small chunks
     bool whu;          // W_hh^T packed for gru_recur_unit_kernel: whenever that kernel serves H, on every path
     int ru_wpg, ru_ht; // gru_recur_unit_kernel: warps per group, compile-time H (102 or 21) or 0
+    int ru_rmax;       // gru_recur_unit_kernel: the largest R (sequences per group) whose shared memory fits
+    int rc_ts;         // gru_recur_kernel: steps of h staged per bulk store (0: every step stored directly)
+    size_t rc_smem;    //                   its dynamic shared memory
     size_t off_wp, off_bias, off_wht, off_whu, off_bhn, off_u, off_gi, off_z, total;
     size_t off_whh_hi, off_whh_lo;   // kRecurTc: W_hh packed as fp16 hi + lo
 };
@@ -105,10 +110,46 @@ long long default_chunk(long long B, size_t bytes_per_seq) {
 }
 
 // gcn_kernel instantiation for the feature widths (the single layer passes F_out as F_hid): the exact 13-wide one
-// with 7 or 4 stations per thread, whichever pads S less (ties: 7), else the generic 16-wide one
+// with 7 or 4 stations per thread, whichever pads S less (ties: 7), else the generic 16-wide one, which
+// dense_gcn_geometry rejects for widths above 16
 GcnKind dense_gcn_kind(int S, int Fi, int Fh, int Fo) {
     if (Fi == 13 && Fh == 13 && Fo == 13) return wg::ceil_div(S, 7) * 7 <= wg::ceil_div(S, 4) * 4 ? kGcn13x7 : kGcn13x4;
-    return Fi <= 16 && Fh <= 16 && Fo <= 16 ? kGcn16x4 : kGcnNone;
+    return kGcn16x4;
+}
+
+// Rows per block and dynamic shared memory of gcn_kernel instantiation k, or the reason why it cannot serve the shape
+// (the single layer passes F_out as F_hid).
+int dense_gcn_geometry(GcnKind k, int S, int Fi, int Fh, int Fo, int& RB, size_t& smem) {
+    const int Fmax = Fi > Fh ? (Fi > Fo ? Fi : Fo) : (Fh > Fo ? Fh : Fo);
+    if (Fmax > 16) return fail(WG_ERR_UNSUPPORTED, "GCN feature width %d > 16 is not built into the dense kernel", Fmax);
+    const int NSG = wg::ceil_div(S, k == kGcn13x7 ? 7 : 4);
+    if (NSG > wg::kGcnThreads)
+        return fail(WG_ERR_UNSUPPORTED, "S=%d too large for the dense GCN kernel", S);
+    auto smem_of = [&](int rb) {
+        const size_t floats = k == kGcn13x7   ? wg::gcn_smem_floats<13, 7>(S, Fmax, rb)
+                              : k == kGcn13x4 ? wg::gcn_smem_floats<13, 4>(S, Fmax, rb)
+                                              : wg::gcn_smem_floats<16, 4>(S, Fmax, rb);
+        return floats * 4;
+    };
+    // rows per block: as many as the 128 threads cover, rounded down so that whole blocks are
+    // 16-byte multiples (bulk-copyable): RB * S * Fi % 4 == 0
+    RB = wg::kGcnThreads / NSG;
+    const int in_cols = S * Fi;
+    const int need = (in_cols % 4 == 0) ? 1 : (in_cols % 2 == 0 ? 2 : 4);
+    if (RB > need) RB -= RB % need;
+    smem = smem_of(RB);
+    // aim for >= 3 resident CTAs per SM when the slabs allow it
+    while (smem > (size_t)wg::kMaxSmemOptin / 3 && RB > 2 * need && RB > 8) {
+        RB -= need > (RB + 7) / 8 ? need : (RB + 7) / 8 / need * need;
+        smem = smem_of(RB);
+    }
+    while (smem > (size_t)wg::kMaxSmemOptin && RB > 1) {
+        RB = RB / 2;
+        smem = smem_of(RB);
+    }
+    if (smem > (size_t)wg::kMaxSmemOptin)
+        return fail(WG_ERR_UNSUPPORTED, "dense GCN needs %zu B of shared memory (S=%d); use the sparse path", smem, S);
+    return WG_OK;
 }
 
 // Testing knob: WG_FORCE_LEGACY=1 runs the fused two-layer GCN on gcn_kernel where gcn_rows_kernel would run, so
@@ -118,8 +159,9 @@ bool force_legacy() {
     return e && e[0] == '1';
 }
 
-int make_plan(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int H, long long chunk,
-              bool sparse = false, int flags = 0) {
+// The shapes, the kernel of every stage and the workspace layout (plan_launch completes the plan).
+int plan_layout(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int H, long long chunk, bool sparse,
+                int flags) {
     if (B < 0 || T <= 0 || S <= 0 || Fi <= 0 || Fh <= 0 || Fo <= 0 || H <= 0 || chunk < 0)
         return fail(WG_ERR_BAD_ARG, "non-positive dimension (B=%lld T=%d S=%d F=%d/%d/%d H=%d chunk=%lld)",
                     B, T, S, Fi, Fh, Fo, H, chunk);
@@ -148,9 +190,9 @@ int make_plan(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int H,
     }
     // GCN: the CSR graph on the second-generation kernel when its weights fit the constant bank and its slab fits
     // shared memory; the dense graph on gcn_rows_kernel when that kernel serves the shape
-    p.sq_smem = wg::gcn_sparse_plan_smem_bytes(S, Fi, Fo);
     if (sparse)
-        p.gcn = Fi <= wg::kSpF && Fo <= wg::kSpF && Fh <= wg::kSqMaxFh && p.sq_smem <= (size_t)wg::kMaxSmemOptin
+        p.gcn = Fi <= wg::kSpF && Fo <= wg::kSpF && Fh <= wg::kSqMaxFh &&
+                        wg::gcn_sparse_plan_smem_bytes(S, Fi, Fo) <= (size_t)wg::kMaxSmemOptin
                     ? kGcnSparsePlan : kGcnSparseLanes;
     else if (wg::gcn_rows_applies(S, Fi, Fh, Fo) && wg::gcn_rows_smem_floats(S) * 4 <= (size_t)wg::kMaxSmemOptin &&
              !force_legacy())
@@ -203,6 +245,62 @@ int make_plan(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int H,
     if (sq) o = align_up(o + wg::sq_plan_bytes(S));
     p.total = o;
     return WG_OK;
+}
+
+// The launch geometry of the plan's kernels that depends only on the shape, and their limits, checked in stage order
+// (GCN, projection, recurrence).  A shape that passes runs every chunk: the checks that grow with the rows take the
+// plan's full chunk, the largest a call runs.
+int plan_launch(Plan& p) {
+    const long long rows = p.chunk * p.T;
+    switch (p.gcn) {
+    case kGcnRows:
+        p.gcn_smem = wg::gcn_rows_smem_floats(p.S) * 4;
+        p.gcn_threads = wg::gcn_rows_warps(p.S) * 32;
+        break;
+    case kGcnSparsePlan: {
+        p.gcn_smem = wg::gcn_sparse_plan_smem_bytes(p.S, p.Fi, p.Fo);
+        // fmajor_to_tiles_kernel: one grid row per 32 rows of whole tiles
+        const long long rt = (rows + wg::kSpThreads - 1) / wg::kSpThreads * wg::kSpThreads;
+        if (rt / 32 > 65535) return fail(WG_ERR_UNSUPPORTED, "sparse GCN: chunk of %lld rows too large", rows);
+        break;
+    }
+    case kGcnSparseLanes:
+        if (p.Fi > wg::kSpF || p.Fo > wg::kSpF)
+            return fail(WG_ERR_UNSUPPORTED, "sparse GCN: F_in / F_out must be <= %d (got %d / %d)", wg::kSpF, p.Fi, p.Fo);
+        p.gcn_smem = ((size_t)2 * p.Fh * wg::kSpF + p.Fh) * 4;
+        if (p.gcn_smem > (size_t)wg::kMaxSmemOptin)
+            return fail(WG_ERR_UNSUPPORTED, "sparse GCN: hidden width %d too large", p.Fh);
+        break;
+    default: {
+        const int rc = dense_gcn_geometry(p.gcn, p.S, p.Fi, p.Fh, p.Fo, p.gcn_rb, p.gcn_smem);
+        if (rc) return rc;
+    }
+    }
+    if (!p.tc && (rows + wg::kIpBM - 1) / wg::kIpBM * (p.NPB / wg::kIpBN) > 0x7fffffffLL)
+        return fail(WG_ERR_UNSUPPORTED, "projection grid too large");
+    if (p.recur == kRecurUnit) {
+        p.ru_rmax = wg::kRuMaxR;
+        while (p.ru_rmax > wg::kRuMinR && wg::recur_u_smem_floats(p.H, p.ru_rmax) * 4 > (size_t)wg::kMaxSmemOptin)
+            --p.ru_rmax;
+    } else if (p.recur == kRecurWide) {
+        // stage h in shared memory for bulk stores when it fits, else store every step directly
+        p.rc_ts = wg::recur_stage_steps(p.H);
+        p.rc_smem = wg::recur_smem_floats(p.KP, p.GP, p.H, p.rc_ts) * 4;
+        if (p.rc_smem > (size_t)wg::kMaxSmemOptin) {
+            p.rc_ts = 0;
+            p.rc_smem = wg::recur_smem_floats(p.KP, p.GP) * 4;
+        }
+        if (p.rc_smem > (size_t)wg::kMaxSmemOptin)
+            return fail(WG_ERR_UNSUPPORTED, "GRU hidden size %d: state does not fit shared memory", p.H);
+    }
+    return WG_OK;
+}
+
+// The whole plan of a forward: every shape it rejects is rejected here, before any launch.
+int make_plan(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int H, long long chunk,
+              bool sparse = false, int flags = 0) {
+    const int rc = plan_layout(p, B, T, S, Fi, Fh, Fo, H, chunk, sparse, flags);
+    return rc ? rc : plan_launch(p);
 }
 
 int check_ws(const void* ws, size_t bytes, size_t need) {
@@ -263,32 +361,11 @@ __global__ void pack_params_kernel(const float* __restrict__ w_ih, const float* 
 // ---------------------------------------------------------------------------------------------
 // stage launchers
 // ---------------------------------------------------------------------------------------------
+// RB, smem: from dense_gcn_geometry
 template <int FP, int SG, bool EXACT, int LAYERS, bool TILED>
 int launch_gcn_t(const float* X, const float* adj, const float* W1, const float* b1, const float* W2,
-                 const float* b2, float* out, long long R, int S, int Fi, int Fh, int Fo, int ldo, cudaStream_t st) {
-    const int NSG = wg::ceil_div(S, SG);
-    if (NSG > wg::kGcnThreads)
-        return fail(WG_ERR_UNSUPPORTED, "S=%d too large for the dense GCN kernel", S);
-    int Fmax = Fi > Fh ? Fi : Fh;
-    if (LAYERS == 2 && Fo > Fmax) Fmax = Fo;
-    // rows per block: as many as the 128 threads cover, rounded down so that whole blocks are
-    // 16-byte multiples (bulk-copyable): RB * S * Fi % 4 == 0
-    int RB = wg::kGcnThreads / NSG;
-    const int in_cols = S * Fi;
-    const int need = (in_cols % 4 == 0) ? 1 : (in_cols % 2 == 0 ? 2 : 4);
-    if (RB > need) RB -= RB % need;
-    size_t smem = wg::gcn_smem_floats<FP, SG>(S, Fmax, RB) * 4;
-    // aim for >= 3 resident CTAs per SM when the slabs allow it
-    while (smem > (size_t)wg::kMaxSmemOptin / 3 && RB > 2 * need && RB > 8) {
-        RB -= need > (RB + 7) / 8 ? need : (RB + 7) / 8 / need * need;
-        smem = wg::gcn_smem_floats<FP, SG>(S, Fmax, RB) * 4;
-    }
-    while (smem > (size_t)wg::kMaxSmemOptin && RB > 1) {
-        RB = RB / 2;
-        smem = wg::gcn_smem_floats<FP, SG>(S, Fmax, RB) * 4;
-    }
-    if (smem > (size_t)wg::kMaxSmemOptin)
-        return fail(WG_ERR_UNSUPPORTED, "dense GCN needs %zu B of shared memory (S=%d); use the sparse path", smem, S);
+                 const float* b2, float* out, long long R, int S, int Fi, int Fh, int Fo, int ldo, int RB, size_t smem,
+                 cudaStream_t st) {
     auto kern = wg::gcn_kernel<FP, SG, EXACT, LAYERS, TILED>;
     WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
@@ -304,33 +381,29 @@ int launch_gcn_t(const float* X, const float* adj, const float* W1, const float*
 }
 
 template <int LAYERS, bool TILED>
-int launch_gcn_dense(GcnKind k, const float* X, const float* adj, const float* W1, const float* b1, const float* W2,
-                     const float* b2, float* out, long long R, int S, int Fi, int Fh, int Fo, int ldo,
-                     cudaStream_t st) {
+int launch_gcn_dense(GcnKind k, int RB, size_t smem, const float* X, const float* adj, const float* W1,
+                     const float* b1, const float* W2, const float* b2, float* out, long long R, int S, int Fi, int Fh,
+                     int Fo, int ldo, cudaStream_t st) {
 #define WG_GCN(FP, SG, EX) \
-    launch_gcn_t<FP, SG, EX, LAYERS, TILED>(X, adj, W1, b1, W2, b2, out, R, S, Fi, Fh, Fo, ldo, st)
+    launch_gcn_t<FP, SG, EX, LAYERS, TILED>(X, adj, W1, b1, W2, b2, out, R, S, Fi, Fh, Fo, ldo, RB, smem, st)
     if (k == kGcn13x7) return WG_GCN(13, 7, true);
     if (k == kGcn13x4) return WG_GCN(13, 4, true);
-    if (k == kGcn16x4) return WG_GCN(16, 4, false);
+    return WG_GCN(16, 4, false);
 #undef WG_GCN
-    const int fmax = Fi > Fh ? (Fi > Fo ? Fi : Fo) : (Fh > Fo ? Fh : Fo);
-    return fail(WG_ERR_UNSUPPORTED, "GCN feature width %d > 16 is not built into the dense kernel", fmax);
 }
 
 // second-generation fused two-layer kernel (gcn_rows.cuh): lane = row, output straight into the tiles
-int launch_gcn_rows(const float* X, const float* adj, const float* W1, const float* b1, const float* W2,
-                    const float* b2, float* out, long long R, int S, int ldo, cudaStream_t st) {
-    const size_t smem = wg::gcn_rows_smem_floats(S) * 4;
-    const int threads = wg::gcn_rows_warps(S) * 32;
-    WG_CUDA(cudaFuncSetAttribute(wg::gcn_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+int launch_gcn_rows(const Plan& p, const float* X, const float* adj, const float* W1, const float* b1,
+                    const float* W2, const float* b2, float* out, long long R, cudaStream_t st) {
+    WG_CUDA(cudaFuncSetAttribute(wg::gcn_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.gcn_smem));
     int per_sm = 0;
-    WG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wg::gcn_rows_kernel, threads, smem));
+    WG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wg::gcn_rows_kernel, p.gcn_threads, p.gcn_smem));
     if (per_sm < 1) per_sm = 1;
     const long long nblocks = (R + wg::kGrRows - 1) / wg::kGrRows;
     long long grid = (long long)wg::kNumSMs * per_sm;
     if (grid > nblocks) grid = nblocks;
     if (grid < 1) return WG_OK;
-    wg::gcn_rows_kernel<<<(unsigned)grid, threads, smem, st>>>(X, adj, W1, b1, W2, b2, out, R, S, ldo);
+    wg::gcn_rows_kernel<<<(unsigned)grid, p.gcn_threads, p.gcn_smem, st>>>(X, adj, W1, b1, W2, b2, out, R, p.S, p.IP);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
@@ -345,23 +418,21 @@ struct Graph {
 
 int launch_gcn_sparse(const Plan& p, void* ws, const Graph& g, const float* x, const float* w1, const float* b1,
                       const float* w2, const float* b2, long long rows, cudaStream_t st) {
-    if (p.Fi > wg::kSpF || p.Fo > wg::kSpF)
-        return fail(WG_ERR_UNSUPPORTED, "sparse GCN: F_in / F_out must be <= %d (got %d / %d)", wg::kSpF, p.Fi, p.Fo);
-    if (p.gcn == kGcnSparsePlan && rows >= 1) {   // constant-bank weights + gather plan (prepare_sparse ran)
+    if (rows < 1) return WG_OK;
+    if (p.gcn == kGcnSparsePlan) {   // constant-bank weights + gather plan (prepare_sparse ran)
         const bool narrow = p.Fi <= 13 && p.Fo <= 13, exact = p.Fi == 13 && p.Fo == 13;
         auto kern = exact ? wg::gcn_sparse_plan_kernel<13, true>
                           : narrow ? wg::gcn_sparse_plan_kernel<13, false> : wg::gcn_sparse_plan_kernel<16, false>;
-        WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.sq_smem));
+        WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.gcn_smem));
         const unsigned grid = (unsigned)(rows < wg::kNumSMs ? rows : wg::kNumSMs);
         float* urow = ws_ptr<float>(ws, p.off_z);   // [rows][Fo][S] f-major U, then gridDim per-CTA Z rows
         float* zscr = urow + (size_t)rows * p.S * p.Fo;
-        kern<<<grid, wg::kSqThreads, p.sq_smem, st>>>(x, g.rowptr, g.colidx, g.vals, ws_ptr<int>(ws, p.off_sqsteps),
-                                                      ws_ptr<int2>(ws, p.off_sqpairs), zscr, urow, rows, p.S, p.Fi,
-                                                      p.Fh, p.Fo);
+        kern<<<grid, wg::kSqThreads, p.gcn_smem, st>>>(x, g.rowptr, g.colidx, g.vals, ws_ptr<int>(ws, p.off_sqsteps),
+                                                       ws_ptr<int2>(ws, p.off_sqpairs), zscr, urow, rows, p.S, p.Fi,
+                                                       p.Fh, p.Fo);
         WG_CUDA(cudaGetLastError());
         const long long rt = (rows + wg::kSpThreads - 1) / wg::kSpThreads * wg::kSpThreads;  // whole tiles (zero rows)
         const dim3 tg((unsigned)((p.S + 31) / 32), (unsigned)(rt / 32));
-        if (tg.y > 65535u) return fail(WG_ERR_UNSUPPORTED, "sparse GCN: chunk of %lld rows too large", rows);
         const size_t tsmem = wg::fmajor_to_tiles_smem_bytes(p.Fo);
         WG_CUDA(cudaFuncSetAttribute(wg::fmajor_to_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsmem));
         wg::fmajor_to_tiles_kernel<<<tg, 256, tsmem, st>>>(urow, ws_ptr<float>(ws, p.off_u), rows, p.S, p.Fo, p.IP);
@@ -370,21 +441,18 @@ int launch_gcn_sparse(const Plan& p, void* ws, const Graph& g, const float* x, c
     }
     // gcn_sparse_plan_kernel does not apply (hidden width above its constant bank, or a slab too large for
     // shared memory): the two lane = row kernels
-    const size_t smem = ((size_t)2 * p.Fh * wg::kSpF + p.Fh) * 4;
-    if (smem > (size_t)wg::kMaxSmemOptin)
-        return fail(WG_ERR_UNSUPPORTED, "sparse GCN: hidden width %d too large", p.Fh);
     const long long tiles = (rows + wg::kSpThreads - 1) / wg::kSpThreads;
-    if (tiles < 1) return WG_OK;
     // split the stations so that the grid fills the machine a few times over
     int chunks = (int)((4LL * wg::kNumSMs * 4 + tiles - 1) / tiles);
     if (chunks < 1) chunks = 1;
     if (chunks > p.S) chunks = p.S;
     const int s_chunk = (p.S + chunks - 1) / chunks;
     const dim3 grid((unsigned)tiles, (unsigned)((p.S + s_chunk - 1) / s_chunk));
-    WG_CUDA(cudaFuncSetAttribute(wg::gcn_sparse_l1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    wg::gcn_sparse_l1_kernel<<<grid, wg::kSpThreads, smem, st>>>(x, g.rowptr, g.colidx, g.vals, w1, b1, w2,
-                                                                ws_ptr<float>(ws, p.off_z), rows, p.S, p.Fi, p.Fh,
-                                                                p.Fo, s_chunk);
+    WG_CUDA(cudaFuncSetAttribute(wg::gcn_sparse_l1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)p.gcn_smem));
+    wg::gcn_sparse_l1_kernel<<<grid, wg::kSpThreads, p.gcn_smem, st>>>(x, g.rowptr, g.colidx, g.vals, w1, b1, w2,
+                                                                       ws_ptr<float>(ws, p.off_z), rows, p.S, p.Fi,
+                                                                       p.Fh, p.Fo, s_chunk);
     WG_CUDA(cudaGetLastError());
     wg::gcn_sparse_l2_kernel<<<grid, wg::kSpThreads, 0, st>>>(ws_ptr<float>(ws, p.off_z), g.rowptr, g.colidx, g.vals,
                                                              b2, ws_ptr<float>(ws, p.off_u), rows, p.S, p.Fo, p.IP,
@@ -397,9 +465,10 @@ int launch_gcn_sparse(const Plan& p, void* ws, const Graph& g, const float* x, c
 int launch_gcn(const Plan& p, void* ws, const Graph& g, const float* x, const float* w1, const float* b1,
                const float* w2, const float* b2, long long rows, cudaStream_t st) {
     float* u = ws_ptr<float>(ws, p.off_u);
-    if (p.gcn == kGcnRows) return launch_gcn_rows(x, g.adj, w1, b1, w2, b2, u, rows, p.S, p.IP, st);
+    if (p.gcn == kGcnRows) return launch_gcn_rows(p, x, g.adj, w1, b1, w2, b2, u, rows, st);
     if (p.sparse) return launch_gcn_sparse(p, ws, g, x, w1, b1, w2, b2, rows, st);
-    return launch_gcn_dense<2, true>(p.gcn, x, g.adj, w1, b1, w2, b2, u, rows, p.S, p.Fi, p.Fh, p.Fo, p.IP, st);
+    return launch_gcn_dense<2, true>(p.gcn, p.gcn_rb, p.gcn_smem, x, g.adj, w1, b1, w2, b2, u, rows, p.S, p.Fi, p.Fh,
+                                     p.Fo, p.IP, st);
 }
 
 int launch_inproj_tc(const Plan& p, void* ws, long long rows, cudaStream_t st) {
@@ -423,7 +492,6 @@ int launch_inproj(const Plan& p, void* ws, long long rows, cudaStream_t st) {
     const int n_tiles = p.NPB / wg::kIpBN;
     const long long grid = m_tiles * n_tiles;
     if (grid < 1) return WG_OK;
-    if (grid > 0x7fffffffLL) return fail(WG_ERR_UNSUPPORTED, "projection grid too large");
     WG_CUDA(cudaFuncSetAttribute(wg::inproj_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  wg::kIpSmemBytes));
     wg::inproj_kernel<<<(unsigned)grid, wg::kIpThreads, wg::kIpSmemBytes, st>>>(
@@ -435,21 +503,12 @@ int launch_inproj(const Plan& p, void* ws, long long rows, cudaStream_t st) {
 
 // FP32 recurrence of the hidden sizes gru_recur_unit_kernel cannot fit (H = 125 .. 360): W_hh^T read through L1 / L2
 int launch_recur_wide(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st) {
-    // stage h in shared memory for bulk stores when it fits, else store every step directly
-    int TS = wg::recur_stage_steps(p.H);
-    size_t smem = wg::recur_smem_floats(p.KP, p.GP, p.H, TS) * 4;
-    if (smem > (size_t)wg::kMaxSmemOptin) {
-        TS = 0;
-        smem = wg::recur_smem_floats(p.KP, p.GP) * 4;
-    }
-    if (smem > (size_t)wg::kMaxSmemOptin)
-        return fail(WG_ERR_UNSUPPORTED, "GRU hidden size %d: state does not fit shared memory", p.H);
-    WG_CUDA(cudaFuncSetAttribute(wg::gru_recur_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    WG_CUDA(cudaFuncSetAttribute(wg::gru_recur_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.rc_smem));
     const long long grid = (Bc + wg::kRcBT - 1) / wg::kRcBT;
     if (grid < 1) return WG_OK;
-    wg::gru_recur_kernel<<<(unsigned)grid, wg::kRcWarps * 32, smem, st>>>(
+    wg::gru_recur_kernel<<<(unsigned)grid, wg::kRcWarps * 32, p.rc_smem, st>>>(
         ws_ptr<float>(ws, p.off_gi), ws_ptr<float>(ws, p.off_wht), ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H,
-        p.GP, p.KP, p.NPR, TS);
+        p.GP, p.KP, p.NPR, p.rc_ts);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
@@ -547,9 +606,8 @@ bool regw_serves(const Plan& p, long long Bc) {
 int launch_recur(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
     if (regw_serves(p, Bc)) return launch_recur_regw(p, ws, out, Bc, Bc >= 4 ? 4 : (int)Bc, st, gsave, ldsave);
     if (p.recur == kRecurUnit) {
-        int r = recur_u_pick_r(Bc, wg::kRuWarps / p.ru_wpg);
-        while (r > wg::kRuMinR && wg::recur_u_smem_floats(p.H, r) * 4 > (size_t)wg::kMaxSmemOptin) --r;
-        return launch_recur_unit(p, ws, out, Bc, r, st, gsave, ldsave);
+        const int r = recur_u_pick_r(Bc, wg::kRuWarps / p.ru_wpg);
+        return launch_recur_unit(p, ws, out, Bc, r < p.ru_rmax ? r : p.ru_rmax, st, gsave, ldsave);
     }
     if (p.recur == kRecurTc) return launch_recur_tc(p, ws, out, Bc, st);   // the tensor path: every batch size
     return launch_recur_wide(p, ws, out, Bc, st);
@@ -764,7 +822,7 @@ constexpr int kTrainMaxH = 106;
 
 int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, int Fo, int H) {
     const long long Bn = B > 0 ? B : 1;   // B = 0 plans one sequence: the backward then only zeroes the gradients
-    int rc = make_plan(tp.f, B, T, S, Fi, Fh, Fo, H, Bn, false, 0);
+    int rc = plan_layout(tp.f, B, T, S, Fi, Fh, Fo, H, Bn, false, 0);
     if (rc) return rc;
     const Plan& p = tp.f;
     if (Fi > 16 || Fh > 16 || Fo > 16)
@@ -864,7 +922,7 @@ int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, in
     if ((size_t)tp.splits_ih * p.I * tp.nt_ih * wg::KbWih::kBN > sk) sk = (size_t)tp.splits_ih * p.I * tp.nt_ih * wg::KbWih::kBN;
     tp.off_splitk = o; o = align_up(o + sk * 4);
     tp.total = o;
-    return WG_OK;
+    return plan_launch(tp.f);   // last: a shape outside the training limits reports those
 }
 
 bool aligned16(const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; }
@@ -1159,8 +1217,13 @@ int wg_gcn_layer_f32(const float* adj, const float* attr, const float* weight, c
     DeviceGuard g(device);
     WG_CUDA(g.err);
     // single layer: "hidden" plays the role of the output width
-    return launch_gcn_dense<1, false>(dense_gcn_kind(S, F_in, F_out, F_out), attr, adj, weight, bias, nullptr, nullptr,
-                                      out, R, S, F_in, F_out, F_out, S * F_out, static_cast<cudaStream_t>(stream));
+    const GcnKind k = dense_gcn_kind(S, F_in, F_out, F_out);
+    int RB = 0;
+    size_t smem = 0;
+    const int rc = dense_gcn_geometry(k, S, F_in, F_out, F_out, RB, smem);
+    if (rc) return rc;
+    return launch_gcn_dense<1, false>(k, RB, smem, attr, adj, weight, bias, nullptr, nullptr, out, R, S, F_in, F_out,
+                                      F_out, S * F_out, static_cast<cudaStream_t>(stream));
 }
 
 

@@ -114,10 +114,8 @@ def gcn_gru_forward(
     out = torch.empty((B, T, H), dtype=torch.float32, device=dev)
     if B == 0 or T == 0:
         return out
+    # 0 bytes: the shape is rejected, and the call below returns the library's code and reason without launching
     nbytes = lib.wg_gcn_gru_workspace_bytes(B, T, S, F_in, F_hid, F_out, H, chunk, flags)
-    if nbytes == 0:
-        raise _lib.WindGNNError(_lib.WG_ERR_UNSUPPORTED if "tensor-core" in _lib.last_error() else _lib.WG_ERR_BAD_ARG,
-                                _lib.last_error())
     ws = _workspace(dev, nbytes)
     stream = torch.cuda.current_stream(dev).cuda_stream
     _lib.check(
@@ -180,10 +178,7 @@ def gcn_gru_forward_csr(
     out = torch.empty((B, T, H), dtype=torch.float32, device=dev)
     if B == 0 or T == 0:
         return out
-    nbytes = lib.wg_gcn_gru_csr_workspace_bytes(B, T, S, F_in, F_hid, F_out, H, chunk, flags)
-    if nbytes == 0:
-        raise _lib.WindGNNError(_lib.WG_ERR_UNSUPPORTED if "tensor-core" in _lib.last_error() else _lib.WG_ERR_BAD_ARG,
-                                _lib.last_error())
+    nbytes = lib.wg_gcn_gru_csr_workspace_bytes(B, T, S, F_in, F_hid, F_out, H, chunk, flags)  # 0: see gcn_gru_forward
     ws = _workspace(dev, nbytes)
     stream = torch.cuda.current_stream(dev).cuda_stream
     _lib.check(
@@ -267,9 +262,7 @@ def gcn_gru_forward_host(adj, x_host, params, out_host=None, chunk: int = 0, dev
         raise RuntimeError(f"out_host must be a contiguous float32 CPU tensor {list(shape)}")
     if B == 0:
         return out_host
-    nbytes = lib.wg_gcn_gru_host_workspace_bytes(B, T, S, F_in, F_hid, F_out, H, chunk, flags)
-    if nbytes == 0:
-        raise _lib.WindGNNError(_lib.WG_ERR_BAD_ARG, _lib.last_error())
+    nbytes = lib.wg_gcn_gru_host_workspace_bytes(B, T, S, F_in, F_hid, F_out, H, chunk, flags)  # 0: see gcn_gru_forward
     ws = _workspace(dev, nbytes, "host")
     torch.cuda.current_stream(dev).synchronize()  # parameters / adj may have been produced on it
     ptrs = (adj.data_ptr(), x_host.data_ptr(), w1.data_ptr(), b1.data_ptr(), w2.data_ptr(), b2.data_ptr(),

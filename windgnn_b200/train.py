@@ -50,14 +50,12 @@ def forward_train(adj, x, params: Sequence[torch.Tensor]):
     params = [_require_cuda_f32(n, p, dev) for n, p in zip(PARAM_NAMES, params)]
     B, T, S, F_in, F_hid, F_out, H = _dims(adj, x, *params)
     out = torch.empty((B, T, H), dtype=torch.float32, device=dev)
+    # 0 bytes: the shape is rejected, and the call below returns the library's code and reason without launching
     nbytes = lib.wg_gcn_gru_train_workspace_bytes(B, T, S, F_in, F_hid, F_out, H)
-    if nbytes == 0:
-        raise _lib.WindGNNError(_lib.WG_ERR_UNSUPPORTED, _lib.last_error())
     ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-    if B > 0 and T > 0:
-        _lib.check(lib.wg_gcn_gru_forward_train_f32(
-            adj.data_ptr(), x.data_ptr(), *(p.data_ptr() for p in params), out.data_ptr(),
-            B, T, S, F_in, F_hid, F_out, H, ws.data_ptr(), ws.numel(), dev.index or 0, _stream(dev)))
+    _lib.check(lib.wg_gcn_gru_forward_train_f32(
+        adj.data_ptr(), x.data_ptr(), *(p.data_ptr() for p in params), out.data_ptr(),
+        B, T, S, F_in, F_hid, F_out, H, ws.data_ptr(), ws.numel(), dev.index or 0, _stream(dev)))
     return out, ws
 
 
