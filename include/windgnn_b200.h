@@ -101,6 +101,41 @@ int wg_gcn_gru_forward_csr_f32(const int32_t* rowptr, const int32_t* colidx, con
                                int F_hid, int F_out, int H, int64_t chunk, int flags, void* workspace,
                                size_t workspace_bytes, int device, void* stream);
 
+/* Rolling forecasts from one table — every window's last hidden state, without materialising the windows.
+ * Stands in for the reference's windowing (src/step4_sequence_preparer.py:7-27) followed by its evaluation
+ * (src/main.py:101-116, which reads the last timestep of each window), for windows that may overlap:
+ *   table  [Ttot, S, F_in]  device: the pivoted table (wg_pivot_table_f32)
+ *   starts int64 [N]        HOST: window n is table[starts[n] : starts[n] + L]; any order, repeats allowed
+ *   out    [N, H]           device: out[n] = h_{L-1} of window n
+ * out[n] is bit-identical to out[n, L-1, :] of wg_gcn_gru_forward_f32 (same flags) on the materialised window:
+ * GCN and input projection depend only on a table row, so they run once per row of [min start, max start + L),
+ * in pieces of at most chunk * L rows, and each window's recurrence (h0 = 0) reads its L rows of input-gate values in
+ * place, on the kernel the forward would choose for the same N and chunk.
+ *
+ * The shapes, chunk and flags are planned as for the forward with T = L and B = N, and rejected with the
+ * forward's code and text; the workspace query also returns 0 for N < 0, L < 1 and L > Ttot.  N == 0 returns
+ * WG_OK.  The entry point validates `starts` before it looks at the workspace: NULL (N > 0) or a start outside
+ * [0, Ttot - L] returns WG_ERR_BAD_ARG naming the window and the value.  The starts are copied to the
+ * workspace on `stream` before the call returns, so the caller may reuse the array at once.
+ * Workspace: the forward's packed parameters and U scratch of one piece, input-gate values of up to Ttot
+ * rows (Ttot * 3H floats, rounded up), N int64 starts. */
+size_t wg_gcn_gru_forecast_workspace_bytes(int64_t N, int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out,
+                                           int H, int64_t chunk, int flags);
+int wg_gcn_gru_forecast_f32(const float* adj, const float* table, const int64_t* starts, const float* w1,
+                            const float* b1, const float* w2, const float* b2, const float* w_ih, const float* w_hh,
+                            const float* b_ih, const float* b_hh, float* out, int64_t N, int64_t Ttot, int L, int S,
+                            int F_in, int F_hid, int F_out, int H, int64_t chunk, int flags, void* workspace,
+                            size_t workspace_bytes, int device, void* stream);
+/* The same with the adjacency as CSR (rowptr, colidx, vals as for wg_gcn_gru_forward_csr_f32). */
+size_t wg_gcn_gru_forecast_csr_workspace_bytes(int64_t N, int64_t Ttot, int L, int S, int F_in, int F_hid,
+                                               int F_out, int H, int64_t chunk, int flags);
+int wg_gcn_gru_forecast_csr_f32(const int32_t* rowptr, const int32_t* colidx, const float* vals, const float* table,
+                                const int64_t* starts, const float* w1, const float* b1, const float* w2,
+                                const float* b2, const float* w_ih, const float* w_hh, const float* b_ih,
+                                const float* b_hh, float* out, int64_t N, int64_t Ttot, int L, int S, int F_in,
+                                int F_hid, int F_out, int H, int64_t chunk, int flags, void* workspace,
+                                size_t workspace_bytes, int device, void* stream);
+
 /* Same computation with HOST buffers for x (pinned for full overlap) and out: the batch is
  * streamed through the device in `chunk`-sized pieces, H2D copy / compute / D2H copy of
  * consecutive pieces overlapped on internal streams (two compute lanes, so the latency-bound

@@ -5,6 +5,7 @@ Public surface (mirrors the reference's step5/step6 modules and step2 graph buil
     GCN_GRU, GraphConvLayer      drop-in nn.Modules (windgnn_b200.model)
     build_graph, knn_graph, ...  bit-exact graph build on the GPU (windgnn_b200.graph)
     ops.gcn_gru_forward, ...     torch custom ops over the C-ABI (windgnn_b200.ops)
+    window_starts, forecast_targets  rolling-forecast windows for GCN_GRU.forecast (windgnn_b200.sequences)
 
 CUDA only.  ``import windgnn_b200`` works without a GPU (so that the package can be built and
 its host logic tested), but every compute call raises unless the in-tree library is built and a
@@ -24,7 +25,14 @@ from .graph import (  # noqa: F401
     synthetic_coordinates,
 )
 
-from .sequences import create_sequences, denormalise_last_step, num_windows, pivot_long_table  # noqa: F401
+from .sequences import (  # noqa: F401
+    create_sequences,
+    denormalise_last_step,
+    forecast_targets,
+    num_windows,
+    pivot_long_table,
+    window_starts,
+)
 
 __all__ = [
     "pivot_long_table",
@@ -34,6 +42,8 @@ __all__ = [
     "create_sequences",
     "denormalise_last_step",
     "num_windows",
+    "window_starts",
+    "forecast_targets",
     "GCN_GRU",
     "GraphConvLayer",
     "build_graph",

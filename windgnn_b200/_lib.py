@@ -41,6 +41,13 @@ _SIGNATURES = {
     "wg_gcn_gru_forward_f32": (c_int, [_P] * 11 + [c_int64, *_DIMS, c_int64, c_int, _P, c_size_t, c_int, _P]),
     "wg_gcn_gru_csr_workspace_bytes": (c_size_t, [c_int64, *_DIMS, c_int64, c_int]),
     "wg_gcn_gru_forward_csr_f32": (c_int, [_P] * 13 + [c_int64, *_DIMS, c_int64, c_int, _P, c_size_t, c_int, _P]),
+    # N, Ttot, then the dims with T = L
+    "wg_gcn_gru_forecast_workspace_bytes": (c_size_t, [c_int64, c_int64, *_DIMS, c_int64, c_int]),
+    "wg_gcn_gru_forecast_f32": (c_int, [_P] * 12 + [c_int64, c_int64, *_DIMS, c_int64, c_int, _P, c_size_t, c_int,
+                                                    _P]),
+    "wg_gcn_gru_forecast_csr_workspace_bytes": (c_size_t, [c_int64, c_int64, *_DIMS, c_int64, c_int]),
+    "wg_gcn_gru_forecast_csr_f32": (c_int, [_P] * 14 + [c_int64, c_int64, *_DIMS, c_int64, c_int, _P, c_size_t,
+                                                        c_int, _P]),
     "wg_gcn_gru_host_workspace_bytes": (c_size_t, [c_int64, *_DIMS, c_int64, c_int]),
     "wg_gcn_gru_forward_host_f32": (c_int, [_P] * 11 + [c_int64, *_DIMS, c_int64, c_int, _P, c_size_t, c_int]),
     "wg_gcn_gru_predict_host_f32": (c_int, [_P] * 11 + [c_int64, *_DIMS, c_int64, c_int, c_double, c_double, _P,

@@ -9,6 +9,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
+#include <vector>
 
 #include "gcn.cuh"
 #include "gcn_bwd.cuh"
@@ -159,9 +160,17 @@ bool force_legacy() {
     return e && e[0] == '1';
 }
 
+// Table rows per GCN + projection piece of a forecast: a chunk of windows' worth, at most the table.
+long long forecast_piece_rows(const Plan& p, long long Ttot) {
+    const long long r = p.chunk * p.T;
+    return r < Ttot ? r : Ttot;
+}
+
 // The shapes, the kernel of every stage and the workspace layout (plan_launch completes the plan).
+// table_rows > 0 (the forecast): GI holds that many rows, and the GCN / projection scratch (U, Z) pieces of
+// forecast_piece_rows rows instead of a chunk's.
 int plan_layout(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int H, long long chunk, bool sparse,
-                int flags) {
+                int flags, long long table_rows = 0) {
     if (B < 0 || T <= 0 || S <= 0 || Fi <= 0 || Fh <= 0 || Fo <= 0 || H <= 0 || chunk < 0)
         return fail(WG_ERR_BAD_ARG, "non-positive dimension (B=%lld T=%d S=%d F=%d/%d/%d H=%d chunk=%lld)",
                     B, T, S, Fi, Fh, Fo, H, chunk);
@@ -228,11 +237,12 @@ int plan_layout(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int 
     const bool tc_recur = p.recur == kRecurTc;
     p.off_whh_hi = o; if (tc_recur) o = align_up(o + wg::recur_tc_w_halves(H) * 2);
     p.off_whh_lo = o; if (tc_recur) o = align_up(o + wg::recur_tc_w_halves(H) * 2);
-    const size_t rows = (size_t)p.chunk * T;
+    const size_t rows = table_rows > 0 ? (size_t)forecast_piece_rows(p, table_rows) : (size_t)p.chunk * T;
     const size_t rows_tiled = (rows + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows;
     p.off_u = o;    o = align_up(o + rows_tiled * p.IP * 4);  // K-major 128-row tiles
     // GI: the tensor-core recurrence reads whole groups of kRtSeqs sequences (rows past the batch are scratch)
-    const size_t rows_gi = (size_t)((p.chunk + wg::kRtSeqs - 1) / wg::kRtSeqs * wg::kRtSeqs) * T;
+    const size_t rows_gi =
+        table_rows > 0 ? (size_t)table_rows : (size_t)((p.chunk + wg::kRtSeqs - 1) / wg::kRtSeqs * wg::kRtSeqs) * T;
     p.off_gi = o;   o = align_up(o + rows_gi * p.GP * 4);
     // sparse path scratch: row-major U (rows x S*Fo) + one [Fo][S] row per resident CTA
     p.off_z = o;    if (sparse) o = align_up(o + (rows + wg::kNumSMs) * (size_t)S * Fo * 4);
@@ -471,7 +481,8 @@ int launch_gcn(const Plan& p, void* ws, const Graph& g, const float* x, const fl
                                      p.Fo, p.IP, st);
 }
 
-int launch_inproj_tc(const Plan& p, void* ws, long long rows, cudaStream_t st) {
+// The projection of the `rows` U rows into GI rows gi[0 .. rows) (row stride p.GP).
+int launch_inproj_tc(const Plan& p, void* ws, long long rows, cudaStream_t st, float* gi) {
     const long long m_tiles = (rows + wg::kT2BM - 1) / wg::kT2BM;
     if (m_tiles < 1) return WG_OK;
     const wg::Tc2Shape& t = p.tc2;
@@ -480,14 +491,14 @@ int launch_inproj_tc(const Plan& p, void* ws, long long rows, cudaStream_t st) {
     const long long tiles = m_tiles * t.n_nt;
     const unsigned grid = (unsigned)(tiles < wg::kNumSMs ? tiles : wg::kNumSMs);
     wg::inproj_tc2_kernel<<<grid, wg::kT2Threads, t.smem_bytes, st>>>(
-        ws_ptr<float>(ws, p.off_u), ws_ptr<__half>(ws, p.off_wp), ws_ptr<float>(ws, p.off_bias),
-        ws_ptr<float>(ws, p.off_gi), rows, p.IP, t.KP, p.GP, t.n_nt, t.N_each, t.stages);
+        ws_ptr<float>(ws, p.off_u), ws_ptr<__half>(ws, p.off_wp), ws_ptr<float>(ws, p.off_bias), gi, rows, p.IP,
+        t.KP, p.GP, t.n_nt, t.N_each, t.stages);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
 
-int launch_inproj(const Plan& p, void* ws, long long rows, cudaStream_t st) {
-    if (p.tc) return launch_inproj_tc(p, ws, rows, st);
+int launch_inproj(const Plan& p, void* ws, long long rows, cudaStream_t st, float* gi) {
+    if (p.tc) return launch_inproj_tc(p, ws, rows, st, gi);
     const long long m_tiles = (rows + wg::kIpBM - 1) / wg::kIpBM;
     const int n_tiles = p.NPB / wg::kIpBN;
     const long long grid = m_tiles * n_tiles;
@@ -495,20 +506,25 @@ int launch_inproj(const Plan& p, void* ws, long long rows, cudaStream_t st) {
     WG_CUDA(cudaFuncSetAttribute(wg::inproj_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  wg::kIpSmemBytes));
     wg::inproj_kernel<<<(unsigned)grid, wg::kIpThreads, wg::kIpSmemBytes, st>>>(
-        ws_ptr<float>(ws, p.off_u), ws_ptr<float>(ws, p.off_wp), ws_ptr<float>(ws, p.off_bias),
-        ws_ptr<float>(ws, p.off_gi), rows, p.IP, p.GP, n_tiles);
+        ws_ptr<float>(ws, p.off_u), ws_ptr<float>(ws, p.off_wp), ws_ptr<float>(ws, p.off_bias), gi, rows, p.IP, p.GP,
+        n_tiles);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
 
+// The recurrence launchers take row0 = NULL for a chunk of sequences laid out one after another in GI (the
+// forward), or the device array of each window's first GI row (the forecast: the windowed instantiations, which
+// store only h at the last step, out [Bc][H]).
+
 // FP32 recurrence of the hidden sizes gru_recur_unit_kernel cannot fit (H = 125 .. 360): W_hh^T read through L1 / L2
-int launch_recur_wide(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st) {
-    WG_CUDA(cudaFuncSetAttribute(wg::gru_recur_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.rc_smem));
+int launch_recur_wide(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, const long long* row0) {
+    auto kern = row0 ? wg::gru_recur_kernel<true> : wg::gru_recur_kernel<false>;
+    WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.rc_smem));
     const long long grid = (Bc + wg::kRcBT - 1) / wg::kRcBT;
     if (grid < 1) return WG_OK;
-    wg::gru_recur_kernel<<<(unsigned)grid, wg::kRcWarps * 32, p.rc_smem, st>>>(
-        ws_ptr<float>(ws, p.off_gi), ws_ptr<float>(ws, p.off_wht), ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H,
-        p.GP, p.KP, p.NPR, p.rc_ts);
+    kern<<<(unsigned)grid, wg::kRcWarps * 32, p.rc_smem, st>>>(ws_ptr<float>(ws, p.off_gi), ws_ptr<float>(ws, p.off_wht),
+                                                              ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H, p.GP,
+                                                              p.KP, p.NPR, row0 ? 0 : p.rc_ts, row0);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
@@ -528,44 +544,48 @@ int recur_u_pick_r(long long Bc, int ngrp) {
 }
 
 using RegwKernel = decltype(&wg::gru_recur_regw_kernel<false, 1, 24>);
-template <bool SAVE, int KPT>
+template <bool SAVE, int KPT, bool WIN = false>
 RegwKernel regw_kernel(int nb) {
-    const RegwKernel k[4] = {wg::gru_recur_regw_kernel<SAVE, 1, KPT>, wg::gru_recur_regw_kernel<SAVE, 2, KPT>,
-                             wg::gru_recur_regw_kernel<SAVE, 3, KPT>, wg::gru_recur_regw_kernel<SAVE, 4, KPT>};
+    const RegwKernel k[4] = {wg::gru_recur_regw_kernel<SAVE, 1, KPT, WIN>, wg::gru_recur_regw_kernel<SAVE, 2, KPT, WIN>,
+                             wg::gru_recur_regw_kernel<SAVE, 3, KPT, WIN>, wg::gru_recur_regw_kernel<SAVE, 4, KPT, WIN>};
     return k[nb - 1];
 }
 int launch_recur_regw(const Plan& p, void* ws, float* out, long long Bc, int nb, cudaStream_t st, float* gsave,
-                      int ldsave) {
+                      int ldsave, const long long* row0) {
     if (Bc < 1) return WG_OK;
-    const RegwKernel kern = gsave ? (p.KP == 104 ? regw_kernel<true, 104>(nb) : regw_kernel<true, 24>(nb))
-                                  : (p.KP == 104 ? regw_kernel<false, 104>(nb) : regw_kernel<false, 24>(nb));
+    const RegwKernel kern =
+        row0    ? (p.KP == 104 ? regw_kernel<false, 104, true>(nb) : regw_kernel<false, 24, true>(nb))
+        : gsave ? (p.KP == 104 ? regw_kernel<true, 104>(nb) : regw_kernel<true, 24>(nb))
+                : (p.KP == 104 ? regw_kernel<false, 104>(nb) : regw_kernel<false, 24>(nb));
     const size_t smem = wg::recur_regw_smem_floats(p.KP, p.NPR, p.GP) * 4;
     WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const long long grid = (Bc + wg::kRsBT - 1) / wg::kRsBT;
     kern<<<(unsigned)grid, wg::kRwThreads, smem, st>>>(ws_ptr<float>(ws, p.off_gi), ws_ptr<float>(ws, p.off_wht),
                                                       ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H, p.GP, p.NPR,
-                                                      gsave, ldsave);
+                                                      gsave, ldsave, row0);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
 
 using UnitKernel = decltype(&wg::gru_recur_unit_kernel<4, 1, false, 0>);
-template <int WPG, bool SAVE, int HT>
+template <int WPG, bool SAVE, int HT, bool WIN>
 UnitKernel unit_kernel(int r) {
-    const UnitKernel k[5] = {wg::gru_recur_unit_kernel<4, WPG, SAVE, HT>, wg::gru_recur_unit_kernel<5, WPG, SAVE, HT>,
-                             wg::gru_recur_unit_kernel<6, WPG, SAVE, HT>, wg::gru_recur_unit_kernel<7, WPG, SAVE, HT>,
-                             wg::gru_recur_unit_kernel<8, WPG, SAVE, HT>};
+    const UnitKernel k[5] = {
+        wg::gru_recur_unit_kernel<4, WPG, SAVE, HT, WIN>, wg::gru_recur_unit_kernel<5, WPG, SAVE, HT, WIN>,
+        wg::gru_recur_unit_kernel<6, WPG, SAVE, HT, WIN>, wg::gru_recur_unit_kernel<7, WPG, SAVE, HT, WIN>,
+        wg::gru_recur_unit_kernel<8, WPG, SAVE, HT, WIN>};
     return k[r - wg::kRuMinR];
 }
-template <bool SAVE>
+template <bool SAVE, bool WIN = false>
 UnitKernel unit_kernel(const Plan& p, int r) {
-    if (p.ru_ht == 102) return unit_kernel<2, SAVE, 102>(r);
-    if (p.ru_ht == 21) return unit_kernel<1, SAVE, 21>(r);
-    return p.ru_wpg == 1 ? unit_kernel<1, SAVE, 0>(r) : unit_kernel<2, SAVE, 0>(r);
+    if (p.ru_ht == 102) return unit_kernel<2, SAVE, 102, WIN>(r);
+    if (p.ru_ht == 21) return unit_kernel<1, SAVE, 21, WIN>(r);
+    return p.ru_wpg == 1 ? unit_kernel<1, SAVE, 0, WIN>(r) : unit_kernel<2, SAVE, 0, WIN>(r);
 }
 int launch_recur_unit(const Plan& p, void* ws, float* out, long long Bc, int r, cudaStream_t st, float* gsave,
-                      int ldsave) {
-    const UnitKernel kern = gsave ? unit_kernel<true>(p, r) : unit_kernel<false>(p, r);
+                      int ldsave, const long long* row0) {
+    const UnitKernel kern =
+        row0 ? unit_kernel<false, true>(p, r) : gsave ? unit_kernel<true>(p, r) : unit_kernel<false>(p, r);
     const size_t smem = wg::recur_u_smem_floats(p.H, r) * 4;
     WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int per_cta = (wg::kRuWarps / p.ru_wpg) * r;
@@ -576,19 +596,20 @@ int launch_recur_unit(const Plan& p, void* ws, float* out, long long Bc, int r, 
     const int handover = p.ru_wpg == 1 ? 1 : 0;
     kern<<<(unsigned)grid, wg::kRuThreads, smem, st>>>(ws_ptr<float>(ws, p.off_gi), ws_ptr<float>(ws, p.off_whu),
                                                       ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H, gsave, ldsave,
-                                                      handover);
+                                                      handover, row0);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
 
-int launch_recur_tc(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st) {
+int launch_recur_tc(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, const long long* row0) {
+    auto kern = row0 ? wg::gru_recur_tc_kernel<true> : wg::gru_recur_tc_kernel<false>;
     const size_t smem = wg::recur_tc_smem_bytes(p.H);
-    WG_CUDA(cudaFuncSetAttribute(wg::gru_recur_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const long long grid = (Bc + wg::kRtSeqs - 1) / wg::kRtSeqs;
     if (grid < 1) return WG_OK;
-    wg::gru_recur_tc_kernel<<<(unsigned)grid, wg::kRtThreads, smem, st>>>(
-        ws_ptr<float>(ws, p.off_gi), ws_ptr<__half>(ws, p.off_whh_hi), ws_ptr<__half>(ws, p.off_whh_lo),
-        ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H, p.GP);
+    kern<<<(unsigned)grid, wg::kRtThreads, smem, st>>>(ws_ptr<float>(ws, p.off_gi), ws_ptr<__half>(ws, p.off_whh_hi),
+                                                      ws_ptr<__half>(ws, p.off_whh_lo), ws_ptr<float>(ws, p.off_bhn),
+                                                      out, Bc, p.T, p.H, p.GP, row0);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
@@ -602,15 +623,16 @@ bool regw_serves(const Plan& p, long long Bc) {
 // gru_recur_regw_kernel where it serves the contraction length (FMA chains per thread = sequences per CTA that can
 // exist: the reference's batch-1 calls run one).  gsave: the training forward, which also saves [r | z | n | hn] per
 // (sequence, step), row stride ldsave; only the regw and unit kernels save gates, and make_train_plan accepts only the
-// shapes that reach one of them.
-int launch_recur(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave) {
-    if (regw_serves(p, Bc)) return launch_recur_regw(p, ws, out, Bc, Bc >= 4 ? 4 : (int)Bc, st, gsave, ldsave);
+// shapes that reach one of them.  row0: the forecast's windows (see launch_recur_wide), which save no gates.
+int launch_recur(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave,
+                 const long long* row0 = nullptr) {
+    if (regw_serves(p, Bc)) return launch_recur_regw(p, ws, out, Bc, Bc >= 4 ? 4 : (int)Bc, st, gsave, ldsave, row0);
     if (p.recur == kRecurUnit) {
         const int r = recur_u_pick_r(Bc, wg::kRuWarps / p.ru_wpg);
-        return launch_recur_unit(p, ws, out, Bc, r < p.ru_rmax ? r : p.ru_rmax, st, gsave, ldsave);
+        return launch_recur_unit(p, ws, out, Bc, r < p.ru_rmax ? r : p.ru_rmax, st, gsave, ldsave, row0);
     }
-    if (p.recur == kRecurTc) return launch_recur_tc(p, ws, out, Bc, st);   // the tensor path: every batch size
-    return launch_recur_wide(p, ws, out, Bc, st);
+    if (p.recur == kRecurTc) return launch_recur_tc(p, ws, out, Bc, st, row0);   // the tensor path: every batch size
+    return launch_recur_wide(p, ws, out, Bc, st, row0);
 }
 
 int launch_pack(const Plan& p, void* ws, const float* w_ih, const float* w_hh, const float* b_ih,
@@ -640,7 +662,7 @@ int run_chunk(const Plan& p, void* ws, const Graph& g, const float* x, const flo
     const long long rows = Bc * p.T;
     int rc = launch_gcn(p, ws, g, x, w1, b1, w2, b2, rows, st);
     if (rc) return rc;
-    rc = launch_inproj(p, ws, rows, st);
+    rc = launch_inproj(p, ws, rows, st, ws_ptr<float>(ws, p.off_gi));
     if (rc) return rc;
     return launch_recur(p, ws, out, Bc, st, gsave, ldsave);
 }
@@ -692,15 +714,14 @@ bool any_null(std::initializer_list<const void*> ps) {
     return false;
 }
 
-// The device-buffer forward of a finished plan, on either graph form: pack the parameters, then every chunk through
-// the three stages.  need: the workspace bytes to check (the training plan adds its regions to the forward's);
-// gsave / ldsave: see launch_recur.  On gcn_sparse_plan_kernel the CSR graph also holds the constant bank from
-// prepare_sparse to finish_sparse.
-int forward(const Plan& p, size_t need, const Graph& g, const float* x, const float* w1, const float* b1,
-            const float* w2, const float* b2, const float* w_ih, const float* w_hh, const float* b_ih,
-            const float* b_hh, float* out, long long B, void* ws, size_t ws_bytes, int device, void* stream,
-            float* gsave = nullptr, int ldsave = 0) {
-    if (B == 0) return WG_OK;
+// The frame of a device-buffer forward or forecast, on either graph form: check the pointers (x: the input windows or
+// the table) and the workspace (need bytes), switch to the device, pack the parameters, then run `stages` on the
+// stream.  On gcn_sparse_plan_kernel the CSR graph also holds the constant bank from prepare_sparse to finish_sparse.
+template <typename Stages>
+int run_packed(const Plan& p, size_t need, const Graph& g, const float* x, const float* w1, const float* b1,
+               const float* w2, const float* b2, const float* w_ih, const float* w_hh, const float* b_ih,
+               const float* b_hh, const float* out, void* ws, size_t ws_bytes, int device, void* stream,
+               Stages stages) {
     const bool no_graph = p.sparse ? any_null({g.rowptr, g.colidx, g.vals}) : !g.adj;
     if (no_graph || any_null({x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out}))
         return fail(WG_ERR_BAD_ARG, "null pointer argument");
@@ -716,14 +737,94 @@ int forward(const Plan& p, size_t need, const Graph& g, const float* x, const fl
         sq_lock.lock();
         if ((rc = prepare_sparse(p, ws, g, w1, b1, w2, b2, device, st))) return rc;
     }
-    const size_t x_seq = (size_t)p.T * p.S * p.Fi, o_seq = (size_t)p.T * p.H;
-    for (long long b0 = 0; b0 < B; b0 += p.chunk) {
-        const long long Bc = (B - b0) < p.chunk ? (B - b0) : p.chunk;
-        rc = run_chunk(p, ws, g, x + (size_t)b0 * x_seq, w1, b1, w2, b2, out + (size_t)b0 * o_seq, Bc, st,
-                       gsave ? gsave + (size_t)b0 * p.T * ldsave : nullptr, ldsave);
-        if (rc) return rc;
-    }
+    if ((rc = stages(st))) return rc;
     return sq ? finish_sparse(device, st) : WG_OK;
+}
+
+// The device-buffer forward of a finished plan: every chunk through the three stages.  need: the workspace bytes to
+// check (the training plan adds its regions to the forward's); gsave / ldsave: see launch_recur.
+int forward(const Plan& p, size_t need, const Graph& g, const float* x, const float* w1, const float* b1,
+            const float* w2, const float* b2, const float* w_ih, const float* w_hh, const float* b_ih,
+            const float* b_hh, float* out, long long B, void* ws, size_t ws_bytes, int device, void* stream,
+            float* gsave = nullptr, int ldsave = 0) {
+    if (B == 0) return WG_OK;
+    auto stages = [&](cudaStream_t st) {
+        const size_t x_seq = (size_t)p.T * p.S * p.Fi, o_seq = (size_t)p.T * p.H;
+        for (long long b0 = 0; b0 < B; b0 += p.chunk) {
+            const long long Bc = (B - b0) < p.chunk ? (B - b0) : p.chunk;
+            const int rc = run_chunk(p, ws, g, x + (size_t)b0 * x_seq, w1, b1, w2, b2, out + (size_t)b0 * o_seq, Bc,
+                                     st, gsave ? gsave + (size_t)b0 * p.T * ldsave : nullptr, ldsave);
+            if (rc) return rc;
+        }
+        return (int)WG_OK;
+    };
+    return run_packed(p, need, g, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, ws, ws_bytes, device, stream,
+                      stages);
+}
+
+// ---- rolling forecasts: windows over one table --------------------------------------------------
+// GCN and input projection depend only on a table row, the recurrence on the window (h0 = 0 at its first row): the
+// rows the windows cover run the first two stages once, each into a GI row of its own, and every window's recurrence
+// reads its L rows in place.  The plan is the forward's for N windows of L steps, with a GI region of Ttot rows and
+// the windows' first GI rows (int64, relative to the first row covered) after it.
+struct ForecastPlan {
+    Plan p;
+    size_t off_row0, total;
+};
+
+int make_forecast_plan(ForecastPlan& f, long long N, long long Ttot, int L, int S, int Fi, int Fh, int Fo, int H,
+                       long long chunk, bool sparse, int flags) {
+    if (N < 0 || L < 1 || Ttot < L)
+        return fail(WG_ERR_BAD_ARG, "forecast: need N >= 0 and 1 <= L <= Ttot (N=%lld L=%d Ttot=%lld)", N, L, Ttot);
+    int rc = plan_layout(f.p, N, L, S, Fi, Fh, Fo, H, chunk, sparse, flags, Ttot);
+    if (rc || (rc = plan_launch(f.p))) return rc;
+    f.off_row0 = f.p.total;
+    f.total = align_up(f.off_row0 + (size_t)N * sizeof(long long));
+    return WG_OK;
+}
+
+// starts: HOST [N], validated before anything else is looked at; out [N][H] = h at the last step of each window.
+int forecast(const ForecastPlan& f, const Graph& g, const float* table, const int64_t* starts, const float* w1,
+             const float* b1, const float* w2, const float* b2, const float* w_ih, const float* w_hh,
+             const float* b_ih, const float* b_hh, float* out, long long N, long long Ttot, void* ws,
+             size_t ws_bytes, int device, void* stream) {
+    const Plan& p = f.p;
+    if (N == 0) return WG_OK;
+    if (!starts) return fail(WG_ERR_BAD_ARG, "starts is NULL (N=%lld)", N);
+    const long long last = Ttot - p.T;
+    long long lo = 0, hi = 0;
+    for (long long n = 0; n < N; ++n) {
+        const long long s = starts[n];
+        if (s < 0 || s > last)
+            return fail(WG_ERR_BAD_ARG, "starts[%lld] = %lld outside [0, Ttot - L] = [0, %lld]", n, s, last);
+        if (n == 0 || s < lo) lo = s;
+        if (n == 0 || s > hi) hi = s;
+    }
+    auto stages = [&](cudaStream_t st) {
+        // first GI rows relative to the span; a pageable source is staged before cudaMemcpyAsync returns
+        std::vector<long long> row0((size_t)N);
+        for (long long n = 0; n < N; ++n) row0[(size_t)n] = starts[n] - lo;
+        long long* row0_dev = ws_ptr<long long>(ws, f.off_row0);
+        WG_CUDA(cudaMemcpyAsync(row0_dev, row0.data(), (size_t)N * sizeof(long long), cudaMemcpyHostToDevice, st));
+        // GCN + projection over table rows [lo, hi + L), in pieces of the U scratch's rows
+        float* gi = ws_ptr<float>(ws, p.off_gi);
+        const size_t x_row = (size_t)p.S * p.Fi;
+        const long long span = hi + p.T - lo, piece = forecast_piece_rows(p, Ttot);
+        for (long long r0 = 0; r0 < span; r0 += piece) {
+            const long long rows = span - r0 < piece ? span - r0 : piece;
+            int rc = launch_gcn(p, ws, g, table + (size_t)(lo + r0) * x_row, w1, b1, w2, b2, rows, st);
+            if (rc || (rc = launch_inproj(p, ws, rows, st, gi + (size_t)r0 * p.GP))) return rc;
+        }
+        // the recurrence in the forward's chunks, so that every chunk runs the kernel the forward would
+        for (long long b0 = 0; b0 < N; b0 += p.chunk) {
+            const long long Bc = (N - b0) < p.chunk ? (N - b0) : p.chunk;
+            const int rc = launch_recur(p, ws, out + (size_t)b0 * p.H, Bc, st, nullptr, 0, row0_dev + b0);
+            if (rc) return rc;
+        }
+        return (int)WG_OK;
+    };
+    return run_packed(p, f.total, g, table, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, ws, ws_bytes, device, stream,
+                      stages);
 }
 
 // The wg_stage_* entry points: plan one chunk, check Bc, the workspace and the device, then run `launch`.
@@ -997,7 +1098,9 @@ int wg_stage_gcn_f32(const float* adj, const float* x, const float* w1, const fl
 
 int wg_stage_inproj_f32(int64_t Bc, int T, int S, int F_in, int F_hid, int F_out, int H, int64_t chunk,
                         int flags, void* workspace, size_t workspace_bytes, int device, void* stream) {
-    auto launch = [&](const Plan& p, cudaStream_t st) { return launch_inproj(p, workspace, Bc * T, st); };
+    auto launch = [&](const Plan& p, cudaStream_t st) {
+        return launch_inproj(p, workspace, Bc * T, st, ws_ptr<float>(workspace, p.off_gi));
+    };
     return run_stage(Bc, T, S, F_in, F_hid, F_out, H, chunk, flags, workspace, workspace_bytes, device, stream, launch);
 }
 
@@ -1036,6 +1139,43 @@ int wg_gcn_gru_forward_csr_f32(const int32_t* rowptr, const int32_t* colidx, con
     const int rc = make_plan(p, B, T, S, F_in, F_hid, F_out, H, chunk, true, flags);
     return rc ? rc : forward(p, p.total, Graph{nullptr, rowptr, colidx, vals}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih,
                              b_hh, out, B, workspace, workspace_bytes, device, stream);
+}
+
+size_t wg_gcn_gru_forecast_workspace_bytes(int64_t N, int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out,
+                                           int H, int64_t chunk, int flags) {
+    ForecastPlan f;
+    if (make_forecast_plan(f, N, Ttot, L, S, F_in, F_hid, F_out, H, chunk, false, flags)) return 0;
+    return f.total;
+}
+
+int wg_gcn_gru_forecast_f32(const float* adj, const float* table, const int64_t* starts, const float* w1,
+                            const float* b1, const float* w2, const float* b2, const float* w_ih, const float* w_hh,
+                            const float* b_ih, const float* b_hh, float* out, int64_t N, int64_t Ttot, int L, int S,
+                            int F_in, int F_hid, int F_out, int H, int64_t chunk, int flags, void* workspace,
+                            size_t workspace_bytes, int device, void* stream) {
+    ForecastPlan f;
+    const int rc = make_forecast_plan(f, N, Ttot, L, S, F_in, F_hid, F_out, H, chunk, false, flags);
+    return rc ? rc : forecast(f, Graph{adj}, table, starts, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, N, Ttot,
+                              workspace, workspace_bytes, device, stream);
+}
+
+size_t wg_gcn_gru_forecast_csr_workspace_bytes(int64_t N, int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out,
+                                               int H, int64_t chunk, int flags) {
+    ForecastPlan f;
+    if (make_forecast_plan(f, N, Ttot, L, S, F_in, F_hid, F_out, H, chunk, true, flags)) return 0;
+    return f.total;
+}
+
+int wg_gcn_gru_forecast_csr_f32(const int32_t* rowptr, const int32_t* colidx, const float* vals, const float* table,
+                                const int64_t* starts, const float* w1, const float* b1, const float* w2,
+                                const float* b2, const float* w_ih, const float* w_hh, const float* b_ih,
+                                const float* b_hh, float* out, int64_t N, int64_t Ttot, int L, int S, int F_in,
+                                int F_hid, int F_out, int H, int64_t chunk, int flags, void* workspace,
+                                size_t workspace_bytes, int device, void* stream) {
+    ForecastPlan f;
+    const int rc = make_forecast_plan(f, N, Ttot, L, S, F_in, F_hid, F_out, H, chunk, true, flags);
+    return rc ? rc : forecast(f, Graph{nullptr, rowptr, colidx, vals}, table, starts, w1, b1, w2, b2, w_ih, w_hh,
+                              b_ih, b_hh, out, N, Ttot, workspace, workspace_bytes, device, stream);
 }
 
 }  // extern "C"

@@ -67,10 +67,13 @@ struct RcFrag {
     float2 wc[4];     // W[k + kk][cC .. cC+1]
 };
 
+// WIN: windows over one table's gi rows (see gru_recur_unit_kernel): row rbase + 4i of the CTA reads its gi from
+// GI + row0[b] * ldg, and only h at t = T-1 is stored, directly to out [B][H] (the launch passes TS = 0: no staging)
+template <bool WIN = false>
 __global__ void __launch_bounds__(kRcWarps * 32, 1)
     gru_recur_kernel(const float* __restrict__ GI, const float* __restrict__ WhT,
                      const float* __restrict__ bhn, float* __restrict__ out, long long B, int T, int H,
-                     int ldg, int KP, int NP, int TS) {
+                     int ldg, int KP, int NP, int TS, const long long* __restrict__ row0) {
     constexpr int NT = kRcWarps * 32;
     constexpr int WG = kRcWarps / 2;   // warps per group
     constexpr int NG = WG * 32;      // threads per group
@@ -106,6 +109,15 @@ __global__ void __launch_bounds__(kRcWarps * 32, 1)
     const int n_cb = NP / kRcCB;           // 80-column blocks; this warp takes gwarp, gwarp + WG, ...
     const int rbase = grp * GB + bg;       // rows rbase + 4 i
 
+    // WIN: gi row 0 of this thread's rows rbase + 4i
+    const float* gwin[WIN ? 4 : 1];
+    if (WIN) {
+#pragma unroll
+        for (int i = 0; i < (WIN ? 4 : 1); ++i) {
+            const long long b = b0 + rbase + 4 * i;
+            gwin[i] = GI + (size_t)(b < B ? row0[b] : 0) * ldg;
+        }
+    }
     // this thread's chunks of the gi tile of step t: per row 16 + 16 + 8 bytes per column block
     auto prefetch_gi = [&](int t) {
         for (int cb = gwarp; cb < n_cb; cb += WG) {
@@ -115,6 +127,7 @@ __global__ void __launch_bounds__(kRcWarps * 32, 1)
             const size_t src_step = (size_t)4 * T * ldg;
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
+                if (WIN) src = gwin[WIN ? i : 0] + (size_t)t * ldg;
                 if (b0 + rbase + 4 * i < B) {
                     if (cA < ldg) cp_async16(dst + cA, src + cA, true);
                     if (cB < ldg) cp_async16(dst + cB, src + cB, true);
@@ -264,8 +277,8 @@ __global__ void __launch_bounds__(kRcWarps * 32, 1)
             const float* __restrict__ gn = ghn + (grp * GB) * KP + j;
             float* __restrict__ hp = hs + (grp * GB) * RS + j;
             float* __restrict__ sp = stage + (grp * GB) * TS * H + (TS > 0 ? (t % TS) * H : 0) + j;
-            float* __restrict__ op = out + ((size_t)(b0 + grp * GB) * T + t) * H + j;
-            const size_t o_step = (size_t)T * H;
+            float* __restrict__ op = out + ((size_t)(b0 + grp * GB) * (WIN ? 1 : T) + (WIN ? 0 : t)) * H + j;
+            const size_t o_step = (size_t)(WIN ? 1 : T) * H;
             const int s_step = TS * H;
             // pass 1: all 16 new states into registers (no store in between, so the loads and MUFU
             // chains of different sequences overlap); pass 2: the stores
@@ -282,7 +295,7 @@ __global__ void __launch_bounds__(kRcWarps * 32, 1)
             for (int bl = 0; bl < GB; ++bl) {
                 hp[bl * RS] = hnew[bl];
                 if (TS > 0) sp[bl * s_step] = hnew[bl];
-                else if (b0 + grp * GB + bl < B) op[bl * o_step] = hnew[bl];
+                else if ((!WIN || t == T - 1) && b0 + grp * GB + bl < B) op[bl * o_step] = hnew[bl];
             }
         }
         if (TS > 0) asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");  // staged h -> async proxy
@@ -334,11 +347,13 @@ __host__ __device__ inline size_t recur_regw_smem_floats(int KP, int NP, int GP)
     return (size_t)kRsBT * (KP + 4) + 2 * (size_t)kRsBT * GP + (size_t)kRsBT * NP + (size_t)KP;
 }
 
-template <bool SAVE, int NB, int KPT>
+// WIN: windows over one table's gi rows (see gru_recur_unit_kernel): sequence b's gi rows start at GI + row0[b] * ldg,
+// only h at t = T-1 is stored, to out [B][H]
+template <bool SAVE, int NB, int KPT, bool WIN = false>
 __global__ void __launch_bounds__(kRwThreads, 1)
     gru_recur_regw_kernel(const float* __restrict__ GI, const float* __restrict__ WhT, const float* __restrict__ bhn,
                           float* __restrict__ out, long long B, int T, int H, int ldg, int NP, float* __restrict__ gsave,
-                          int ldsave) {
+                          int ldsave, const long long* __restrict__ row0) {
     extern __shared__ __align__(16) float smem[];
     constexpr int RS = KPT + 4;
     float* hs = smem;                          // [4][RS]
@@ -373,7 +388,8 @@ __global__ void __launch_bounds__(kRwThreads, 1)
         const int b = mine ? e / chunks : 0, c = mine ? e - b * chunks : 0;
         pf_ok[q] = mine && (b0 + b < B);
         pf_off[q] = mine ? b * ldg + 4 * c : -1;
-        pf_src[q] = GI + ((size_t)(pf_ok[q] ? b0 + b : 0) * T) * ldg + 4 * c;
+        pf_src[q] = WIN ? GI + (size_t)(pf_ok[q] ? row0[b0 + b] : 0) * ldg + 4 * c
+                        : GI + ((size_t)(pf_ok[q] ? b0 + b : 0) * T) * ldg + 4 * c;
     }
 #define WG_RW_PREFETCH(t_)                                                                              \
     do {                                                                                                \
@@ -423,7 +439,9 @@ __global__ void __launch_bounds__(kRwThreads, 1)
                 const float n = tanh_f(gr[H2] + r * hn);
                 const float hnew = (hs[b * RS + j] - n) * z + n;
                 hs[b * RS + j] = hnew;
-                if (b0 + b < B) {
+                if (WIN) {
+                    if (b0 + b < B && t == T - 1) out[(size_t)(b0 + b) * H + j] = hnew;
+                } else if (b0 + b < B) {
                     out[((size_t)(b0 + b) * T + t) * H + j] = hnew;
                     if (SAVE) {
                         float* gs = gsave + ((size_t)(b0 + b) * T + t) * ldsave + j;

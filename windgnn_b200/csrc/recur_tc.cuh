@@ -117,9 +117,13 @@ __global__ void pack_whh_tc_kernel(const float* __restrict__ w_hh, __half* __res
 
 // GI [rows][ldg] (b_ih, and b_hh of r / z, folded in; readable up to the next multiple of kRtSeqs sequences);
 // Whi / Wlo: pack_whh_tc_kernel's output; out [B][T][H]
+// WIN: windows over one table's gi rows (see gru_recur_unit_kernel): sequence b's gi rows start at GI + row0[b] * ldg
+// (the padding sequences of the last group read the last window's rows), only h at t = T-1 is stored, to out [B][H]
+template <bool WIN = false>
 __global__ void __launch_bounds__(kRtThreads, 1)
     gru_recur_tc_kernel(const float* __restrict__ GI, const __half* __restrict__ Whi, const __half* __restrict__ Wlo,
-                        const float* __restrict__ bhn, float* __restrict__ out, long long B, int T, int H, int ldg) {
+                        const float* __restrict__ bhn, float* __restrict__ out, long long B, int T, int H, int ldg,
+                        const long long* __restrict__ row0) {
     extern __shared__ __align__(1024) unsigned char smem_rt[];
     const int KP = recur_tc_kp(H), NCH = KP / 8, NKS = KP / 16;
     const uint32_t a_part = (uint32_t)(3 * NCH * 2048);           // bytes of A_hi (= A_lo)
@@ -182,9 +186,15 @@ __global__ void __launch_bounds__(kRtThreads, 1)
     const long long left = B - bg0;
     const int nvalid = left >= 8 ? 8 : (left > 0 ? (int)left : 0);
     // running pointers (advance one step at a time); sequences are T * ldg / T * H floats apart
+    // (WIN: out rows H floats apart, written at the last step; gi rows from gw)
     const float* gp = GI + (size_t)bg0 * T * ldg + jc;
-    float* op = out + (size_t)bg0 * T * H + j;
-    const int g_seq = T * ldg, o_seq = T * H;
+    float* op = out + (size_t)bg0 * (WIN ? 1 : T) * H + j;
+    const int g_seq = T * ldg, o_seq = (WIN ? 1 : T) * H;
+    const float* gw[WIN ? 8 : 1];
+    if (WIN) {
+#pragma unroll
+        for (int n = 0; n < (WIN ? 8 : 1); ++n) gw[n] = GI + (size_t)row0[bg0 + n < B ? bg0 + n : B - 1] * ldg + jc;
+    }
     uint32_t ph = 0;
     // MMA issue (one thread per group): operand bases
     const uint32_t idesc32 = umma_idesc_f16(128, 2 * kRtN), idesc16 = umma_idesc_f16(128, kRtN);
@@ -192,18 +202,20 @@ __global__ void __launch_bounds__(kRtThreads, 1)
     const uint32_t dcol = tmem_base + (uint32_t)(g * 6 * kRtN);
 
     // gi of this thread's 8 sequences: [gate][seq]; rows beyond B are readable scratch (never stored)
-    auto load_gi = [&](float (&gi)[3][8], const float* p) {
+    // (WIN: step t of sequence n at gw[n] + t * ldg)
+    auto load_gi = [&](float (&gi)[3][8], const float* p, int t) {
 #pragma unroll
         for (int n = 0; n < 8; ++n) {
-            gi[0][n] = __ldg(p + n * g_seq);
-            gi[1][n] = __ldg(p + n * g_seq + H);
-            gi[2][n] = __ldg(p + n * g_seq + H2);
+            const float* s = WIN ? gw[WIN ? n : 0] + (size_t)t * ldg : p + n * g_seq;
+            gi[0][n] = __ldg(s);
+            gi[1][n] = __ldg(s + H);
+            gi[2][n] = __ldg(s + H2);
         }
     };
     float gi[3][8], gi_nxt[3][8];
-    load_gi(gi, gp);
+    load_gi(gi, gp, 0);
     for (int t = 0; t < T; ++t) {
-        if (t + 1 < T) load_gi(gi_nxt, gp + ldg);   // a whole step ahead: lands during this step's gates + product
+        if (t + 1 < T) load_gi(gi_nxt, gp + ldg, t + 1);   // a whole step ahead: lands during this step's gates + product
         float rr[8], zz[8], hn[8];
         if (t > 0) {
             mbar_wait(&acc_full[g], ph);   // this group's product of step t is complete
@@ -249,11 +261,11 @@ __global__ void __launch_bounds__(kRtThreads, 1)
                 const __half hl = __float2half_rn(hnew - __half2float(hh));
                 *reinterpret_cast<__half*>(bh + n * 16) = hh;
                 *reinterpret_cast<__half*>(bl + n * 16) = hl;
-                if (n < nvalid) op[n * o_seq] = hnew;
+                if (n < nvalid && (!WIN || t == T - 1)) op[n * o_seq] = hnew;
             }
         }
         gp += ldg;
-        op += H;
+        if (!WIN) op += H;
         if (t + 1 < T) {
             // h_t of the group is in shared memory (generic-proxy writes -> visible to the tensor core), every
             // warp of the group has read its accumulators: one thread issues the next step's product

@@ -94,15 +94,8 @@ class GCN_GRU(nn.Module):
         if torch.is_grad_enabled() and (attr_matrix.requires_grad or (not is_csr and adj_matrix.requires_grad)):
             # the reference never differentiates w.r.t. its data (main.py:66-77); the library has no such gradient
             raise RuntimeError("windgnn_b200.GCN_GRU: gradients w.r.t. attr_matrix / adj_matrix are not implemented")
-        if is_csr or adj_matrix.shape[0] > self.DENSE_MAX_STATIONS or max(widths) > 16:
-            # scaled shapes (thousands of stations, wide hidden layer): CSR adjacency path
-            if is_csr:
-                csr = (adj_matrix.rowptr, adj_matrix.colidx, adj_matrix.vals)
-            else:
-                key = (adj_matrix.data_ptr(), adj_matrix._version, tuple(adj_matrix.shape))
-                if self._csr_cache is None or self._csr_cache[0] != key:
-                    self._csr_cache = (key, ops.dense_to_csr(adj_matrix))
-                csr = self._csr_cache[1]
+        csr = self._csr_of(adj_matrix)
+        if csr is not None:
             if needs_grad:
                 # forward works under grad mode (main.py:66 style calls); backward() explains the limit
                 out = _InferenceOnly.apply(
@@ -135,6 +128,48 @@ class GCN_GRU(nn.Module):
         )
         return ops.gcn_gru_forward_host(adj_matrix, attr_host, [p.detach() for p in params], out_host, self.chunk,
                                         flags=self._flags(), last_step_range=last_step_range)
+
+    @torch.no_grad()
+    def forecast(self, adj_matrix, table, starts=None, seq_length=168, stride=1, last_step_range=None):
+        """Rolling forecasts from one table: the last hidden state ``[N, H]`` of every window
+        ``table[starts[n] : starts[n] + seq_length]`` of ``table [Ttot, S, F_in]`` (on the GPU), without
+        materialising the windows: GCN and input projection run once per table row.  Row ``n`` is bit-identical to
+        ``self(adj_matrix, window_n)[-1]`` under ``torch.no_grad()``.
+
+        ``starts``: int64 first rows (any order, repeats allowed); ``None`` = every ``stride``-th window,
+        ``window_starts(Ttot, seq_length, stride)``.  Same adjacency forms, routing, ``precision`` and ``chunk`` as
+        ``forward``.  ``last_step_range=(wind_min, wind_max)``: de-normalised as ``denormalise_last_step`` does
+        (src/main.py:103,116)."""
+        from .sequences import denormalise_last_step, window_starts
+
+        if starts is None:
+            starts = window_starts(table.shape[0], seq_length, stride)
+        params = [p.detach() for p in (
+            self.conv1.weight, self.conv1.bias, self.conv2.weight, self.conv2.bias,
+            self.gru.weight_ih_l0, self.gru.weight_hh_l0, self.gru.bias_ih_l0, self.gru.bias_hh_l0,
+        )]
+        csr = self._csr_of(adj_matrix)
+        if csr is not None:
+            out = ops.gcn_gru_forecast_csr(*csr, table, starts, *params, seq_length, self.chunk, self._flags())
+        else:
+            out = ops.gcn_gru_forecast(adj_matrix, table, starts, *params, seq_length, self.chunk, self._flags())
+        if last_step_range is not None:
+            out = denormalise_last_step(out.unsqueeze(1), *last_step_range)
+        return out
+
+    def _csr_of(self, adj_matrix):
+        """The CSR arrays the library takes for ``adj_matrix``, or ``None`` for the dense path: a ``CsrGraph``, more
+        than DENSE_MAX_STATIONS stations or GCN widths above 16 (the scaled shapes) go to CSR, a dense matrix
+        through a cached conversion."""
+        widths = (self.conv1.weight.shape[0], self.conv1.weight.shape[1], self.conv2.weight.shape[1])
+        if isinstance(adj_matrix, CsrGraph):
+            return (adj_matrix.rowptr, adj_matrix.colidx, adj_matrix.vals)
+        if adj_matrix.shape[0] <= self.DENSE_MAX_STATIONS and max(widths) <= 16:
+            return None
+        key = (adj_matrix.data_ptr(), adj_matrix._version, tuple(adj_matrix.shape))
+        if self._csr_cache is None or self._csr_cache[0] != key:
+            self._csr_cache = (key, ops.dense_to_csr(adj_matrix))
+        return self._csr_cache[1]
 
     def _flags(self) -> int:
         from . import _lib

@@ -2,6 +2,8 @@
 
 ``windgnn::gcn_gru_forward``  the fused forward of ``GCN_GRU`` (reference:
                               src/step6_gcn_gru_combined_model.py:13-27)
+``windgnn::gcn_gru_forecast``  the last hidden state of windows over one table, GCN and projection once per
+                              table row (``GCN_GRU.forecast``)
 ``windgnn::gcn_layer``        one ``GraphConvLayer`` (reference: src/step5_gcn_layer_model.py:13-23)
 
 PyTorch is the plumbing here: it owns device memory (inputs, output, the cached workspace)
@@ -195,6 +197,142 @@ def gcn_gru_forward_csr(
 @gcn_gru_forward_csr.register_fake
 def _(rowptr, colidx, vals, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, chunk=0, flags=0):
     return x.new_empty((x.shape[0], x.shape[1], w_hh.shape[1]))
+
+
+def _forecast_starts(starts: torch.Tensor) -> torch.Tensor:
+    """The windows' first table rows as the contiguous HOST int64 array the library reads."""
+    if not isinstance(starts, torch.Tensor) or starts.dtype != torch.int64 or starts.dim() != 1:
+        raise RuntimeError("starts must be a 1-D int64 tensor")
+    return starts.cpu().contiguous()
+
+
+def _forecast_dims(adj, table, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh):
+    if table.dim() != 3:
+        raise RuntimeError(f"table must be [Ttot, S, F_in], got {tuple(table.shape)}")
+    _, Ttot, S, F_in, F_hid, F_out, H = _dims(adj, table.unsqueeze(0), w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh)
+    return Ttot, S, F_in, F_hid, F_out, H
+
+
+@torch.library.custom_op("windgnn::gcn_gru_forecast", mutates_args=())
+def gcn_gru_forecast(
+    adj: torch.Tensor,
+    table: torch.Tensor,
+    starts: torch.Tensor,
+    w1: torch.Tensor,
+    b1: torch.Tensor,
+    w2: torch.Tensor,
+    b2: torch.Tensor,
+    w_ih: torch.Tensor,
+    w_hh: torch.Tensor,
+    b_ih: torch.Tensor,
+    b_hh: torch.Tensor,
+    seq_length: int,
+    chunk: int = 0,
+    flags: int = 0,
+) -> torch.Tensor:
+    """Rolling forecasts: ``table [Ttot, S, F_in]`` and int64 ``starts [N]`` -> ``[N, H]``, row ``n`` the last
+    hidden state of the window ``table[starts[n] : starts[n] + seq_length]``, bit-identical to
+    ``gcn_gru_forward(window)[:, -1]`` with the same ``chunk`` and ``flags``.  GCN and input projection run once
+    per table row.  ``starts`` may live on either device (the library reads it from the host)."""
+    lib = _lib.load()
+    table = _require_cuda_f32("table", table)
+    dev = table.device
+    adj, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh = (
+        _require_cuda_f32(n, t, dev)
+        for n, t in (
+            ("adj_matrix", adj), ("conv1.weight", w1), ("conv1.bias", b1), ("conv2.weight", w2),
+            ("conv2.bias", b2), ("gru.weight_ih_l0", w_ih), ("gru.weight_hh_l0", w_hh),
+            ("gru.bias_ih_l0", b_ih), ("gru.bias_hh_l0", b_hh),
+        )
+    )
+    Ttot, S, F_in, F_hid, F_out, H = _forecast_dims(adj, table, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh)
+    starts = _forecast_starts(starts)
+    N = starts.numel()
+    out = torch.empty((N, H), dtype=torch.float32, device=dev)
+    # 0 bytes: the shape is rejected, and the call below returns the library's code and reason without launching
+    nbytes = lib.wg_gcn_gru_forecast_workspace_bytes(N, Ttot, seq_length, S, F_in, F_hid, F_out, H, chunk, flags)
+    ws = _workspace(dev, nbytes, "forecast")
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    _lib.check(
+        lib.wg_gcn_gru_forecast_f32(
+            adj.data_ptr(), table.data_ptr(), starts.data_ptr(), w1.data_ptr(), b1.data_ptr(), w2.data_ptr(),
+            b2.data_ptr(), w_ih.data_ptr(), w_hh.data_ptr(), b_ih.data_ptr(), b_hh.data_ptr(), out.data_ptr(),
+            N, Ttot, seq_length, S, F_in, F_hid, F_out, H, chunk, flags, ws.data_ptr(), ws.numel(), dev.index or 0,
+            stream,
+        )
+    )
+    return out
+
+
+@gcn_gru_forecast.register_fake
+def _(adj, table, starts, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, seq_length, chunk=0, flags=0):
+    return table.new_empty((starts.shape[0], w_hh.shape[1]))
+
+
+@torch.library.custom_op("windgnn::gcn_gru_forecast_csr", mutates_args=())
+def gcn_gru_forecast_csr(
+    rowptr: torch.Tensor,
+    colidx: torch.Tensor,
+    vals: torch.Tensor,
+    table: torch.Tensor,
+    starts: torch.Tensor,
+    w1: torch.Tensor,
+    b1: torch.Tensor,
+    w2: torch.Tensor,
+    b2: torch.Tensor,
+    w_ih: torch.Tensor,
+    w_hh: torch.Tensor,
+    b_ih: torch.Tensor,
+    b_hh: torch.Tensor,
+    seq_length: int,
+    chunk: int = 0,
+    flags: int = 0,
+) -> torch.Tensor:
+    """``gcn_gru_forecast`` with the adjacency in CSR form (as for ``gcn_gru_forward_csr``); bit-identical to
+    ``gcn_gru_forward_csr(window)[:, -1]``."""
+    lib = _lib.load()
+    table = _require_cuda_f32("table", table)
+    dev = table.device
+    w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, vals = (
+        _require_cuda_f32(n, t, dev)
+        for n, t in (
+            ("conv1.weight", w1), ("conv1.bias", b1), ("conv2.weight", w2), ("conv2.bias", b2),
+            ("gru.weight_ih_l0", w_ih), ("gru.weight_hh_l0", w_hh), ("gru.bias_ih_l0", b_ih),
+            ("gru.bias_hh_l0", b_hh), ("adjacency values", vals),
+        )
+    )
+    if table.dim() != 3:
+        raise RuntimeError(f"table must be [Ttot, S, F_in], got {tuple(table.shape)}")
+    S = table.shape[1]
+    for n, t in (("rowptr", rowptr), ("colidx", colidx)):
+        if not t.is_cuda or t.dtype != torch.int32 or t.device != dev:
+            raise RuntimeError(f"windgnn_b200: {n} must be a CUDA int32 tensor on {dev}")
+    rowptr, colidx = rowptr.contiguous(), colidx.contiguous()
+    if rowptr.numel() != S + 1 or colidx.numel() != vals.numel():
+        raise RuntimeError("CSR arrays do not match the number of stations")
+    adj_shape = torch.empty((S, S), device="meta")
+    Ttot, S, F_in, F_hid, F_out, H = _forecast_dims(adj_shape, table, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh)
+    starts = _forecast_starts(starts)
+    N = starts.numel()
+    out = torch.empty((N, H), dtype=torch.float32, device=dev)
+    nbytes = lib.wg_gcn_gru_forecast_csr_workspace_bytes(N, Ttot, seq_length, S, F_in, F_hid, F_out, H, chunk,
+                                                         flags)  # 0: see gcn_gru_forecast
+    ws = _workspace(dev, nbytes, "forecast")
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    _lib.check(
+        lib.wg_gcn_gru_forecast_csr_f32(
+            rowptr.data_ptr(), colidx.data_ptr(), vals.data_ptr(), table.data_ptr(), starts.data_ptr(),
+            w1.data_ptr(), b1.data_ptr(), w2.data_ptr(), b2.data_ptr(), w_ih.data_ptr(), w_hh.data_ptr(),
+            b_ih.data_ptr(), b_hh.data_ptr(), out.data_ptr(), N, Ttot, seq_length, S, F_in, F_hid, F_out, H, chunk,
+            flags, ws.data_ptr(), ws.numel(), dev.index or 0, stream,
+        )
+    )
+    return out
+
+
+@gcn_gru_forecast_csr.register_fake
+def _(rowptr, colidx, vals, table, starts, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, seq_length, chunk=0, flags=0):
+    return table.new_empty((starts.shape[0], w_hh.shape[1]))
 
 
 def dense_to_csr(adj: torch.Tensor):

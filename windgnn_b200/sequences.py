@@ -106,6 +106,34 @@ def create_sequences(table: torch.Tensor, seq_length: int = SEQ_LENGTH, perm: to
     return x, y
 
 
+def window_starts(n_rows: int, seq_length: int = SEQ_LENGTH, stride: int = 1, horizons: int = 0) -> torch.Tensor:
+    """CPU int64 first rows ``0, stride, 2 stride, ...`` of every window of ``seq_length`` rows that has
+    ``horizons`` label rows after it in a table of ``n_rows`` rows (``GCN_GRU.forecast``).  ``stride=1``: one
+    forecast per hour; ``stride=seq_length, horizons=3``: the reference's non-overlapping windows (step4:10-16),
+    ``num_windows`` of them."""
+    if seq_length < 1 or stride < 1 or horizons < 0:
+        raise ValueError("seq_length and stride must be >= 1, horizons >= 0")
+    return torch.arange(0, max(n_rows - seq_length - horizons + 1, 0), stride, dtype=torch.int64)
+
+
+def forecast_targets(table: torch.Tensor, starts: torch.Tensor, seq_length: int = SEQ_LENGTH,
+                     label_feature: int = LABEL_FEATURE, horizons: int = HORIZONS) -> torch.Tensor:
+    """``[N, horizons * S]`` targets of each window's last step, ``y[n, k*S + s] = table[starts[n] + L + k, s,
+    label_feature]``: what ``create_sequences(...)[1][:, -1]`` holds for ``starts = perm * L`` (step4:14-18), for
+    any starts.  Index plumbing only, on ``table``'s device."""
+    if table.dim() != 3:
+        raise RuntimeError("table must be [time, station, feature]")
+    if starts.dtype != torch.int64 or starts.dim() != 1:
+        raise RuntimeError("starts must be a 1-D int64 tensor")
+    Ttot, S, _ = table.shape
+    starts = starts.to(table.device)
+    if starts.numel() and (int(starts.min()) < 0 or int(starts.max()) + seq_length + horizons > Ttot):
+        raise RuntimeError(f"starts must lie in [0, {Ttot - seq_length - horizons}] so that every window has "
+                           f"{horizons} label rows after it")
+    rows = starts[:, None] + seq_length + torch.arange(horizons, device=table.device)
+    return table[rows, :, label_feature].reshape(starts.numel(), horizons * S)
+
+
 def denormalise_last_step(outputs: torch.Tensor, wind_min: float, wind_max: float) -> torch.Tensor:
     """``outputs [B, T, H]`` (or ``[T, H]``) -> ``[B, H]``: ``out[:, -1] * (max - min) + min`` in
     fp32 with NumPy's rounding (main.py:103) — only ``3S`` floats per window leave the GPU."""
