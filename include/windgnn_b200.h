@@ -66,12 +66,15 @@ const char* wg_last_error(void);
  * `chunk` = sequences processed per internal pass (bounds the workspace); 0 = default.
  * `flags`: 0 = every contraction as FP32 FMA (the reference's arithmetic, different summation
  *   order).  WG_FLAG_TENSOR_CORES = the GRU input projection (65 % of the FLOPs) and, for H <= 128,
- *   the recurrent product h.W_hh^T run on the tcgen05 tensor cores: each operand is split into two
- *   fp16 parts (x = hi + lo, 22 significant bits) and a product is hi*hi + hi*lo + lo*hi with fp32
- *   accumulation; the error against fp64 is the same size as the FP32 path's and the path is held
- *   to the same 1e-5 parity bar.  Operand magnitudes must stay inside the fp16 range (|x| < 65504;
- *   the GCN outputs and the weights of the shipped models are O(1)).  Results do not depend on how
- *   a batch is split.  The workspace must be sized with the same flags.
+ *   the recurrent product h.W_hh^T run on the tcgen05 tensor cores: each operand row (a row of
+ *   U = the GCN output, of W_ih, of W_hh; h as a whole) is scaled by a power of two that puts its
+ *   largest magnitude in [2^14, 2^15), then split into two fp16 parts (x = hi + lo, 22 significant
+ *   bits for every element down to 2^-17 of its row's largest), and a product is hi*hi + hi*lo +
+ *   lo*hi with fp32 accumulation, unscaled once in fp32.  The error against fp64 is therefore the
+ *   same size as the FP32 path's at any operand scale (row maxima from 2^-49 to 2^78; beyond, the
+ *   scale stops at 2^+-63), no operand overflows fp16, and rescaling a model's operands by powers
+ *   of two leaves the result bit-identical.  The path is held to the same 1e-5 parity bar.  Results
+ *   do not depend on how a batch is split.  The workspace must be sized with the same flags.
  *
  * The workspace queries of the forward (this one, the CSR and the host-buffer ones below) return 0
  * for every shape (dims, chunk and flags) their entry point rejects, and wg_last_error() says why.

@@ -301,19 +301,33 @@ def test_tensor_core_path_full_size(full34):
     assert normalised_max_error(yt[idx].cpu().numpy(), ref) <= TOL
 
 
-@pytest.mark.parametrize("S,H,B,T", [(3, 9, 33, 7), (12, 36, 70, 11), (20, 50, 31, 6), (40, 150, 9, 5)])
+@pytest.mark.parametrize("S,H,B,T", [(3, 9, 33, 7), (12, 36, 70, 11), (20, 50, 31, 6), (40, 150, 9, 5),
+                                     (10, 128, 40, 5),    # three 128-column projection slices, largest tcgen05 recurrence
+                                     (10, 129, 20, 4),    # tensor projection feeding the FP32 recurrence
+                                     (5, 11, 25, 6),      # N = 48: the epilogue's second column half is partial
+                                     (1, 8, 37, 5),       # K = 13: less than one 32-k stage
+                                     (32, 96, 19, 3),     # K = 416: whole 32-k stages, no padding
+                                     (34, 102, 1, 1), (34, 102, 17, 1), (34, 102, 33, 1)])   # T = 1, ragged groups
 def test_tensor_core_path_ragged_shapes(S, H, B, T):
+    """Against float32 and float64 oracles; a chunked call (17 sequences per pass) is bit-identical."""
     m = _random_model(S, seed=S * 7 + B, H=H)
     sd = {k: v.detach().clone() for k, v in m.state_dict().items()}
     rng = np.random.default_rng(B + 1)
     adj = (rng.random((S, S), dtype=np.float32) / S).astype(np.float32)
     x = rng.random((B, T, S, 13), dtype=np.float32)
     ref = gcn_gru_forward(adj, x, sd, dtype=np.float32)
+    ref64 = gcn_gru_forward(adj, x, sd, dtype=np.float64)
     m = m.to(DEV)
     m.precision = "tf32x3"
+    a, xd = torch.from_numpy(adj).to(DEV), torch.from_numpy(x).to(DEV)
     with torch.no_grad():
-        y = m(torch.from_numpy(adj).to(DEV), torch.from_numpy(x).to(DEV)).reshape(B, T, H).cpu().numpy()
+        y = m(a, xd).reshape(B, T, H)
+        m.chunk = 17
+        yc = m(a, xd).reshape(B, T, H)
+    assert torch.equal(yc, y)
+    y = y.cpu().numpy()
     assert normalised_max_error(y, ref) <= TOL
+    assert normalised_max_error(y, ref64) <= TOL
 
 
 def _scaled_model(S, Fh, H, seed):

@@ -97,6 +97,9 @@ struct Plan {
     size_t rc_smem;    //                   its dynamic shared memory
     size_t off_wp, off_bias, off_wht, off_whu, off_bhn, off_u, off_gi, off_z, total;
     size_t off_whh_hi, off_whh_lo;   // kRecurTc: W_hh packed as fp16 hi + lo
+    // tensor path: the inverse power-of-two scales of the split operands (tc_scale_exp), per packed W_ih row (tc2.NP)
+    // then per packed W_hh row ([3][128], h's scale folded in); the largest element of every U row (float bits)
+    size_t off_tcs, off_umax;
 };
 
 long long default_chunk(long long B, size_t bytes_per_seq) {
@@ -230,6 +233,7 @@ int plan_layout(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int 
     // packed w_ih: fp32 [N/64][K][64] for the FFMA GEMM, or fp16 hi + lo stage blocks for the tensor cores
     p.off_wp = o;   o = align_up(o + (p.tc ? wg::tc2_w_halves(p.tc2) * 2 : (size_t)p.NPB * p.IP * 4));
     p.off_bias = o; o = align_up(o + (size_t)p.n_bias * 4);
+    p.off_tcs = o;  if (p.tc) o = align_up(o + ((size_t)p.tc2.NP + 3 * 128) * 4);
     p.off_wht = o;  o = align_up(o + (size_t)p.KP * p.NPR * 4);
     p.off_whu = o;  // [k][gate][unit] (recur_unit.cuh)
     if (p.whu) o = align_up(o + (size_t)p.KP * 3 * wg::recur_u_hp2(H) * 4);
@@ -240,6 +244,7 @@ int plan_layout(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int 
     const size_t rows = table_rows > 0 ? (size_t)forecast_piece_rows(p, table_rows) : (size_t)p.chunk * T;
     const size_t rows_tiled = (rows + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows;
     p.off_u = o;    o = align_up(o + rows_tiled * p.IP * 4);  // K-major 128-row tiles
+    p.off_umax = o; if (p.tc) o = align_up(o + rows_tiled * 4);
     // GI: the tensor-core recurrence reads whole groups of kRtSeqs sequences (rows past the batch are scratch)
     const size_t rows_gi =
         table_rows > 0 ? (size_t)table_rows : (size_t)((p.chunk + wg::kRtSeqs - 1) / wg::kRtSeqs * wg::kRtSeqs) * T;
@@ -403,17 +408,20 @@ int launch_gcn_dense(GcnKind k, int RB, size_t smem, const float* X, const float
 }
 
 // second-generation fused two-layer kernel (gcn_rows.cuh): lane = row, output straight into the tiles
+// (the tensor path's instantiation also records the U row maxima in umax, cleared here)
 int launch_gcn_rows(const Plan& p, const float* X, const float* adj, const float* W1, const float* b1,
-                    const float* W2, const float* b2, float* out, long long R, cudaStream_t st) {
-    WG_CUDA(cudaFuncSetAttribute(wg::gcn_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.gcn_smem));
+                    const float* W2, const float* b2, float* out, int* umax, long long R, cudaStream_t st) {
+    auto kern = p.tc ? wg::gcn_rows_kernel<true> : wg::gcn_rows_kernel<false>;
+    if (p.tc) WG_CUDA(cudaMemsetAsync(umax, 0, (size_t)(R + wg::kT2BM - 1) / wg::kT2BM * wg::kT2BM * 4, st));
+    WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.gcn_smem));
     int per_sm = 0;
-    WG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wg::gcn_rows_kernel, p.gcn_threads, p.gcn_smem));
+    WG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, p.gcn_threads, p.gcn_smem));
     if (per_sm < 1) per_sm = 1;
     const long long nblocks = (R + wg::kGrRows - 1) / wg::kGrRows;
     long long grid = (long long)wg::kNumSMs * per_sm;
     if (grid > nblocks) grid = nblocks;
     if (grid < 1) return WG_OK;
-    wg::gcn_rows_kernel<<<(unsigned)grid, p.gcn_threads, p.gcn_smem, st>>>(X, adj, W1, b1, W2, b2, out, R, p.S, p.IP);
+    kern<<<(unsigned)grid, p.gcn_threads, p.gcn_smem, st>>>(X, adj, W1, b1, W2, b2, out, R, p.S, p.IP, umax);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
@@ -471,14 +479,22 @@ int launch_gcn_sparse(const Plan& p, void* ws, const Graph& g, const float* x, c
     return WG_OK;
 }
 
-// The plan's two-layer GCN over `rows` = sequences x steps, into the projection's U tiles.
+// The plan's two-layer GCN over `rows` = sequences x steps, into the projection's U tiles; on the tensor path also
+// the largest element of every U row, which sets the row's scale in the projection (gcn_rows_kernel records it while
+// it writes U, u_rowmax_kernel reads it back after the other GCN kernels).
 int launch_gcn(const Plan& p, void* ws, const Graph& g, const float* x, const float* w1, const float* b1,
                const float* w2, const float* b2, long long rows, cudaStream_t st) {
     float* u = ws_ptr<float>(ws, p.off_u);
-    if (p.gcn == kGcnRows) return launch_gcn_rows(p, x, g.adj, w1, b1, w2, b2, u, rows, st);
-    if (p.sparse) return launch_gcn_sparse(p, ws, g, x, w1, b1, w2, b2, rows, st);
-    return launch_gcn_dense<2, true>(p.gcn, p.gcn_rb, p.gcn_smem, x, g.adj, w1, b1, w2, b2, u, rows, p.S, p.Fi, p.Fh,
-                                     p.Fo, p.IP, st);
+    int* umax = ws_ptr<int>(ws, p.off_umax);
+    if (p.gcn == kGcnRows) return launch_gcn_rows(p, x, g.adj, w1, b1, w2, b2, u, umax, rows, st);
+    const int rc = p.sparse ? launch_gcn_sparse(p, ws, g, x, w1, b1, w2, b2, rows, st)
+                            : launch_gcn_dense<2, true>(p.gcn, p.gcn_rb, p.gcn_smem, x, g.adj, w1, b1, w2, b2, u, rows,
+                                                        p.S, p.Fi, p.Fh, p.Fo, p.IP, st);
+    if (rc || !p.tc || rows < 1) return rc;
+    const long long rt = (rows + wg::kT2BM - 1) / wg::kT2BM * wg::kT2BM;
+    wg::u_rowmax_kernel<<<(unsigned)((rt + 255) / 256), 256, 0, st>>>(u, umax, rows, p.IP);
+    WG_CUDA(cudaGetLastError());
+    return WG_OK;
 }
 
 // The projection of the `rows` U rows into GI rows gi[0 .. rows) (row stride p.GP).
@@ -491,8 +507,9 @@ int launch_inproj_tc(const Plan& p, void* ws, long long rows, cudaStream_t st, f
     const long long tiles = m_tiles * t.n_nt;
     const unsigned grid = (unsigned)(tiles < wg::kNumSMs ? tiles : wg::kNumSMs);
     wg::inproj_tc2_kernel<<<grid, wg::kT2Threads, t.smem_bytes, st>>>(
-        ws_ptr<float>(ws, p.off_u), ws_ptr<__half>(ws, p.off_wp), ws_ptr<float>(ws, p.off_bias), gi, rows, p.IP,
-        t.KP, p.GP, t.n_nt, t.N_each, t.stages);
+        ws_ptr<float>(ws, p.off_u), ws_ptr<int>(ws, p.off_umax), ws_ptr<__half>(ws, p.off_wp),
+        ws_ptr<float>(ws, p.off_tcs), ws_ptr<float>(ws, p.off_bias), gi, rows, p.IP, t.KP, p.GP, t.n_nt, t.N_each,
+        t.stages);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
@@ -608,8 +625,9 @@ int launch_recur_tc(const Plan& p, void* ws, float* out, long long Bc, cudaStrea
     const long long grid = (Bc + wg::kRtSeqs - 1) / wg::kRtSeqs;
     if (grid < 1) return WG_OK;
     kern<<<(unsigned)grid, wg::kRtThreads, smem, st>>>(ws_ptr<float>(ws, p.off_gi), ws_ptr<__half>(ws, p.off_whh_hi),
-                                                      ws_ptr<__half>(ws, p.off_whh_lo), ws_ptr<float>(ws, p.off_bhn),
-                                                      out, Bc, p.T, p.H, p.GP, row0);
+                                                      ws_ptr<__half>(ws, p.off_whh_lo),
+                                                      ws_ptr<float>(ws, p.off_tcs) + p.tc2.NP,
+                                                      ws_ptr<float>(ws, p.off_bhn), out, Bc, p.T, p.H, p.GP, row0);
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
@@ -643,13 +661,15 @@ int launch_pack(const Plan& p, void* ws, const float* w_ih, const float* w_hh, c
         p.I, p.H, p.IP, p.NPB, p.KP, p.NPR, p.tc ? 0 : 1, p.n_bias);
     WG_CUDA(cudaGetLastError());
     if (p.tc) {
-        wg::pack_wih_tc2_kernel<<<wg::kNumSMs * 2, 256, 0, st>>>(w_ih, ws_ptr<__half>(ws, p.off_wp), p.G, p.I, p.tc2.KP,
-                                                                p.tc2.n_nt, p.tc2.N_each);
+        wg::pack_wih_tc2_kernel<<<wg::kNumSMs, 256, 0, st>>>(w_ih, ws_ptr<__half>(ws, p.off_wp),
+                                                            ws_ptr<float>(ws, p.off_tcs), p.G, p.I, p.tc2.KP,
+                                                            p.tc2.n_nt, p.tc2.N_each);
         WG_CUDA(cudaGetLastError());
     }
     if (p.recur == kRecurTc) {
-        wg::pack_whh_tc_kernel<<<wg::kNumSMs, 256, 0, st>>>(w_hh, ws_ptr<__half>(ws, p.off_whh_hi),
-                                                           ws_ptr<__half>(ws, p.off_whh_lo), p.H);
+        wg::pack_whh_tc_kernel<<<48, 256, 0, st>>>(w_hh, ws_ptr<__half>(ws, p.off_whh_hi),
+                                                  ws_ptr<__half>(ws, p.off_whh_lo),
+                                                  ws_ptr<float>(ws, p.off_tcs) + p.tc2.NP, p.H);
         WG_CUDA(cudaGetLastError());
     }
     return WG_OK;

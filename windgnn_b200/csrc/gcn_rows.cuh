@@ -234,13 +234,15 @@ __device__ __forceinline__ float2 gr_bias(float2 o, float b) { return __fadd2_rn
 // One row block through both layers for a warp that owns NPW station pairs starting at station s0.
 // SHARED (balanced mode): additionally this warp's feature / column slice f0 .. f0 + 3 of the shared pair
 // (stations 32, 33); xch = this lane's two exchange rows (layer 1, layer 2: kGrRows * kGrXS floats apart).
-template <int NPW, bool SHARED>
+// ROWMAX (tensor path): the largest value this warp writes to the lane's row goes to *umax_row (atomicMax of the
+// float bits, which order like integers for U >= 0).
+template <int NPW, bool SHARED, bool ROWMAX>
 __device__ __forceinline__ void gr_block(float* __restrict__ buf, const float* __restrict__ arow, int astride,
                                          const float* __restrict__ w1d, const float* __restrict__ b1s,
                                          const float* __restrict__ w2d, const float* __restrict__ b2s, int S, int s0,
                                          int lane, bool row_ok, float* __restrict__ out_col0, int ldo, bool pad_warp,
                                          const float* __restrict__ next_src, unsigned next_bytes, uint64_t* bar,
-                                         float* __restrict__ xch, int f0) {
+                                         float* __restrict__ xch, int f0, int* __restrict__ umax_row) {
     constexpr int SNF = kGrSliceW;
     constexpr int SS = 32;   // the shared pair's first station (pair 16)
     const int SF0 = f0;
@@ -304,6 +306,7 @@ __device__ __forceinline__ void gr_block(float* __restrict__ buf, const float* _
         mbar_expect_tx(bar, next_bytes);
         bulk_g2s(buf, next_src, next_bytes, bar);
     }
+    float vmax = 0.0f;   // ROWMAX
     auto store_u = [&](const float2 (&o)[NPW][4], int c0, auto width) {
         constexpr int W = decltype(width)::value;
         const float4 bb = *reinterpret_cast<const float4*>(b2s + c0);
@@ -319,6 +322,7 @@ __device__ __forceinline__ void gr_block(float* __restrict__ buf, const float* _
                     const float2 u = gr_bias(o[p][c], bv[c]);
                     c_lo[(size_t)c * kUTileRows] = gr_relu(u.x);
                     if (s + 1 < S) c_lo[(size_t)(kGrF + c) * kUTileRows] = gr_relu(u.y);
+                    if (ROWMAX) vmax = fmaxf(vmax, s + 1 < S ? fmaxf(gr_relu(u.x), gr_relu(u.y)) : gr_relu(u.x));
                 }
             }
         }
@@ -343,18 +347,23 @@ __device__ __forceinline__ void gr_block(float* __restrict__ buf, const float* _
                 const float2 u = gr_bias(o[j], b2s[SF0 + j]);
                 c_lo[(size_t)j * kUTileRows] = gr_relu(u.x);
                 if (SS + 1 < S) c_lo[(size_t)(kGrF + j) * kUTileRows] = gr_relu(u.y);
+                if (ROWMAX) vmax = fmaxf(vmax, SS + 1 < S ? fmaxf(gr_relu(u.x), gr_relu(u.y)) : gr_relu(u.x));
             }
         }
     }
     if (pad_warp && row_ok)   // zero the K padding of the projection GEMM
         for (int c = in_cols; c < ldo; ++c) out_col0[(size_t)c * kUTileRows] = 0.0f;
+    if (ROWMAX && row_ok) atomicMax(umax_row, __float_as_int(vmax));
 }
 
 // X [R][S][13] -> out [ceil(R/128)][ldo][128] (K-major row tiles, columns >= S*13 zero)
+// ROWMAX (the tensor path's instantiation): also umax[r] = max(umax[r], the largest element of U row r), float bits
+// (umax cleared by the caller)
+template <bool ROWMAX>
 __global__ void __launch_bounds__(kGrMaxWarps * 32, 1)
     gcn_rows_kernel(const float* __restrict__ X, const float* __restrict__ adj, const float* __restrict__ W1,
                     const float* __restrict__ b1, const float* __restrict__ W2, const float* __restrict__ b2,
-                    float* __restrict__ out, long long R, int S, int ldo) {
+                    float* __restrict__ out, long long R, int S, int ldo, int* __restrict__ umax) {
     extern __shared__ __align__(16) float smem[];
     const int NW = gcn_rows_warps(S);
     const int nthreads = NW * 32;
@@ -446,14 +455,15 @@ __global__ void __launch_bounds__(kGrMaxWarps * 32, 1)
         float* out_col0 = out + (size_t)(r / kUTileRows) * ldo * kUTileRows + (r % kUTileRows);
         const bool row_ok = lane < nrows;
         const bool pad_warp = w == NW - 1;
+        int* umax_row = ROWMAX ? umax + r : nullptr;
 #define WG_GR(N)                                                                                              \
     case N:                                                                                                   \
-        gr_block<N, false>(buf, arow, astride, w1d, b1s, w2d, b2s, S, s0, lane, row_ok, out_col0, ldo,        \
-                           pad_warp, nsrc, nbytes, bar, xch, 0);                                              \
+        gr_block<N, false, ROWMAX>(buf, arow, astride, w1d, b1s, w2d, b2s, S, s0, lane, row_ok, out_col0, ldo, \
+                                   pad_warp, nsrc, nbytes, bar, xch, 0, umax_row);                            \
         break;
         if (balanced) {   // one instruction stream for the four warps; the slice offset is a runtime value
-            gr_block<4, true>(buf, arow, astride, w1d, b1s, w2d, b2s, S, s0, lane, row_ok, out_col0, ldo, pad_warp,
-                              nsrc, nbytes, bar, xch, kGrSliceStep * w);
+            gr_block<4, true, ROWMAX>(buf, arow, astride, w1d, b1s, w2d, b2s, S, s0, lane, row_ok, out_col0, ldo,
+                                      pad_warp, nsrc, nbytes, bar, xch, kGrSliceStep * w, umax_row);
         } else {
             switch (npw) {   // warp-uniform
                 WG_GR(1) WG_GR(2) WG_GR(3) WG_GR(4) WG_GR(5)

@@ -2,6 +2,12 @@
 //     GI = U . W_ih^T + b,   x = hi + lo with hi = fp16(x), lo = fp16(x - hi)   (22 significant bits)
 //     U.W ~= U_hi.W_hi + U_hi.W_lo + U_lo.W_hi        (kind::f16: fp16 x fp16 products are exact in the
 //                                                      fp32 accumulator; the dropped lo.lo term is 2^-22)
+// Before the split each U row and each W_ih row (gate column) is scaled by a power of two (tc_scale_exp, recur_tc.cuh)
+// that maps its largest magnitude into [2^14, 2^15); the epilogue undoes both with one factor per output,
+//     GI[r][c] = (acc_hi + acc_corr) * 2^-(e_r + e_c) + b[c],
+// so the relative error of the split does not depend on the scale of U or W_ih and no operand leaves the fp16 range.
+// The largest element of each U row (U >= 0 after the ReLU: float bits compare as integers) is recorded in umax by
+// the GCN kernel that writes the row, or by u_rowmax_kernel.
 //
 // Reference: the `gi = W_ih u + b_ih` half of nn.GRU, src/step6_gcn_gru_combined_model.py:11,23.
 //
@@ -14,14 +20,14 @@
 //
 // One persistent CTA per SM, 14 warps:
 //   warp 12      producer: per stage two bulk async copies (A fp32 16 KB, B hi+lo 20 KB at N = 160)
-//   warps 8-11   converters: a thread takes 2 rows x 8 k's (8-byte loads), splits fp32 -> fp16 hi / lo and
+//   warps 8-11   converters: a thread takes 2 rows x 8 k's (8-byte loads), scales them by 2^e_r, splits fp32 -> fp16 hi / lo and
 //                writes 16-byte chunks into the canonical layout ([k / 8][row][8 halves]: 8-row x 16-byte
 //                core matrices, SBO = 128 B, LBO = rows * 16 B)
 //   warp 13      MMA issuer: 6 x tcgen05.mma.kind::f16 (M = 128, N <= 160, K = 16) per stage;
 //                hi.hi into one TMEM accumulator, the corrections into a second one (TMEM accumulation
 //                truncates: the small terms are kept apart and added in fp32 in the epilogue)
 //   warps 0-7    epilogue: warp w reads TMEM lanes 32 (w % 4) .. and the column half w / 4: tcgen05.ld, sum,
-//                + bias, 32-byte stores (GI rows are 32-byte aligned); the accumulators are released to the
+//                x 2^-(e_r + e_c) + bias (one FMA), 32-byte stores (GI rows are 32-byte aligned); the accumulators are released to the
 //                issuer as soon as a warp's last block is in registers
 #pragma once
 
@@ -68,31 +74,54 @@ __host__ inline Tc2Shape tc2_shape(int G, int I) {
 // halves of the packed W_ih (hi and lo together): [n_nt][KP / 32 stages][hi | lo][4 chunks][N_each][8]
 __host__ inline size_t tc2_w_halves(const Tc2Shape& s) { return (size_t)2 * s.NP * s.KP; }
 
-// w_ih [G][I] fp32 -> per (column slice, stage) one contiguous block [hi | lo][k chunk][n][8 halves]
-__global__ void pack_wih_tc2_kernel(const float* __restrict__ w_ih, __half* __restrict__ wp, int G, int I, int KP,
-                                    int n_nt, int N_each) {
-    const long long total = (long long)2 * n_nt * N_each * KP;
-    const int nst = KP / kT2BK;
-    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total;
-         e += (long long)gridDim.x * blockDim.x) {
-        long long r = e;
-        const int kk = (int)(r & 7); r >>= 3;
-        const int nl = (int)(r % N_each); r /= N_each;
-        const int c = (int)(r & 3); r >>= 2;
-        const int part = (int)(r & 1); r >>= 1;
-        const int kb = (int)(r % nst), nt = (int)(r / nst);
-        const int n = nt * N_each + nl, k = kb * kT2BK + c * 8 + kk;
-        const float v = (n < G && k < I) ? w_ih[(size_t)n * I + k] : 0.0f;
-        const __half h = __float2half_rn(v);
-        wp[e] = part == 0 ? h : __float2half_rn(v - __half2float(h));
+// w_ih [G][I] fp32 -> per (column slice, stage) one contiguous block [hi | lo][k chunk][n][8 halves], gate column n
+// scaled by 2^e(n) before the split; colinv [NP] = 2^-e(n).  One warp per gate column.
+__global__ void pack_wih_tc2_kernel(const float* __restrict__ w_ih, __half* __restrict__ wp, float* __restrict__ colinv,
+                                    int G, int I, int KP, int n_nt, int N_each) {
+    const int nst = KP / kT2BK, NP = n_nt * N_each, lane = threadIdx.x & 31;
+    const int nwarps = gridDim.x * blockDim.x / 32;
+    for (int n = (blockIdx.x * blockDim.x + threadIdx.x) / 32; n < NP; n += nwarps) {
+        const float* w = w_ih + (size_t)(n < G ? n : 0) * I;
+        float m = 0.0f;
+        if (n < G)
+            for (int k = lane; k < I; k += 32) m = fmaxf(m, fabsf(w[k]));
+        const int e = tc_scale_exp(warp_max(m));
+        const float sc = tc_exp2(e);
+        if (lane == 0) colinv[n] = tc_exp2(-e);
+        const int nt = n / N_each, nl = n % N_each;
+        for (int k = lane; k < KP; k += 32) {
+            const float v = (n < G && k < I) ? w[k] * sc : 0.0f;
+            // [nt][k / 32][part][k % 32 / 8][nl][k % 8]; the lo part is 4 chunks further
+            const size_t idx = ((((size_t)nt * nst + k / kT2BK) * 2 * 4 + (k % kT2BK) / 8) * N_each + nl) * 8 + k % 8;
+            const __half h = __float2half_rn(v);
+            wp[idx] = h;
+            wp[idx + (size_t)4 * N_each * 8] = __float2half_rn(v - __half2float(h));
+        }
     }
 }
 
+// umax[r] = the largest element of U row r (>= 0: float bits), for whole 128-row tiles (0 past `rows`); for the GCN
+// kernels that do not record it while they write U.  A thread per row: a warp reads 128 contiguous bytes per k.
+__global__ void __launch_bounds__(256) u_rowmax_kernel(const float* __restrict__ U, int* __restrict__ umax,
+                                                       long long rows, int ldk) {
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= (rows + kT2BM - 1) / kT2BM * kT2BM) return;
+    float m = 0.0f;
+    if (r < rows) {
+        const float* u = U + (size_t)(r / kT2BM) * ldk * kT2BM + r % kT2BM;
+#pragma unroll 8
+        for (int k = 0; k < ldk; ++k) m = fmaxf(m, __ldg(u + (size_t)k * kT2BM));
+    }
+    umax[r] = __float_as_int(m);
+}
+
 // A: U tiles [M/128][lda][128] fp32 (lda >= KP, K-major 128-row tiles written by the GCN kernels);
-// Wp: pack_wih_tc2_kernel's output;  C: [M][ldc] row-major (GI)
+// umax: [whole tiles of M rows] row maxima (float bits); Wp, colinv: pack_wih_tc2_kernel's output;
+// C: [M][ldc] row-major (GI)
 __global__ void __launch_bounds__(kT2Threads, 1)
-    inproj_tc2_kernel(const float* __restrict__ A, const __half* __restrict__ Wp, const float* __restrict__ bias,
-                      float* __restrict__ C, long long M, int lda, int KP, int ldc, int n_nt, int N_each, int stages) {
+    inproj_tc2_kernel(const float* __restrict__ A, const int* __restrict__ umax, const __half* __restrict__ Wp,
+                      const float* __restrict__ colinv, const float* __restrict__ bias, float* __restrict__ C,
+                      long long M, int lda, int KP, int ldc, int n_nt, int N_each, int stages) {
     extern __shared__ __align__(1024) unsigned char smem_t2[];
     const uint32_t a32_bytes = kT2BM * kT2BK * 4;                   // 16 KB
     const uint32_t a16_bytes = kT2BM * kT2BK * 2;                   // 8 KB per part
@@ -160,6 +189,10 @@ __global__ void __launch_bounds__(kT2Threads, 1)
         int s = 0;
         uint32_t phase = 0;
         for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+            // this thread's rows 2 rp, 2 rp + 1 (rp = ct % 64 for both items): their scales 2^e_r
+            const long long r0 = tile / n_nt * kT2BM + 2 * (ct & 63);
+            const float sc0 = tc_exp2(tc_scale_exp(__int_as_float(__ldg(umax + r0))));
+            const float sc1 = tc_exp2(tc_scale_exp(__int_as_float(__ldg(umax + r0 + 1))));
             for (int kb = 0; kb < KB; ++kb) {
                 mbar_wait(&full_ld[s], phase);
                 unsigned char* st = smem_t2 + (size_t)s * stage_bytes;
@@ -172,7 +205,11 @@ __global__ void __launch_bounds__(kT2Threads, 1)
                     unsigned char* lo = hi + a16_bytes;
                     float2 v[8];
 #pragma unroll
-                    for (int kk = 0; kk < 8; ++kk) v[kk] = *reinterpret_cast<const float2*>(a32 + kk * kT2BM);
+                    for (int kk = 0; kk < 8; ++kk) {
+                        v[kk] = *reinterpret_cast<const float2*>(a32 + kk * kT2BM);
+                        v[kk].x *= sc0;
+                        v[kk].y *= sc1;
+                    }
                     __half2 h0[4], l0[4], h1[4], l1[4];   // row 2 rp / row 2 rp + 1: k pairs
 #pragma unroll
                     for (int q = 0; q < 4; ++q) {
@@ -245,6 +282,7 @@ __global__ void __launch_bounds__(kT2Threads, 1)
             tc_fence_after();
             const long long row = mt * kT2BM + lq * 32 + lane;
             float* crow = C + (size_t)(row < M ? row : 0) * ldc;
+            const float rinv = tc_exp2(-tc_scale_exp(__int_as_float(__ldg(umax + row))));   // 2^-e_r
             const uint32_t lane_base = tmem_base + ((uint32_t)(lq * 32) << 16);
             for (int c0 = cbeg; c0 < cend; c0 += 32) {
                 float v0[32], v1[32];
@@ -260,26 +298,28 @@ __global__ void __launch_bounds__(kT2Threads, 1)
                     for (int q = 0; q < 4; ++q) {
                         const int cl = c0 + 8 * q;            // column inside the slice
                         const int c = nt * N_each + cl;       // gate column
+                        // bias and colinv hold NP >= c + 8 entries
+                        const float4 b0 = __ldg(reinterpret_cast<const float4*>(bias + c));
+                        const float4 b1 = __ldg(reinterpret_cast<const float4*>(bias + c + 4));
+                        const float4 f0 = __ldg(reinterpret_cast<const float4*>(colinv + c));
+                        const float4 f1 = __ldg(reinterpret_cast<const float4*>(colinv + c + 4));
+                        const float bb[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+                        const float ff[8] = {f0.x, f0.y, f0.z, f0.w, f1.x, f1.y, f1.z, f1.w};
                         float o[8];
 #pragma unroll
-                        for (int e = 0; e < 8; ++e) o[e] = v0[8 * q + e] + v1[8 * q + e];
+                        for (int e = 0; e < 8; ++e) o[e] = fmaf(v0[8 * q + e] + v1[8 * q + e], rinv * ff[e], bb[e]);
                         if (cl + 8 <= cend && c + 8 <= ldc && wide) {
-                            const float4 b0 = __ldg(reinterpret_cast<const float4*>(bias + c));
-                            const float4 b1 = __ldg(reinterpret_cast<const float4*>(bias + c + 4));
                             asm volatile("st.global.v8.f32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};\n" ::"l"(crow + c),
-                                         "f"(o[0] + b0.x), "f"(o[1] + b0.y), "f"(o[2] + b0.z), "f"(o[3] + b0.w),
-                                         "f"(o[4] + b1.x), "f"(o[5] + b1.y), "f"(o[6] + b1.z), "f"(o[7] + b1.w)
+                                         "f"(o[0]), "f"(o[1]), "f"(o[2]), "f"(o[3]), "f"(o[4]), "f"(o[5]), "f"(o[6]),
+                                         "f"(o[7])
                                          : "memory");
                         } else {
 #pragma unroll
                             for (int hq = 0; hq < 2; ++hq) {
                                 const int c4 = c + 4 * hq;
-                                if (cl + 4 * hq < cend && c4 < ldc) {
-                                    const float4 b4 = __ldg(reinterpret_cast<const float4*>(bias + c4));
+                                if (cl + 4 * hq < cend && c4 < ldc)
                                     *reinterpret_cast<float4*>(crow + c4) =
-                                        make_float4(o[4 * hq] + b4.x, o[4 * hq + 1] + b4.y, o[4 * hq + 2] + b4.z,
-                                                    o[4 * hq + 3] + b4.w);
-                                }
+                                        make_float4(o[4 * hq], o[4 * hq + 1], o[4 * hq + 2], o[4 * hq + 3]);
                             }
                         }
                     }

@@ -10,6 +10,9 @@
 // with both operands split into two fp16 parts, x = hi + lo (hi = fp16(x), lo = fp16(x - hi): 22
 // significant bits, and fp16 x fp16 products are exact in the fp32 accumulator):
 //     D ~= A_hi.B_hi + A_hi.B_lo + A_lo.B_hi          (kind::f16, M = 128, N = 16, K = 16)
+// Both operands are scaled by powers of two before the split (tc_scale_exp: a W_hh row by its own exponent, h by
+// the fixed 2^kTcHExp) and the gate phase undoes both with one factor per gate and hidden unit, so the split keeps
+// its 22 bits whatever the magnitude of W_hh or h.
 // The A_hi.B_hi products go to one TMEM accumulator, the two corrections to a second one (TMEM
 // accumulation truncates — tcgen05.cuh — so the small terms are kept apart from the big ones and the
 // two are added with round-to-nearest in the epilogue).  The dropped lo.lo term is 2^-22 relative.
@@ -95,35 +98,63 @@ __device__ __forceinline__ void tmem_ld_wait(float (&v)[8]) {
 }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory"); }
 
-// w_hh [3H][H] fp32 -> hi / lo fp16 parts in the UMMA K-major layout [gate][k / 8][128 rows][k % 8]
+// Power-of-two scales of the split fp16 operands.  Unscaled, lo = fp16(x - hi) is an fp16 subnormal below |x| = 2^-3
+// (a fixed absolute error of 2^-25, so the relative precision falls with the magnitude) and hi overflows above 65504.
+// A row whose largest magnitude is m is multiplied by 2^e with m 2^e in [2^14, 2^15) before the split and the
+// product by 2^-e after it, in fp32: every element down to 2^-17 m keeps 22 significant bits, at any m, and a row
+// rescaled by a power of two splits into exactly rescaled parts.  e is clamped to [-kTcExpMax, kTcExpMax] so that
+// the product of two inverse factors is a normal fp32; a zero, infinite or NaN m gets e = 0.
+constexpr int kTcExpMax = 63;
+constexpr int kTcHExp = 14;   // the GRU state: |h| < 1, a fixed 2^14
+__device__ __forceinline__ int tc_scale_exp(float m) {
+    if (!(m > 0.0f) || !(m <= 3.402823466e38f)) return 0;
+    int E;
+    frexpf(m, &E);   // m = f 2^E, f in [0.5, 1)
+    const int e = 15 - E;
+    return e < -kTcExpMax ? -kTcExpMax : (e > kTcExpMax ? kTcExpMax : e);
+}
+__device__ __forceinline__ float tc_exp2(int e) { return __int_as_float((127 + e) << 23); }   // e in [-126, 127]
+__device__ __forceinline__ float warp_max(float v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
+    return v;
+}
+
+// w_hh [3H][H] fp32 -> hi / lo fp16 parts in the UMMA K-major layout [gate][k / 8][128 rows][k % 8], each row
+// (gate g, hidden unit j) scaled by 2^e(row) before the split; funit [3][128] = 2^-(e(row) + kTcHExp), the factor
+// that undoes the row's and h's scales.  One warp per row.
 __global__ void pack_whh_tc_kernel(const float* __restrict__ w_hh, __half* __restrict__ hi, __half* __restrict__ lo,
-                                   int H) {
-    const int nch = recur_tc_kp(H) / 8;
-    const long long total = (long long)3 * nch * 128 * 8;
-    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total;
-         e += (long long)gridDim.x * blockDim.x) {
-        const int kk = (int)(e & 7);
-        long long r = e >> 3;
-        const int j = (int)(r % 128);
-        r /= 128;
-        const int c = (int)(r % nch), g = (int)(r / nch);
-        const int k = c * 8 + kk;
-        const float v = (j < H && k < H) ? w_hh[((size_t)g * H + j) * H + k] : 0.0f;
-        const __half h = __float2half_rn(v);
-        hi[e] = h;
-        lo[e] = __float2half_rn(v - __half2float(h));
+                                   float* __restrict__ funit, int H) {
+    const int nch = recur_tc_kp(H) / 8, KP = nch * 8, lane = threadIdx.x & 31;
+    const int nwarps = gridDim.x * blockDim.x / 32;
+    for (int row = (blockIdx.x * blockDim.x + threadIdx.x) / 32; row < 3 * 128; row += nwarps) {
+        const int g = row / 128, j = row % 128;
+        const float* w = w_hh + ((size_t)g * H + (j < H ? j : 0)) * H;
+        float m = 0.0f;
+        if (j < H)
+            for (int k = lane; k < H; k += 32) m = fmaxf(m, fabsf(w[k]));
+        const int e = tc_scale_exp(warp_max(m));
+        const float sc = tc_exp2(e);
+        if (lane == 0) funit[row] = tc_exp2(-e - kTcHExp);
+        for (int k = lane; k < KP; k += 32) {
+            const float v = (j < H && k < H) ? w[k] * sc : 0.0f;
+            const size_t idx = (((size_t)g * nch + k / 8) * 128 + j) * 8 + k % 8;
+            const __half h = __float2half_rn(v);
+            hi[idx] = h;
+            lo[idx] = __float2half_rn(v - __half2float(h));
+        }
     }
 }
 
 // GI [rows][ldg] (b_ih, and b_hh of r / z, folded in; readable up to the next multiple of kRtSeqs sequences);
-// Whi / Wlo: pack_whh_tc_kernel's output; out [B][T][H]
+// Whi / Wlo / funit: pack_whh_tc_kernel's output; out [B][T][H]
 // WIN: windows over one table's gi rows (see gru_recur_unit_kernel): sequence b's gi rows start at GI + row0[b] * ldg
 // (the padding sequences of the last group read the last window's rows), only h at t = T-1 is stored, to out [B][H]
 template <bool WIN = false>
 __global__ void __launch_bounds__(kRtThreads, 1)
     gru_recur_tc_kernel(const float* __restrict__ GI, const __half* __restrict__ Whi, const __half* __restrict__ Wlo,
-                        const float* __restrict__ bhn, float* __restrict__ out, long long B, int T, int H, int ldg,
-                        const long long* __restrict__ row0) {
+                        const float* __restrict__ funit, const float* __restrict__ bhn, float* __restrict__ out,
+                        long long B, int T, int H, int ldg, const long long* __restrict__ row0) {
     extern __shared__ __align__(1024) unsigned char smem_rt[];
     const int KP = recur_tc_kp(H), NCH = KP / 8, NKS = KP / 16;
     const uint32_t a_part = (uint32_t)(3 * NCH * 2048);           // bytes of A_hi (= A_lo)
@@ -174,6 +205,7 @@ __global__ void __launch_bounds__(kRtThreads, 1)
     const bool unit_ok = j < H;
     const int jc = unit_ok ? j : H - 1;
     const float bn = __ldg(bhn + jc);
+    const float fr = __ldg(funit + jc), fz = __ldg(funit + 128 + jc), fn = __ldg(funit + 256 + jc);   // 2^-(e + 14)
     const uint32_t tcol = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(g * 6 * kRtN + half * 8);
     // byte address of this unit inside the group's B operand: chunk j / 8, element j % 8 (row n adds n * 16)
     unsigned char* bh = sB + (size_t)g * b_grp + (size_t)(jc >> 3) * kRtBLbo + (size_t)(jc & 7) * 2 + half * 8 * 16;
@@ -227,19 +259,19 @@ __global__ void __launch_bounds__(kRtThreads, 1)
             tmem_ld_wait(m);
             tmem_ld_wait(c);
 #pragma unroll
-            for (int n = 0; n < 8; ++n) rr[n] = gi[0][n] + (m[n] + c[n]);
+            for (int n = 0; n < 8; ++n) rr[n] = fmaf(m[n] + c[n], fr, gi[0][n]);
             tmem_ld8(tcol + 2 * kRtN, m);
             tmem_ld8(tcol + 3 * kRtN, c);
             tmem_ld_wait(m);
             tmem_ld_wait(c);
 #pragma unroll
-            for (int n = 0; n < 8; ++n) zz[n] = gi[1][n] + (m[n] + c[n]);
+            for (int n = 0; n < 8; ++n) zz[n] = fmaf(m[n] + c[n], fz, gi[1][n]);
             tmem_ld8(tcol + 4 * kRtN, m);
             tmem_ld8(tcol + 5 * kRtN, c);
             tmem_ld_wait(m);
             tmem_ld_wait(c);
 #pragma unroll
-            for (int n = 0; n < 8; ++n) hn[n] = (m[n] + c[n]) + bn;
+            for (int n = 0; n < 8; ++n) hn[n] = fmaf(m[n] + c[n], fn, bn);
             tc_fence_before();   // the accumulators have been read: the next product may overwrite them
         } else {
 #pragma unroll
@@ -257,8 +289,9 @@ __global__ void __launch_bounds__(kRtThreads, 1)
             const float hnew = (hprev[n] - nv) * z + nv;
             hprev[n] = hnew;
             if (unit_ok) {
-                const __half hh = __float2half_rn(hnew);
-                const __half hl = __float2half_rn(hnew - __half2float(hh));
+                const float hs = hnew * (float)(1 << kTcHExp);
+                const __half hh = __float2half_rn(hs);
+                const __half hl = __float2half_rn(hs - __half2float(hh));
                 *reinterpret_cast<__half*>(bh + n * 16) = hh;
                 *reinterpret_cast<__half*>(bl + n * 16) = hl;
                 if (n < nvalid && (!WIN || t == T - 1)) op[n * o_seq] = hnew;
