@@ -24,6 +24,13 @@ def test_shipped_checkpoints_load_unchanged(S):
         assert torch.equal(model.state_dict()[k], sd[k])
 
 
+def test_parameters_reach_the_library_in_state_dict_order():
+    model = windgnn_b200.GCN_GRU(13, 13, 13, 91, 21)
+    named = dict(model.named_parameters())
+    assert list(windgnn_b200.ops.PARAM_NAMES) == REFERENCE_KEYS
+    assert all(p is named[n] for n, p in zip(REFERENCE_KEYS, model._params(), strict=True))
+
+
 def test_graph_conv_layer_init_matches_reference_shapes():
     layer = windgnn_b200.GraphConvLayer(13, 5)
     assert layer.weight.shape == (13, 5) and layer.bias.shape == (5,)

@@ -84,11 +84,7 @@ class GCN_GRU(nn.Module):
             raise RuntimeError(
                 f"attr_matrix must be [B, T, S, F_in], got {tuple(attr_matrix.shape)}"
             )
-        params = (
-            self.conv1.weight, self.conv1.bias, self.conv2.weight, self.conv2.bias,
-            self.gru.weight_ih_l0, self.gru.weight_hh_l0, self.gru.bias_ih_l0, self.gru.bias_hh_l0,
-        )
-        widths = (self.conv1.weight.shape[0], self.conv1.weight.shape[1], self.conv2.weight.shape[1])
+        params = self._params()
         needs_grad = torch.is_grad_enabled() and any(p.requires_grad for p in params)
         is_csr = isinstance(adj_matrix, CsrGraph)
         if torch.is_grad_enabled() and (attr_matrix.requires_grad or (not is_csr and adj_matrix.requires_grad)):
@@ -101,7 +97,7 @@ class GCN_GRU(nn.Module):
                 out = _InferenceOnly.apply(
                     "windgnn_b200.GCN_GRU: training is implemented for dense graphs with at most "
                     f"{self.DENSE_MAX_STATIONS} stations and GCN widths <= 16 (got {adj_matrix.shape[0]} stations, "
-                    f"widths {widths}); the scaled shapes are inference-only",
+                    f"widths {self._widths()}); the scaled shapes are inference-only",
                     lambda: ops.gcn_gru_forward_csr(*csr, attr_matrix, *[p.detach() for p in params], self.chunk,
                                                     self._flags()),
                     *params)
@@ -122,12 +118,8 @@ class GCN_GRU(nn.Module):
         """Host-buffer end-to-end forward (H2D, compute, D2H overlapped chunk by chunk).  With
         ``last_step_range=(wind_min, wind_max)`` only the de-normalised last timestep ``[B, 3S]`` comes back
         (the evaluation of main.py:101-116 in one call)."""
-        params = (
-            self.conv1.weight, self.conv1.bias, self.conv2.weight, self.conv2.bias,
-            self.gru.weight_ih_l0, self.gru.weight_hh_l0, self.gru.bias_ih_l0, self.gru.bias_hh_l0,
-        )
-        return ops.gcn_gru_forward_host(adj_matrix, attr_host, [p.detach() for p in params], out_host, self.chunk,
-                                        flags=self._flags(), last_step_range=last_step_range)
+        return ops.gcn_gru_forward_host(adj_matrix, attr_host, [p.detach() for p in self._params()], out_host,
+                                        self.chunk, flags=self._flags(), last_step_range=last_step_range)
 
     @torch.no_grad()
     def forecast(self, adj_matrix, table, starts=None, seq_length=168, stride=1, last_step_range=None):
@@ -144,10 +136,7 @@ class GCN_GRU(nn.Module):
 
         if starts is None:
             starts = window_starts(table.shape[0], seq_length, stride)
-        params = [p.detach() for p in (
-            self.conv1.weight, self.conv1.bias, self.conv2.weight, self.conv2.bias,
-            self.gru.weight_ih_l0, self.gru.weight_hh_l0, self.gru.bias_ih_l0, self.gru.bias_hh_l0,
-        )]
+        params = [p.detach() for p in self._params()]
         csr = self._csr_of(adj_matrix)
         if csr is not None:
             out = ops.gcn_gru_forecast_csr(*csr, table, starts, *params, seq_length, self.chunk, self._flags())
@@ -161,15 +150,23 @@ class GCN_GRU(nn.Module):
         """The CSR arrays the library takes for ``adj_matrix``, or ``None`` for the dense path: a ``CsrGraph``, more
         than DENSE_MAX_STATIONS stations or GCN widths above 16 (the scaled shapes) go to CSR, a dense matrix
         through a cached conversion."""
-        widths = (self.conv1.weight.shape[0], self.conv1.weight.shape[1], self.conv2.weight.shape[1])
         if isinstance(adj_matrix, CsrGraph):
             return (adj_matrix.rowptr, adj_matrix.colidx, adj_matrix.vals)
-        if adj_matrix.shape[0] <= self.DENSE_MAX_STATIONS and max(widths) <= 16:
+        if adj_matrix.shape[0] <= self.DENSE_MAX_STATIONS and max(self._widths()) <= 16:
             return None
         key = (adj_matrix.data_ptr(), adj_matrix._version, tuple(adj_matrix.shape))
         if self._csr_cache is None or self._csr_cache[0] != key:
             self._csr_cache = (key, ops.dense_to_csr(adj_matrix))
         return self._csr_cache[1]
+
+    def _params(self):
+        """The eight parameters in state_dict order (``ops.PARAM_NAMES``), the order the library takes them in."""
+        return (self.conv1.weight, self.conv1.bias, self.conv2.weight, self.conv2.bias,
+                self.gru.weight_ih_l0, self.gru.weight_hh_l0, self.gru.bias_ih_l0, self.gru.bias_hh_l0)
+
+    def _widths(self):
+        """The GCN widths ``(F_in, F_hid, F_out)``."""
+        return self.conv1.weight.shape[0], self.conv1.weight.shape[1], self.conv2.weight.shape[1]
 
     def _flags(self) -> int:
         from . import _lib

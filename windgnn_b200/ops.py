@@ -22,6 +22,12 @@ from . import _lib
 _WORKSPACES: Dict[Tuple[int, int, str], torch.Tensor] = {}
 _WS_LOCK = threading.Lock()
 
+# the GCN_GRU parameters in state_dict order, the order every entry point takes them in
+PARAM_NAMES = (
+    "conv1.weight", "conv1.bias", "conv2.weight", "conv2.bias",
+    "gru.weight_ih_l0", "gru.weight_hh_l0", "gru.bias_ih_l0", "gru.bias_hh_l0",
+)
+
 
 def _workspace(device: torch.device, nbytes: int, tag: str = "fwd") -> torch.Tensor:
     """Scratch per (device, CUDA stream, tag), grown on demand and reused.  The library calls are
@@ -56,12 +62,14 @@ def _require_cuda_f32(name: str, t: torch.Tensor, device=None) -> torch.Tensor:
     return t.contiguous()
 
 
-def _dims(adj, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh):
-    if x.dim() != 4:
-        raise RuntimeError(f"attr_matrix must be [B, T, S, F_in], got {tuple(x.shape)}")
-    B, T, S, F_in = x.shape
-    if adj.shape != (S, S):
-        raise RuntimeError(f"adj_matrix must be [{S}, {S}], got {tuple(adj.shape)}")
+def _params(params, device: torch.device) -> list:
+    """The eight parameters (``PARAM_NAMES`` order), checked to be float32 on ``device``, contiguous."""
+    return [_require_cuda_f32(n, p, device) for n, p in zip(PARAM_NAMES, params, strict=True)]
+
+
+def _param_dims(S: int, F_in: int, params) -> Tuple[int, int, int]:
+    """``(F_hid, F_out, H)`` of the eight parameters, checked against ``S`` stations of ``F_in`` features."""
+    w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh = params
     if w1.dim() != 2 or w1.shape[0] != F_in:
         raise RuntimeError(f"conv1.weight must be [{F_in}, F_hid], got {tuple(w1.shape)}")
     F_hid = w1.shape[1]
@@ -81,7 +89,86 @@ def _dims(adj, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh):
         )
     if b_ih.shape != (3 * H,) or b_hh.shape != (3 * H,):
         raise RuntimeError("gru biases must be [3H]")
-    return B, T, S, F_in, F_hid, F_out, H
+    return F_hid, F_out, H
+
+
+def _graph(graph, S: int, device: torch.device) -> tuple:
+    """The adjacency as the library takes it, checked for ``S`` stations on ``device``: a dense fp32 ``adj [S, S]``
+    gives ``(adj,)``; CSR ``(rowptr, colidx, vals)`` (int32 ``[S+1]``, int32 ``[nnz]``, fp32 ``[nnz]``) gives the
+    same three.  The tensors come back contiguous."""
+    if isinstance(graph, torch.Tensor):
+        adj = _require_cuda_f32("adj_matrix", graph, device)
+        if adj.shape != (S, S):
+            raise RuntimeError(f"adj_matrix must be [{S}, {S}], got {tuple(adj.shape)}")
+        return (adj,)
+    rowptr, colidx, vals = graph
+    vals = _require_cuda_f32("adjacency values", vals, device)
+    for n, t in (("rowptr", rowptr), ("colidx", colidx)):
+        if not t.is_cuda or t.dtype != torch.int32 or t.device != device:
+            raise RuntimeError(f"windgnn_b200: {n} must be a CUDA int32 tensor on {device}")
+    rowptr, colidx = rowptr.contiguous(), colidx.contiguous()
+    if rowptr.numel() != S + 1 or colidx.numel() != vals.numel():
+        raise RuntimeError("CSR arrays do not match the number of stations")
+    return rowptr, colidx, vals
+
+
+def _attr_shape(x: torch.Tensor) -> torch.Size:
+    if x.dim() != 4:
+        raise RuntimeError(f"attr_matrix must be [B, T, S, F_in], got {tuple(x.shape)}")
+    return x.shape
+
+
+def _run(query: str, entry: str, tensors, dims, device: torch.device, tag: str, extra=(), host: bool = False):
+    """``entry(*pointers of tensors, *dims, *extra, workspace, its bytes, device index, current stream)`` with the
+    cached workspace ``query(*dims)`` asks for; a non-zero status raises ``_lib.WindGNNError``.  A query returns 0
+    bytes for a shape its entry point rejects, and the entry point then returns the library's code and reason
+    without launching anything.  ``host``: the host-buffer entry points, which take no stream and run on streams of
+    their own."""
+    lib = _lib.load()
+    ws = _workspace(device, getattr(lib, query)(*dims), tag)
+    stream = torch.cuda.current_stream(device)
+    args = (*(t.data_ptr() for t in tensors), *dims, *extra, ws.data_ptr(), ws.numel(), device.index or 0)
+    if host:
+        stream.synchronize()  # parameters / adj may have been produced on it
+        _lib.check(getattr(lib, entry)(*args))
+    else:
+        _lib.check(getattr(lib, entry)(*args, stream.cuda_stream))
+
+
+def _forward(query: str, entry: str, graph, x, params, chunk: int, flags: int) -> torch.Tensor:
+    x = _require_cuda_f32("attr_matrix", x)
+    dev = x.device
+    B, T, S, F_in = _attr_shape(x)
+    graph = _graph(graph, S, dev)
+    params = _params(params, dev)
+    F_hid, F_out, H = _param_dims(S, F_in, params)
+    out = torch.empty((B, T, H), dtype=torch.float32, device=dev)
+    if B == 0 or T == 0:
+        return out
+    _run(query, entry, (*graph, x, *params, out), (B, T, S, F_in, F_hid, F_out, H, chunk, flags), dev, "fwd")
+    return out
+
+
+def _forecast(query: str, entry: str, graph, table, starts, params, seq_length: int, chunk: int,
+              flags: int) -> torch.Tensor:
+    table = _require_cuda_f32("table", table)
+    dev = table.device
+    if table.dim() != 3:
+        raise RuntimeError(f"table must be [Ttot, S, F_in], got {tuple(table.shape)}")
+    Ttot, S, F_in = table.shape
+    graph = _graph(graph, S, dev)
+    params = _params(params, dev)
+    F_hid, F_out, H = _param_dims(S, F_in, params)
+    # the windows' first table rows as the contiguous HOST int64 array the library reads
+    if not isinstance(starts, torch.Tensor) or starts.dtype != torch.int64 or starts.dim() != 1:
+        raise RuntimeError("starts must be a 1-D int64 tensor")
+    starts = starts.cpu().contiguous()
+    N = starts.numel()
+    out = torch.empty((N, H), dtype=torch.float32, device=dev)
+    # N == 0 goes to the library too: it still rejects a bad seq_length / Ttot
+    _run(query, entry, (*graph, table, starts, *params, out),
+         (N, Ttot, seq_length, S, F_in, F_hid, F_out, H, chunk, flags), dev, "forecast")
+    return out
 
 
 @torch.library.custom_op("windgnn::gcn_gru_forward", mutates_args=())
@@ -101,33 +188,8 @@ def gcn_gru_forward(
 ) -> torch.Tensor:
     """``x [B,T,S,F_in] -> [B,T,H]`` (every GRU hidden state), fused on the GPU.
     ``flags``: 0 = FP32 FMA everywhere, ``_lib.FLAG_TENSOR_CORES`` = 3xTF32 tcgen05 input projection."""
-    lib = _lib.load()
-    x = _require_cuda_f32("attr_matrix", x)
-    dev = x.device
-    adj, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh = (
-        _require_cuda_f32(n, t, dev)
-        for n, t in (
-            ("adj_matrix", adj), ("conv1.weight", w1), ("conv1.bias", b1), ("conv2.weight", w2),
-            ("conv2.bias", b2), ("gru.weight_ih_l0", w_ih), ("gru.weight_hh_l0", w_hh),
-            ("gru.bias_ih_l0", b_ih), ("gru.bias_hh_l0", b_hh),
-        )
-    )
-    B, T, S, F_in, F_hid, F_out, H = _dims(adj, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh)
-    out = torch.empty((B, T, H), dtype=torch.float32, device=dev)
-    if B == 0 or T == 0:
-        return out
-    # 0 bytes: the shape is rejected, and the call below returns the library's code and reason without launching
-    nbytes = lib.wg_gcn_gru_workspace_bytes(B, T, S, F_in, F_hid, F_out, H, chunk, flags)
-    ws = _workspace(dev, nbytes)
-    stream = torch.cuda.current_stream(dev).cuda_stream
-    _lib.check(
-        lib.wg_gcn_gru_forward_f32(
-            adj.data_ptr(), x.data_ptr(), w1.data_ptr(), b1.data_ptr(), w2.data_ptr(), b2.data_ptr(),
-            w_ih.data_ptr(), w_hh.data_ptr(), b_ih.data_ptr(), b_hh.data_ptr(), out.data_ptr(),
-            B, T, S, F_in, F_hid, F_out, H, chunk, flags, ws.data_ptr(), ws.numel(), dev.index or 0, stream,
-        )
-    )
-    return out
+    return _forward("wg_gcn_gru_workspace_bytes", "wg_gcn_gru_forward_f32", adj, x,
+                    (w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh), chunk, flags)
 
 
 @gcn_gru_forward.register_fake
@@ -155,62 +217,13 @@ def gcn_gru_forward_csr(
     """The same forward with the adjacency in CSR form (int32 ``rowptr [S+1]``, ``colidx [nnz]``,
     fp32 ``vals [nnz]``): the large-sparse-graph path (thousands of stations, wide GCN hidden layer).
     ``flags``: as for ``gcn_gru_forward`` (the tensor path serves the projection and the recurrence)."""
-    lib = _lib.load()
-    x = _require_cuda_f32("attr_matrix", x)
-    dev = x.device
-    w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, vals = (
-        _require_cuda_f32(n, t, dev)
-        for n, t in (
-            ("conv1.weight", w1), ("conv1.bias", b1), ("conv2.weight", w2), ("conv2.bias", b2),
-            ("gru.weight_ih_l0", w_ih), ("gru.weight_hh_l0", w_hh), ("gru.bias_ih_l0", b_ih),
-            ("gru.bias_hh_l0", b_hh), ("adjacency values", vals),
-        )
-    )
-    if x.dim() != 4:
-        raise RuntimeError(f"attr_matrix must be [B, T, S, F_in], got {tuple(x.shape)}")
-    S = x.shape[2]
-    for n, t in (("rowptr", rowptr), ("colidx", colidx)):
-        if not t.is_cuda or t.dtype != torch.int32 or t.device != dev:
-            raise RuntimeError(f"windgnn_b200: {n} must be a CUDA int32 tensor on {dev}")
-    rowptr, colidx = rowptr.contiguous(), colidx.contiguous()
-    if rowptr.numel() != S + 1 or colidx.numel() != vals.numel():
-        raise RuntimeError("CSR arrays do not match the number of stations")
-    adj_shape = torch.empty((S, S), device="meta")
-    B, T, S, F_in, F_hid, F_out, H = _dims(adj_shape, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh)
-    out = torch.empty((B, T, H), dtype=torch.float32, device=dev)
-    if B == 0 or T == 0:
-        return out
-    nbytes = lib.wg_gcn_gru_csr_workspace_bytes(B, T, S, F_in, F_hid, F_out, H, chunk, flags)  # 0: see gcn_gru_forward
-    ws = _workspace(dev, nbytes)
-    stream = torch.cuda.current_stream(dev).cuda_stream
-    _lib.check(
-        lib.wg_gcn_gru_forward_csr_f32(
-            rowptr.data_ptr(), colidx.data_ptr(), vals.data_ptr(), x.data_ptr(), w1.data_ptr(), b1.data_ptr(),
-            w2.data_ptr(), b2.data_ptr(), w_ih.data_ptr(), w_hh.data_ptr(), b_ih.data_ptr(), b_hh.data_ptr(),
-            out.data_ptr(), B, T, S, F_in, F_hid, F_out, H, chunk, flags, ws.data_ptr(), ws.numel(), dev.index or 0,
-            stream,
-        )
-    )
-    return out
+    return _forward("wg_gcn_gru_csr_workspace_bytes", "wg_gcn_gru_forward_csr_f32", (rowptr, colidx, vals), x,
+                    (w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh), chunk, flags)
 
 
 @gcn_gru_forward_csr.register_fake
 def _(rowptr, colidx, vals, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, chunk=0, flags=0):
     return x.new_empty((x.shape[0], x.shape[1], w_hh.shape[1]))
-
-
-def _forecast_starts(starts: torch.Tensor) -> torch.Tensor:
-    """The windows' first table rows as the contiguous HOST int64 array the library reads."""
-    if not isinstance(starts, torch.Tensor) or starts.dtype != torch.int64 or starts.dim() != 1:
-        raise RuntimeError("starts must be a 1-D int64 tensor")
-    return starts.cpu().contiguous()
-
-
-def _forecast_dims(adj, table, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh):
-    if table.dim() != 3:
-        raise RuntimeError(f"table must be [Ttot, S, F_in], got {tuple(table.shape)}")
-    _, Ttot, S, F_in, F_hid, F_out, H = _dims(adj, table.unsqueeze(0), w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh)
-    return Ttot, S, F_in, F_hid, F_out, H
 
 
 @torch.library.custom_op("windgnn::gcn_gru_forecast", mutates_args=())
@@ -234,34 +247,8 @@ def gcn_gru_forecast(
     hidden state of the window ``table[starts[n] : starts[n] + seq_length]``, bit-identical to
     ``gcn_gru_forward(window)[:, -1]`` with the same ``chunk`` and ``flags``.  GCN and input projection run once
     per table row.  ``starts`` may live on either device (the library reads it from the host)."""
-    lib = _lib.load()
-    table = _require_cuda_f32("table", table)
-    dev = table.device
-    adj, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh = (
-        _require_cuda_f32(n, t, dev)
-        for n, t in (
-            ("adj_matrix", adj), ("conv1.weight", w1), ("conv1.bias", b1), ("conv2.weight", w2),
-            ("conv2.bias", b2), ("gru.weight_ih_l0", w_ih), ("gru.weight_hh_l0", w_hh),
-            ("gru.bias_ih_l0", b_ih), ("gru.bias_hh_l0", b_hh),
-        )
-    )
-    Ttot, S, F_in, F_hid, F_out, H = _forecast_dims(adj, table, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh)
-    starts = _forecast_starts(starts)
-    N = starts.numel()
-    out = torch.empty((N, H), dtype=torch.float32, device=dev)
-    # 0 bytes: the shape is rejected, and the call below returns the library's code and reason without launching
-    nbytes = lib.wg_gcn_gru_forecast_workspace_bytes(N, Ttot, seq_length, S, F_in, F_hid, F_out, H, chunk, flags)
-    ws = _workspace(dev, nbytes, "forecast")
-    stream = torch.cuda.current_stream(dev).cuda_stream
-    _lib.check(
-        lib.wg_gcn_gru_forecast_f32(
-            adj.data_ptr(), table.data_ptr(), starts.data_ptr(), w1.data_ptr(), b1.data_ptr(), w2.data_ptr(),
-            b2.data_ptr(), w_ih.data_ptr(), w_hh.data_ptr(), b_ih.data_ptr(), b_hh.data_ptr(), out.data_ptr(),
-            N, Ttot, seq_length, S, F_in, F_hid, F_out, H, chunk, flags, ws.data_ptr(), ws.numel(), dev.index or 0,
-            stream,
-        )
-    )
-    return out
+    return _forecast("wg_gcn_gru_forecast_workspace_bytes", "wg_gcn_gru_forecast_f32", adj, table, starts,
+                     (w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh), seq_length, chunk, flags)
 
 
 @gcn_gru_forecast.register_fake
@@ -290,44 +277,9 @@ def gcn_gru_forecast_csr(
 ) -> torch.Tensor:
     """``gcn_gru_forecast`` with the adjacency in CSR form (as for ``gcn_gru_forward_csr``); bit-identical to
     ``gcn_gru_forward_csr(window)[:, -1]``."""
-    lib = _lib.load()
-    table = _require_cuda_f32("table", table)
-    dev = table.device
-    w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, vals = (
-        _require_cuda_f32(n, t, dev)
-        for n, t in (
-            ("conv1.weight", w1), ("conv1.bias", b1), ("conv2.weight", w2), ("conv2.bias", b2),
-            ("gru.weight_ih_l0", w_ih), ("gru.weight_hh_l0", w_hh), ("gru.bias_ih_l0", b_ih),
-            ("gru.bias_hh_l0", b_hh), ("adjacency values", vals),
-        )
-    )
-    if table.dim() != 3:
-        raise RuntimeError(f"table must be [Ttot, S, F_in], got {tuple(table.shape)}")
-    S = table.shape[1]
-    for n, t in (("rowptr", rowptr), ("colidx", colidx)):
-        if not t.is_cuda or t.dtype != torch.int32 or t.device != dev:
-            raise RuntimeError(f"windgnn_b200: {n} must be a CUDA int32 tensor on {dev}")
-    rowptr, colidx = rowptr.contiguous(), colidx.contiguous()
-    if rowptr.numel() != S + 1 or colidx.numel() != vals.numel():
-        raise RuntimeError("CSR arrays do not match the number of stations")
-    adj_shape = torch.empty((S, S), device="meta")
-    Ttot, S, F_in, F_hid, F_out, H = _forecast_dims(adj_shape, table, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh)
-    starts = _forecast_starts(starts)
-    N = starts.numel()
-    out = torch.empty((N, H), dtype=torch.float32, device=dev)
-    nbytes = lib.wg_gcn_gru_forecast_csr_workspace_bytes(N, Ttot, seq_length, S, F_in, F_hid, F_out, H, chunk,
-                                                         flags)  # 0: see gcn_gru_forecast
-    ws = _workspace(dev, nbytes, "forecast")
-    stream = torch.cuda.current_stream(dev).cuda_stream
-    _lib.check(
-        lib.wg_gcn_gru_forecast_csr_f32(
-            rowptr.data_ptr(), colidx.data_ptr(), vals.data_ptr(), table.data_ptr(), starts.data_ptr(),
-            w1.data_ptr(), b1.data_ptr(), w2.data_ptr(), b2.data_ptr(), w_ih.data_ptr(), w_hh.data_ptr(),
-            b_ih.data_ptr(), b_hh.data_ptr(), out.data_ptr(), N, Ttot, seq_length, S, F_in, F_hid, F_out, H, chunk,
-            flags, ws.data_ptr(), ws.numel(), dev.index or 0, stream,
-        )
-    )
-    return out
+    return _forecast("wg_gcn_gru_forecast_csr_workspace_bytes", "wg_gcn_gru_forecast_csr_f32",
+                     (rowptr, colidx, vals), table, starts, (w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh), seq_length,
+                     chunk, flags)
 
 
 @gcn_gru_forecast_csr.register_fake
@@ -382,17 +334,20 @@ def gcn_gru_forward_host(adj, x_host, params, out_host=None, chunk: int = 0, dev
                          last_step_range=None):
     """End-to-end variant: ``x_host`` / ``out_host`` are HOST tensors (pin them for full
     copy/compute overlap); the batch is streamed through the GPU in chunks.  Blocks until
-    ``out_host`` is complete.  ``params`` = the 8 tensors in state_dict order, on the GPU.
+    ``out_host`` is complete.  ``params`` = the 8 tensors in state_dict order, on the GPU (``device``, by default
+    the device of ``adj``).
 
     ``last_step_range=(wind_min, wind_max)``: only the last timestep of every window, de-normalised
     (what the reference's evaluation reads, main.py:103,116), comes back: ``out_host`` is ``[B, H]``."""
-    lib = _lib.load()
     if x_host.is_cuda or x_host.dtype != torch.float32 or not x_host.is_contiguous():
         raise RuntimeError("x_host must be a contiguous float32 CPU tensor")
-    adj = _require_cuda_f32("adj_matrix", adj)
+    B, T, S, F_in = _attr_shape(x_host)
+    if not isinstance(adj, torch.Tensor):  # the host entry points take the dense adjacency only
+        raise TypeError("adj_matrix must be a torch.Tensor")
     dev = adj.device if device is None else torch.device(device)
-    w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh = (_require_cuda_f32(f"param{i}", t, dev) for i, t in enumerate(params))
-    B, T, S, F_in, F_hid, F_out, H = _dims(adj, x_host, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh)
+    (adj,) = _graph(adj, S, dev)
+    params = _params(params, dev)
+    F_hid, F_out, H = _param_dims(S, F_in, params)
     shape = (B, H) if last_step_range is not None else (B, T, H)
     if out_host is None:
         out_host = torch.empty(shape, dtype=torch.float32, pin_memory=True)
@@ -400,16 +355,10 @@ def gcn_gru_forward_host(adj, x_host, params, out_host=None, chunk: int = 0, dev
         raise RuntimeError(f"out_host must be a contiguous float32 CPU tensor {list(shape)}")
     if B == 0:
         return out_host
-    nbytes = lib.wg_gcn_gru_host_workspace_bytes(B, T, S, F_in, F_hid, F_out, H, chunk, flags)  # 0: see gcn_gru_forward
-    ws = _workspace(dev, nbytes, "host")
-    torch.cuda.current_stream(dev).synchronize()  # parameters / adj may have been produced on it
-    ptrs = (adj.data_ptr(), x_host.data_ptr(), w1.data_ptr(), b1.data_ptr(), w2.data_ptr(), b2.data_ptr(),
-            w_ih.data_ptr(), w_hh.data_ptr(), b_ih.data_ptr(), b_hh.data_ptr(), out_host.data_ptr())
+    tensors, dims = (adj, x_host, *params, out_host), (B, T, S, F_in, F_hid, F_out, H, chunk, flags)
     if last_step_range is None:
-        _lib.check(lib.wg_gcn_gru_forward_host_f32(*ptrs, B, T, S, F_in, F_hid, F_out, H, chunk, flags, ws.data_ptr(),
-                                                   ws.numel(), dev.index or 0))
+        _run("wg_gcn_gru_host_workspace_bytes", "wg_gcn_gru_forward_host_f32", tensors, dims, dev, "host", host=True)
     else:
-        _lib.check(lib.wg_gcn_gru_predict_host_f32(*ptrs, B, T, S, F_in, F_hid, F_out, H, chunk, flags,
-                                                   float(last_step_range[0]), float(last_step_range[1]),
-                                                   ws.data_ptr(), ws.numel(), dev.index or 0))
+        _run("wg_gcn_gru_host_workspace_bytes", "wg_gcn_gru_predict_host_f32", tensors, dims, dev, "host",
+             extra=(float(last_step_range[0]), float(last_step_range[1])), host=True)
     return out_host

@@ -29,12 +29,7 @@ from typing import Optional, Sequence
 import torch
 
 from . import _lib
-from .ops import _dims, _require_cuda_f32
-
-PARAM_NAMES = (
-    "conv1.weight", "conv1.bias", "conv2.weight", "conv2.bias",
-    "gru.weight_ih_l0", "gru.weight_hh_l0", "gru.bias_ih_l0", "gru.bias_hh_l0",
-)
+from .ops import _attr_shape, _graph, _param_dims, _params, _require_cuda_f32
 
 
 def _stream(dev: torch.device) -> int:
@@ -46,9 +41,10 @@ def forward_train(adj, x, params: Sequence[torch.Tensor]):
     lib = _lib.load()
     x = _require_cuda_f32("attr_matrix", x)
     dev = x.device
-    adj = _require_cuda_f32("adj_matrix", adj, dev)
-    params = [_require_cuda_f32(n, p, dev) for n, p in zip(PARAM_NAMES, params)]
-    B, T, S, F_in, F_hid, F_out, H = _dims(adj, x, *params)
+    B, T, S, F_in = _attr_shape(x)
+    (adj,) = _graph(adj, S, dev)
+    params = _params(params, dev)
+    F_hid, F_out, H = _param_dims(S, F_in, params)
     out = torch.empty((B, T, H), dtype=torch.float32, device=dev)
     # 0 bytes: the shape is rejected, and the call below returns the library's code and reason without launching
     nbytes = lib.wg_gcn_gru_train_workspace_bytes(B, T, S, F_in, F_hid, F_out, H)
@@ -64,11 +60,12 @@ def backward(adj, x, params: Sequence[torch.Tensor], out, d_out, ws, grads: Opti
     lib = _lib.load()
     x = _require_cuda_f32("attr_matrix", x)
     dev = x.device
-    adj = _require_cuda_f32("adj_matrix", adj, dev)
-    params = [_require_cuda_f32(n, p, dev) for n, p in zip(PARAM_NAMES, params)]
+    B, T, S, F_in = _attr_shape(x)
+    (adj,) = _graph(adj, S, dev)
+    params = _params(params, dev)
+    F_hid, F_out, H = _param_dims(S, F_in, params)
     out = _require_cuda_f32("out", out, dev)
     d_out = _require_cuda_f32("d_out", d_out, dev)
-    B, T, S, F_in, F_hid, F_out, H = _dims(adj, x, *params)
     if out.shape != (B, T, H) or d_out.shape != (B, T, H):
         raise RuntimeError(f"out / d_out must be [{B}, {T}, {H}]")
     n = lib.wg_gcn_gru_param_count(S, F_in, F_hid, F_out, H)
@@ -176,13 +173,9 @@ class Trainer:
         self.adj = _require_cuda_f32("adj_matrix", adj)
         self.lr, self.betas, self.eps, self.group = float(lr), (float(betas[0]), float(betas[1])), float(eps), group
         self.step_count = 0
-        self.params = [
-            model.conv1.weight, model.conv1.bias, model.conv2.weight, model.conv2.bias,
-            model.gru.weight_ih_l0, model.gru.weight_hh_l0, model.gru.bias_ih_l0, model.gru.bias_hh_l0,
-        ]
+        self.params = list(model._params())
         dev = self.adj.device
-        for n, p in zip(PARAM_NAMES, self.params):
-            _require_cuda_f32(n, p, dev)
+        _params(self.params, dev)
         shapes = [tuple(p.shape) for p in self.params]
         n = sum(p.numel() for p in self.params)
         self.flat = torch.empty(n, dtype=torch.float32, device=dev)
