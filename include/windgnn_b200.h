@@ -307,6 +307,44 @@ size_t wg_mse_workspace_bytes(void);
 int wg_mse_loss_grad_f32(const float* out, const float* y, int64_t n, float* d_out, float* loss, void* workspace,
                          size_t workspace_bytes, int device, void* stream);
 
+/* Training on windows over one table — the rolling windows table[starts[n] : starts[n] + L] of `table` [Ttot, S, F_in]
+ * (device), without materialising them.  GCN and input projection depend only on a table row, and their backward is
+ * linear in the input-gate gradient: the forward runs them once over the table rows [min start, max start + L) the
+ * windows cover, the backward sums every (window, step)'s input-gate gradient per table row and runs dW_ih, dU and
+ * the GCN backward once per row of that span.  The recurrence, BPTT and dW_hh run per window as in
+ * wg_gcn_gru_forward_train_f32 / wg_gcn_gru_backward_f32.
+ *
+ * The shapes, limits and error texts are the training path's for N sequences of T = L steps (see above); in addition
+ * L <= Ttot, and Ttot may be at most 2,097,024 rows.  A workspace query of 0 means the entry points reject the shape.
+ * `starts` [N] is a HOST int64 array (any order, repeats allowed), each in [0, Ttot - L]; a NULL array or a start
+ * outside that range returns WG_ERR_BAD_ARG naming the window before anything launches.  The backward takes the
+ * forward's starts.  out [N, L, H] (every hidden state) and d_out as for the materialised windows; grads: the same
+ * flat buffer, bit-reproducible run to run.  For the non-overlapping windows starts[n] = n L (what
+ * wg_make_windows_f32 materialises), out, grads and the loss below are bit-identical to the materialised path's.
+ * N = 0: the forward does nothing and the backward zeroes grads. */
+size_t wg_gcn_gru_train_windows_workspace_bytes(int64_t N, int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out,
+                                                int H);
+int wg_gcn_gru_forward_train_windows_f32(const float* adj, const float* table, const int64_t* starts, const float* w1,
+                                         const float* b1, const float* w2, const float* b2, const float* w_ih,
+                                         const float* w_hh, const float* b_ih, const float* b_hh, float* out,
+                                         int64_t N, int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out, int H,
+                                         void* workspace, size_t workspace_bytes, int device, void* stream);
+int wg_gcn_gru_backward_windows_f32(const float* adj, const float* table, const int64_t* starts, const float* w1,
+                                    const float* b1, const float* w2, const float* b2, const float* w_ih,
+                                    const float* w_hh, const float* out, const float* d_out, float* grads, int64_t N,
+                                    int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out, int H, void* workspace,
+                                    size_t workspace_bytes, int device, void* stream);
+
+/* wg_mse_loss_grad_f32 of out [N, L, horizons * S] against the targets of the table windows, read from the table in
+ * place: y[n, l, k*S + s] = table[starts[n] + l + 1 + k, s, label_f] (table [Ttot, S, F], device), what
+ * wg_make_windows_f32 builds for starts[n] = n L.  The same loss bit for bit.  starts: HOST int64 [N], each in
+ * [0, Ttot - L - horizons] (else WG_ERR_BAD_ARG naming the window); N = 0 is rejected.  workspace:
+ * wg_mse_window_labels_workspace_bytes(N) bytes, 8-byte aligned. */
+size_t wg_mse_window_labels_workspace_bytes(int64_t N);
+int wg_mse_window_labels_f32(const float* out, const float* table, const int64_t* starts, int64_t N, int L, int64_t Ttot,
+                             int S, int F, int label_f, int horizons, float* d_out, float* loss, void* workspace,
+                             size_t workspace_bytes, int device, void* stream);
+
 /* One torch.optim.Adam step (no weight decay / amsgrad) over flat buffers of n floats; `step` is
  * the 1-based step count, `grad_scale` multiplies the gradient first (1 / world size after a
  * sum all-reduce). */

@@ -71,6 +71,13 @@ _SIGNATURES = {
     "wg_gcn_gru_train_workspace_bytes": (c_size_t, [c_int64, *_DIMS]),
     "wg_gcn_gru_forward_train_f32": (c_int, [_P] * 11 + [c_int64, *_DIMS, _P, c_size_t, c_int, _P]),
     "wg_gcn_gru_backward_f32": (c_int, [_P] * 11 + [c_int64, *_DIMS, _P, c_size_t, c_int, _P]),
+    # N, Ttot, L, S, F_in, F_hid, F_out, H
+    "wg_gcn_gru_train_windows_workspace_bytes": (c_size_t, [c_int64, c_int64, *_DIMS]),
+    "wg_gcn_gru_forward_train_windows_f32": (c_int, [_P] * 12 + [c_int64, c_int64, *_DIMS, _P, c_size_t, c_int, _P]),
+    "wg_gcn_gru_backward_windows_f32": (c_int, [_P] * 12 + [c_int64, c_int64, *_DIMS, _P, c_size_t, c_int, _P]),
+    "wg_mse_window_labels_workspace_bytes": (c_size_t, [c_int64]),
+    "wg_mse_window_labels_f32": (c_int, [_P, _P, _P, c_int64, c_int, c_int64, c_int, c_int, c_int, c_int, _P, _P, _P,
+                                         c_size_t, c_int, _P]),
     "wg_mse_workspace_bytes": (c_size_t, []),
     "wg_mse_loss_grad_f32": (c_int, [_P, _P, c_int64, _P, _P, _P, c_size_t, c_int, _P]),
     "wg_adam_step_f32": (c_int, [_P, _P, _P, _P, c_int64, c_double, c_double, c_double, c_double, c_int64,

@@ -3,6 +3,7 @@
 
 #include "../../include/windgnn_b200.h"
 
+#include <algorithm>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -26,6 +27,7 @@
 #include "recur_unit.cuh"
 #include "sgemm.cuh"
 #include "train_misc.cuh"
+#include "train_windows.cuh"
 #include "wg_common.cuh"
 
 namespace {
@@ -170,10 +172,11 @@ long long forecast_piece_rows(const Plan& p, long long Ttot) {
 }
 
 // The shapes, the kernel of every stage and the workspace layout (plan_launch completes the plan).
-// table_rows > 0 (the forecast): GI holds that many rows, and the GCN / projection scratch (U, Z) pieces of
-// forecast_piece_rows rows instead of a chunk's.
+// table_rows > 0 (windows over one table): GI holds that many rows, and the GCN / projection scratch (U, Z) pieces of
+// forecast_piece_rows rows instead of a chunk's (the forecast), or all table_rows of them (whole_table: training,
+// whose dW_ih reads U in place).
 int plan_layout(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int H, long long chunk, bool sparse,
-                int flags, long long table_rows = 0) {
+                int flags, long long table_rows = 0, bool whole_table = false) {
     if (B < 0 || T <= 0 || S <= 0 || Fi <= 0 || Fh <= 0 || Fo <= 0 || H <= 0 || chunk < 0)
         return fail(WG_ERR_BAD_ARG, "non-positive dimension (B=%lld T=%d S=%d F=%d/%d/%d H=%d chunk=%lld)",
                     B, T, S, Fi, Fh, Fo, H, chunk);
@@ -241,7 +244,8 @@ int plan_layout(Plan& p, long long B, int T, int S, int Fi, int Fh, int Fo, int 
     const bool tc_recur = p.recur == kRecurTc;
     p.off_whh_hi = o; if (tc_recur) o = align_up(o + wg::recur_tc_w_halves(H) * 2);
     p.off_whh_lo = o; if (tc_recur) o = align_up(o + wg::recur_tc_w_halves(H) * 2);
-    const size_t rows = table_rows > 0 ? (size_t)forecast_piece_rows(p, table_rows) : (size_t)p.chunk * T;
+    const size_t rows = table_rows > 0 ? (size_t)(whole_table ? table_rows : forecast_piece_rows(p, table_rows))
+                                       : (size_t)p.chunk * T;
     const size_t rows_tiled = (rows + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows;
     p.off_u = o;    o = align_up(o + rows_tiled * p.IP * 4);  // K-major 128-row tiles
     p.off_umax = o; if (p.tc) o = align_up(o + rows_tiled * 4);
@@ -530,8 +534,9 @@ int launch_inproj(const Plan& p, void* ws, long long rows, cudaStream_t st, floa
 }
 
 // The recurrence launchers take row0 = NULL for a chunk of sequences laid out one after another in GI (the
-// forward), or the device array of each window's first GI row (the forecast: the windowed instantiations, which
-// store only h at the last step, out [Bc][H]).
+// forward), or the device array of each window's first GI row: the forecast (gsave = NULL: the kWinLast
+// instantiations, which store only h at the last step, out [Bc][H]) or training on table windows (gsave set: the
+// kWinAll instantiations of gru_recur_regw_kernel and gru_recur_unit_kernel, out [Bc][T][H] and the gates).
 
 // FP32 recurrence of the hidden sizes gru_recur_unit_kernel cannot fit (H = 125 .. 360): W_hh^T read through L1 / L2
 int launch_recur_wide(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, const long long* row0) {
@@ -561,7 +566,7 @@ int recur_u_pick_r(long long Bc, int ngrp) {
 }
 
 using RegwKernel = decltype(&wg::gru_recur_regw_kernel<false, 1, 24>);
-template <bool SAVE, int KPT, bool WIN = false>
+template <bool SAVE, int KPT, int WIN = wg::kWinOff>
 RegwKernel regw_kernel(int nb) {
     const RegwKernel k[4] = {wg::gru_recur_regw_kernel<SAVE, 1, KPT, WIN>, wg::gru_recur_regw_kernel<SAVE, 2, KPT, WIN>,
                              wg::gru_recur_regw_kernel<SAVE, 3, KPT, WIN>, wg::gru_recur_regw_kernel<SAVE, 4, KPT, WIN>};
@@ -571,7 +576,8 @@ int launch_recur_regw(const Plan& p, void* ws, float* out, long long Bc, int nb,
                       int ldsave, const long long* row0) {
     if (Bc < 1) return WG_OK;
     const RegwKernel kern =
-        row0    ? (p.KP == 104 ? regw_kernel<false, 104, true>(nb) : regw_kernel<false, 24, true>(nb))
+        row0 && gsave ? (p.KP == 104 ? regw_kernel<true, 104, wg::kWinAll>(nb) : regw_kernel<true, 24, wg::kWinAll>(nb))
+        : row0 ? (p.KP == 104 ? regw_kernel<false, 104, wg::kWinLast>(nb) : regw_kernel<false, 24, wg::kWinLast>(nb))
         : gsave ? (p.KP == 104 ? regw_kernel<true, 104>(nb) : regw_kernel<true, 24>(nb))
                 : (p.KP == 104 ? regw_kernel<false, 104>(nb) : regw_kernel<false, 24>(nb));
     const size_t smem = wg::recur_regw_smem_floats(p.KP, p.NPR, p.GP) * 4;
@@ -585,7 +591,7 @@ int launch_recur_regw(const Plan& p, void* ws, float* out, long long Bc, int nb,
 }
 
 using UnitKernel = decltype(&wg::gru_recur_unit_kernel<4, 1, false, 0>);
-template <int WPG, bool SAVE, int HT, bool WIN>
+template <int WPG, bool SAVE, int HT, int WIN>
 UnitKernel unit_kernel(int r) {
     const UnitKernel k[5] = {
         wg::gru_recur_unit_kernel<4, WPG, SAVE, HT, WIN>, wg::gru_recur_unit_kernel<5, WPG, SAVE, HT, WIN>,
@@ -593,7 +599,7 @@ UnitKernel unit_kernel(int r) {
         wg::gru_recur_unit_kernel<8, WPG, SAVE, HT, WIN>};
     return k[r - wg::kRuMinR];
 }
-template <bool SAVE, bool WIN = false>
+template <bool SAVE, int WIN = wg::kWinOff>
 UnitKernel unit_kernel(const Plan& p, int r) {
     if (p.ru_ht == 102) return unit_kernel<2, SAVE, 102, WIN>(r);
     if (p.ru_ht == 21) return unit_kernel<1, SAVE, 21, WIN>(r);
@@ -601,8 +607,10 @@ UnitKernel unit_kernel(const Plan& p, int r) {
 }
 int launch_recur_unit(const Plan& p, void* ws, float* out, long long Bc, int r, cudaStream_t st, float* gsave,
                       int ldsave, const long long* row0) {
-    const UnitKernel kern =
-        row0 ? unit_kernel<false, true>(p, r) : gsave ? unit_kernel<true>(p, r) : unit_kernel<false>(p, r);
+    const UnitKernel kern = row0 && gsave ? unit_kernel<true, wg::kWinAll>(p, r)
+                            : row0        ? unit_kernel<false, wg::kWinLast>(p, r)
+                            : gsave       ? unit_kernel<true>(p, r)
+                                          : unit_kernel<false>(p, r);
     const size_t smem = wg::recur_u_smem_floats(p.H, r) * 4;
     WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int per_cta = (wg::kRuWarps / p.ru_wpg) * r;
@@ -641,7 +649,8 @@ bool regw_serves(const Plan& p, long long Bc) {
 // gru_recur_regw_kernel where it serves the contraction length (FMA chains per thread = sequences per CTA that can
 // exist: the reference's batch-1 calls run one).  gsave: the training forward, which also saves [r | z | n | hn] per
 // (sequence, step), row stride ldsave; only the regw and unit kernels save gates, and make_train_plan accepts only the
-// shapes that reach one of them.  row0: the forecast's windows (see launch_recur_wide), which save no gates.
+// shapes that reach one of them.  row0: windows over one table's GI rows (see launch_recur_wide): the forecast, or with
+// gsave training on table windows.
 int launch_recur(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave,
                  const long long* row0 = nullptr) {
     if (regw_serves(p, Bc)) return launch_recur_regw(p, ws, out, Bc, Bc >= 4 ? 4 : (int)Bc, st, gsave, ldsave, row0);
@@ -803,6 +812,20 @@ int make_forecast_plan(ForecastPlan& f, long long N, long long Ttot, int L, int 
     return WG_OK;
 }
 
+// The first and last of the HOST starts [N] (N > 0) of windows, each checked to lie in [0, last]; `bound` names the
+// interval in the error text.
+int window_span(const int64_t* starts, long long N, long long last, const char* bound, long long& lo, long long& hi) {
+    if (!starts) return fail(WG_ERR_BAD_ARG, "starts is NULL (N=%lld)", N);
+    for (long long n = 0; n < N; ++n) {
+        const long long s = starts[n];
+        if (s < 0 || s > last)
+            return fail(WG_ERR_BAD_ARG, "starts[%lld] = %lld outside %s = [0, %lld]", n, s, bound, last);
+        if (n == 0 || s < lo) lo = s;
+        if (n == 0 || s > hi) hi = s;
+    }
+    return WG_OK;
+}
+
 // starts: HOST [N], validated before anything else is looked at; out [N][H] = h at the last step of each window.
 int forecast(const ForecastPlan& f, const Graph& g, const float* table, const int64_t* starts, const float* w1,
              const float* b1, const float* w2, const float* b2, const float* w_ih, const float* w_hh,
@@ -810,16 +833,9 @@ int forecast(const ForecastPlan& f, const Graph& g, const float* table, const in
              size_t ws_bytes, int device, void* stream) {
     const Plan& p = f.p;
     if (N == 0) return WG_OK;
-    if (!starts) return fail(WG_ERR_BAD_ARG, "starts is NULL (N=%lld)", N);
-    const long long last = Ttot - p.T;
     long long lo = 0, hi = 0;
-    for (long long n = 0; n < N; ++n) {
-        const long long s = starts[n];
-        if (s < 0 || s > last)
-            return fail(WG_ERR_BAD_ARG, "starts[%lld] = %lld outside [0, Ttot - L] = [0, %lld]", n, s, last);
-        if (n == 0 || s < lo) lo = s;
-        if (n == 0 || s > hi) hi = s;
-    }
+    const int rc = window_span(starts, N, Ttot - p.T, "[0, Ttot - L]", lo, hi);
+    if (rc) return rc;
     auto stages = [&](cudaStream_t st) {
         // first GI rows relative to the span; a pageable source is staged before cudaMemcpyAsync returns
         std::vector<long long> row0((size_t)N);
@@ -896,10 +912,21 @@ GbRegwKernel gb_regw_kernel(int i) {
 // features everywhere) or gcn_bwd_kernel<16>
 enum GcnBwdKind { kGcnBwdRows, kGcnBwd13, kGcnBwd16 };
 
+// The launch geometry of backward stages 3-5 (dW_ih, dU, GCN backward) over `rows` rows of U, dGI and x: B*T for
+// materialised windows, the span of the table rows the windows cover for table windows.
+struct RowStages {
+    long long rows;
+    int splits_ih;          // 3. dW_ih: splits of the rows, k-tiles (16 rows) per split
+    long long kt_per_ih;
+    dim3 tg_du;             // 4. rows_to_tiles_kernel: dGI into K-major 128-row tiles
+    long long mt_du;        //    inproj_kernel: row tiles
+    int grid_gcn, parts_gcn;   // 5. GCN backward CTAs; parts_gcn: partial gradient sets they write
+};
+
 struct TrainPlan {
     Plan f;            // the forward's plan (chunk == B, FP32 path, dense graph)
     int LD4;           // row stride of the gate / DG buffers: 4H rounded up to 4
-    long long rows;    // B * T
+    long long rows;    // B * T: the rows of stages 1-2
     // 1. BPTT: exactly one of gb_regw and gb is set
     GbRegwKernel gb_regw;
     GbKernel gb;
@@ -908,19 +935,20 @@ struct TrainPlan {
     size_t gb_smem;
     // 2. dW_hh on sgemm_kernel: K splits of the r / z and of the n product
     int splits_hh_a, splits_hh_b;
-    // 3. dW_ih on gemm_kb_kernel: tiles over the input features / the gate columns, splits of the B*T rows
-    int mt_ih, nt_ih, splits_ih;
-    long long kt_per_ih;    // k-tiles (16 rows) per split
+    // 3. dW_ih on gemm_kb_kernel: tiles over the input features / the gate columns
+    int mt_ih, nt_ih;
     // 4. dU on inproj_kernel
     int ldu, KPd, NPd;  // dU row stride (I rounded up to 4); K / N of the dU GEMM padded for inproj_kernel
-    dim3 tg_du;         // rows_to_tiles_kernel: dGI into K-major 128-row tiles
-    long long mt_du;    // inproj_kernel: row tiles
-    int nt_du;          //                column tiles
+    int nt_du;          // inproj_kernel: column tiles
     // 5. GCN backward
     GcnBwdKind gcn;
-    int grid_gcn, rb_gcn, parts_gcn;   // parts_gcn: partial gradient sets the GCN backward writes
+    int rb_gcn;
     size_t smem_gcn;
-    size_t off_gates, off_dg, off_dgt, off_wpb, off_zb, off_du, off_biasp, off_gcnp, off_splitk, total;
+    RowStages rs;       // stages 3-5 over the rows the workspace holds: B * T, or the table's rows (table windows)
+    long long table_rows;   // training on windows over one table: its rows Ttot; else 0
+    size_t off_gates, off_dg, off_dgt, off_wpb, off_zb, off_du, off_biasp, off_gcnp, off_splitk;
+    size_t off_dgi, off_row0, off_ssort, off_wsort;   // table windows only (sizes 0 otherwise)
+    size_t total;
 };
 
 int pick_splits(long long M, long long N, long long K) {
@@ -936,14 +964,52 @@ size_t param_count(int S, int Fi, int Fh, int Fo, int H) {
     return (size_t)Fi * Fh + Fh + (size_t)Fh * Fo + Fo + G * I + G * H + G + G;
 }
 
+// dW_ih on gemm_kb_kernel<64, 160, 0>: the most row splits, those that make the grid one wave at 3 CTAs per SM
+long long ih_split_cap(const TrainPlan& tp) {
+    const long long sp = (3LL * wg::kNumSMs) / ((long long)tp.mt_ih * tp.nt_ih);
+    return sp < 1 ? 1 : sp;
+}
+
+RowStages row_stages(const TrainPlan& tp, long long rows) {
+    RowStages r;
+    r.rows = rows;
+    {   // tiles over (i, g), the rows split so that the grid is one wave
+        const long long ktall = (rows + wg::kKbBK - 1) / wg::kKbBK;
+        long long sp = ih_split_cap(tp);
+        if (sp > ktall) sp = ktall;
+        r.kt_per_ih = (ktall + sp - 1) / sp;
+        r.splits_ih = (int)((ktall + r.kt_per_ih - 1) / r.kt_per_ih);
+    }
+    const long long rt = (rows + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows;
+    r.tg_du = dim3((unsigned)((tp.KPd + 31) / 32), (unsigned)(rt / 32));
+    r.mt_du = rt / wg::kIpBM;
+    if (tp.gcn == kGcnBwdRows) {
+        const long long nblk = (rows + wg::kGb2Rows - 1) / wg::kGb2Rows;
+        const int per_sm = tp.smem_gcn + 1024 <= (size_t)(228 * 1024) / 2 ? 2 : 1;   // 228 KB per SM, 1 KB reserved per CTA
+        r.grid_gcn = (int)(nblk < (long long)per_sm * wg::kNumSMs ? nblk : (long long)per_sm * wg::kNumSMs);
+        r.parts_gcn = r.grid_gcn * wg::kGb2Slices;
+    } else {
+        const long long nblk = (rows + tp.rb_gcn - 1) / tp.rb_gcn;
+        r.grid_gcn = (int)(nblk < wg::kNumSMs ? nblk : wg::kNumSMs);
+        r.parts_gcn = r.grid_gcn * (wg::kGbwThreads / 16);
+    }
+    return r;
+}
+
 // Largest GRU hidden size training accepts: the bound of the recurrence it was built and tested with (W_hh^T resident
 // in shared memory beside the state of 32 sequences).  The gate-saving recurrence that runs now
 // (gru_recur_unit_kernel or gru_recur_regw_kernel) serves every H up to it.
 constexpr int kTrainMaxH = 106;
 
-int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, int Fo, int H) {
+// dU stage: dGI re-laid into K-major 128-row tiles by one pass of 32-row blocks (at most 65535 of them, 2,097,024 rows)
+bool du_one_pass(long long rows) { return (rows + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows / 32 <= 65535; }
+
+// table_rows > 0: training on windows over a table of that many rows (make_train_windows_plan).  U, GI and the
+// regions of stages 3-5 then hold table_rows rows (the span of the windows is at most that), and the plan adds the
+// per-row dGI, the windows' first GI rows and their sorted order.
+int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, int Fo, int H, long long table_rows = 0) {
     const long long Bn = B > 0 ? B : 1;   // B = 0 plans one sequence: the backward then only zeroes the gradients
-    int rc = plan_layout(tp.f, B, T, S, Fi, Fh, Fo, H, Bn, false, 0);
+    int rc = plan_layout(tp.f, B, T, S, Fi, Fh, Fo, H, Bn, false, 0, table_rows, true);
     if (rc) return rc;
     const Plan& p = tp.f;
     if (Fi > 16 || Fh > 16 || Fo > 16)
@@ -979,6 +1045,7 @@ int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, in
     if (H > kTrainMaxH || !(regw_serves(p, B) || p.recur == kRecurUnit))
         return fail(WG_ERR_UNSUPPORTED, "training: GRU hidden size %d does not fit the shared-memory recurrence", H);
     tp.rows = Bn * T;
+    tp.table_rows = table_rows > 0 ? table_rows : 0;
     tp.ldu = wg::round_up(p.I, 4);
     tp.KPd = wg::round_up(p.G, wg::kIpBK);
     tp.NPd = wg::round_up(p.I, wg::kIpBN);
@@ -988,10 +1055,6 @@ int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, in
         tp.gcn = kGcnBwdRows;
         tp.rb_gcn = wg::kGb2Rows;
         tp.smem_gcn = wg::gcn_bwd_rows_smem_floats(S, tp.ldu) * 4;
-        const long long nblk = (tp.rows + wg::kGb2Rows - 1) / wg::kGb2Rows;
-        const int per_sm = tp.smem_gcn + 1024 <= (size_t)(228 * 1024) / 2 ? 2 : 1;   // 228 KB per SM, 1 KB reserved per CTA
-        tp.grid_gcn = (int)(nblk < (long long)per_sm * wg::kNumSMs ? nblk : (long long)per_sm * wg::kNumSMs);
-        tp.parts_gcn = tp.grid_gcn * wg::kGb2Slices;
     } else {
         tp.gcn = Fi == 13 && Fh == 13 && Fo == 13 ? kGcnBwd13 : kGcnBwd16;
         const int NSG = wg::ceil_div(S, wg::kGbwSG);
@@ -1006,44 +1069,54 @@ int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, in
             return fail(WG_ERR_UNSUPPORTED, "training: S=%d does not fit the shared-memory GCN backward", S);
         tp.rb_gcn = RB;
         tp.smem_gcn = smem_of(RB);
-        const long long nblk = (tp.rows + RB - 1) / RB;
-        tp.grid_gcn = (int)(nblk < wg::kNumSMs ? nblk : wg::kNumSMs);
-        tp.parts_gcn = tp.grid_gcn * (wg::kGbwThreads / 16);
     }
-    // dU stage: dGI re-laid into K-major 128-row tiles by one pass of 32-row blocks (at most 65535 of them)
-    const long long rt = (tp.rows + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows;
-    if (rt / 32 > 65535) return fail(WG_ERR_UNSUPPORTED, "training: B*T = %lld rows exceed one pass", tp.rows);
-    tp.tg_du = dim3((unsigned)((tp.KPd + 31) / 32), (unsigned)(rt / 32));
-    tp.mt_du = rt / wg::kIpBM;
+    if (!du_one_pass(tp.rows)) return fail(WG_ERR_UNSUPPORTED, "training: B*T = %lld rows exceed one pass", tp.rows);
+    if (tp.table_rows && !du_one_pass(tp.table_rows))
+        return fail(WG_ERR_UNSUPPORTED, "training: a table of %lld rows exceeds one pass", tp.table_rows);
     tp.nt_du = tp.NPd / wg::kIpBN;
     tp.splits_hh_a = pick_splits(2 * H, H, tp.rows);
     tp.splits_hh_b = pick_splits(H, H, tp.rows);
-    // dW_ih on gemm_kb_kernel<64, 160, 0>: tiles over (i, g), the B*T rows split so that the grid is one wave
     tp.mt_ih = (p.IP + wg::KbWih::kBM - 1) / wg::KbWih::kBM;
     tp.nt_ih = (p.G + wg::KbWih::kBN - 1) / wg::KbWih::kBN;
-    {
-        const long long ktall = (tp.rows + wg::kKbBK - 1) / wg::kKbBK;
-        long long sp = (3LL * wg::kNumSMs) / ((long long)tp.mt_ih * tp.nt_ih);   // one wave at 3 CTAs per SM
-        if (sp < 1) sp = 1;
-        if (sp > ktall) sp = ktall;
-        tp.kt_per_ih = (ktall + sp - 1) / sp;
-        tp.splits_ih = (int)((ktall + tp.kt_per_ih - 1) / tp.kt_per_ih);
+    const long long rows3 = tp.table_rows ? tp.table_rows : tp.rows;   // the rows of stages 3-5
+    tp.rs = row_stages(tp, rows3);
+    // the split-K partials of dW_ih: a table's spans take the splits of their own row count, at most the cap
+    long long ih_parts = tp.rs.splits_ih;
+    if (tp.table_rows) {
+        const long long ktall = (rows3 + wg::kKbBK - 1) / wg::kKbBK;
+        ih_parts = ih_split_cap(tp) < ktall ? ih_split_cap(tp) : ktall;
     }
+    const long long rt = (rows3 + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows;
     size_t o = p.total;
     tp.off_gates = o; o = align_up(o + (size_t)tp.rows * tp.LD4 * 4);
     tp.off_dg = o;    o = align_up(o + (size_t)tp.rows * tp.LD4 * 4);
     tp.off_dgt = o;   o = align_up(o + (size_t)rt * tp.KPd * 4);              // dGI in K-major 128-row tiles
     tp.off_wpb = o;   o = align_up(o + (size_t)tp.NPd * tp.KPd * 4);          // w_ih packed for dU = dGI . w_ih
     tp.off_zb = o;    o = align_up(o + (size_t)tp.NPd * 4);                   // zero bias (written by the pack kernel)
-    tp.off_du = o;    o = align_up(o + (size_t)tp.rows * tp.ldu * 4);
+    tp.off_du = o;    o = align_up(o + (size_t)rows3 * tp.ldu * 4);
     tp.off_biasp = o; o = align_up(o + (size_t)tp.gb_grid * 3 * tp.LD4 * 4);  // 3 partial sets per CTA (regw), else 2
-    tp.off_gcnp = o;  o = align_up(o + (size_t)tp.parts_gcn * (2 * 256 + 32) * 4);
+    tp.off_gcnp = o;  o = align_up(o + (size_t)tp.rs.parts_gcn * (2 * 256 + 32) * 4);
     size_t sk = (size_t)tp.splits_hh_a * 2 * H * H;
     if ((size_t)tp.splits_hh_b * H * H > sk) sk = (size_t)tp.splits_hh_b * H * H;
-    if ((size_t)tp.splits_ih * p.I * tp.nt_ih * wg::KbWih::kBN > sk) sk = (size_t)tp.splits_ih * p.I * tp.nt_ih * wg::KbWih::kBN;
+    if ((size_t)ih_parts * p.I * tp.nt_ih * wg::KbWih::kBN > sk) sk = (size_t)ih_parts * p.I * tp.nt_ih * wg::KbWih::kBN;
     tp.off_splitk = o; o = align_up(o + sk * 4);
+    // table windows: dGI summed per table row (dgi_rows_kernel), the windows' first GI rows, their sorted starts and
+    // order (int64 each)
+    const size_t nt = tp.table_rows ? 1 : 0;
+    tp.off_dgi = o;   o = align_up(o + nt * rows3 * tp.LD4 * 4);
+    tp.off_row0 = o;  o = align_up(o + nt * Bn * 8);
+    tp.off_ssort = o; o = align_up(o + nt * Bn * 8);
+    tp.off_wsort = o; o = align_up(o + nt * Bn * 8);
     tp.total = o;
     return plan_launch(tp.f);   // last: a shape outside the training limits reports those
+}
+
+// Training on N windows of L steps over a table of Ttot rows: the training plan of N sequences of L steps (every limit
+// and error text is the training path's) with the table's regions.
+int make_train_windows_plan(TrainPlan& tp, long long N, long long Ttot, int L, int S, int Fi, int Fh, int Fo, int H) {
+    if (L >= 1 && Ttot < L)
+        return fail(WG_ERR_BAD_ARG, "training windows: need L <= Ttot (L=%d Ttot=%lld)", L, Ttot);
+    return make_train_plan(tp, N, L, S, Fi, Fh, Fo, H, Ttot);
 }
 
 bool aligned16(const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; }
@@ -1065,6 +1138,123 @@ int splitk_gemm(const wg::SgOperand& A, const wg::SgOperand& Bo, long long M, in
     WG_CUDA(cudaGetLastError());
     return WG_OK;
 }
+
+// The training backward after a forward that left its gates and hidden states in the workspace.  Stages 1-2 (BPTT,
+// bias gradients, dW_hh) run over the B sequences of tp.rows = B*T rows; stages 3-5 (dW_ih, dU, GCN backward) over
+// the rs.rows rows of U, of the gate gradients dgi_rows(st, DG, dgi) points dgi at, and of x (their GCN input rows).
+// Materialised windows pass B*T rows and DG itself; table windows the span of rows the windows cover, its first table
+// row as x and DG summed per table row.  grads: flat, state_dict order.
+template <typename DgiRows>
+int backward(const TrainPlan& tp, const RowStages& rs, const float* adj, const float* x, const float* w1,
+             const float* b1, const float* w2, const float* b2, const float* w_ih, const float* w_hh, const float* out,
+             const float* d_out, float* grads, long long B, void* workspace, cudaStream_t st, DgiRows dgi_rows) {
+    const Plan& p = tp.f;
+    const int T = p.T, H = p.H, F_in = p.Fi, F_hid = p.Fh, F_out = p.Fo;
+    int rc;
+    // flat gradient layout = state_dict order
+    float* d_w1 = grads;
+    float* d_b1 = d_w1 + (size_t)F_in * F_hid;
+    float* d_w2 = d_b1 + F_hid;
+    float* d_b2 = d_w2 + (size_t)F_hid * F_out;
+    float* d_wih = d_b2 + F_out;
+    float* d_whh = d_wih + (size_t)p.G * p.I;
+    float* d_bih = d_whh + (size_t)p.G * H;
+    float* d_bhh = d_bih + p.G;
+
+    float* gates = ws_ptr<float>(workspace, tp.off_gates);
+    float* DG = ws_ptr<float>(workspace, tp.off_dg);
+    float* dU = ws_ptr<float>(workspace, tp.off_du);
+    float* biasp = ws_ptr<float>(workspace, tp.off_biasp);
+    float* skp = ws_ptr<float>(workspace, tp.off_splitk);
+    const long long rows = tp.rows;
+
+    // 1. BPTT through the recurrence: DG = [da_r | da_z | da_n | da_n r], bias partials
+    if (tp.gb_regw) {
+        WG_CUDA(cudaFuncSetAttribute(tp.gb_regw, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.gb_smem));
+        tp.gb_regw<<<tp.gb_grid, tp.gb_threads, tp.gb_smem, st>>>(gates, out, d_out, w_hh, DG, biasp, B, T, H, tp.LD4);
+    } else {
+        WG_CUDA(cudaFuncSetAttribute(tp.gb, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.gb_smem));
+        tp.gb<<<tp.gb_grid, tp.gb_threads, tp.gb_smem, st>>>(gates, out, d_out, w_hh, DG, biasp, B, T, H, tp.LD4, tp.HP,
+                                                              tp.GR);
+    }
+    WG_CUDA(cudaGetLastError());
+    wg::gru_bias_grad_kernel<<<(4 * H + 127) / 128, 128, 0, st>>>(biasp, tp.gb_parts, H, tp.LD4, d_bih, d_bhh);
+    WG_CUDA(cudaGetLastError());
+    const int dg_vec = (tp.LD4 % 4 == 0) && aligned16(DG);
+    // 2. dW_hh = dGH^T . H_prev   (H_prev[b, t] = out[b, t-1], 0 at t = 0)
+    {
+        const wg::SgOperand hprev{out, H, 0, 0, (H % 4 == 0) && aligned16(out), T};
+        const wg::SgOperand a_rz{DG, tp.LD4, 0, 0, dg_vec, 0};
+        if ((rc = splitk_gemm(a_rz, hprev, 2 * H, H, rows, tp.splits_hh_a, skp, d_whh, H, 1, st))) return rc;
+        const wg::SgOperand a_n{DG + 3 * (size_t)H, tp.LD4, 0, 0, dg_vec && ((3 * H) % 4 == 0), 0};
+        if ((rc = splitk_gemm(a_n, hprev, H, H, rows, tp.splits_hh_b, skp, d_whh + 2 * (size_t)H * H, H, 1, st)))
+            return rc;
+    }
+    // the gate gradients of stages 3-5, one row per U row
+    const float* dgi = nullptr;
+    if ((rc = dgi_rows(st, DG, dgi))) return rc;
+    // 3. dW_ih [3H x I] = dGI^T . U: gemm_kb_kernel reads dGI (row-major, as the BPTT kernel or dgi_rows_kernel wrote
+    //    it) and U (the forward's K-major tiles) in place; one wave of CTAs over (tile, row split), fixed-order reduction
+    {
+        using Cfg = wg::KbWih;
+        auto kern = wg::gemm_kb_kernel<Cfg::kBM, Cfg::kBN, Cfg::kTN>;
+        WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
+        wg::KbArgs a{};
+        a.a = ws_ptr<float>(workspace, p.off_u);
+        a.b = dgi;
+        a.c = skp;
+        a.R = rs.rows;
+        a.I = p.I;
+        a.IP = p.IP;
+        a.ld_dg = tp.LD4;
+        a.ldc = tp.nt_ih * Cfg::kBN;
+        a.m_tiles = tp.mt_ih;
+        a.n_tiles = tp.nt_ih;
+        a.kt_per_split = rs.kt_per_ih;
+        const dim3 grid((unsigned)(tp.mt_ih * tp.nt_ih), (unsigned)rs.splits_ih);
+        kern<<<grid, Cfg::kThreads, Cfg::kSmemBytes, st>>>(a);
+        WG_CUDA(cudaGetLastError());
+        // d_wih[g][i] = sum_z part[z][i][g]
+        const long long total = (long long)p.G * p.I;
+        wg::sg_reduce_kernel<<<(unsigned)((total * 8 + 255) / 256), 256, 0, st>>>(skp, rs.splits_ih, p.I, p.G, d_wih, 1, p.I,
+                                                                             a.ldc);
+        WG_CUDA(cudaGetLastError());
+    }
+    // 4. dU [BT x I] = dGI . W_ih on the forward's projection kernel (bulk-copy pipeline, 87 % of the FMA
+    //    peak): dGI re-laid into K-major 128-row tiles, w_ih packed as [N/64][K][64], zero bias.  (A variant
+    //    of gemm_kb_kernel that reads dGI in place ran this product in 3.60 ms against 0.32 + 3.01 ms here.)
+    {
+        float* DGt = ws_ptr<float>(workspace, tp.off_dgt);
+        float* wpb = ws_ptr<float>(workspace, tp.off_wpb);
+        float* zb = ws_ptr<float>(workspace, tp.off_zb);
+        wg::rows_to_tiles_kernel<<<rs.tg_du, 256, 0, st>>>(dgi, DGt, rs.rows, p.G, tp.LD4, tp.KPd);
+        WG_CUDA(cudaGetLastError());
+        pack_wih_bwd_kernel<<<wg::kNumSMs, 256, 0, st>>>(w_ih, wpb, zb, p.G, p.I, tp.KPd, tp.NPd);
+        WG_CUDA(cudaGetLastError());
+        WG_CUDA(cudaFuncSetAttribute(wg::inproj_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, wg::kIpSmemBytes));
+        wg::inproj_kernel<<<(unsigned)(rs.mt_du * tp.nt_du), wg::kIpThreads, wg::kIpSmemBytes, st>>>(
+            DGt, wpb, zb, dU, rs.rows, tp.KPd, tp.ldu, tp.nt_du);
+        WG_CUDA(cudaGetLastError());
+    }
+    // 5. GCN backward: dW1, db1, dW2, db2
+    float* gcnp = ws_ptr<float>(workspace, tp.off_gcnp);
+    if (tp.gcn == kGcnBwdRows) {
+        WG_CUDA(cudaFuncSetAttribute(wg::gcn_bwd_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_gcn));
+        wg::gcn_bwd_rows_kernel<<<rs.grid_gcn, wg::kGb2Threads, tp.smem_gcn, st>>>(x, dU, adj, w1, b1, w2, b2, gcnp,
+                                                                                 rs.rows, p.S, tp.ldu);
+    } else {
+        auto kern = tp.gcn == kGcnBwd13 ? wg::gcn_bwd_kernel<13> : wg::gcn_bwd_kernel<16>;
+        WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_gcn));
+        kern<<<rs.grid_gcn, wg::kGbwThreads, tp.smem_gcn, st>>>(x, dU, adj, w1, b1, w2, b2, gcnp, rs.rows, p.S, p.Fi,
+                                                               p.Fh, p.Fo, tp.rb_gcn, tp.ldu);
+    }
+    WG_CUDA(cudaGetLastError());
+    wg::gcn_bwd_finish_kernel<<<(2 * 256 + 32 + 7) / 8, 256, 0, st>>>(
+        gcnp, rs.parts_gcn, F_in, F_hid, F_out, d_w1, d_b1, d_w2, d_b2);
+    WG_CUDA(cudaGetLastError());
+    return WG_OK;
+}
+
 
 // FFMA peak microbenchmark: 8 independent chains per thread, register resident.
 __global__ void __launch_bounds__(256) ffma_peak_kernel(float* sink, int iters, float a, float b) {
@@ -1424,112 +1614,96 @@ int wg_gcn_gru_backward_f32(const float* adj, const float* x, const float* w1, c
     DeviceGuard g(device);
     WG_CUDA(g.err);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const Plan& p = tp.f;
-    const size_t n_params = param_count(S, F_in, F_hid, F_out, H);
     if (B == 0) {
-        WG_CUDA(cudaMemsetAsync(grads, 0, n_params * 4, st));
+        WG_CUDA(cudaMemsetAsync(grads, 0, param_count(S, F_in, F_hid, F_out, H) * 4, st));
         return WG_OK;
     }
     if ((rc = check_ws(workspace, workspace_bytes, tp.total))) return rc;
-    // flat gradient layout = state_dict order
-    float* d_w1 = grads;
-    float* d_b1 = d_w1 + (size_t)F_in * F_hid;
-    float* d_w2 = d_b1 + F_hid;
-    float* d_b2 = d_w2 + (size_t)F_hid * F_out;
-    float* d_wih = d_b2 + F_out;
-    float* d_whh = d_wih + (size_t)p.G * p.I;
-    float* d_bih = d_whh + (size_t)p.G * H;
-    float* d_bhh = d_bih + p.G;
+    // stages 3-5 over the B*T rows of the windows, on the BPTT's DG rows themselves
+    auto dgi_rows = [](cudaStream_t, const float* DG, const float*& dgi) { dgi = DG; return (int)WG_OK; };
+    return backward(tp, tp.rs, adj, x, w1, b1, w2, b2, w_ih, w_hh, out, d_out, grads, B, workspace, st, dgi_rows);
+}
 
-    float* gates = ws_ptr<float>(workspace, tp.off_gates);
-    float* DG = ws_ptr<float>(workspace, tp.off_dg);
-    float* dU = ws_ptr<float>(workspace, tp.off_du);
-    float* biasp = ws_ptr<float>(workspace, tp.off_biasp);
-    float* skp = ws_ptr<float>(workspace, tp.off_splitk);
-    const long long rows = tp.rows;
+// ---- training on windows over one table ------------------------------------------------------------------
+size_t wg_gcn_gru_train_windows_workspace_bytes(int64_t N, int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out,
+                                                int H) {
+    TrainPlan tp;
+    if (make_train_windows_plan(tp, N, Ttot, L, S, F_in, F_hid, F_out, H)) return 0;
+    return tp.total;
+}
 
-    // 1. BPTT through the recurrence: DG = [da_r | da_z | da_n | da_n r], bias partials
-    if (tp.gb_regw) {
-        WG_CUDA(cudaFuncSetAttribute(tp.gb_regw, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.gb_smem));
-        tp.gb_regw<<<tp.gb_grid, tp.gb_threads, tp.gb_smem, st>>>(gates, out, d_out, w_hh, DG, biasp, B, T, H, tp.LD4);
-    } else {
-        WG_CUDA(cudaFuncSetAttribute(tp.gb, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.gb_smem));
-        tp.gb<<<tp.gb_grid, tp.gb_threads, tp.gb_smem, st>>>(gates, out, d_out, w_hh, DG, biasp, B, T, H, tp.LD4, tp.HP,
-                                                              tp.GR);
+int wg_gcn_gru_forward_train_windows_f32(const float* adj, const float* table, const int64_t* starts, const float* w1,
+                                         const float* b1, const float* w2, const float* b2, const float* w_ih,
+                                         const float* w_hh, const float* b_ih, const float* b_hh, float* out,
+                                         int64_t N, int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out, int H,
+                                         void* workspace, size_t workspace_bytes, int device, void* stream) {
+    TrainPlan tp;
+    int rc = make_train_windows_plan(tp, N, Ttot, L, S, F_in, F_hid, F_out, H);
+    if (rc) return rc;
+    if (N == 0) return WG_OK;
+    long long lo = 0, hi = 0;
+    if ((rc = window_span(starts, N, Ttot - L, "[0, Ttot - L]", lo, hi))) return rc;
+    const Plan& p = tp.f;
+    auto stages = [&](cudaStream_t st) {
+        // the windows' first GI rows relative to the span (a pageable source is staged before cudaMemcpyAsync returns)
+        std::vector<long long> row0((size_t)N);
+        for (long long n = 0; n < N; ++n) row0[(size_t)n] = starts[n] - lo;
+        long long* row0_dev = ws_ptr<long long>(workspace, tp.off_row0);
+        WG_CUDA(cudaMemcpyAsync(row0_dev, row0.data(), (size_t)N * sizeof(long long), cudaMemcpyHostToDevice, st));
+        // GCN + projection once over table rows [lo, hi + L): U (kept whole for dW_ih) and GI
+        const long long span = hi + L - lo;
+        int rc2 = launch_gcn(p, workspace, Graph{adj}, table + (size_t)lo * S * F_in, w1, b1, w2, b2, span, st);
+        if (rc2 || (rc2 = launch_inproj(p, workspace, span, st, ws_ptr<float>(workspace, p.off_gi)))) return rc2;
+        // every window's recurrence over its GI rows in place: every step stored, the gates saved
+        return launch_recur(p, workspace, out, N, st, ws_ptr<float>(workspace, tp.off_gates), tp.LD4, row0_dev);
+    };
+    return run_packed(p, tp.total, Graph{adj}, table, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, workspace,
+                      workspace_bytes, device, stream, stages);
+}
+
+int wg_gcn_gru_backward_windows_f32(const float* adj, const float* table, const int64_t* starts, const float* w1,
+                                    const float* b1, const float* w2, const float* b2, const float* w_ih,
+                                    const float* w_hh, const float* out, const float* d_out, float* grads, int64_t N,
+                                    int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out, int H, void* workspace,
+                                    size_t workspace_bytes, int device, void* stream) {
+    TrainPlan tp;
+    int rc = make_train_windows_plan(tp, N, Ttot, L, S, F_in, F_hid, F_out, H);
+    if (rc) return rc;
+    long long lo = 0, hi = 0;
+    if (N > 0 && (rc = window_span(starts, N, Ttot - L, "[0, Ttot - L]", lo, hi))) return rc;
+    if (any_null({adj, table, w1, b1, w2, b2, w_ih, w_hh, out, d_out, grads}))
+        return fail(WG_ERR_BAD_ARG, "null pointer argument");
+    DeviceGuard g(device);
+    WG_CUDA(g.err);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (N == 0) {
+        WG_CUDA(cudaMemsetAsync(grads, 0, param_count(S, F_in, F_hid, F_out, H) * 4, st));
+        return WG_OK;
     }
-    WG_CUDA(cudaGetLastError());
-    wg::gru_bias_grad_kernel<<<(4 * H + 127) / 128, 128, 0, st>>>(biasp, tp.gb_parts, H, tp.LD4, d_bih, d_bhh);
-    WG_CUDA(cudaGetLastError());
-    const int dg_vec = (tp.LD4 % 4 == 0) && aligned16(DG);
-    // 2. dW_hh = dGH^T . H_prev   (H_prev[b, t] = out[b, t-1], 0 at t = 0)
-    {
-        const wg::SgOperand hprev{out, H, 0, 0, (H % 4 == 0) && aligned16(out), T};
-        const wg::SgOperand a_rz{DG, tp.LD4, 0, 0, dg_vec, 0};
-        if ((rc = splitk_gemm(a_rz, hprev, 2 * H, H, rows, tp.splits_hh_a, skp, d_whh, H, 1, st))) return rc;
-        const wg::SgOperand a_n{DG + 3 * (size_t)H, tp.LD4, 0, 0, dg_vec && ((3 * H) % 4 == 0), 0};
-        if ((rc = splitk_gemm(a_n, hprev, H, H, rows, tp.splits_hh_b, skp, d_whh + 2 * (size_t)H * H, H, 1, st)))
-            return rc;
-    }
-    // 3. dW_ih [3H x I] = dGI^T . U: gemm_kb_kernel reads dGI (row-major, as the BPTT kernel wrote it) and U (the
-    //    forward's K-major tiles) in place; one wave of CTAs over (tile, row split), fixed-order reduction
-    {
-        using Cfg = wg::KbWih;
-        auto kern = wg::gemm_kb_kernel<Cfg::kBM, Cfg::kBN, Cfg::kTN>;
-        WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
-        wg::KbArgs a{};
-        a.a = ws_ptr<float>(workspace, p.off_u);
-        a.b = DG;
-        a.c = skp;
-        a.R = rows;
-        a.I = p.I;
-        a.IP = p.IP;
-        a.ld_dg = tp.LD4;
-        a.ldc = tp.nt_ih * Cfg::kBN;
-        a.m_tiles = tp.mt_ih;
-        a.n_tiles = tp.nt_ih;
-        a.kt_per_split = tp.kt_per_ih;
-        const dim3 grid((unsigned)(tp.mt_ih * tp.nt_ih), (unsigned)tp.splits_ih);
-        kern<<<grid, Cfg::kThreads, Cfg::kSmemBytes, st>>>(a);
+    if ((rc = check_ws(workspace, workspace_bytes, tp.total))) return rc;
+    // the windows ordered by (start, n): those covering a span row are then a contiguous range (dgi_rows_kernel)
+    std::vector<long long> order((size_t)N), ssort((size_t)N);
+    for (long long n = 0; n < N; ++n) order[(size_t)n] = n;
+    std::sort(order.begin(), order.end(),
+              [&](long long a, long long b) { return starts[a] != starts[b] ? starts[a] < starts[b] : a < b; });
+    for (long long k = 0; k < N; ++k) ssort[(size_t)k] = starts[order[(size_t)k]] - lo;
+    long long* ssort_dev = ws_ptr<long long>(workspace, tp.off_ssort);
+    long long* wsort_dev = ws_ptr<long long>(workspace, tp.off_wsort);
+    WG_CUDA(cudaMemcpyAsync(ssort_dev, ssort.data(), (size_t)N * sizeof(long long), cudaMemcpyHostToDevice, st));
+    WG_CUDA(cudaMemcpyAsync(wsort_dev, order.data(), (size_t)N * sizeof(long long), cudaMemcpyHostToDevice, st));
+    const long long span = hi + L - lo;
+    float* dgi_buf = ws_ptr<float>(workspace, tp.off_dgi);
+    // stages 3-5 over the span's rows, on DG summed per table row
+    auto dgi_rows = [&](cudaStream_t s, const float* DG, const float*& dgi) {
+        const long long grid = (span + wg::kDgiWarps - 1) / wg::kDgiWarps;
+        wg::dgi_rows_kernel<<<(unsigned)grid, wg::kDgiWarps * 32, 0, s>>>(DG, ssort_dev, wsort_dev, N, L, span, tp.LD4,
+                                                                        wg::round_up(tp.f.G, 4), dgi_buf);
         WG_CUDA(cudaGetLastError());
-        // d_wih[g][i] = sum_z part[z][i][g]
-        const long long total = (long long)p.G * p.I;
-        wg::sg_reduce_kernel<<<(unsigned)((total * 8 + 255) / 256), 256, 0, st>>>(skp, tp.splits_ih, p.I, p.G, d_wih, 1, p.I,
-                                                                             a.ldc);
-        WG_CUDA(cudaGetLastError());
-    }
-    // 4. dU [BT x I] = dGI . W_ih on the forward's projection kernel (bulk-copy pipeline, 87 % of the FMA
-    //    peak): dGI re-laid into K-major 128-row tiles, w_ih packed as [N/64][K][64], zero bias.  (A variant
-    //    of gemm_kb_kernel that reads dGI in place ran this product in 3.60 ms against 0.32 + 3.01 ms here.)
-    {
-        float* DGt = ws_ptr<float>(workspace, tp.off_dgt);
-        float* wpb = ws_ptr<float>(workspace, tp.off_wpb);
-        float* zb = ws_ptr<float>(workspace, tp.off_zb);
-        wg::rows_to_tiles_kernel<<<tp.tg_du, 256, 0, st>>>(DG, DGt, rows, p.G, tp.LD4, tp.KPd);
-        WG_CUDA(cudaGetLastError());
-        pack_wih_bwd_kernel<<<wg::kNumSMs, 256, 0, st>>>(w_ih, wpb, zb, p.G, p.I, tp.KPd, tp.NPd);
-        WG_CUDA(cudaGetLastError());
-        WG_CUDA(cudaFuncSetAttribute(wg::inproj_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, wg::kIpSmemBytes));
-        wg::inproj_kernel<<<(unsigned)(tp.mt_du * tp.nt_du), wg::kIpThreads, wg::kIpSmemBytes, st>>>(
-            DGt, wpb, zb, dU, rows, tp.KPd, tp.ldu, tp.nt_du);
-        WG_CUDA(cudaGetLastError());
-    }
-    // 5. GCN backward: dW1, db1, dW2, db2
-    float* gcnp = ws_ptr<float>(workspace, tp.off_gcnp);
-    if (tp.gcn == kGcnBwdRows) {
-        WG_CUDA(cudaFuncSetAttribute(wg::gcn_bwd_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_gcn));
-        wg::gcn_bwd_rows_kernel<<<tp.grid_gcn, wg::kGb2Threads, tp.smem_gcn, st>>>(x, dU, adj, w1, b1, w2, b2, gcnp, rows,
-                                                                                 p.S, tp.ldu);
-    } else {
-        auto kern = tp.gcn == kGcnBwd13 ? wg::gcn_bwd_kernel<13> : wg::gcn_bwd_kernel<16>;
-        WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.smem_gcn));
-        kern<<<tp.grid_gcn, wg::kGbwThreads, tp.smem_gcn, st>>>(x, dU, adj, w1, b1, w2, b2, gcnp, rows, p.S, p.Fi, p.Fh,
-                                                               p.Fo, tp.rb_gcn, tp.ldu);
-    }
-    WG_CUDA(cudaGetLastError());
-    wg::gcn_bwd_finish_kernel<<<(2 * 256 + 32 + 7) / 8, 256, 0, st>>>(
-        gcnp, tp.parts_gcn, F_in, F_hid, F_out, d_w1, d_b1, d_w2, d_b2);
-    WG_CUDA(cudaGetLastError());
-    return WG_OK;
+        dgi = dgi_buf;
+        return (int)WG_OK;
+    };
+    return backward(tp, row_stages(tp, span), adj, table + (size_t)lo * S * F_in, w1, b1, w2, b2, w_ih, w_hh, out,
+                    d_out, grads, N, workspace, st, dgi_rows);
 }
 
 size_t wg_mse_workspace_bytes(void) { return (size_t)2 * wg::kNumSMs * sizeof(double); }
@@ -1544,6 +1718,45 @@ int wg_mse_loss_grad_f32(const float* out, const float* y, int64_t n, float* d_o
     WG_CUDA(g.err);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int grid = 2 * wg::kNumSMs;
+    wg::mse_grad_kernel<<<grid, wg::kMseThreads, 0, st>>>(out, wg::LabelBuffer{y}, d_out, static_cast<double*>(workspace),
+                                                         n, (float)(2.0 / (double)n));
+    WG_CUDA(cudaGetLastError());
+    wg::mse_finish_kernel<<<1, 32, 0, st>>>(static_cast<double*>(workspace), grid, n, loss);
+    WG_CUDA(cudaGetLastError());
+    return WG_OK;
+}
+
+// [partials | starts]: the partials of wg_mse_loss_grad_f32, then the windows' starts on the device
+size_t wg_mse_window_labels_workspace_bytes(int64_t N) {
+    if (N <= 0) return 0;
+    return align_up(wg_mse_workspace_bytes()) + (size_t)N * sizeof(long long);
+}
+
+int wg_mse_window_labels_f32(const float* out, const float* table, const int64_t* starts, int64_t N, int L, int64_t Ttot,
+                             int S, int F, int label_f, int horizons, float* d_out, float* loss, void* workspace,
+                             size_t workspace_bytes, int device, void* stream) {
+    if (N <= 0) return fail(WG_ERR_BAD_ARG, "mse: N must be positive");
+    if (L < 1 || S < 1 || F < 1 || horizons < 1 || label_f < 0 || label_f >= F)
+        return fail(WG_ERR_BAD_ARG, "mse: bad dimension (L=%d S=%d F=%d label_f=%d horizons=%d)", L, S, F, label_f,
+                    horizons);
+    long long lo = 0, hi = 0;
+    const int rc = window_span(starts, N, Ttot - L - horizons, "[0, Ttot - L - horizons]", lo, hi);
+    if (rc) return rc;
+    if (any_null({out, table, loss})) return fail(WG_ERR_BAD_ARG, "null pointer argument");
+    const size_t need = wg_mse_window_labels_workspace_bytes(N);
+    if (!workspace || workspace_bytes < need || reinterpret_cast<uintptr_t>(workspace) % 8)
+        return fail(WG_ERR_WORKSPACE, "mse: workspace of %zu bytes (8-byte aligned) needed", need);
+    DeviceGuard g(device);
+    WG_CUDA(g.err);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    // through a pageable copy, which cudaMemcpyAsync stages before it returns: the caller may free starts at once
+    const std::vector<long long> starts_h(starts, starts + N);
+    long long* starts_dev = reinterpret_cast<long long*>(static_cast<char*>(workspace) + align_up(wg_mse_workspace_bytes()));
+    WG_CUDA(cudaMemcpyAsync(starts_dev, starts_h.data(), (size_t)N * sizeof(long long), cudaMemcpyHostToDevice, st));
+    // the grid, the grid-stride order and the partials of wg_mse_loss_grad_f32: the same loss bit for bit
+    const long long n = N * L * (long long)horizons * S;
+    const int grid = 2 * wg::kNumSMs;
+    const wg::LabelTable y{table, starts_dev, L, S, F, label_f, horizons * S};
     wg::mse_grad_kernel<<<grid, wg::kMseThreads, 0, st>>>(out, y, d_out, static_cast<double*>(workspace), n,
                                                          (float)(2.0 / (double)n));
     WG_CUDA(cudaGetLastError());

@@ -347,13 +347,21 @@ __host__ __device__ inline size_t recur_regw_smem_floats(int KP, int NP, int GP)
     return (size_t)kRsBT * (KP + 4) + 2 * (size_t)kRsBT * GP + (size_t)kRsBT * NP + (size_t)KP;
 }
 
-// WIN: windows over one table's gi rows (see gru_recur_unit_kernel): sequence b's gi rows start at GI + row0[b] * ldg,
-// only h at t = T-1 is stored, to out [B][H]
-template <bool SAVE, int NB, int KPT, bool WIN = false>
+// Where gru_recur_regw_kernel and gru_recur_unit_kernel read gi and what they store (template argument WIN):
+//   kWinOff   the sequences' gi rows one after another, h of every step stored to out [B][T][H] (the forward)
+//   kWinLast  windows over one table's gi rows: sequence b's gi rows start at GI + row0[b] * ldg, and only h at
+//             t = T-1 is stored, to out [B][H] (the forecast)
+//   kWinAll   gi rows through row0 as kWinLast, h of every step stored to out [B][T][H] and, with SAVE, the gates
+//             (training on table windows)
+enum WinMode { kWinOff = 0, kWinLast = 1, kWinAll = 2 };
+
+// WIN: a WinMode
+template <bool SAVE, int NB, int KPT, int WIN = kWinOff>
 __global__ void __launch_bounds__(kRwThreads, 1)
     gru_recur_regw_kernel(const float* __restrict__ GI, const float* __restrict__ WhT, const float* __restrict__ bhn,
                           float* __restrict__ out, long long B, int T, int H, int ldg, int NP, float* __restrict__ gsave,
                           int ldsave, const long long* __restrict__ row0) {
+    constexpr bool ROW0 = WIN != kWinOff, LAST = WIN == kWinLast;
     extern __shared__ __align__(16) float smem[];
     constexpr int RS = KPT + 4;
     float* hs = smem;                          // [4][RS]
@@ -388,8 +396,8 @@ __global__ void __launch_bounds__(kRwThreads, 1)
         const int b = mine ? e / chunks : 0, c = mine ? e - b * chunks : 0;
         pf_ok[q] = mine && (b0 + b < B);
         pf_off[q] = mine ? b * ldg + 4 * c : -1;
-        pf_src[q] = WIN ? GI + (size_t)(pf_ok[q] ? row0[b0 + b] : 0) * ldg + 4 * c
-                        : GI + ((size_t)(pf_ok[q] ? b0 + b : 0) * T) * ldg + 4 * c;
+        pf_src[q] = ROW0 ? GI + (size_t)(pf_ok[q] ? row0[b0 + b] : 0) * ldg + 4 * c
+                         : GI + ((size_t)(pf_ok[q] ? b0 + b : 0) * T) * ldg + 4 * c;
     }
 #define WG_RW_PREFETCH(t_)                                                                              \
     do {                                                                                                \
@@ -439,7 +447,7 @@ __global__ void __launch_bounds__(kRwThreads, 1)
                 const float n = tanh_f(gr[H2] + r * hn);
                 const float hnew = (hs[b * RS + j] - n) * z + n;
                 hs[b * RS + j] = hnew;
-                if (WIN) {
+                if (LAST) {
                     if (b0 + b < B && t == T - 1) out[(size_t)(b0 + b) * H + j] = hnew;
                 } else if (b0 + b < B) {
                     out[((size_t)(b0 + b) * T + t) * H + j] = hnew;

@@ -83,14 +83,15 @@ struct RuFrag {
 // out [B][T][H];   gsave (SAVE): [B*T][ldsave] = [r | z | n | W_hn h + b_hn]
 // HT > 0: the hidden size is the compile-time constant HT (every shared-memory offset becomes an
 // immediate); HT == 0: H is the runtime argument.
-// WIN (windows over one table's gi rows, wg_gcn_gru_forecast_f32): sequence b's gi rows start at GI + row0[b] * ldg,
-// and only h at t = T-1 is stored, to out [B][H].  The product and the gate math are unchanged.
-template <int R, int WPG, bool SAVE, int HT, bool WIN = false>
+// WIN: a WinMode (recur.cuh).  kWinLast and kWinAll read sequence b's gi rows from GI + row0[b] * ldg (windows over one
+// table's gi rows); kWinLast stores only h at t = T-1, to out [B][H].  The product and the gate math are unchanged.
+template <int R, int WPG, bool SAVE, int HT, int WIN = kWinOff>
 __global__ void __launch_bounds__(kRuThreads, 1)
     gru_recur_unit_kernel(const float* __restrict__ GI, const float* __restrict__ Whu, const float* __restrict__ bhn,
                           float* __restrict__ out, long long B, int T, int H_rt,
                           float* __restrict__ gsave, int ldsave, int handover,
                           const long long* __restrict__ row0) {
+    constexpr bool ROW0 = WIN != kWinOff, LAST = WIN == kWinLast;
     constexpr int NGRP = kRuWarps / WPG;   // groups per CTA
     constexpr int NG = WPG * 32;           // threads per group
     constexpr int NB = WPG == 1 ? kRuGiRing : 1;   // gi ring slots per group (recur_u_nb)
@@ -146,19 +147,19 @@ __global__ void __launch_bounds__(kRuThreads, 1)
     // group barrier that ends step t - NB, i.e. when every thread of the group has read gi(t - NB).
     float* gi_ring = gis + grp * R * ldg;        // slot stride: NGRP * R * ldg
     uint64_t* gi_bar = gbar + grp * NB;
-    const float* gwin[WIN ? R : 1];              // WIN: gi row 0 of each of the group's sequences
-    if (WIN && p == 0) {
+    const float* gwin[ROW0 ? R : 1];             // ROW0: gi row 0 of each of the group's sequences
+    if (ROW0 && p == 0) {
 #pragma unroll
-        for (int i = 0; i < (WIN ? R : 1); ++i) gwin[i] = GI + (size_t)(i < nvalid ? row0[b0 + i] : 0) * ldg;
+        for (int i = 0; i < (ROW0 ? R : 1); ++i) gwin[i] = GI + (size_t)(i < nvalid ? row0[b0 + i] : 0) * ldg;
     }
     auto fetch_gi = [&](int t) {
         if (nvalid > 0) {
             const int slot = NB == 1 ? 0 : t % NB;
             float* tile = gi_ring + slot * (NGRP * R * ldg);
             mbar_expect_tx(&gi_bar[slot], (unsigned)(nvalid * ldg * 4));
-            if (WIN) {
+            if (ROW0) {
 #pragma unroll
-                for (int i = 0; i < (WIN ? R : 1); ++i)
+                for (int i = 0; i < (ROW0 ? R : 1); ++i)
                     if (i < nvalid)
                         bulk_g2s(tile + i * ldg, gwin[i] + (size_t)t * ldg, (unsigned)(ldg * 4), &gi_bar[slot]);
             } else {
@@ -181,9 +182,9 @@ __global__ void __launch_bounds__(kRuThreads, 1)
     const bool out_vec = (reinterpret_cast<uintptr_t>(out) & 7) == 0 && (H & 1) == 0;
     const bool save_vec = SAVE && (reinterpret_cast<uintptr_t>(gsave) & 7) == 0 && (ldsave & 1) == 0 && (H & 1) == 0;
     const bool gi_vec = (H & 1) == 0;      // g*H + j0 even: 8-byte reads of the gi tile
-    // running output pointers: + H per step (WIN: one row per sequence, written at the last step)
-    float* op0 = out + (size_t)b0 * (WIN ? 1 : T) * H + j0;
-    const size_t o_seq = (size_t)(WIN ? 1 : T) * H;
+    // running output pointers: + H per step (LAST: one row per sequence, written at the last step)
+    float* op0 = out + (size_t)b0 * (LAST ? 1 : T) * H + j0;
+    const size_t o_seq = (size_t)(LAST ? 1 : T) * H;
     float* gs0 = SAVE ? gsave + (size_t)b0 * T * ldsave + j0 : nullptr;
     const size_t s_seq = (size_t)T * ldsave;
 
@@ -287,7 +288,7 @@ __global__ void __launch_bounds__(kRuThreads, 1)
             hprev[i] = hnew;
             if (active) {
                 *reinterpret_cast<float2*>(hnxt + i * RS + j0) = hnew;
-                if (i < nvalid && (!WIN || t == T - 1)) {
+                if (i < nvalid && (!LAST || t == T - 1)) {
                     float* op = op0 + i * o_seq;
                     if (out_vec) {
                         *reinterpret_cast<float2*>(op) = hnew;
@@ -310,7 +311,7 @@ __global__ void __launch_bounds__(kRuThreads, 1)
                 }
             }
         }
-        if (!WIN) op0 += H;
+        if (!LAST) op0 += H;
         if (SAVE) gs0 += ldsave;
         // h_t complete for the group before anyone reads it; the buffer written at step t+1 is the one
         // read at step t, which every warp of the group has finished with once it arrives here.  The same

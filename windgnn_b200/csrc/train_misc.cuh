@@ -10,15 +10,39 @@ namespace wg {
 
 constexpr int kMseThreads = 256;
 
+// Where the targets y[e] of mse_grad_kernel come from: a buffer laid out as out ...
+struct LabelBuffer {
+    const float* __restrict__ y;
+    __device__ float operator()(long long e) const { return y[e]; }
+};
+
+// ... or the table itself, for out [N][L][K*S] over the windows table[starts[n] : starts[n] + L]: the target of
+// (n, l, k*S + s) is the label feature k + 1 rows after the window's row l, as wg_make_windows_f32 builds y:
+// y[n][l][k*S + s] = table[starts[n] + l + 1 + k][s][label_f].
+struct LabelTable {
+    const float* __restrict__ table;
+    const long long* __restrict__ starts;   // device, [N]
+    int L, S, F, label_f, KS;               // KS = K * S: the width of out
+    __device__ float operator()(long long e) const {
+        const long long row = e / KS;        // n * L + l
+        const int c = (int)(e - row * KS);
+        const long long n = row / L;
+        const int l = (int)(row - n * L);
+        const int k = c / S, s = c - k * S;
+        return table[((starts[n] + l + 1 + k) * S + s) * F + label_f];
+    }
+};
+
 // d_out = 2 (out - y) / n ; partial[cta] = sum of (out - y)^2 over the CTA's grid-stride slice.
+template <typename Labels>
 __global__ void __launch_bounds__(kMseThreads)
-    mse_grad_kernel(const float* __restrict__ out, const float* __restrict__ y, float* __restrict__ d_out,
+    mse_grad_kernel(const float* __restrict__ out, Labels y, float* __restrict__ d_out,
                     double* __restrict__ partial, long long n, float scale) {
     __shared__ double red[kMseThreads / 32];
     double s = 0.0;
     for (long long e = (long long)blockIdx.x * kMseThreads + threadIdx.x; e < n;
          e += (long long)gridDim.x * kMseThreads) {
-        const float d = out[e] - y[e];
+        const float d = out[e] - y(e);
         if (d_out) d_out[e] = d * scale;
         s += (double)d * (double)d;
     }

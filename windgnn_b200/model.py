@@ -95,9 +95,7 @@ class GCN_GRU(nn.Module):
             if needs_grad:
                 # forward works under grad mode (main.py:66 style calls); backward() explains the limit
                 out = _InferenceOnly.apply(
-                    "windgnn_b200.GCN_GRU: training is implemented for dense graphs with at most "
-                    f"{self.DENSE_MAX_STATIONS} stations and GCN widths <= 16 (got {adj_matrix.shape[0]} stations, "
-                    f"widths {self._widths()}); the scaled shapes are inference-only",
+                    self._no_training_message(adj_matrix),
                     lambda: ops.gcn_gru_forward_csr(*csr, attr_matrix, *[p.detach() for p in params], self.chunk,
                                                     self._flags()),
                     *params)
@@ -145,6 +143,33 @@ class GCN_GRU(nn.Module):
         if last_step_range is not None:
             out = denormalise_last_step(out.unsqueeze(1), *last_step_range)
         return out
+
+    def forward_windows(self, adj_matrix, table, starts=None, seq_length=168, stride=1):
+        """Every hidden state ``[N, L, H]`` of the windows ``table[starts[n] : starts[n] + seq_length]`` of ``table
+        [Ttot, S, F_in]`` (on the GPU), without materialising them: GCN and input projection run once per table row
+        the windows cover, and under grad mode so do their gradients (``GcnGruWindowsFunction``), so the reference's
+        loop (``nn.MSELoss``, ``backward``, ``torch.optim.Adam``) trains on table windows.  ``starts``: as in
+        ``forecast``.  Row ``n`` equals ``self(adj_matrix, window_n)`` on the materialised window.  The training path:
+        FP32, a dense graph and the training limits, in grad mode or not."""
+        from .sequences import window_starts
+        from .train import GcnGruWindowsFunction, forward_train_windows
+
+        if starts is None:
+            starts = window_starts(table.shape[0], seq_length, stride)
+        params = self._params()
+        if torch.is_grad_enabled() and table.requires_grad:
+            raise RuntimeError("windgnn_b200.GCN_GRU: gradients w.r.t. the table are not implemented")
+        if self._csr_of(adj_matrix) is not None:
+            raise RuntimeError(self._no_training_message(adj_matrix))
+        if torch.is_grad_enabled() and any(p.requires_grad for p in params):
+            return GcnGruWindowsFunction.apply(adj_matrix, table, starts, seq_length, *params)
+        out, _ = forward_train_windows(adj_matrix, table, starts, [p.detach() for p in params], seq_length)
+        return out
+
+    def _no_training_message(self, adj_matrix) -> str:
+        return ("windgnn_b200.GCN_GRU: training is implemented for dense graphs with at most "
+                f"{self.DENSE_MAX_STATIONS} stations and GCN widths <= 16 (got {adj_matrix.shape[0]} stations, "
+                f"widths {self._widths()}); the scaled shapes are inference-only")
 
     def _csr_of(self, adj_matrix):
         """The CSR arrays the library takes for ``adj_matrix``, or ``None`` for the dense path: a ``CsrGraph``, more

@@ -149,20 +149,28 @@ def _forward(query: str, entry: str, graph, x, params, chunk: int, flags: int) -
     return out
 
 
+def _forecast_starts(starts) -> torch.Tensor:
+    """The windows' first table rows as the contiguous HOST int64 array the library reads (and range-checks)."""
+    if not isinstance(starts, torch.Tensor) or starts.dtype != torch.int64 or starts.dim() != 1:
+        raise RuntimeError("starts must be a 1-D int64 tensor")
+    return starts.cpu().contiguous()
+
+
+def _table_shape(table: torch.Tensor) -> torch.Size:
+    if table.dim() != 3:
+        raise RuntimeError(f"table must be [Ttot, S, F_in], got {tuple(table.shape)}")
+    return table.shape
+
+
 def _forecast(query: str, entry: str, graph, table, starts, params, seq_length: int, chunk: int,
               flags: int) -> torch.Tensor:
     table = _require_cuda_f32("table", table)
     dev = table.device
-    if table.dim() != 3:
-        raise RuntimeError(f"table must be [Ttot, S, F_in], got {tuple(table.shape)}")
-    Ttot, S, F_in = table.shape
+    Ttot, S, F_in = _table_shape(table)
     graph = _graph(graph, S, dev)
     params = _params(params, dev)
     F_hid, F_out, H = _param_dims(S, F_in, params)
-    # the windows' first table rows as the contiguous HOST int64 array the library reads
-    if not isinstance(starts, torch.Tensor) or starts.dtype != torch.int64 or starts.dim() != 1:
-        raise RuntimeError("starts must be a 1-D int64 tensor")
-    starts = starts.cpu().contiguous()
+    starts = _forecast_starts(starts)
     N = starts.numel()
     out = torch.empty((N, H), dtype=torch.float32, device=dev)
     # N == 0 goes to the library too: it still rejects a bad seq_length / Ttot

@@ -17,6 +17,10 @@ Two ways in:
 * ``Trainer.step(x, y)`` is the fused step: forward, MSE loss + its gradient, backward into ONE flat
   gradient bucket, one all-reduce of that bucket across the data-parallel ranks (NCCL over NVLink;
   identity for a single process), one fused Adam kernel over the flat parameter buffer.
+* Windows over one table (``table[starts[n] : starts[n] + L]``) train without being materialised:
+  ``GCN_GRU.forward_windows`` under grad mode (``GcnGruWindowsFunction``) and ``Trainer.step_table``, whose
+  loss reads the targets from the table.  GCN, input projection and their gradients run once per table row
+  (``wg_gcn_gru_forward_train_windows_f32`` / ``wg_gcn_gru_backward_windows_f32``, DESIGN.md section 10).
 
 PyTorch is plumbing here (device memory, streams, ``torch.distributed``); every arithmetic step is a
 kernel of ``libwindgnn_b200.so``.  CUDA only — no CPU fallback.
@@ -29,7 +33,7 @@ from typing import Optional, Sequence
 import torch
 
 from . import _lib
-from .ops import _attr_shape, _graph, _param_dims, _params, _require_cuda_f32
+from .ops import _attr_shape, _forecast_starts, _graph, _param_dims, _params, _require_cuda_f32, _table_shape
 
 
 def _stream(dev: torch.device) -> int:
@@ -81,6 +85,59 @@ def backward(adj, x, params: Sequence[torch.Tensor], out, d_out, ws, grads: Opti
     return grads
 
 
+def _table_args(adj, table, params):
+    """The checked table, ``(adj,)``, parameters and dims ``(S, F_in, F_hid, F_out, H)`` of a table-window call."""
+    table = _require_cuda_f32("table", table)
+    dev = table.device
+    _, S, F_in = _table_shape(table)
+    (adj,) = _graph(adj, S, dev)
+    params = _params(params, dev)
+    return table, adj, params, (S, F_in, *_param_dims(S, F_in, params))
+
+
+def forward_train_windows(adj, table, starts, params: Sequence[torch.Tensor], seq_length: int):
+    """``forward_train`` of the windows ``table[starts[n] : starts[n] + seq_length]`` of ``table [Ttot, S, F_in]``
+    without materialising them: GCN and input projection run once per table row the windows cover.  ``starts``:
+    int64 first rows (any order, repeats allowed; read from the host).  Returns ``(out [N, L, H], workspace)``."""
+    lib = _lib.load()
+    table, adj, params, dims = _table_args(adj, table, params)
+    starts = _forecast_starts(starts)
+    N, Ttot, dev = starts.numel(), table.shape[0], table.device
+    out = torch.empty((N, max(seq_length, 0), dims[-1]), dtype=torch.float32, device=dev)
+    # 0 bytes: the shape is rejected, and the call below returns the library's code and reason without launching
+    nbytes = lib.wg_gcn_gru_train_windows_workspace_bytes(N, Ttot, seq_length, *dims)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+    _lib.check(lib.wg_gcn_gru_forward_train_windows_f32(
+        adj.data_ptr(), table.data_ptr(), starts.data_ptr(), *(p.data_ptr() for p in params), out.data_ptr(),
+        N, Ttot, seq_length, *dims, ws.data_ptr(), ws.numel(), dev.index or 0, _stream(dev)))
+    return out, ws
+
+
+def backward_windows(adj, table, starts, params: Sequence[torch.Tensor], out, d_out, ws, seq_length: int,
+                     grads: Optional[torch.Tensor] = None):
+    """``backward`` after ``forward_train_windows`` (the same ``starts`` and workspace): the flat gradient bucket.
+    The input-gate gradients are summed per table row, and dW_ih, dU and the GCN backward run once per row."""
+    lib = _lib.load()
+    table, adj, params, dims = _table_args(adj, table, params)
+    starts = _forecast_starts(starts)
+    N, Ttot, dev, H = starts.numel(), table.shape[0], table.device, dims[-1]
+    out = _require_cuda_f32("out", out, dev)
+    d_out = _require_cuda_f32("d_out", d_out, dev)
+    if out.shape != (N, seq_length, H) or d_out.shape != (N, seq_length, H):
+        raise RuntimeError(f"out / d_out must be [{N}, {seq_length}, {H}]")
+    n = lib.wg_gcn_gru_param_count(*dims)
+    if grads is None:
+        grads = torch.empty(n, dtype=torch.float32, device=dev)
+    elif grads.numel() != n or not grads.is_cuda or grads.dtype != torch.float32 or not grads.is_contiguous():
+        raise RuntimeError(f"grads must be a contiguous CUDA float32 buffer of {n} elements")
+    w1, b1, w2, b2, w_ih, w_hh, _, _ = params
+    _lib.check(lib.wg_gcn_gru_backward_windows_f32(
+        adj.data_ptr(), table.data_ptr(), starts.data_ptr(), w1.data_ptr(), b1.data_ptr(), w2.data_ptr(),
+        b2.data_ptr(), w_ih.data_ptr(), w_hh.data_ptr(), out.data_ptr(), d_out.data_ptr(), grads.data_ptr(),
+        N, Ttot, seq_length, *dims, ws.data_ptr(), ws.numel(), dev.index or 0, _stream(dev)))
+    return grads
+
+
 def split_flat(flat: torch.Tensor, shapes):
     """Views of a flat buffer, one per shape, in order."""
     views, o = [], 0
@@ -93,6 +150,27 @@ def split_flat(flat: torch.Tensor, shapes):
     if o != flat.numel():
         raise RuntimeError(f"flat buffer has {flat.numel()} elements, shapes need {o}")
     return views
+
+
+class GcnGruWindowsFunction(torch.autograd.Function):
+    """autograd bridge of the table windows: ``forward_train_windows`` + ``backward_windows``."""
+
+    @staticmethod
+    def forward(ctx, adj, table, starts, seq_length, *params):
+        out, ws = forward_train_windows(adj, table, starts, [p.detach() for p in params], seq_length)
+        ctx.save_for_backward(adj, table, *params, out)
+        ctx.starts, ctx.seq_length, ctx.ws = starts, seq_length, ws
+        return out
+
+    @staticmethod
+    def backward(ctx, d_out):
+        adj, table, *rest = ctx.saved_tensors
+        params, out = rest[:8], rest[8]
+        flat = backward_windows(adj, table, ctx.starts, [p.detach() for p in params], out, d_out.contiguous(),
+                                ctx.ws, ctx.seq_length)
+        ctx.ws = None
+        grads = split_flat(flat, [p.shape for p in params])
+        return (None, None, None, None, *grads)
 
 
 class GcnGruFunction(torch.autograd.Function):
@@ -130,6 +208,29 @@ def mse_loss_grad(out: torch.Tensor, y: torch.Tensor, want_grad: bool = True):
     _lib.check(lib.wg_mse_loss_grad_f32(out.data_ptr(), y.data_ptr(), out.numel(),
                                         d_out.data_ptr() if want_grad else None, loss.data_ptr(), ws.data_ptr(),
                                         ws.numel(), dev.index or 0, _stream(dev)))
+    return loss, d_out
+
+
+def mse_window_labels(out: torch.Tensor, table: torch.Tensor, starts, seq_length: int, label_feature: int = 11,
+                      horizons: int = 3, want_grad: bool = True):
+    """``mse_loss_grad`` of ``out [N, L, horizons * S]`` against the targets of the windows ``table[starts[n] :
+    starts[n] + L]``, read from the table in place: ``y[n, l, k*S + s] = table[starts[n] + l + 1 + k, s,
+    label_feature]``, what ``create_sequences`` builds for ``starts[n] = n L``.  The same loss bit for bit."""
+    lib = _lib.load()
+    out = _require_cuda_f32("out", out)
+    dev = out.device
+    table = _require_cuda_f32("table", table, dev)
+    Ttot, S, F = _table_shape(table)
+    starts = _forecast_starts(starts)
+    N = starts.numel()
+    if out.shape != (N, seq_length, horizons * S):
+        raise RuntimeError(f"out must be [{N}, {seq_length}, {horizons * S}], got {tuple(out.shape)}")
+    d_out = torch.empty_like(out) if want_grad else None
+    loss = torch.empty((), dtype=torch.float32, device=dev)
+    ws = torch.empty(max(lib.wg_mse_window_labels_workspace_bytes(N), 1), dtype=torch.uint8, device=dev)
+    _lib.check(lib.wg_mse_window_labels_f32(out.data_ptr(), table.data_ptr(), starts.data_ptr(), N, seq_length, Ttot,
+                                            S, F, label_feature, horizons, d_out.data_ptr() if want_grad else None,
+                                            loss.data_ptr(), ws.data_ptr(), ws.numel(), dev.index or 0, _stream(dev)))
     return loss, d_out
 
 
@@ -196,8 +297,6 @@ class Trainer:
         mean-squared error when every rank holds the same number of windows.  For uneven shards pass
         ``global_batch`` (the number of windows over all ranks): this rank's upstream gradient is then
         weighted by ``B_local * world / global_batch`` so that the average is the global gradient."""
-        lib = _lib.load()
-        dev = self.flat.device
         ps = [p.data for p in self.params]
         out, ws = forward_train(self.adj, x, ps)
         loss, d_out = mse_loss_grad(out, y)
@@ -206,10 +305,39 @@ class Trainer:
             if w != 1.0:
                 d_out.mul_(w)
         backward(self.adj, x, ps, out, d_out, ws, self.grads)
+        self._update()
+        return loss
+
+    @torch.no_grad()
+    def step_table(self, table: torch.Tensor, starts, seq_length: int = 168, label_feature: int = 11,
+                   horizons: int = 3, global_batch: Optional[int] = None) -> torch.Tensor:
+        """``step`` on this rank's windows ``table[starts[n] : starts[n] + seq_length]`` of ``table [Ttot, S, F]``,
+        without materialising them: the targets are ``create_sequences``' (``label_feature`` ``1 .. horizons``
+        rows after each step), read from the table, and GCN, input projection and their gradients run once per
+        table row the windows cover.  The model's ``H`` must be ``horizons * S``.  Same all-reduce, ``global_batch``
+        weighting and Adam update as ``step``; for ``starts[n] = n seq_length`` the same result bit for bit."""
+        ps = [p.data for p in self.params]
+        S, H = _table_shape(table)[1], ps[5].shape[1]
+        if H != horizons * S:
+            raise RuntimeError(f"step_table: the model's H = {H} is not horizons * S = {horizons} * {S}")
+        starts = _forecast_starts(starts)
+        out, ws = forward_train_windows(self.adj, table, starts, ps, seq_length)
+        loss, d_out = mse_window_labels(out, table, starts, seq_length, label_feature, horizons)
+        if global_batch is not None:
+            w = shard_weight(starts.numel(), global_batch, self.group)
+            if w != 1.0:
+                d_out.mul_(w)
+        backward_windows(self.adj, table, starts, ps, out, d_out, ws, seq_length, self.grads)
+        self._update()
+        return loss
+
+    def _update(self) -> None:
+        """All-reduce of the gradient bucket, then one Adam step over the flat parameters."""
+        lib = _lib.load()
+        dev = self.flat.device
         scale = allreduce_mean_(self.grads, self.group)
         self.step_count += 1
         _lib.check(lib.wg_adam_step_f32(
             self.flat.data_ptr(), self.grads.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(),
             self.flat.numel(), self.lr, self.betas[0], self.betas[1], self.eps, self.step_count, scale,
             dev.index or 0, _stream(dev)))
-        return loss
