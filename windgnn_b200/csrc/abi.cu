@@ -534,9 +534,9 @@ int launch_inproj(const Plan& p, void* ws, long long rows, cudaStream_t st, floa
 }
 
 // The recurrence launchers take row0 = NULL for a chunk of sequences laid out one after another in GI (the
-// forward), or the device array of each window's first GI row: the forecast (gsave = NULL: the kWinLast
-// instantiations, which store only h at the last step, out [Bc][H]) or training on table windows (gsave set: the
-// kWinAll instantiations of gru_recur_regw_kernel and gru_recur_unit_kernel, out [Bc][T][H] and the gates).
+// inference forward), or the device array of each window's first GI row: the forecast (gsave = NULL: the kWinLast
+// instantiations, which store only h at the last step, out [Bc][H]) or the training forward (gsave set: the kWinAll
+// instantiations of gru_recur_regw_kernel and gru_recur_unit_kernel, out [Bc][T][H] and the gates).
 
 // FP32 recurrence of the hidden sizes gru_recur_unit_kernel cannot fit (H = 125 .. 360): W_hh^T read through L1 / L2
 int launch_recur_wide(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, const long long* row0) {
@@ -565,21 +565,20 @@ int recur_u_pick_r(long long Bc, int ngrp) {
     return best;
 }
 
-using RegwKernel = decltype(&wg::gru_recur_regw_kernel<false, 1, 24>);
-template <bool SAVE, int KPT, int WIN = wg::kWinOff>
+using RegwKernel = decltype(&wg::gru_recur_regw_kernel<1, 24>);
+template <int KPT, int WIN>
 RegwKernel regw_kernel(int nb) {
-    const RegwKernel k[4] = {wg::gru_recur_regw_kernel<SAVE, 1, KPT, WIN>, wg::gru_recur_regw_kernel<SAVE, 2, KPT, WIN>,
-                             wg::gru_recur_regw_kernel<SAVE, 3, KPT, WIN>, wg::gru_recur_regw_kernel<SAVE, 4, KPT, WIN>};
+    const RegwKernel k[4] = {wg::gru_recur_regw_kernel<1, KPT, WIN>, wg::gru_recur_regw_kernel<2, KPT, WIN>,
+                             wg::gru_recur_regw_kernel<3, KPT, WIN>, wg::gru_recur_regw_kernel<4, KPT, WIN>};
     return k[nb - 1];
 }
-int launch_recur_regw(const Plan& p, void* ws, float* out, long long Bc, int nb, cudaStream_t st, float* gsave,
-                      int ldsave, const long long* row0) {
+int launch_recur_regw(const Plan& p, void* ws, float* out, long long Bc, int nb, cudaStream_t st,
+                      const long long* row0, float* gsave, int ldsave) {
     if (Bc < 1) return WG_OK;
     const RegwKernel kern =
-        row0 && gsave ? (p.KP == 104 ? regw_kernel<true, 104, wg::kWinAll>(nb) : regw_kernel<true, 24, wg::kWinAll>(nb))
-        : row0 ? (p.KP == 104 ? regw_kernel<false, 104, wg::kWinLast>(nb) : regw_kernel<false, 24, wg::kWinLast>(nb))
-        : gsave ? (p.KP == 104 ? regw_kernel<true, 104>(nb) : regw_kernel<true, 24>(nb))
-                : (p.KP == 104 ? regw_kernel<false, 104>(nb) : regw_kernel<false, 24>(nb));
+        gsave  ? (p.KP == 104 ? regw_kernel<104, wg::kWinAll>(nb) : regw_kernel<24, wg::kWinAll>(nb))
+        : row0 ? (p.KP == 104 ? regw_kernel<104, wg::kWinLast>(nb) : regw_kernel<24, wg::kWinLast>(nb))
+               : (p.KP == 104 ? regw_kernel<104, wg::kWinOff>(nb) : regw_kernel<24, wg::kWinOff>(nb));
     const size_t smem = wg::recur_regw_smem_floats(p.KP, p.NPR, p.GP) * 4;
     WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const long long grid = (Bc + wg::kRsBT - 1) / wg::kRsBT;
@@ -590,27 +589,26 @@ int launch_recur_regw(const Plan& p, void* ws, float* out, long long Bc, int nb,
     return WG_OK;
 }
 
-using UnitKernel = decltype(&wg::gru_recur_unit_kernel<4, 1, false, 0>);
-template <int WPG, bool SAVE, int HT, int WIN>
+using UnitKernel = decltype(&wg::gru_recur_unit_kernel<4, 1, 0>);
+template <int WPG, int HT, int WIN>
 UnitKernel unit_kernel(int r) {
     const UnitKernel k[5] = {
-        wg::gru_recur_unit_kernel<4, WPG, SAVE, HT, WIN>, wg::gru_recur_unit_kernel<5, WPG, SAVE, HT, WIN>,
-        wg::gru_recur_unit_kernel<6, WPG, SAVE, HT, WIN>, wg::gru_recur_unit_kernel<7, WPG, SAVE, HT, WIN>,
-        wg::gru_recur_unit_kernel<8, WPG, SAVE, HT, WIN>};
+        wg::gru_recur_unit_kernel<4, WPG, HT, WIN>, wg::gru_recur_unit_kernel<5, WPG, HT, WIN>,
+        wg::gru_recur_unit_kernel<6, WPG, HT, WIN>, wg::gru_recur_unit_kernel<7, WPG, HT, WIN>,
+        wg::gru_recur_unit_kernel<8, WPG, HT, WIN>};
     return k[r - wg::kRuMinR];
 }
-template <bool SAVE, int WIN = wg::kWinOff>
+template <int WIN>
 UnitKernel unit_kernel(const Plan& p, int r) {
-    if (p.ru_ht == 102) return unit_kernel<2, SAVE, 102, WIN>(r);
-    if (p.ru_ht == 21) return unit_kernel<1, SAVE, 21, WIN>(r);
-    return p.ru_wpg == 1 ? unit_kernel<1, SAVE, 0, WIN>(r) : unit_kernel<2, SAVE, 0, WIN>(r);
+    if (p.ru_ht == 102) return unit_kernel<2, 102, WIN>(r);
+    if (p.ru_ht == 21) return unit_kernel<1, 21, WIN>(r);
+    return p.ru_wpg == 1 ? unit_kernel<1, 0, WIN>(r) : unit_kernel<2, 0, WIN>(r);
 }
-int launch_recur_unit(const Plan& p, void* ws, float* out, long long Bc, int r, cudaStream_t st, float* gsave,
-                      int ldsave, const long long* row0) {
-    const UnitKernel kern = row0 && gsave ? unit_kernel<true, wg::kWinAll>(p, r)
-                            : row0        ? unit_kernel<false, wg::kWinLast>(p, r)
-                            : gsave       ? unit_kernel<true>(p, r)
-                                          : unit_kernel<false>(p, r);
+int launch_recur_unit(const Plan& p, void* ws, float* out, long long Bc, int r, cudaStream_t st,
+                      const long long* row0, float* gsave, int ldsave) {
+    const UnitKernel kern = gsave  ? unit_kernel<wg::kWinAll>(p, r)
+                            : row0 ? unit_kernel<wg::kWinLast>(p, r)
+                                   : unit_kernel<wg::kWinOff>(p, r);
     const size_t smem = wg::recur_u_smem_floats(p.H, r) * 4;
     WG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int per_cta = (wg::kRuWarps / p.ru_wpg) * r;
@@ -647,16 +645,15 @@ bool regw_serves(const Plan& p, long long Bc) {
 
 // The recurrence of one chunk: the plan's kernel, except that up to two waves of 4-sequence CTAs run
 // gru_recur_regw_kernel where it serves the contraction length (FMA chains per thread = sequences per CTA that can
-// exist: the reference's batch-1 calls run one).  gsave: the training forward, which also saves [r | z | n | hn] per
-// (sequence, step), row stride ldsave; only the regw and unit kernels save gates, and make_train_plan accepts only the
-// shapes that reach one of them.  row0: windows over one table's GI rows (see launch_recur_wide): the forecast, or with
-// gsave training on table windows.
-int launch_recur(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, float* gsave, int ldsave,
-                 const long long* row0 = nullptr) {
-    if (regw_serves(p, Bc)) return launch_recur_regw(p, ws, out, Bc, Bc >= 4 ? 4 : (int)Bc, st, gsave, ldsave, row0);
+// exist: the reference's batch-1 calls run one).  row0: windows over one table's GI rows (see launch_recur_wide): the
+// forecast, or with gsave the training forward, which also saves [r | z | n | hn] per (window, step), row stride
+// ldsave; only the regw and unit kernels save gates, and make_train_plan accepts only the shapes that reach one of them.
+int launch_recur(const Plan& p, void* ws, float* out, long long Bc, cudaStream_t st, const long long* row0 = nullptr,
+                 float* gsave = nullptr, int ldsave = 0) {
+    if (regw_serves(p, Bc)) return launch_recur_regw(p, ws, out, Bc, Bc >= 4 ? 4 : (int)Bc, st, row0, gsave, ldsave);
     if (p.recur == kRecurUnit) {
         const int r = recur_u_pick_r(Bc, wg::kRuWarps / p.ru_wpg);
-        return launch_recur_unit(p, ws, out, Bc, r < p.ru_rmax ? r : p.ru_rmax, st, gsave, ldsave, row0);
+        return launch_recur_unit(p, ws, out, Bc, r < p.ru_rmax ? r : p.ru_rmax, st, row0, gsave, ldsave);
     }
     if (p.recur == kRecurTc) return launch_recur_tc(p, ws, out, Bc, st, row0);   // the tensor path: every batch size
     return launch_recur_wide(p, ws, out, Bc, st, row0);
@@ -684,16 +681,38 @@ int launch_pack(const Plan& p, void* ws, const float* w_ih, const float* w_hh, c
     return WG_OK;
 }
 
-// One chunk (Bc <= plan.chunk sequences) through the three stages; gsave / ldsave: see launch_recur.
+// One chunk (Bc <= plan.chunk sequences) through the three stages.
 int run_chunk(const Plan& p, void* ws, const Graph& g, const float* x, const float* w1, const float* b1,
-              const float* w2, const float* b2, float* out, long long Bc, cudaStream_t st, float* gsave = nullptr,
-              int ldsave = 0) {
+              const float* w2, const float* b2, float* out, long long Bc, cudaStream_t st) {
     const long long rows = Bc * p.T;
     int rc = launch_gcn(p, ws, g, x, w1, b1, w2, b2, rows, st);
     if (rc) return rc;
     rc = launch_inproj(p, ws, rows, st, ws_ptr<float>(ws, p.off_gi));
     if (rc) return rc;
-    return launch_recur(p, ws, out, Bc, st, gsave, ldsave);
+    return launch_recur(p, ws, out, Bc, st);
+}
+
+// Windows over one table: GCN + projection of the `span` table rows from x on, in pieces of `piece` rows (what the
+// plan's U scratch holds), table row r into GI row r (at gi + r * GP).
+int run_span_stages(const Plan& p, void* ws, const Graph& g, const float* x, const float* w1, const float* b1,
+                    const float* w2, const float* b2, long long span, long long piece, cudaStream_t st) {
+    float* gi = ws_ptr<float>(ws, p.off_gi);
+    const size_t x_row = (size_t)p.S * p.Fi;
+    for (long long r0 = 0; r0 < span; r0 += piece) {
+        const long long rows = span - r0 < piece ? span - r0 : piece;
+        int rc = launch_gcn(p, ws, g, x + (size_t)r0 * x_row, w1, b1, w2, b2, rows, st);
+        if (rc || (rc = launch_inproj(p, ws, rows, st, gi + (size_t)r0 * p.GP))) return rc;
+    }
+    return WG_OK;
+}
+
+// The first GI rows of the windows with HOST starts [N], relative to the span's first table row lo, into the device
+// array dst [N] (a pageable source is staged before cudaMemcpyAsync returns).
+int upload_row0(const int64_t* starts, long long N, long long lo, long long* dst, cudaStream_t st) {
+    std::vector<long long> row0((size_t)N);
+    for (long long n = 0; n < N; ++n) row0[(size_t)n] = starts[n] - lo;
+    WG_CUDA(cudaMemcpyAsync(dst, row0.data(), (size_t)N * sizeof(long long), cudaMemcpyHostToDevice, st));
+    return WG_OK;
 }
 
 // Per-device tables (constant-bank ordering below, host-path streams): DeviceGuard has rejected a negative index.
@@ -770,24 +789,22 @@ int run_packed(const Plan& p, size_t need, const Graph& g, const float* x, const
     return sq ? finish_sparse(device, st) : WG_OK;
 }
 
-// The device-buffer forward of a finished plan: every chunk through the three stages.  need: the workspace bytes to
-// check (the training plan adds its regions to the forward's); gsave / ldsave: see launch_recur.
-int forward(const Plan& p, size_t need, const Graph& g, const float* x, const float* w1, const float* b1,
-            const float* w2, const float* b2, const float* w_ih, const float* w_hh, const float* b_ih,
-            const float* b_hh, float* out, long long B, void* ws, size_t ws_bytes, int device, void* stream,
-            float* gsave = nullptr, int ldsave = 0) {
+// The device-buffer forward of a finished plan: every chunk through the three stages.
+int forward(const Plan& p, const Graph& g, const float* x, const float* w1, const float* b1, const float* w2,
+            const float* b2, const float* w_ih, const float* w_hh, const float* b_ih, const float* b_hh, float* out,
+            long long B, void* ws, size_t ws_bytes, int device, void* stream) {
     if (B == 0) return WG_OK;
     auto stages = [&](cudaStream_t st) {
         const size_t x_seq = (size_t)p.T * p.S * p.Fi, o_seq = (size_t)p.T * p.H;
         for (long long b0 = 0; b0 < B; b0 += p.chunk) {
             const long long Bc = (B - b0) < p.chunk ? (B - b0) : p.chunk;
-            const int rc = run_chunk(p, ws, g, x + (size_t)b0 * x_seq, w1, b1, w2, b2, out + (size_t)b0 * o_seq, Bc,
-                                     st, gsave ? gsave + (size_t)b0 * p.T * ldsave : nullptr, ldsave);
+            const int rc =
+                run_chunk(p, ws, g, x + (size_t)b0 * x_seq, w1, b1, w2, b2, out + (size_t)b0 * o_seq, Bc, st);
             if (rc) return rc;
         }
         return (int)WG_OK;
     };
-    return run_packed(p, need, g, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, ws, ws_bytes, device, stream,
+    return run_packed(p, p.total, g, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, ws, ws_bytes, device, stream,
                       stages);
 }
 
@@ -837,25 +854,16 @@ int forecast(const ForecastPlan& f, const Graph& g, const float* table, const in
     const int rc = window_span(starts, N, Ttot - p.T, "[0, Ttot - L]", lo, hi);
     if (rc) return rc;
     auto stages = [&](cudaStream_t st) {
-        // first GI rows relative to the span; a pageable source is staged before cudaMemcpyAsync returns
-        std::vector<long long> row0((size_t)N);
-        for (long long n = 0; n < N; ++n) row0[(size_t)n] = starts[n] - lo;
-        long long* row0_dev = ws_ptr<long long>(ws, f.off_row0);
-        WG_CUDA(cudaMemcpyAsync(row0_dev, row0.data(), (size_t)N * sizeof(long long), cudaMemcpyHostToDevice, st));
+        long long* row0 = ws_ptr<long long>(ws, f.off_row0);
         // GCN + projection over table rows [lo, hi + L), in pieces of the U scratch's rows
-        float* gi = ws_ptr<float>(ws, p.off_gi);
-        const size_t x_row = (size_t)p.S * p.Fi;
-        const long long span = hi + p.T - lo, piece = forecast_piece_rows(p, Ttot);
-        for (long long r0 = 0; r0 < span; r0 += piece) {
-            const long long rows = span - r0 < piece ? span - r0 : piece;
-            int rc = launch_gcn(p, ws, g, table + (size_t)(lo + r0) * x_row, w1, b1, w2, b2, rows, st);
-            if (rc || (rc = launch_inproj(p, ws, rows, st, gi + (size_t)r0 * p.GP))) return rc;
-        }
+        int rc = upload_row0(starts, N, lo, row0, st);
+        if (rc || (rc = run_span_stages(p, ws, g, table + (size_t)lo * p.S * p.Fi, w1, b1, w2, b2, hi + p.T - lo,
+                                        forecast_piece_rows(p, Ttot), st)))
+            return rc;
         // the recurrence in the forward's chunks, so that every chunk runs the kernel the forward would
         for (long long b0 = 0; b0 < N; b0 += p.chunk) {
             const long long Bc = (N - b0) < p.chunk ? (N - b0) : p.chunk;
-            const int rc = launch_recur(p, ws, out + (size_t)b0 * p.H, Bc, st, nullptr, 0, row0_dev + b0);
-            if (rc) return rc;
+            if ((rc = launch_recur(p, ws, out + (size_t)b0 * p.H, Bc, st, row0 + b0))) return rc;
         }
         return (int)WG_OK;
     };
@@ -912,8 +920,8 @@ GbRegwKernel gb_regw_kernel(int i) {
 // features everywhere) or gcn_bwd_kernel<16>
 enum GcnBwdKind { kGcnBwdRows, kGcnBwd13, kGcnBwd16 };
 
-// The launch geometry of backward stages 3-5 (dW_ih, dU, GCN backward) over `rows` rows of U, dGI and x: B*T for
-// materialised windows, the span of the table rows the windows cover for table windows.
+// The launch geometry of backward stages 3-5 (dW_ih, dU, GCN backward) over `rows` rows of U, dGI and x: the span of
+// the table rows the windows cover (B*T for a materialised batch).
 struct RowStages {
     long long rows;
     int splits_ih;          // 3. dW_ih: splits of the rows, k-tiles (16 rows) per split
@@ -923,10 +931,13 @@ struct RowStages {
     int grid_gcn, parts_gcn;   // 5. GCN backward CTAs; parts_gcn: partial gradient sets they write
 };
 
+// Training runs N windows of L steps over a table of Ttot rows.  A materialised batch x [B][T] is the table
+// x.view(B*T) with windows that tile it (starts[n] = n*T): a tiled plan, whose backward reads dGI from DG in place.
 struct TrainPlan {
-    Plan f;            // the forward's plan (chunk == B, FP32 path, dense graph)
+    Plan f;            // the forward's plan (N sequences of L steps, chunk == N, FP32 path, dense graph, GI of Ttot rows)
+    bool tiled;        // the windows tile the table: row0[n] = n*L, no per-row dGI
     int LD4;           // row stride of the gate / DG buffers: 4H rounded up to 4
-    long long rows;    // B * T: the rows of stages 1-2
+    long long rows;    // N * L: the rows of stages 1-2
     // 1. BPTT: exactly one of gb_regw and gb is set
     GbRegwKernel gb_regw;
     GbKernel gb;
@@ -944,10 +955,8 @@ struct TrainPlan {
     GcnBwdKind gcn;
     int rb_gcn;
     size_t smem_gcn;
-    RowStages rs;       // stages 3-5 over the rows the workspace holds: B * T, or the table's rows (table windows)
-    long long table_rows;   // training on windows over one table: its rows Ttot; else 0
-    size_t off_gates, off_dg, off_dgt, off_wpb, off_zb, off_du, off_biasp, off_gcnp, off_splitk;
-    size_t off_dgi, off_row0, off_ssort, off_wsort;   // table windows only (sizes 0 otherwise)
+    size_t off_gates, off_dg, off_dgt, off_wpb, off_zb, off_du, off_biasp, off_gcnp, off_splitk, off_row0;
+    size_t off_dgi, off_ssort, off_wsort;   // untiled plans only (sizes 0 otherwise)
     size_t total;
 };
 
@@ -1004,14 +1013,17 @@ constexpr int kTrainMaxH = 106;
 // dU stage: dGI re-laid into K-major 128-row tiles by one pass of 32-row blocks (at most 65535 of them, 2,097,024 rows)
 bool du_one_pass(long long rows) { return (rows + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows / 32 <= 65535; }
 
-// table_rows > 0: training on windows over a table of that many rows (make_train_windows_plan).  U, GI and the
-// regions of stages 3-5 then hold table_rows rows (the span of the windows is at most that), and the plan adds the
-// per-row dGI, the windows' first GI rows and their sorted order.
-int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, int Fo, int H, long long table_rows = 0) {
-    const long long Bn = B > 0 ? B : 1;   // B = 0 plans one sequence: the backward then only zeroes the gradients
-    int rc = plan_layout(tp.f, B, T, S, Fi, Fh, Fo, H, Bn, false, 0, table_rows, true);
+// The training plan of N windows of L steps over a table of Ttot rows (tiled: see TrainPlan).  U, GI and the regions of
+// stages 3-5 hold Ttot rows (the span of the windows is at most that); every plan holds the windows' first GI rows, an
+// untiled one also the per-row dGI and the windows' sorted order.
+int make_train_plan(TrainPlan& tp, long long N, long long Ttot, int L, int S, int Fi, int Fh, int Fo, int H, bool tiled) {
+    if (L >= 1 && Ttot < L)
+        return fail(WG_ERR_BAD_ARG, "training windows: need L <= Ttot (L=%d Ttot=%lld)", L, Ttot);
+    const long long Nn = N > 0 ? N : 1;   // N = 0 plans one sequence: the backward then only zeroes the gradients
+    int rc = plan_layout(tp.f, N, L, S, Fi, Fh, Fo, H, Nn, false, 0, Ttot, true);
     if (rc) return rc;
     const Plan& p = tp.f;
+    tp.tiled = tiled;
     if (Fi > 16 || Fh > 16 || Fo > 16)
         return fail(WG_ERR_UNSUPPORTED, "training: GCN feature widths must be <= 16 (got %d / %d / %d)", Fi, Fh, Fo);
     tp.LD4 = wg::round_up(4 * H, 4);
@@ -1020,7 +1032,7 @@ int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, in
     if (tp.HP == 104 || tp.HP == 24) {
         // W_hh in registers: the smallest CTA size that still makes the grid one wave (28 sequences fit)
         int i = 0;
-        while (i < 3 && (Bn + kGbRegwBT[i] - 1) / kGbRegwBT[i] > wg::kNumSMs) ++i;
+        while (i < 3 && (Nn + kGbRegwBT[i] - 1) / kGbRegwBT[i] > wg::kNumSMs) ++i;
         bt = kGbRegwBT[i];
         tp.gb_regw = tp.HP == 104 ? gb_regw_kernel<104>(i) : gb_regw_kernel<24>(i);
         tp.gb = nullptr;
@@ -1029,7 +1041,7 @@ int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, in
     } else {
         // 16 sequences per CTA when that fills the machine, else 4 (the recurrence is latency-bound: with few
         // sequences per GPU — configs[4]: 512 — more, lighter CTAs shorten every one of the T serial steps)
-        bt = Bn > 4LL * wg::kNumSMs ? wg::kGbBT : 4;
+        bt = Nn > 4LL * wg::kNumSMs ? wg::kGbBT : 4;
         tp.GR = wg::gru_bwd_gr(H, bt);
         tp.gb_smem = wg::gru_bwd_smem_floats(tp.HP, tp.GR, bt) * 4;
         if (tp.HP > 128 || (tp.HP / 4) * (bt / 4) * wg::gru_bwd_ksplit(bt) > wg::kGbThreads ||
@@ -1039,13 +1051,12 @@ int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, in
         tp.gb = bt == 4 ? wg::gru_bwd_kernel<4> : wg::gru_bwd_kernel<wg::kGbBT>;
         tp.gb_threads = wg::kGbThreads;
     }
-    tp.gb_grid = (int)((Bn + bt - 1) / bt);
+    tp.gb_grid = (int)((Nn + bt - 1) / bt);
     tp.gb_parts = tp.gb_grid * (tp.gb_regw ? 3 : 2);
     // the forward's recurrence saves the gates: only gru_recur_regw_kernel and gru_recur_unit_kernel do (launch_recur)
-    if (H > kTrainMaxH || !(regw_serves(p, B) || p.recur == kRecurUnit))
+    if (H > kTrainMaxH || !(regw_serves(p, N) || p.recur == kRecurUnit))
         return fail(WG_ERR_UNSUPPORTED, "training: GRU hidden size %d does not fit the shared-memory recurrence", H);
-    tp.rows = Bn * T;
-    tp.table_rows = table_rows > 0 ? table_rows : 0;
+    tp.rows = Nn * L;
     tp.ldu = wg::round_up(p.I, 4);
     tp.KPd = wg::round_up(p.G, wg::kIpBK);
     tp.NPd = wg::round_up(p.I, wg::kIpBN);
@@ -1070,53 +1081,47 @@ int make_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, in
         tp.rb_gcn = RB;
         tp.smem_gcn = smem_of(RB);
     }
+    // a tiled plan's table is its B*T rows: the first check reports it
     if (!du_one_pass(tp.rows)) return fail(WG_ERR_UNSUPPORTED, "training: B*T = %lld rows exceed one pass", tp.rows);
-    if (tp.table_rows && !du_one_pass(tp.table_rows))
-        return fail(WG_ERR_UNSUPPORTED, "training: a table of %lld rows exceeds one pass", tp.table_rows);
+    if (!du_one_pass(Ttot)) return fail(WG_ERR_UNSUPPORTED, "training: a table of %lld rows exceeds one pass", Ttot);
     tp.nt_du = tp.NPd / wg::kIpBN;
     tp.splits_hh_a = pick_splits(2 * H, H, tp.rows);
     tp.splits_hh_b = pick_splits(H, H, tp.rows);
     tp.mt_ih = (p.IP + wg::KbWih::kBM - 1) / wg::KbWih::kBM;
     tp.nt_ih = (p.G + wg::KbWih::kBN - 1) / wg::KbWih::kBN;
-    const long long rows3 = tp.table_rows ? tp.table_rows : tp.rows;   // the rows of stages 3-5
-    tp.rs = row_stages(tp, rows3);
-    // the split-K partials of dW_ih: a table's spans take the splits of their own row count, at most the cap
-    long long ih_parts = tp.rs.splits_ih;
-    if (tp.table_rows) {
-        const long long ktall = (rows3 + wg::kKbBK - 1) / wg::kKbBK;
-        ih_parts = ih_split_cap(tp) < ktall ? ih_split_cap(tp) : ktall;
-    }
-    const long long rt = (rows3 + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows;
+    // stages 3-5 run over the span of the windows, at most Ttot rows.  The split-K partials of dW_ih: the splits of a
+    // span's row count, at most the cap
+    const RowStages rs = row_stages(tp, Ttot);
+    const long long ktall = (Ttot + wg::kKbBK - 1) / wg::kKbBK;
+    const long long ih_parts = ih_split_cap(tp) < ktall ? ih_split_cap(tp) : ktall;
+    const long long rt = (Ttot + wg::kUTileRows - 1) / wg::kUTileRows * wg::kUTileRows;
     size_t o = p.total;
     tp.off_gates = o; o = align_up(o + (size_t)tp.rows * tp.LD4 * 4);
     tp.off_dg = o;    o = align_up(o + (size_t)tp.rows * tp.LD4 * 4);
     tp.off_dgt = o;   o = align_up(o + (size_t)rt * tp.KPd * 4);              // dGI in K-major 128-row tiles
     tp.off_wpb = o;   o = align_up(o + (size_t)tp.NPd * tp.KPd * 4);          // w_ih packed for dU = dGI . w_ih
     tp.off_zb = o;    o = align_up(o + (size_t)tp.NPd * 4);                   // zero bias (written by the pack kernel)
-    tp.off_du = o;    o = align_up(o + (size_t)rows3 * tp.ldu * 4);
+    tp.off_du = o;    o = align_up(o + (size_t)Ttot * tp.ldu * 4);
     tp.off_biasp = o; o = align_up(o + (size_t)tp.gb_grid * 3 * tp.LD4 * 4);  // 3 partial sets per CTA (regw), else 2
-    tp.off_gcnp = o;  o = align_up(o + (size_t)tp.rs.parts_gcn * (2 * 256 + 32) * 4);
+    tp.off_gcnp = o;  o = align_up(o + (size_t)rs.parts_gcn * (2 * 256 + 32) * 4);
     size_t sk = (size_t)tp.splits_hh_a * 2 * H * H;
     if ((size_t)tp.splits_hh_b * H * H > sk) sk = (size_t)tp.splits_hh_b * H * H;
     if ((size_t)ih_parts * p.I * tp.nt_ih * wg::KbWih::kBN > sk) sk = (size_t)ih_parts * p.I * tp.nt_ih * wg::KbWih::kBN;
     tp.off_splitk = o; o = align_up(o + sk * 4);
-    // table windows: dGI summed per table row (dgi_rows_kernel), the windows' first GI rows, their sorted starts and
-    // order (int64 each)
-    const size_t nt = tp.table_rows ? 1 : 0;
-    tp.off_dgi = o;   o = align_up(o + nt * rows3 * tp.LD4 * 4);
-    tp.off_row0 = o;  o = align_up(o + nt * Bn * 8);
-    tp.off_ssort = o; o = align_up(o + nt * Bn * 8);
-    tp.off_wsort = o; o = align_up(o + nt * Bn * 8);
+    // the windows' first GI rows (int64); untiled: dGI summed per table row (dgi_rows_kernel), the windows' sorted
+    // starts and order (int64 each)
+    const size_t nt = tiled ? 0 : 1;
+    tp.off_dgi = o;   o = align_up(o + nt * Ttot * tp.LD4 * 4);
+    tp.off_row0 = o;  o = align_up(o + Nn * 8);
+    tp.off_ssort = o; o = align_up(o + nt * Nn * 8);
+    tp.off_wsort = o; o = align_up(o + nt * Nn * 8);
     tp.total = o;
     return plan_launch(tp.f);   // last: a shape outside the training limits reports those
 }
 
-// Training on N windows of L steps over a table of Ttot rows: the training plan of N sequences of L steps (every limit
-// and error text is the training path's) with the table's regions.
-int make_train_windows_plan(TrainPlan& tp, long long N, long long Ttot, int L, int S, int Fi, int Fh, int Fo, int H) {
-    if (L >= 1 && Ttot < L)
-        return fail(WG_ERR_BAD_ARG, "training windows: need L <= Ttot (L=%d Ttot=%lld)", L, Ttot);
-    return make_train_plan(tp, N, L, S, Fi, Fh, Fo, H, Ttot);
+// The tiled plan of a materialised batch x [B][T]: the table x.view(B*T) (one sequence's rows at B = 0).
+int make_batch_train_plan(TrainPlan& tp, long long B, int T, int S, int Fi, int Fh, int Fo, int H) {
+    return make_train_plan(tp, B, (B > 0 ? B : 1) * T, T, S, Fi, Fh, Fo, H, true);
 }
 
 bool aligned16(const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; }
@@ -1139,18 +1144,83 @@ int splitk_gemm(const wg::SgOperand& A, const wg::SgOperand& Bo, long long M, in
     return WG_OK;
 }
 
-// The training backward after a forward that left its gates and hidden states in the workspace.  Stages 1-2 (BPTT,
-// bias gradients, dW_hh) run over the B sequences of tp.rows = B*T rows; stages 3-5 (dW_ih, dU, GCN backward) over
-// the rs.rows rows of U, of the gate gradients dgi_rows(st, DG, dgi) points dgi at, and of x (their GCN input rows).
-// Materialised windows pass B*T rows and DG itself; table windows the span of rows the windows cover, its first table
-// row as x and DG summed per table row.  grads: flat, state_dict order.
-template <typename DgiRows>
-int backward(const TrainPlan& tp, const RowStages& rs, const float* adj, const float* x, const float* w1,
-             const float* b1, const float* w2, const float* b2, const float* w_ih, const float* w_hh, const float* out,
-             const float* d_out, float* grads, long long B, void* workspace, cudaStream_t st, DgiRows dgi_rows) {
+// The table rows [lo, lo + span) that N > 0 windows of L steps cover: all N*L of a tiled plan, else those from the
+// smallest to the largest of the HOST starts [N], each checked to lie in [0, Ttot - L].
+int train_span(const TrainPlan& tp, const int64_t* starts, long long N, long long Ttot, long long& lo, long long& span) {
+    const int L = tp.f.T;
+    long long hi = (N - 1) * L;
+    lo = 0;
+    const int rc = tp.tiled ? WG_OK : window_span(starts, N, Ttot - L, "[0, Ttot - L]", lo, hi);
+    span = hi + L - lo;
+    return rc;
+}
+
+// The training forward of N windows over a table x of Ttot rows (starts: see train_span): GCN + projection once over
+// the span's rows into U (kept whole for dW_ih) and GI, then every window's recurrence over its GI rows in place, every
+// step's h stored and the gates saved.
+int train_forward(const TrainPlan& tp, const Graph& g, const float* x, const int64_t* starts, const float* w1,
+                  const float* b1, const float* w2, const float* b2, const float* w_ih, const float* w_hh,
+                  const float* b_ih, const float* b_hh, float* out, long long N, long long Ttot, void* ws,
+                  size_t ws_bytes, int device, void* stream) {
+    const Plan& p = tp.f;
+    if (N == 0) return WG_OK;
+    long long lo, span;
+    int rc = train_span(tp, starts, N, Ttot, lo, span);
+    if (rc) return rc;
+    auto stages = [&](cudaStream_t st) {
+        long long* row0 = ws_ptr<long long>(ws, tp.off_row0);
+        int rc2 = WG_OK;
+        if (tp.tiled) {   // filled on the device: the step issues no host-to-device copy
+            wg::tiled_row0_kernel<<<(unsigned)((N + 255) / 256), 256, 0, st>>>(row0, N, p.T);
+            WG_CUDA(cudaGetLastError());
+        } else {
+            rc2 = upload_row0(starts, N, lo, row0, st);
+        }
+        if (rc2 || (rc2 = run_span_stages(p, ws, g, x + (size_t)lo * p.S * p.Fi, w1, b1, w2, b2, span, span, st)))
+            return rc2;
+        return launch_recur(p, ws, out, N, st, row0, ws_ptr<float>(ws, tp.off_gates), tp.LD4);
+    };
+    return run_packed(p, tp.total, g, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, ws, ws_bytes, device, stream,
+                      stages);
+}
+
+// The training backward after train_forward left its gates and hidden states in the workspace (the same windows).
+// Stages 1-2 (BPTT, bias gradients, dW_hh) run over the N windows' N*L rows; stages 3-5 (dW_ih, dU, GCN backward) over
+// the span's rows of U, of the gate gradients dGI and of x.  dGI: DG itself on a tiled plan, else DG summed per table
+// row.  grads: flat, state_dict order.
+int train_backward(const TrainPlan& tp, const float* adj, const float* x, const int64_t* starts, const float* w1,
+                   const float* b1, const float* w2, const float* b2, const float* w_ih, const float* w_hh,
+                   const float* out, const float* d_out, float* grads, long long N, long long Ttot, void* workspace,
+                   size_t workspace_bytes, int device, void* stream) {
     const Plan& p = tp.f;
     const int T = p.T, H = p.H, F_in = p.Fi, F_hid = p.Fh, F_out = p.Fo;
+    long long lo = 0, span = 0;
     int rc;
+    if (N > 0 && (rc = train_span(tp, starts, N, Ttot, lo, span))) return rc;
+    if (any_null({adj, x, w1, b1, w2, b2, w_ih, w_hh, out, d_out, grads}))
+        return fail(WG_ERR_BAD_ARG, "null pointer argument");
+    DeviceGuard g(device);
+    WG_CUDA(g.err);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (N == 0) {
+        WG_CUDA(cudaMemsetAsync(grads, 0, param_count(p.S, F_in, F_hid, F_out, H) * 4, st));
+        return WG_OK;
+    }
+    if ((rc = check_ws(workspace, workspace_bytes, tp.total))) return rc;
+    long long* ssort_dev = ws_ptr<long long>(workspace, tp.off_ssort);
+    long long* wsort_dev = ws_ptr<long long>(workspace, tp.off_wsort);
+    if (!tp.tiled) {
+        // the windows ordered by (start, n): those covering a span row are then a contiguous range (dgi_rows_kernel)
+        std::vector<long long> order((size_t)N), ssort((size_t)N);
+        for (long long n = 0; n < N; ++n) order[(size_t)n] = n;
+        std::sort(order.begin(), order.end(),
+                  [&](long long a, long long b) { return starts[a] != starts[b] ? starts[a] < starts[b] : a < b; });
+        for (long long k = 0; k < N; ++k) ssort[(size_t)k] = starts[order[(size_t)k]] - lo;
+        WG_CUDA(cudaMemcpyAsync(ssort_dev, ssort.data(), (size_t)N * sizeof(long long), cudaMemcpyHostToDevice, st));
+        WG_CUDA(cudaMemcpyAsync(wsort_dev, order.data(), (size_t)N * sizeof(long long), cudaMemcpyHostToDevice, st));
+    }
+    x += (size_t)lo * p.S * F_in;   // the span's first table row
+    const RowStages rs = row_stages(tp, span);
     // flat gradient layout = state_dict order
     float* d_w1 = grads;
     float* d_b1 = d_w1 + (size_t)F_in * F_hid;
@@ -1171,10 +1241,10 @@ int backward(const TrainPlan& tp, const RowStages& rs, const float* adj, const f
     // 1. BPTT through the recurrence: DG = [da_r | da_z | da_n | da_n r], bias partials
     if (tp.gb_regw) {
         WG_CUDA(cudaFuncSetAttribute(tp.gb_regw, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.gb_smem));
-        tp.gb_regw<<<tp.gb_grid, tp.gb_threads, tp.gb_smem, st>>>(gates, out, d_out, w_hh, DG, biasp, B, T, H, tp.LD4);
+        tp.gb_regw<<<tp.gb_grid, tp.gb_threads, tp.gb_smem, st>>>(gates, out, d_out, w_hh, DG, biasp, N, T, H, tp.LD4);
     } else {
         WG_CUDA(cudaFuncSetAttribute(tp.gb, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tp.gb_smem));
-        tp.gb<<<tp.gb_grid, tp.gb_threads, tp.gb_smem, st>>>(gates, out, d_out, w_hh, DG, biasp, B, T, H, tp.LD4, tp.HP,
+        tp.gb<<<tp.gb_grid, tp.gb_threads, tp.gb_smem, st>>>(gates, out, d_out, w_hh, DG, biasp, N, T, H, tp.LD4, tp.HP,
                                                               tp.GR);
     }
     WG_CUDA(cudaGetLastError());
@@ -1190,9 +1260,16 @@ int backward(const TrainPlan& tp, const RowStages& rs, const float* adj, const f
         if ((rc = splitk_gemm(a_n, hprev, H, H, rows, tp.splits_hh_b, skp, d_whh + 2 * (size_t)H * H, H, 1, st)))
             return rc;
     }
-    // the gate gradients of stages 3-5, one row per U row
-    const float* dgi = nullptr;
-    if ((rc = dgi_rows(st, DG, dgi))) return rc;
+    // the gate gradients of stages 3-5, one row per span row
+    const float* dgi = DG;
+    if (!tp.tiled) {
+        float* dgi_buf = ws_ptr<float>(workspace, tp.off_dgi);
+        const long long grid = (span + wg::kDgiWarps - 1) / wg::kDgiWarps;
+        wg::dgi_rows_kernel<<<(unsigned)grid, wg::kDgiWarps * 32, 0, st>>>(DG, ssort_dev, wsort_dev, N, T, span, tp.LD4,
+                                                                         wg::round_up(p.G, 4), dgi_buf);
+        WG_CUDA(cudaGetLastError());
+        dgi = dgi_buf;
+    }
     // 3. dW_ih [3H x I] = dGI^T . U: gemm_kb_kernel reads dGI (row-major, as the BPTT kernel or dgi_rows_kernel wrote
     //    it) and U (the forward's K-major tiles) in place; one wave of CTAs over (tile, row split), fixed-order reduction
     {
@@ -1328,7 +1405,7 @@ int wg_gcn_gru_forward_f32(const float* adj, const float* x, const float* w1, co
                            size_t workspace_bytes, int device, void* stream) {
     Plan p;
     const int rc = make_plan(p, B, T, S, F_in, F_hid, F_out, H, chunk, false, flags);
-    return rc ? rc : forward(p, p.total, Graph{adj}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, B, workspace,
+    return rc ? rc : forward(p, Graph{adj}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, B, workspace,
                              workspace_bytes, device, stream);
 }
 
@@ -1347,8 +1424,8 @@ int wg_gcn_gru_forward_csr_f32(const int32_t* rowptr, const int32_t* colidx, con
                                void* stream) {
     Plan p;
     const int rc = make_plan(p, B, T, S, F_in, F_hid, F_out, H, chunk, true, flags);
-    return rc ? rc : forward(p, p.total, Graph{nullptr, rowptr, colidx, vals}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih,
-                             b_hh, out, B, workspace, workspace_bytes, device, stream);
+    return rc ? rc : forward(p, Graph{nullptr, rowptr, colidx, vals}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh,
+                             out, B, workspace, workspace_bytes, device, stream);
 }
 
 size_t wg_gcn_gru_forecast_workspace_bytes(int64_t N, int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out,
@@ -1585,7 +1662,7 @@ size_t wg_gcn_gru_param_count(int S, int F_in, int F_hid, int F_out, int H) {
 
 size_t wg_gcn_gru_train_workspace_bytes(int64_t B, int T, int S, int F_in, int F_hid, int F_out, int H) {
     TrainPlan tp;
-    if (make_train_plan(tp, B, T, S, F_in, F_hid, F_out, H)) return 0;
+    if (make_batch_train_plan(tp, B, T, S, F_in, F_hid, F_out, H)) return 0;
     return tp.total;
 }
 
@@ -1595,11 +1672,9 @@ int wg_gcn_gru_forward_train_f32(const float* adj, const float* x, const float* 
                                  int F_in, int F_hid, int F_out, int H, void* workspace, size_t workspace_bytes,
                                  int device, void* stream) {
     TrainPlan tp;
-    const int rc = make_train_plan(tp, B, T, S, F_in, F_hid, F_out, H);
-    if (rc) return rc;
-    float* gates = workspace ? ws_ptr<float>(workspace, tp.off_gates) : nullptr;   // forward() rejects a NULL workspace
-    return forward(tp.f, tp.total, Graph{adj}, x, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, B, workspace,
-                   workspace_bytes, device, stream, gates, tp.LD4);
+    const int rc = make_batch_train_plan(tp, B, T, S, F_in, F_hid, F_out, H);
+    return rc ? rc : train_forward(tp, Graph{adj}, x, nullptr, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, B,
+                                   B * T, workspace, workspace_bytes, device, stream);
 }
 
 int wg_gcn_gru_backward_f32(const float* adj, const float* x, const float* w1, const float* b1, const float* w2,
@@ -1607,28 +1682,16 @@ int wg_gcn_gru_backward_f32(const float* adj, const float* x, const float* w1, c
                             const float* d_out, float* grads, int64_t B, int T, int S, int F_in, int F_hid,
                             int F_out, int H, void* workspace, size_t workspace_bytes, int device, void* stream) {
     TrainPlan tp;
-    int rc = make_train_plan(tp, B, T, S, F_in, F_hid, F_out, H);
-    if (rc) return rc;
-    if (any_null({adj, x, w1, b1, w2, b2, w_ih, w_hh, out, d_out, grads}))
-        return fail(WG_ERR_BAD_ARG, "null pointer argument");
-    DeviceGuard g(device);
-    WG_CUDA(g.err);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (B == 0) {
-        WG_CUDA(cudaMemsetAsync(grads, 0, param_count(S, F_in, F_hid, F_out, H) * 4, st));
-        return WG_OK;
-    }
-    if ((rc = check_ws(workspace, workspace_bytes, tp.total))) return rc;
-    // stages 3-5 over the B*T rows of the windows, on the BPTT's DG rows themselves
-    auto dgi_rows = [](cudaStream_t, const float* DG, const float*& dgi) { dgi = DG; return (int)WG_OK; };
-    return backward(tp, tp.rs, adj, x, w1, b1, w2, b2, w_ih, w_hh, out, d_out, grads, B, workspace, st, dgi_rows);
+    const int rc = make_batch_train_plan(tp, B, T, S, F_in, F_hid, F_out, H);
+    return rc ? rc : train_backward(tp, adj, x, nullptr, w1, b1, w2, b2, w_ih, w_hh, out, d_out, grads, B, B * T,
+                                    workspace, workspace_bytes, device, stream);
 }
 
 // ---- training on windows over one table ------------------------------------------------------------------
 size_t wg_gcn_gru_train_windows_workspace_bytes(int64_t N, int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out,
                                                 int H) {
     TrainPlan tp;
-    if (make_train_windows_plan(tp, N, Ttot, L, S, F_in, F_hid, F_out, H)) return 0;
+    if (make_train_plan(tp, N, Ttot, L, S, F_in, F_hid, F_out, H, false)) return 0;
     return tp.total;
 }
 
@@ -1638,27 +1701,9 @@ int wg_gcn_gru_forward_train_windows_f32(const float* adj, const float* table, c
                                          int64_t N, int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out, int H,
                                          void* workspace, size_t workspace_bytes, int device, void* stream) {
     TrainPlan tp;
-    int rc = make_train_windows_plan(tp, N, Ttot, L, S, F_in, F_hid, F_out, H);
-    if (rc) return rc;
-    if (N == 0) return WG_OK;
-    long long lo = 0, hi = 0;
-    if ((rc = window_span(starts, N, Ttot - L, "[0, Ttot - L]", lo, hi))) return rc;
-    const Plan& p = tp.f;
-    auto stages = [&](cudaStream_t st) {
-        // the windows' first GI rows relative to the span (a pageable source is staged before cudaMemcpyAsync returns)
-        std::vector<long long> row0((size_t)N);
-        for (long long n = 0; n < N; ++n) row0[(size_t)n] = starts[n] - lo;
-        long long* row0_dev = ws_ptr<long long>(workspace, tp.off_row0);
-        WG_CUDA(cudaMemcpyAsync(row0_dev, row0.data(), (size_t)N * sizeof(long long), cudaMemcpyHostToDevice, st));
-        // GCN + projection once over table rows [lo, hi + L): U (kept whole for dW_ih) and GI
-        const long long span = hi + L - lo;
-        int rc2 = launch_gcn(p, workspace, Graph{adj}, table + (size_t)lo * S * F_in, w1, b1, w2, b2, span, st);
-        if (rc2 || (rc2 = launch_inproj(p, workspace, span, st, ws_ptr<float>(workspace, p.off_gi)))) return rc2;
-        // every window's recurrence over its GI rows in place: every step stored, the gates saved
-        return launch_recur(p, workspace, out, N, st, ws_ptr<float>(workspace, tp.off_gates), tp.LD4, row0_dev);
-    };
-    return run_packed(p, tp.total, Graph{adj}, table, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, workspace,
-                      workspace_bytes, device, stream, stages);
+    const int rc = make_train_plan(tp, N, Ttot, L, S, F_in, F_hid, F_out, H, false);
+    return rc ? rc : train_forward(tp, Graph{adj}, table, starts, w1, b1, w2, b2, w_ih, w_hh, b_ih, b_hh, out, N, Ttot,
+                                   workspace, workspace_bytes, device, stream);
 }
 
 int wg_gcn_gru_backward_windows_f32(const float* adj, const float* table, const int64_t* starts, const float* w1,
@@ -1667,43 +1712,9 @@ int wg_gcn_gru_backward_windows_f32(const float* adj, const float* table, const 
                                     int64_t Ttot, int L, int S, int F_in, int F_hid, int F_out, int H, void* workspace,
                                     size_t workspace_bytes, int device, void* stream) {
     TrainPlan tp;
-    int rc = make_train_windows_plan(tp, N, Ttot, L, S, F_in, F_hid, F_out, H);
-    if (rc) return rc;
-    long long lo = 0, hi = 0;
-    if (N > 0 && (rc = window_span(starts, N, Ttot - L, "[0, Ttot - L]", lo, hi))) return rc;
-    if (any_null({adj, table, w1, b1, w2, b2, w_ih, w_hh, out, d_out, grads}))
-        return fail(WG_ERR_BAD_ARG, "null pointer argument");
-    DeviceGuard g(device);
-    WG_CUDA(g.err);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (N == 0) {
-        WG_CUDA(cudaMemsetAsync(grads, 0, param_count(S, F_in, F_hid, F_out, H) * 4, st));
-        return WG_OK;
-    }
-    if ((rc = check_ws(workspace, workspace_bytes, tp.total))) return rc;
-    // the windows ordered by (start, n): those covering a span row are then a contiguous range (dgi_rows_kernel)
-    std::vector<long long> order((size_t)N), ssort((size_t)N);
-    for (long long n = 0; n < N; ++n) order[(size_t)n] = n;
-    std::sort(order.begin(), order.end(),
-              [&](long long a, long long b) { return starts[a] != starts[b] ? starts[a] < starts[b] : a < b; });
-    for (long long k = 0; k < N; ++k) ssort[(size_t)k] = starts[order[(size_t)k]] - lo;
-    long long* ssort_dev = ws_ptr<long long>(workspace, tp.off_ssort);
-    long long* wsort_dev = ws_ptr<long long>(workspace, tp.off_wsort);
-    WG_CUDA(cudaMemcpyAsync(ssort_dev, ssort.data(), (size_t)N * sizeof(long long), cudaMemcpyHostToDevice, st));
-    WG_CUDA(cudaMemcpyAsync(wsort_dev, order.data(), (size_t)N * sizeof(long long), cudaMemcpyHostToDevice, st));
-    const long long span = hi + L - lo;
-    float* dgi_buf = ws_ptr<float>(workspace, tp.off_dgi);
-    // stages 3-5 over the span's rows, on DG summed per table row
-    auto dgi_rows = [&](cudaStream_t s, const float* DG, const float*& dgi) {
-        const long long grid = (span + wg::kDgiWarps - 1) / wg::kDgiWarps;
-        wg::dgi_rows_kernel<<<(unsigned)grid, wg::kDgiWarps * 32, 0, s>>>(DG, ssort_dev, wsort_dev, N, L, span, tp.LD4,
-                                                                        wg::round_up(tp.f.G, 4), dgi_buf);
-        WG_CUDA(cudaGetLastError());
-        dgi = dgi_buf;
-        return (int)WG_OK;
-    };
-    return backward(tp, row_stages(tp, span), adj, table + (size_t)lo * S * F_in, w1, b1, w2, b2, w_ih, w_hh, out,
-                    d_out, grads, N, workspace, st, dgi_rows);
+    const int rc = make_train_plan(tp, N, Ttot, L, S, F_in, F_hid, F_out, H, false);
+    return rc ? rc : train_backward(tp, adj, table, starts, w1, b1, w2, b2, w_ih, w_hh, out, d_out, grads, N, Ttot,
+                                    workspace, workspace_bytes, device, stream);
 }
 
 size_t wg_mse_workspace_bytes(void) { return (size_t)2 * wg::kNumSMs * sizeof(double); }

@@ -348,20 +348,21 @@ __host__ __device__ inline size_t recur_regw_smem_floats(int KP, int NP, int GP)
 }
 
 // Where gru_recur_regw_kernel and gru_recur_unit_kernel read gi and what they store (template argument WIN):
-//   kWinOff   the sequences' gi rows one after another, h of every step stored to out [B][T][H] (the forward)
+//   kWinOff   the sequences' gi rows one after another, h of every step stored to out [B][T][H] (the inference
+//             forward)
 //   kWinLast  windows over one table's gi rows: sequence b's gi rows start at GI + row0[b] * ldg, and only h at
 //             t = T-1 is stored, to out [B][H] (the forecast)
-//   kWinAll   gi rows through row0 as kWinLast, h of every step stored to out [B][T][H] and, with SAVE, the gates
-//             (training on table windows)
+//   kWinAll   gi rows through row0 as kWinLast, h of every step stored to out [B][T][H] and the gates saved to gsave
+//             (the training forward, on table windows or on a batch laid out as windows that tile it)
 enum WinMode { kWinOff = 0, kWinLast = 1, kWinAll = 2 };
 
 // WIN: a WinMode
-template <bool SAVE, int NB, int KPT, int WIN = kWinOff>
+template <int NB, int KPT, int WIN = kWinOff>
 __global__ void __launch_bounds__(kRwThreads, 1)
     gru_recur_regw_kernel(const float* __restrict__ GI, const float* __restrict__ WhT, const float* __restrict__ bhn,
                           float* __restrict__ out, long long B, int T, int H, int ldg, int NP, float* __restrict__ gsave,
                           int ldsave, const long long* __restrict__ row0) {
-    constexpr bool ROW0 = WIN != kWinOff, LAST = WIN == kWinLast;
+    constexpr bool ROW0 = WIN != kWinOff, LAST = WIN == kWinLast, SAVE = WIN == kWinAll;
     extern __shared__ __align__(16) float smem[];
     constexpr int RS = KPT + 4;
     float* hs = smem;                          // [4][RS]

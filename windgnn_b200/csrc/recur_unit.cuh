@@ -80,18 +80,19 @@ struct RuFrag {
 
 // GI  [B*T][ldg]   gi with b_ih (+ b_hh for r, z) folded in, column g*H + j; ldg = 3H rounded up to 8
 // Whu [KP][3][HP2] W_hh^T, Whu[k][g][j] = w_hh[g*H + j][k], zero padded
-// out [B][T][H];   gsave (SAVE): [B*T][ldsave] = [r | z | n | W_hn h + b_hn]
+// out [B][T][H];   gsave (kWinAll): [B*T][ldsave] = [r | z | n | W_hn h + b_hn]
 // HT > 0: the hidden size is the compile-time constant HT (every shared-memory offset becomes an
 // immediate); HT == 0: H is the runtime argument.
 // WIN: a WinMode (recur.cuh).  kWinLast and kWinAll read sequence b's gi rows from GI + row0[b] * ldg (windows over one
-// table's gi rows); kWinLast stores only h at t = T-1, to out [B][H].  The product and the gate math are unchanged.
-template <int R, int WPG, bool SAVE, int HT, int WIN = kWinOff>
+// table's gi rows); kWinLast stores only h at t = T-1, to out [B][H]; kWinAll also saves the gates (the training
+// forward).  The product and the gate math are unchanged.
+template <int R, int WPG, int HT, int WIN = kWinOff>
 __global__ void __launch_bounds__(kRuThreads, 1)
     gru_recur_unit_kernel(const float* __restrict__ GI, const float* __restrict__ Whu, const float* __restrict__ bhn,
                           float* __restrict__ out, long long B, int T, int H_rt,
                           float* __restrict__ gsave, int ldsave, int handover,
                           const long long* __restrict__ row0) {
-    constexpr bool ROW0 = WIN != kWinOff, LAST = WIN == kWinLast;
+    constexpr bool ROW0 = WIN != kWinOff, LAST = WIN == kWinLast, SAVE = WIN == kWinAll;
     constexpr int NGRP = kRuWarps / WPG;   // groups per CTA
     constexpr int NG = WPG * 32;           // threads per group
     constexpr int NB = WPG == 1 ? kRuGiRing : 1;   // gi ring slots per group (recur_u_nb)

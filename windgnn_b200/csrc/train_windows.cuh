@@ -1,15 +1,23 @@
-// Training on windows over one table: the gate gradients of every (window, step) summed per table row.
+// Training on windows over one table: the windows' first GI rows, and the gate gradients of every (window, step)
+// summed per table row.
 //
 // The GCN, the input projection and the backward of both depend only on a table row, and the backward is linear in
 // the input-gate gradient dGI.  So when the windows table[starts[n] : starts[n] + L] overlap, the forward runs those
-// stages once per row of the span the windows cover (abi.cu, wg_gcn_gru_forward_train_windows_f32), and the
-// backward sums, per span row t, the dGI rows of every (n, l) that read it (starts[n] + l = t), then runs dW_ih, dU
-// and the GCN backward once per span row instead of once per (window, step).
+// stages once per row of the span the windows cover (abi.cu, train_forward), and the backward sums, per span row t,
+// the dGI rows of every (n, l) that read it (starts[n] + l = t), then runs dW_ih, dU and the GCN backward once per
+// span row instead of once per (window, step).  A materialised batch x [B][T] is such a table, x.view(B*T), with
+// windows that tile it (starts[n] = n*T): every row has one contributor, and the backward reads dGI in place.
 #pragma once
 
 #include "wg_common.cuh"
 
 namespace wg {
+
+// row0[n] = n * L: the first GI rows of N windows that tile the table (a materialised batch)
+__global__ void tiled_row0_kernel(long long* __restrict__ row0, long long N, int L) {
+    const long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (n < N) row0[n] = n * L;
+}
 
 constexpr int kDgiWarps = 8;   // rows per CTA (one warp each)
 constexpr int kDgiVec = 3;     // float4 columns per lane: 3H <= 384, i.e. H <= 128 (training serves H <= 106)

@@ -59,6 +59,16 @@ def forward_train(adj, x, params: Sequence[torch.Tensor]):
     return out, ws
 
 
+def _grads_bucket(lib, dims, dev, grads: Optional[torch.Tensor]) -> torch.Tensor:
+    """``grads``, checked, or a new flat gradient bucket for the model of ``dims = (S, F_in, F_hid, F_out, H)``."""
+    n = lib.wg_gcn_gru_param_count(*dims)
+    if grads is None:
+        return torch.empty(n, dtype=torch.float32, device=dev)
+    if grads.numel() != n or not grads.is_cuda or grads.dtype != torch.float32 or not grads.is_contiguous():
+        raise RuntimeError(f"grads must be a contiguous CUDA float32 buffer of {n} elements")
+    return grads
+
+
 def backward(adj, x, params: Sequence[torch.Tensor], out, d_out, ws, grads: Optional[torch.Tensor] = None):
     """Flat gradient bucket (state_dict order) of the loss w.r.t. the eight parameter tensors."""
     lib = _lib.load()
@@ -72,11 +82,7 @@ def backward(adj, x, params: Sequence[torch.Tensor], out, d_out, ws, grads: Opti
     d_out = _require_cuda_f32("d_out", d_out, dev)
     if out.shape != (B, T, H) or d_out.shape != (B, T, H):
         raise RuntimeError(f"out / d_out must be [{B}, {T}, {H}]")
-    n = lib.wg_gcn_gru_param_count(S, F_in, F_hid, F_out, H)
-    if grads is None:
-        grads = torch.empty(n, dtype=torch.float32, device=dev)
-    elif grads.numel() != n or not grads.is_cuda or grads.dtype != torch.float32 or not grads.is_contiguous():
-        raise RuntimeError(f"grads must be a contiguous CUDA float32 buffer of {n} elements")
+    grads = _grads_bucket(lib, (S, F_in, F_hid, F_out, H), dev, grads)
     w1, b1, w2, b2, w_ih, w_hh, _, _ = params
     _lib.check(lib.wg_gcn_gru_backward_f32(
         adj.data_ptr(), x.data_ptr(), w1.data_ptr(), b1.data_ptr(), w2.data_ptr(), b2.data_ptr(),
@@ -125,11 +131,7 @@ def backward_windows(adj, table, starts, params: Sequence[torch.Tensor], out, d_
     d_out = _require_cuda_f32("d_out", d_out, dev)
     if out.shape != (N, seq_length, H) or d_out.shape != (N, seq_length, H):
         raise RuntimeError(f"out / d_out must be [{N}, {seq_length}, {H}]")
-    n = lib.wg_gcn_gru_param_count(*dims)
-    if grads is None:
-        grads = torch.empty(n, dtype=torch.float32, device=dev)
-    elif grads.numel() != n or not grads.is_cuda or grads.dtype != torch.float32 or not grads.is_contiguous():
-        raise RuntimeError(f"grads must be a contiguous CUDA float32 buffer of {n} elements")
+    grads = _grads_bucket(lib, dims, dev, grads)
     w1, b1, w2, b2, w_ih, w_hh, _, _ = params
     _lib.check(lib.wg_gcn_gru_backward_windows_f32(
         adj.data_ptr(), table.data_ptr(), starts.data_ptr(), w1.data_ptr(), b1.data_ptr(), w2.data_ptr(),
